@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the ASVGP hot path on B200: ELBO + gradient datapoints/s at N = 1e8, M = 1e4 (BASELINE.json configs[2]).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload 1d|1d-random|...]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload 1d|1d-random|...] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic points:
     accumulate (asvgp_accum_1d, O(N))  ->  [N>1: one NCCL all-reduce of the packed band]  ->  Kuu assembly +
@@ -22,6 +22,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the source tree may be read-only; the benchmark writes nothing into it
 # stdout carries exactly ONE JSON line: library chatter (NCCL's version banner, torchrun notices) goes to stderr instead
 _JSON_OUT = os.fdopen(os.dup(1), "w")
 os.dup2(2, 1)
@@ -61,6 +62,8 @@ def parse():
     ap.add_argument("--n", type=float, default=None, help="override points per rank (debug)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float64), to compare two builds")
     return ap.parse_args()
 
 
@@ -69,6 +72,22 @@ def launch_count():
     from asvgp_b200 import _lib
 
     return int(_lib.load().asvgp_launch_count())
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """Writes every tensor of `arrays` as dirname/<name>.npy in float64.  The inputs are seeded, so two builds run with
+    the same arguments can be compared output for output."""
+    import numpy as np
+
+    host = {name: np.asarray(t.detach().cpu().numpy(), dtype=np.float64) for name, t in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    assert total <= DUMP_LIMIT_BYTES, "outputs of %d bytes exceed the dump limit" % total
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -315,9 +334,9 @@ def workload_config_2d(name, n1, n2, m, k):
                             "no on-device classification pass; every point is still verified against the statement"}
 
 
-def run_2d(args, name, torch, dist, world, rank, steps, warmup, with_e2e=True):
+def run_2d(args, name, torch, dist, world, rank, steps, warmup, with_e2e=True, dump=None):
     """Times the 2-D path; returns the summary dict (rank 0) — used as the main line for --workload 2d* and as the
-    `kron_2d` appendix of the default 1-D line."""
+    `kron_2d` appendix of the default 1-D line.  dump: directory for the outputs of the last timed step (rank 0)."""
     import numpy as np
 
     from asvgp_b200 import basis as B, kernels as Kn, ops
@@ -402,6 +421,11 @@ def run_2d(args, name, torch, dist, world, rank, steps, warmup, with_e2e=True):
         t1.record()
         barrier()
         launches = launch_count() - launches0
+    if dump and rank == 0:
+        dump_outputs(dump, {
+            "elbo": torch.tensor([result["elbo"]], dtype=torch.float64),
+            "grad": torch.tensor([float(result["grads"][id(p)]) for p in model.trainable_variables], dtype=torch.float64),
+            "KufKfu_stencil": model._Gs, "Kuf_y": model._b, "tr_yTy_count": model._scal})
     total_ms = torch.tensor([t0.elapsed_time(t1)], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(total_ms, op=dist.ReduceOp.MAX)
@@ -651,7 +675,8 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     if args.workload in WORKLOADS_2D:
-        line = run_2d(args, args.workload, torch, dist, world, rank, args.steps, args.warmup, with_e2e=not args.no_e2e)
+        line = run_2d(args, args.workload, torch, dist, world, rank, args.steps, args.warmup, with_e2e=not args.no_e2e,
+                      dump=args.dump_outputs)
         if rank == 0:
             if world == 1 and not args.no_cpu_baseline:
                 v, dt, n_sample, t_acc, t_fac = run_cpu_2d(args.workload, 1, 0, 1)
@@ -751,6 +776,11 @@ def main():
         host_enqueue_ms = (time.perf_counter() - h0) * 1e3 / args.steps      # must stay below ms_per_step, else the host is the bound
         barrier()
         launches = launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        # out[9:15] holds clock counters, not results; acc holds the all-reduced statistics the bound was evaluated on
+        G_band, Kuf_y, scal = ops.split_accum_1d(acc, basis)
+        dump_outputs(args.dump_outputs, {"elbo": out[0:1], "grad": out[1:4], "bound_terms": torch.cat([out[4:9], out[15:16]]),
+                                         "KufKfu_band": G_band, "Kuf_y": Kuf_y, "tr_yTy_count": scal})
     total_ms = torch.tensor([t0.elapsed_time(t1)], dtype=torch.float64, device="cuda")
     kuu_asm_ms = float(np.mean([e[0].elapsed_time(e[1]) for e in phase_ev]))
     accum_ms = float(np.mean([e[1].elapsed_time(e[2]) for e in phase_ev]))

@@ -11,6 +11,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+import scale_cases as SC  # noqa: E402
 from oracle import ref_under_shim  # noqa: E402
 
 OUT = os.path.join(ROOT, "tests", "golden")
@@ -82,17 +84,16 @@ def basis_eval(ns):
 
 
 def synth_1d(ns):
-    """C2-shaped small case: x ~ U(0, m) on (a,b)=(-1, m+1) (int endpoints -> f64 mesh), random order."""
+    """C2-shaped small case: x ~ U(0, m) on (a,b)=(-1, m+1) (int endpoints -> f64 mesh), random order.  The inputs come
+    from tests/scale_cases.py (seeded numpy); the tests regenerate them, so only every SYNTH_1D_SAMPLE-th point is stored."""
     out = {}
-    rng = np.random.default_rng(1997)
-    n = 20000
-    for k, m in ((1, 50), (2, 50), (3, 60), (4, 60), (5, 64)):
-        x = rng.uniform(0.0, m, n)
-        y = np.sin(2 * np.pi * x / 37) + 0.5 * np.sin(2 * np.pi * x / 3.1) + 0.3 * rng.standard_normal(n)
-        y = (y - y.mean()) / y.std()
+    inputs = SC.synth_1d_inputs()
+    for k, m in SC.SYNTH_1D:
+        x, y, xs = inputs[k]
         basis = getattr(ns.basis, "B%dSpline" % k)(-1, m + 1, m)
         key = "k%d" % k
-        out[key + "_x"], out[key + "_y"], out[key + "_m"] = x, y, m
+        out[key + "_x_sample"], out[key + "_y_sample"] = x[::SC.SYNTH_1D_SAMPLE], y[::SC.SYNTH_1D_SAMPLE]
+        out[key + "_m"] = m
         for kind in KINDS:
             need = {"Matern12": 1, "Matern32": 2, "Matern52": 3}[kind]
             if k < need:
@@ -106,7 +107,6 @@ def synth_1d(ns):
         out[key + "_G"] = np.asarray(model.KufKfu)
         out[key + "_Kuf_y"] = np.asarray(model.Kuf_y)
         out[key + "_tr_yTy"] = float(model.tr_yTy)
-        xs = rng.uniform(0.5, m - 0.5, 64).reshape(-1, 1)
         mu, var = model.predict_f(xs)
         out[key + "_xs"], out[key + "_mean"], out[key + "_var"] = xs, np.asarray(mu), np.asarray(var)
         out[key + "_pred_hypers"] = np.array([1.3, 2.5, 0.7])

@@ -1,9 +1,8 @@
-"""Import the UNMODIFIED reference package from /root/reference under the numpy/SciPy stand-ins of
-`oracle/shim/` ("reference-under-shim", SURVEY §8(c)).
+"""Import the UNMODIFIED reference package (a checkout of the original ASVGP sources at $ASVGP_REFERENCE_ROOT) under the
+numpy/SciPy stand-ins of `oracle/shim/` ("reference-under-shim", SURVEY §8(c)).
 
-TEST INFRASTRUCTURE ONLY, and build-container only: /root/reference does not exist on the GPU box, so this
-module is used solely by `oracle/make_golden.py` (which writes tests/golden/*.npz) and by the CPU tests that
-re-validate the restatement when the reference happens to be present.
+TEST INFRASTRUCTURE ONLY: the reference sources are not part of this repository, so this module is used solely by
+`oracle/make_golden.py`, which writes tests/golden/*.npz; the tests compare with those stored vectors.
 """
 import importlib
 import os

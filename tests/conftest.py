@@ -14,12 +14,40 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
 
 
+class _Arrays(dict):
+    """A golden file's arrays by name, with the `files` list of the NpzFile that np.load returns."""
+
+    @property
+    def files(self):
+        return list(self)
+
+
+def _with_synth_1d_inputs(npz):
+    """synth_1d.npz stores every SYNTH_1D_SAMPLE-th input point only: the full inputs k*_x, k*_y are regenerated from their
+    seed and must match those samples."""
+    import numpy as np
+
+    if os.path.join(ROOT, "tests") not in sys.path:
+        sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import scale_cases as SC
+
+    out = _Arrays((name, npz[name]) for name in npz.files)
+    for k, (x, y, xs) in SC.synth_1d_inputs().items():
+        key = "k%d" % k
+        np.testing.assert_array_equal(x[::SC.SYNTH_1D_SAMPLE], out[key + "_x_sample"])
+        np.testing.assert_allclose(y[::SC.SYNTH_1D_SAMPLE], out[key + "_y_sample"], rtol=0, atol=1e-14)   # np.sin may differ by an ulp
+        np.testing.assert_array_equal(xs, out[key + "_xs"])
+        out[key + "_x"], out[key + "_y"] = x, y
+    return out
+
+
 @pytest.fixture(scope="session")
 def golden():
     import numpy as np
 
     def load(name):
-        return np.load(os.path.join(GOLDEN, name + ".npz"), allow_pickle=False)
+        npz = np.load(os.path.join(GOLDEN, name + ".npz"), allow_pickle=False)
+        return _with_synth_1d_inputs(npz) if name == "synth_1d" else npz
 
     return load
 

@@ -1,7 +1,25 @@
 """Seeded synthetic inputs of the BASELINE-sized parity cases (SURVEY §8(d) C3 / C4 / C5 shapes).  Pure numpy, shared by
 the generator of the golden fixtures (oracle/make_golden_scale.py, run in the build container where the oracle's
-LAPACK-band evaluations take minutes) and by the GPU tests that compare the CUDA path with those fixtures."""
+LAPACK-band evaluations take minutes) and by the GPU tests that compare the CUDA path with those fixtures.
+Also the inputs of tests/golden/synth_1d.npz (oracle/make_golden.py), which are too many to store."""
 import numpy as np
+
+# ---- 1-D, C2-shaped small case of synth_1d.npz: 20 000 points in random order per (spline order, M) --------------------------
+SYNTH_1D = ((1, 50), (2, 50), (3, 60), (4, 60), (5, 64))
+SYNTH_1D_SAMPLE = 97                # synth_1d.npz keeps every 97th input point to check the regenerated ones
+
+
+def synth_1d_inputs(n=20_000, seed=1997):
+    """{order: (x, y, xs)} drawn in sequence from one generator: x ~ U(0, M), standardised y, 64 test points xs."""
+    rng = np.random.default_rng(seed)
+    out = {}
+    for k, m in SYNTH_1D:
+        x = rng.uniform(0.0, m, n)
+        y = np.sin(2 * np.pi * x / 37) + 0.5 * np.sin(2 * np.pi * x / 3.1) + 0.3 * rng.standard_normal(n)
+        y = (y - y.mean()) / y.std()
+        xs = rng.uniform(0.5, m - 0.5, 64).reshape(-1, 1)
+        out[k] = x, y, xs
+    return out
 
 # ---- 1-D, C3-shaped: M = 1e4 cubic B-splines on (-1, M + 1), N = 2e7 sorted points ---------------------------------------
 C3_M, C3_N, C3_ORDER = 10_000, 20_000_000, 3
