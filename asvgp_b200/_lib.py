@@ -20,6 +20,9 @@ SIGNATURES = {
     "asvgp_accum_1d": [_vp, _vp, _c_i64, _vp, _c_int, _c_int, _vp, _vp],
     "asvgp_accum_1d_binned": [_vp, _vp, _c_i64, _vp, _c_int, _c_int, _vp, _vp, _c_i64, _vp],
     "asvgp_order_probe_1d": [_vp, _c_i64, _vp, _c_int, _vp, _vp],
+    "asvgp_accum_1d_typed": [_vp, _c_int, _vp, _c_int, _c_i64, _vp, _c_int, _c_int, _vp, _vp],
+    "asvgp_accum_1d_binned_typed": [_vp, _c_int, _vp, _c_int, _c_i64, _vp, _c_int, _c_int, _vp, _vp, _c_i64, _vp],
+    "asvgp_order_probe_1d_typed": [_vp, _c_int, _c_i64, _vp, _c_int, _vp, _vp],
     "asvgp_predict_1d": [_vp, _c_i64, _vp, _c_int, _c_int, _vp, _vp, _c_dbl, _vp, _vp, _vp],
     "asvgp_kuu_assemble": [_vp, _c_int, _vp, _vp, _c_int, _c_int, _vp, _vp, _vp],
     "asvgp_elbo_grad_1d": [_vp, _vp, _vp, _c_int, _c_int, _c_dbl, _c_dbl, _c_int, _vp, _vp, _c_i64, _vp],
@@ -34,6 +37,11 @@ SIGNATURES = {
     "asvgp_predict_2d_apply": [_vp, _c_i64, _c_i64, _vp, _c_int, _vp, _c_int, _c_int, _c_dbl, _vp, _vp, _vp, _vp],
     "asvgp_accum_2d_binned": [_vp, _vp, _c_i64, _vp, _c_int, _vp, _c_int, _c_int, _vp, _vp, _vp, _c_i64, _vp],
     "asvgp_order_probe_2d": [_vp, _c_i64, _vp, _c_int, _vp, _c_int, _vp, _vp],
+    "asvgp_accum_2d_typed": [_vp, _c_int, _vp, _c_int, _c_i64, _vp, _c_int, _vp, _c_int, _c_int, _vp, _vp, _vp],
+    "asvgp_accum_2d_raster_typed": [_vp, _c_int, _vp, _c_int, _c_i64, _c_i64, _vp, _c_int, _vp, _c_int, _c_int, _vp, _vp, _vp],
+    "asvgp_accum_2d_binned_typed": [_vp, _c_int, _vp, _c_int, _c_i64, _vp, _c_int, _vp, _c_int, _c_int, _vp, _vp, _vp, _c_i64,
+                                    _vp],
+    "asvgp_order_probe_2d_typed": [_vp, _c_int, _c_i64, _vp, _c_int, _vp, _c_int, _vp, _vp],
     "asvgp_expand_moments_2d": [_vp, _vp, _vp, _c_int, _c_int, _c_int, _vp, _vp, _vp],
     "asvgp_kron_factor": [_vp, _vp, _vp, _c_int, _c_int, _c_int, _c_dbl, _vp, _vp, _vp, _vp],
     "asvgp_kron_selinv": [_vp, _c_int, _c_int, _c_int, _vp, _vp, _vp, _vp, _vp],

@@ -76,13 +76,39 @@ __device__ __forceinline__ double2 ldg_stream2(const double* p, uint64_t pol) {
     return v;
 }
 
+__device__ __forceinline__ float4 ldg_stream4f(const float* p, uint64_t pol) {
+    float4 v;
+    asm volatile("ld.global.nc.L1::no_allocate.L2::cache_hint.v4.f32 {%0, %1, %2, %3}, [%4], %5;"
+                 : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p), "l"(pol));
+    return v;
+}
+
 __device__ __forceinline__ void cp_async_16_stream(unsigned dst_smem, const void* src, uint64_t pol) {
     asm volatile("cp.async.cg.shared.global.L2::cache_hint [%0], [%1], 16, %2;" ::"r"(dst_smem), "l"(src), "l"(pol) : "memory");
 }
 __device__ __forceinline__ void cp_async_8_stream(unsigned dst_smem, const void* src, uint64_t pol) {
     asm volatile("cp.async.ca.shared.global.L2::cache_hint [%0], [%1], 8, %2;" ::"r"(dst_smem), "l"(src), "l"(pol) : "memory");
 }
+__device__ __forceinline__ void cp_async_4_stream(unsigned dst_smem, const void* src, uint64_t pol) {
+    asm volatile("cp.async.ca.shared.global.L2::cache_hint [%0], [%1], 4, %2;" ::"r"(dst_smem), "l"(src), "l"(pol) : "memory");
+}
 #endif
+
+// ---- element types of the training points (ASVGP_F64 / ASVGP_F32 of the C ABI) ----------------------------------------
+// The point-reading kernels are templated on the element types of x / X and y and convert every loaded value to double in
+// registers (exact for float), so all arithmetic after the load is the float64 code.
+template <class T> struct TypeTag { using type = T; };
+ASVGP_HD bool valid_elem_type(int t) { return t == 0 || t == 1; }
+// the element-type check of a typed entry point taking two arrays (before any CUDA call)
+#define ASVGP_REQUIRE_TYPES(what, xt, yt) \
+    ASVGP_REQUIRE(::asvgp::valid_elem_type(xt) && ::asvgp::valid_elem_type(yt), \
+                  what ": element types %d, %d (0 = float64, 1 = float32)", xt, yt)
+// f(TypeTag<TX>(), TypeTag<TY>()) for the two type codes (checked with valid_elem_type beforehand)
+template <class F>
+int with_elem_types(int x_type, int y_type, F&& f) {
+    if (x_type == 1) return y_type == 1 ? f(TypeTag<float>(), TypeTag<float>()) : f(TypeTag<float>(), TypeTag<double>());
+    return y_type == 1 ? f(TypeTag<double>(), TypeTag<float>()) : f(TypeTag<double>(), TypeTag<double>());
+}
 
 template <class LoadFn>
 ASVGP_HD int locate_interval(const Mesh& mesh, double x, LoadFn load) {

@@ -12,6 +12,8 @@
 // with warp shuffles and issues one fp64 RED per band entry, then switches interval.  Points that belong to neither
 // the old nor the new interval (only possible for unsorted input) are added with per-point REDs, so any input order
 // gives the right answer; sorted input costs ~(k+1)(k+4)/2 REDs per warp per interval crossing, i.e. nothing.
+// x and y may each be float32 or float64 (asvgp_accum_1d_typed): they are loaded in their own type and converted to double in
+// registers, so a float32 pair streams 8 B per point instead of 16 through the same fp64 arithmetic.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -221,13 +223,38 @@ __device__ __forceinline__ void scatter_point(const Mesh& mesh, int idx, double 
     }
 }
 
-// VEC = 2: x and y are 16-byte aligned and read as double2; VEC = 1: scalar loads (misaligned views).
-template <int K, int VEC>
+// VEC consecutive points of one array from a 16-byte aligned address, evict-first: double2 loads, or one float4
+template <int VEC>
+__device__ __forceinline__ void ldg_stream_vec(const double* p, double (&v)[VEC], uint64_t pol) {
+#pragma unroll
+    for (int h = 0; h < VEC; h += 2) {
+        const double2 d = ldg_stream2(p + h, pol);
+        v[h] = d.x; v[h + 1] = d.y;
+    }
+}
+template <int VEC>
+__device__ __forceinline__ void ldg_stream_vec(const float* p, float (&v)[VEC], uint64_t pol) {
+    static_assert(VEC == 4, "float32 points are read four at a time");
+    const float4 f = ldg_stream4f(p, pol);
+    v[0] = f.x; v[1] = f.y; v[2] = f.z; v[3] = f.w;
+}
+
+// Slots in flight per lane.  2-point float64 slots: 8 (256 B).  4-point slots carry four copies of the per-point code, so
+// fewer of them fit the 128 registers of two CTAs per SM without spilling at k = 3: 6 for a float32 pair (24 points,
+// 192 B), 4 for a mixed pair (16 points, 192 B).
+template <int VEC, class TX, class TY>
+constexpr int accum_unroll() { return VEC == 4 ? (sizeof(TX) == sizeof(TY) ? 6 : 4) : kAccumUnroll; }
+
+// x and y hold float64 or float32 (TX, TY); the values stay in their own type until they are used and are converted to
+// double there (exact).  VEC = 2: both arrays are float64 and 16-byte aligned and are read as double2; VEC = 4: at least
+// one is float32, both are 16-byte aligned, a slot is 4 points (float4, or 2 x double2); VEC = 1: scalar loads
+// (misaligned views).
+template <int K, int VEC, class TX, class TY>
 __global__ void __launch_bounds__(kAccumThreads, 2)
-accum_1d_kernel(const double* __restrict__ x, const double* __restrict__ y, int64_t n,
+accum_1d_kernel(const TX* __restrict__ x, const TY* __restrict__ y, int64_t n,
                 const double* __restrict__ knots, int n_knots, int M,
                 double* __restrict__ G, double* __restrict__ b, double* __restrict__ scal) {
-    constexpr int U = kAccumUnroll;
+    constexpr int U = accum_unroll<VEC, TX, TY>();
     const Mesh mesh = load_mesh(knots, n_knots);
     const int lane = threadIdx.x & 31;
     const int warp = threadIdx.x >> 5;
@@ -258,45 +285,49 @@ accum_1d_kernel(const double* __restrict__ x, const double* __restrict__ y, int6
     const int64_t w_end = imin64(w_begin + per_warp, t_end);
 
     for (int64_t tl = w_begin; tl < w_end; ++tl) {
-        double xs[U][VEC], ys[U][VEC];
+        TX xs[U][VEC];
+        TY ys[U][VEC];
         const int64_t slot0 = tl * tile + lane;
 #pragma unroll
         for (int j = 0; j < U; ++j) {
             const int64_t slot = slot0 + j * 32;
             const int64_t p = slot * VEC;
-            if (VEC == 2) {
-                if (p + 1 < n) {
-                    const double2 xv = ldg_stream2(x + p, stream_policy);
-                    const double2 yv = ldg_stream2(y + p, stream_policy);
-                    xs[j][0] = xv.x; xs[j][VEC - 1] = xv.y;
-                    ys[j][0] = yv.x; ys[j][VEC - 1] = yv.y;
+            if constexpr (VEC > 1) {
+                if (p + VEC - 1 < n) {
+                    ldg_stream_vec<VEC>(x + p, xs[j], stream_policy);
+                    ldg_stream_vec<VEC>(y + p, ys[j], stream_policy);
                 } else {
-                    xs[j][0] = (p < n) ? __ldg(x + p) : 0.0;
-                    ys[j][0] = (p < n) ? __ldg(y + p) : 0.0;
-                    xs[j][VEC - 1] = xs[j][0];
-                    ys[j][VEC - 1] = 0.0;
+                    // the array's tail: entries past n (never added) repeat the slot's first x
+#pragma unroll
+                    for (int e = 0; e < VEC; ++e) {
+                        xs[j][e] = (p + e < n) ? __ldg(x + p + e) : (e ? xs[j][0] : (TX)0);
+                        ys[j][e] = (p + e < n) ? __ldg(y + p + e) : (TY)0;
+                    }
                 }
             } else {
-                xs[j][0] = (p < n) ? __ldg(x + p) : 0.0;
-                ys[j][0] = (p < n) ? __ldg(y + p) : 0.0;
+                xs[j][0] = (p < n) ? __ldg(x + p) : (TX)0;
+                ys[j][0] = (p < n) ? __ldg(y + p) : (TY)0;
             }
         }
 #pragma unroll
         for (int j = 0; j < U; ++j) {
             const int64_t p = (slot0 + j * 32) * VEC;
+            double xd[VEC], yd[VEC];
+#pragma unroll
+            for (int e = 0; e < VEC; ++e) { xd[e] = (double)xs[j][e]; yd[e] = (double)ys[j][e]; }
             bool valid[VEC], in[VEC];
             bool all_in = true;
 #pragma unroll
             for (int e = 0; e < VEC; ++e) {
                 valid[e] = (p + e) < n;
-                in[e] = wa.inside(xs[j][e]);
+                in[e] = wa.inside(xd[e]);
                 all_in = all_in && (in[e] || !valid[e]);
-                if (valid[e]) yy = fma(ys[j][e], ys[j][e], yy);
+                if (valid[e]) yy = fma(yd[e], yd[e], yy);
             }
             if (__all_sync(0xffffffffu, all_in)) {
 #pragma unroll
                 for (int e = 0; e < VEC; ++e)
-                    if (valid[e]) wa.add(mesh, xs[j][e], ys[j][e]);
+                    if (valid[e]) wa.add(mesh, xd[e], yd[e]);
                 wa.dirty = true;
             } else {
                 // interval crossing (or unsorted input)
@@ -307,9 +338,9 @@ accum_1d_kernel(const double* __restrict__ x, const double* __restrict__ y, int6
                 for (int e = 0; e < VEC; ++e) {
                     where[e] = -1;
                     if (valid[e]) {
-                        if (in[e]) { wa.add(mesh, xs[j][e], ys[j][e]); added_old = true; }
+                        if (in[e]) { wa.add(mesh, xd[e], yd[e]); added_old = true; }
                         else {
-                            where[e] = locate_interval(mesh, xs[j][e], LdgLoader());
+                            where[e] = locate_interval(mesh, xd[e], LdgLoader());
                             pending = true;
                             cand = where[e];
                         }
@@ -325,8 +356,8 @@ accum_1d_kernel(const double* __restrict__ x, const double* __restrict__ y, int6
 #pragma unroll
                 for (int e = 0; e < VEC; ++e) {
                     if (where[e] >= 0) {
-                        if (where[e] == wa.cur) { wa.add(mesh, xs[j][e], ys[j][e]); added = true; }
-                        else scatter_point<K>(mesh, where[e], xs[j][e], ys[j][e], G, b, M);
+                        if (where[e] == wa.cur) { wa.add(mesh, xd[e], yd[e]); added = true; }
+                        else scatter_point<K>(mesh, where[e], xd[e], yd[e], G, b, M);
                     }
                 }
                 wa.dirty = __any_sync(0xffffffffu, added);
@@ -355,9 +386,10 @@ constexpr int kUnitPoints1 = 4096;  // points per unit (2048-point units at thre
 constexpr int kUnitMargin = 2;      // intervals either side of a bucket the exact interval may fall into (a float32-built
                                     // mesh is not the uniform grid the bucket guess assumes); beyond: per-point REDs
 
+template <class TX, class TY>
 struct Points1D {
-    const double* x;
-    const double* y;
+    const TX* x;
+    const TY* y;
     const double* knots;
     int n_knots;
     int ipb;            // knot intervals per bucket
@@ -368,8 +400,8 @@ struct Points1D {
         const int hi = n_knots - 2;
         return g < 0.0 ? 0 : (g > (double)hi ? hi : (int)g);
     }
-    __device__ __forceinline__ int bucket(int64_t i) const { return guess(__ldg(x + i)) / ipb; }
-    __device__ __forceinline__ void load(int64_t i, double (&v)[2]) const { v[0] = __ldg(x + i); v[1] = __ldg(y + i); }
+    __device__ __forceinline__ int bucket(int64_t i) const { return guess((double)__ldg(x + i)) / ipb; }
+    __device__ __forceinline__ void load(int64_t i, double (&v)[2]) const { v[0] = (double)__ldg(x + i); v[1] = (double)__ldg(y + i); }
     __device__ __forceinline__ int bucket_of(const double (&v)[2]) const { return guess(v[0]) / ipb; }
 };
 
@@ -508,13 +540,14 @@ static size_t accum_1d_units_smem(int n_bins) { return (size_t)2 * kUnitPoints1 
 
 // Fraction of sampled neighbours (x[i], x[i+1]) that lie more than one knot interval apart: ~0 for time-series order,
 // ~1 for shuffled input.  out[0] += jumps / samples.
-__global__ void __launch_bounds__(256) order_probe_1d_kernel(const double* __restrict__ x, int64_t n, const double* __restrict__ knots,
+template <class TX>
+__global__ void __launch_bounds__(256) order_probe_1d_kernel(const TX* __restrict__ x, int64_t n, const double* __restrict__ knots,
                                                              int n_knots, int samples, double* __restrict__ out) {
     const Mesh mesh = load_mesh(knots, n_knots);
     int jumps = 0;
     for (int s = threadIdx.x; s < samples; s += blockDim.x) {
         const int64_t i = (int64_t)((double)s * (double)(n - 1) / (double)samples);
-        const int a = locate_interval(mesh, __ldg(x + i), LdgLoader()), c = locate_interval(mesh, __ldg(x + i + 1), LdgLoader());
+        const int a = locate_interval(mesh, (double)__ldg(x + i), LdgLoader()), c = locate_interval(mesh, (double)__ldg(x + i + 1), LdgLoader());
         jumps += (a - c > 1 || c - a > 1) ? 1 : 0;
     }
     jumps = __reduce_add_sync(0xffffffffu, jumps);
@@ -724,41 +757,66 @@ extern "C" int asvgp_basis_eval_1d(const double* x, int64_t n, const double* mes
     return kOk;
 }
 
-extern "C" int asvgp_accum_1d(const double* x, const double* y, int64_t n, const double* mesh, int n_knots, int order,
-                              double* acc, void* stream) {
-    ASVGP_REQUIRE(n >= 0 && n_knots >= 2, "accum_1d: n=%lld n_knots=%d", (long long)n, n_knots);
-    ASVGP_REQUIRE(order >= 1 && order <= kMaxOrder, "accum_1d: spline order %d not in 1..6", order);
-    if (n == 0) return kOk;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
+template <class TX, class TY>
+static int launch_accum_1d(const TX* x, const TY* y, int64_t n, const double* mesh, int n_knots, int order, double* acc,
+                           cudaStream_t st) {
     const int M = n_knots + order - 1;
     double* G = acc;
     double* b = acc + (int64_t)(order + 1) * M;
     double* scal = b + M;
     const bool vec = ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) & 15u) == 0;
-    const int64_t per_tile = 32 * kAccumUnroll * (vec ? 2 : 1);
+    constexpr int VV = (sizeof(TX) == 8 && sizeof(TY) == 8) ? 2 : 4;      // points per slot of the vector path
+    const int64_t per_tile = 32 * (vec ? (int64_t)accum_unroll<VV, TX, TY>() * VV : (int64_t)accum_unroll<1, TX, TY>());
     const int64_t n_tiles = (n + per_tile - 1) / per_tile;
     // (tools/accum_sweep.py: 2 and 4 CTAs' worth of ranges per SM both give 0.258 ms at N = 1e8; 3, 8, 16 are slower)
     const int blocks = (int)std::min<int64_t>((n_tiles + 7) / 8, (int64_t)accum_sm_budget() * 2);
     if (vec) {
-        ASVGP_DISPATCH_ORDER(order, (accum_1d_kernel<K, 2><<<blocks, kAccumThreads, 0, st>>>(x, y, n, mesh, n_knots, M, G, b, scal))); ASVGP_LAUNCHED();
+        ASVGP_DISPATCH_ORDER(order, (accum_1d_kernel<K, VV, TX, TY><<<blocks, kAccumThreads, 0, st>>>(x, y, n, mesh, n_knots, M, G, b, scal))); ASVGP_LAUNCHED();
     } else {
-        ASVGP_DISPATCH_ORDER(order, (accum_1d_kernel<K, 1><<<blocks, kAccumThreads, 0, st>>>(x, y, n, mesh, n_knots, M, G, b, scal))); ASVGP_LAUNCHED();
+        ASVGP_DISPATCH_ORDER(order, (accum_1d_kernel<K, 1, TX, TY><<<blocks, kAccumThreads, 0, st>>>(x, y, n, mesh, n_knots, M, G, b, scal))); ASVGP_LAUNCHED();
     }
     ASVGP_CUDA_OK(cudaGetLastError());
     return kOk;
 }
 
+extern "C" int asvgp_accum_1d_typed(const void* x, int x_type, const void* y, int y_type, int64_t n, const double* mesh,
+                                    int n_knots, int order, double* acc, void* stream) {
+    ASVGP_REQUIRE_TYPES("accum_1d", x_type, y_type);
+    ASVGP_REQUIRE(n >= 0 && n_knots >= 2, "accum_1d: n=%lld n_knots=%d", (long long)n, n_knots);
+    ASVGP_REQUIRE(order >= 1 && order <= kMaxOrder, "accum_1d: spline order %d not in 1..6", order);
+    if (n == 0) return kOk;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    return with_elem_types(x_type, y_type, [&](auto tx, auto ty) -> int {
+        using TX = typename decltype(tx)::type;
+        using TY = typename decltype(ty)::type;
+        return launch_accum_1d(static_cast<const TX*>(x), static_cast<const TY*>(y), n, mesh, n_knots, order, acc, st);
+    });
+}
+
+extern "C" int asvgp_accum_1d(const double* x, const double* y, int64_t n, const double* mesh, int n_knots, int order,
+                              double* acc, void* stream) {
+    return asvgp_accum_1d_typed(x, ASVGP_F64, y, ASVGP_F64, n, mesh, n_knots, order, acc, stream);
+}
+
 extern "C" int64_t asvgp_accum_1d_binned_work_bytes(int64_t n) { return PartWork::bytes(n < 0 ? 0 : n, 2); }
 
-extern "C" int asvgp_order_probe_1d(const double* x, int64_t n, const double* mesh, int n_knots, double* out, void* stream) {
+extern "C" int asvgp_order_probe_1d_typed(const void* x, int x_type, int64_t n, const double* mesh, int n_knots, double* out,
+                                          void* stream) {
+    ASVGP_REQUIRE(valid_elem_type(x_type), "order_probe_1d: element type %d (0 = float64, 1 = float32)", x_type);
     ASVGP_REQUIRE(n >= 0 && n_knots >= 2 && out != nullptr, "order_probe_1d: n=%lld n_knots=%d", (long long)n, n_knots);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     ASVGP_CUDA_OK(cudaMemsetAsync(out, 0, sizeof(double), st));
     if (n < 2) return kOk;
     const int samples = (int)std::min<int64_t>(n - 1, 4096);
-    order_probe_1d_kernel<<<1, 256, 0, st>>>(x, n, mesh, n_knots, samples, out); ASVGP_LAUNCHED();
+    if (x_type == ASVGP_F32) order_probe_1d_kernel<<<1, 256, 0, st>>>(static_cast<const float*>(x), n, mesh, n_knots, samples, out);
+    else order_probe_1d_kernel<<<1, 256, 0, st>>>(static_cast<const double*>(x), n, mesh, n_knots, samples, out);
+    ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     return kOk;
+}
+
+extern "C" int asvgp_order_probe_1d(const double* x, int64_t n, const double* mesh, int n_knots, double* out, void* stream) {
+    return asvgp_order_probe_1d_typed(x, ASVGP_F64, n, mesh, n_knots, out, stream);
 }
 
 template <int K>
@@ -776,14 +834,15 @@ static int launch_accum_1d_units(const PartWork& w, int64_t n, const double* mes
     return kOk;
 }
 
-extern "C" int asvgp_accum_1d_binned(const double* x, const double* y, int64_t n, const double* mesh, int n_knots, int order,
-                                     double* acc, void* work, int64_t work_bytes, void* stream) {
+extern "C" int asvgp_accum_1d_binned_typed(const void* x, int x_type, const void* y, int y_type, int64_t n, const double* mesh,
+                                           int n_knots, int order, double* acc, void* work, int64_t work_bytes, void* stream) {
+    ASVGP_REQUIRE_TYPES("accum_1d_binned", x_type, y_type);
     ASVGP_REQUIRE(n >= 0 && n_knots >= 2, "accum_1d_binned: n=%lld n_knots=%d", (long long)n, n_knots);
     ASVGP_REQUIRE(order >= 1 && order <= kMaxOrder, "accum_1d_binned: spline order %d not in 1..6", order);
     const int n_int = n_knots - 1;
     const int ipb = (n_int + kPartBuckets - 1) / kPartBuckets;
     if (ipb + 2 * kUnitMargin > kUnitMaxBins)  // more than ~2^20 knot intervals: the general kernel handles any order
-        return asvgp_accum_1d(x, y, n, mesh, n_knots, order, acc, stream);
+        return asvgp_accum_1d_typed(x, x_type, y, y_type, n, mesh, n_knots, order, acc, stream);
     ASVGP_REQUIRE(work != nullptr && work_bytes >= PartWork::bytes(n, 2), "accum_1d_binned: work_bytes=%lld < %lld",
                   (long long)work_bytes, (long long)PartWork::bytes(n, 2));
     if (n == 0) return kOk;
@@ -794,13 +853,25 @@ extern "C" int asvgp_accum_1d_binned(const double* x, const double* y, int64_t n
     double* scal = b + M;
     const PartWork w = PartWork::carve(work);
     ASVGP_CUDA_OK(cudaMemsetAsync(w.count, 0, kPartBuckets * sizeof(u64), st));
-    Points1D src;
-    src.x = x; src.y = y; src.knots = mesh; src.n_knots = n_knots; src.ipb = ipb;
     const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>((n + kPartTile - 1) / kPartTile, (int64_t)sm_count() * 2));
-    ASVGP_CUDA_OK((launch_partition<Points1D, 2>(src, n, w, kUnitPoints1, blocks, st)));
+    // the partition reads the points in their own types and writes float64 records: the units kernel is type-free
+    const int prc = with_elem_types(x_type, y_type, [&](auto tx, auto ty) -> int {
+        using TX = typename decltype(tx)::type;
+        using TY = typename decltype(ty)::type;
+        Points1D<TX, TY> src;
+        src.x = static_cast<const TX*>(x); src.y = static_cast<const TY*>(y); src.knots = mesh; src.n_knots = n_knots; src.ipb = ipb;
+        ASVGP_CUDA_OK((launch_partition<Points1D<TX, TY>, 2>(src, n, w, kUnitPoints1, blocks, st)));
+        return kOk;
+    });
+    if (prc != kOk) return prc;
     int rc = kOk;
     ASVGP_DISPATCH_ORDER(order, (rc = launch_accum_1d_units<K>(w, n, mesh, n_knots, ipb, M, G, b, scal, st)));
     return rc;
+}
+
+extern "C" int asvgp_accum_1d_binned(const double* x, const double* y, int64_t n, const double* mesh, int n_knots, int order,
+                                     double* acc, void* work, int64_t work_bytes, void* stream) {
+    return asvgp_accum_1d_binned_typed(x, ASVGP_F64, y, ASVGP_F64, n, mesh, n_knots, order, acc, work, work_bytes, stream);
 }
 
 extern "C" int asvgp_predict_1d(const double* xnew, int64_t n, const double* mesh, int n_knots, int order,

@@ -15,6 +15,8 @@
 // move to another cell.  A second, tiny kernel expands the moment table into the Gram stencil and the projection.
 // Every thread walks its own contiguous slice of the points, so raster-ordered data (x1 slow) gives runs of
 // ~n2/(m2-k) points per flush; any order gives the right answer.
+// X and y may each be float32 or float64 (asvgp_accum_2d_typed): every kernel that reads points is templated on the two
+// element types and converts each loaded value to double in registers (12 B per point for float32 data instead of 24).
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -41,6 +43,23 @@ __device__ __forceinline__ Mesh load_mesh2(const double* knots, int n_knots) {
     m.x0 = __ldg(knots);
     m.inv_delta = 1.0 / (__ldg(knots + 1) - m.x0);
     return m;
+}
+
+// Loads of the training points, which are float64 or float32 (X and y independently): every value is converted to double
+// in registers (exact), so everything after the load is the float64 code.
+__device__ __forceinline__ double ldg_d(const double* p) { return __ldg(p); }
+__device__ __forceinline__ double ldg_d(const float* p) { return (double)__ldg(p); }
+// point i (x1, x2) of a row-major [n, 2] array
+__device__ __forceinline__ double2 ldg_point(const double* X, int64_t i) { return __ldg(reinterpret_cast<const double2*>(X) + i); }
+__device__ __forceinline__ double2 ldg_point(const float* X, int64_t i) {
+    const float2 p = __ldg(reinterpret_cast<const float2*>(X) + i);
+    return make_double2(p.x, p.y);
+}
+// targets i and i + 1, i even (one 16-byte / 8-byte load)
+__device__ __forceinline__ double2 ldg_pair(const double* y, int64_t i) { return __ldg(reinterpret_cast<const double2*>(y + i)); }
+__device__ __forceinline__ double2 ldg_pair(const float* y, int64_t i) {
+    const float2 p = __ldg(reinterpret_cast<const float2*>(y + i));
+    return make_double2(p.x, p.y);
 }
 
 struct Interval {            // cached knot interval of one dimension
@@ -78,9 +97,9 @@ __device__ __forceinline__ void powers(double t, double (&tp)[N + 1], double (&u
 // Thread-private accumulation over a contiguous slice of points.  [P0, P1) is the range of the dim-1 moment index
 // this launch handles (register budget: one launch for k <= 3, split launches for k >= 4); WITH_Y: also the
 // projection moments, sum y^2 and the count.
-template <int K, int P0, int P1, bool WITH_Y>
+template <int K, int P0, int P1, bool WITH_Y, class TX, class TY>
 __global__ void __launch_bounds__(256, 1)
-accum_2d_kernel(const double* __restrict__ X, const double* __restrict__ y, int64_t n,
+accum_2d_kernel(const TX* __restrict__ X, const TY* __restrict__ y, int64_t n,
                 const double* __restrict__ knots1, int nk1, const double* __restrict__ knots2, int nk2,
                 double* __restrict__ cellmom, double* __restrict__ scal, const int* __restrict__ select, int want) {
     if (select != nullptr && *select != want) return;
@@ -159,15 +178,14 @@ accum_2d_kernel(const double* __restrict__ X, const double* __restrict__ y, int6
         dirty = true;
     };
 
-    // X is row-major [n, 2]: one 16-byte load per point; begin is even so y pairs are 16-byte aligned too
-    const double2* __restrict__ X2 = reinterpret_cast<const double2*>(X);
+    // X is row-major [n, 2]: one 16-byte (float32: 8-byte) load per point; begin is even so y pairs are aligned too
     int64_t i = begin;
     for (; i + 4 <= end; i += 4) {
-        const double2 pa = __ldg(X2 + i), pb = __ldg(X2 + i + 1), pc = __ldg(X2 + i + 2), pd = __ldg(X2 + i + 3);
+        const double2 pa = ldg_point(X, i), pb = ldg_point(X, i + 1), pc = ldg_point(X, i + 2), pd = ldg_point(X, i + 3);
         double2 ya = make_double2(0.0, 0.0), yb = ya;
         if (WITH_Y) {
-            ya = __ldg(reinterpret_cast<const double2*>(y + i));
-            yb = __ldg(reinterpret_cast<const double2*>(y + i + 2));
+            ya = ldg_pair(y, i);
+            yb = ldg_pair(y, i + 2);
         }
         add(pa.x, pa.y, ya.x);
         add(pb.x, pb.y, ya.y);
@@ -175,8 +193,8 @@ accum_2d_kernel(const double* __restrict__ X, const double* __restrict__ y, int6
         add(pd.x, pd.y, yb.y);
     }
     for (; i < end; ++i) {
-        const double2 pa = __ldg(X2 + i);
-        add(pa.x, pa.y, WITH_Y ? __ldg(y + i) : 0.0);
+        const double2 pa = ldg_point(X, i);
+        add(pa.x, pa.y, WITH_Y ? ldg_d(y + i) : 0.0);
     }
     flush();
 
@@ -205,9 +223,9 @@ accum_2d_kernel(const double* __restrict__ X, const double* __restrict__ y, int6
 // handled correctly (a run may have length 1); asvgp_accum_2d picks this kernel when a probe finds the input
 // gridded.
 // ------------------------------------------------------------------------------------------------------------------
-template <int K>
+template <int K, class TX, class TY>
 __global__ void __launch_bounds__(256, 2)
-accum_2d_run_kernel(const double* __restrict__ X, const double* __restrict__ y, int64_t n,
+accum_2d_run_kernel(const TX* __restrict__ X, const TY* __restrict__ y, int64_t n,
                     const double* __restrict__ knots1, int nk1, const double* __restrict__ knots2, int nk2,
                     double* __restrict__ cellmom, double* __restrict__ scal, const int* __restrict__ select,
                     int want) {
@@ -283,22 +301,20 @@ accum_2d_run_kernel(const double* __restrict__ X, const double* __restrict__ y, 
         dirty = true;
     };
 
-    // X is row-major [n, 2]: one 16-byte load per point; begin is a multiple of 4 so y pairs are 16-byte aligned.
+    // X is row-major [n, 2]: one 16-byte (float32: 8-byte) load per point; begin is a multiple of 4 so y pairs are aligned.
     // The next group's loads are issued before the current group is processed.
-    const double2* __restrict__ X2 = reinterpret_cast<const double2*>(X);
-    const double2* __restrict__ Y2 = reinterpret_cast<const double2*>(y);
     const int64_t n_full = begin + ((end - begin) & ~(int64_t)3);
     double2 pa, pb, pc, pd, ya, yb;
     int64_t i = begin;
     if (i < n_full) {
-        pa = __ldg(X2 + i); pb = __ldg(X2 + i + 1); pc = __ldg(X2 + i + 2); pd = __ldg(X2 + i + 3);
-        ya = __ldg(Y2 + (i >> 1)); yb = __ldg(Y2 + (i >> 1) + 1);
+        pa = ldg_point(X, i); pb = ldg_point(X, i + 1); pc = ldg_point(X, i + 2); pd = ldg_point(X, i + 3);
+        ya = ldg_pair(y, i); yb = ldg_pair(y, i + 2);
     }
     for (; i < n_full; i += 4) {
         const double2 ca = pa, cb = pb, cc = pc, cd = pd, cya = ya, cyb = yb;
         if (i + 4 < n_full) {
-            pa = __ldg(X2 + i + 4); pb = __ldg(X2 + i + 5); pc = __ldg(X2 + i + 6); pd = __ldg(X2 + i + 7);
-            ya = __ldg(Y2 + (i >> 1) + 2); yb = __ldg(Y2 + (i >> 1) + 3);
+            pa = ldg_point(X, i + 4); pb = ldg_point(X, i + 5); pc = ldg_point(X, i + 6); pd = ldg_point(X, i + 7);
+            ya = ldg_pair(y, i + 4); yb = ldg_pair(y, i + 6);
         }
         add(ca.x, ca.y, cya.x);
         add(cb.x, cb.y, cya.y);
@@ -306,8 +322,8 @@ accum_2d_run_kernel(const double* __restrict__ X, const double* __restrict__ y, 
         add(cd.x, cd.y, cyb.y);
     }
     for (; i < end; ++i) {
-        const double2 p = __ldg(X2 + i);
-        add(p.x, p.y, __ldg(y + i));
+        const double2 p = ldg_point(X, i);
+        add(p.x, p.y, ldg_d(y + i));
     }
     flush();
 
@@ -355,13 +371,19 @@ __device__ __forceinline__ void prefetch_l2_span(const double* first, int64_t n_
 __device__ __forceinline__ void ldg256(const double* p, double (&v)[4]) {
     asm volatile("ld.global.nc.v4.f64 {%0,%1,%2,%3}, [%4];" : "=d"(v[0]), "=d"(v[1]), "=d"(v[2]), "=d"(v[3]) : "l"(p));
 }
+// four consecutive values as double: one 256-bit load of float64, one 128-bit load of float32
+__device__ __forceinline__ void ldg4(const double* p, double (&v)[4]) { ldg256(p, v); }
+__device__ __forceinline__ void ldg4(const float* p, double (&v)[4]) {
+    const float4 f = __ldg(reinterpret_cast<const float4*>(p));
+    v[0] = f.x; v[1] = f.y; v[2] = f.z; v[3] = f.w;
+}
 
 constexpr int kRasterWarps = 8;          // 256 threads, two CTAs per SM (<= 128 registers per thread): occupancy beats
                                          // a deeper register-staged prefetch here (measured: 6 warps x 8-point groups was slower)
 
-template <int K, bool VEC256>
+template <int K, bool VEC256, class TX, class TY>
 __global__ void __launch_bounds__(kRasterWarps * 32, 2)
-accum_2d_raster_kernel(const double* __restrict__ X, const double* __restrict__ y, int64_t n,
+accum_2d_raster_kernel(const TX* __restrict__ X, const TY* __restrict__ y, int64_t n,
                        const double* __restrict__ knots1, int nk1, const double* __restrict__ knots2, int nk2,
                        double* __restrict__ cellmom, double* __restrict__ scal, const ProbeResult* __restrict__ probe) {
     if (probe->select != (VEC256 ? 3 : 2)) return;
@@ -396,8 +418,8 @@ accum_2d_raster_kernel(const double* __restrict__ X, const double* __restrict__ 
         const int64_t row = g * 32 + lane;
         const bool active = row < n1;
         const int64_t c_begin = sg * seg_len, c_end = c_begin + seg_len < n2 ? c_begin + seg_len : n2;
-        const double* xr = X + 2 * (row * n2);
-        const double* yr = y + row * n2;
+        const TX* xr = X + 2 * (row * n2);
+        const TY* yr = y + row * n2;
 #pragma unroll
         for (int i = 0; i < NB; ++i) s[i] = 0.0;
 #pragma unroll
@@ -478,30 +500,29 @@ accum_2d_raster_kernel(const double* __restrict__ X, const double* __restrict__ 
         };
 
         if (VEC256) {
-            // n2 % 4 == 0 and 32-byte aligned bases: four points = two 256-bit loads of X and one of y, the next group's
-            // loads in flight while the current one is processed
+            // n2 % 4 == 0 and 32-byte aligned bases: four points = two 256-bit loads of X and one of y (float32: 128-bit
+            // loads), the next group's loads in flight while the current one is processed
             double xa[4], xb[4], ya[4];
             int64_t c = c_begin;
-            if (active && c < c_end) { ldg256(xr + 2 * c, xa); ldg256(xr + 2 * c + 4, xb); ldg256(yr + c, ya); }
+            if (active && c < c_end) { ldg4(xr + 2 * c, xa); ldg4(xr + 2 * c + 4, xb); ldg4(yr + c, ya); }
             for (; c < c_end; c += 4) {
                 double ca[4], cb[4], cy[4];
 #pragma unroll
                 for (int i = 0; i < 4; ++i) { ca[i] = xa[i]; cb[i] = xb[i]; cy[i] = ya[i]; }
-                if (active && c + 4 < c_end) { ldg256(xr + 2 * (c + 4), xa); ldg256(xr + 2 * (c + 4) + 4, xb); ldg256(yr + c + 4, ya); }
+                if (active && c + 4 < c_end) { ldg4(xr + 2 * (c + 4), xa); ldg4(xr + 2 * (c + 4) + 4, xb); ldg4(yr + c + 4, ya); }
                 add(ca[0], ca[1], cy[0], active);
                 add(ca[2], ca[3], cy[1], active);
                 add(cb[0], cb[1], cy[2], active);
                 add(cb[2], cb[3], cy[3], active);
             }
         } else {
-            const double2* __restrict__ X2 = reinterpret_cast<const double2*>(xr);
             double2 pn = make_double2(0.0, 0.0);
             double yn = 0.0;
-            if (active && c_begin < c_end) { pn = __ldg(X2 + c_begin); yn = __ldg(yr + c_begin); }
+            if (active && c_begin < c_end) { pn = ldg_point(xr, c_begin); yn = ldg_d(yr + c_begin); }
             for (int64_t c = c_begin; c < c_end; ++c) {
                 const double2 pc = pn;
                 const double yc = yn;
-                if (active && c + 1 < c_end) { pn = __ldg(X2 + c + 1); yn = __ldg(yr + c + 1); }
+                if (active && c + 1 < c_end) { pn = ldg_point(xr, c + 1); yn = ldg_d(yr + c + 1); }
                 add(pc.x, pc.y, yc, active);
             }
         }
@@ -634,10 +655,27 @@ __device__ __forceinline__ void cp_async_8(void* dst_smem, const void* src) {
 }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+template <int BYTES> __device__ __forceinline__ void cp_async_stream(unsigned dst_smem, const void* src, uint64_t pol) {
+    static_assert(BYTES == 16 || BYTES == 8 || BYTES == 4, "cp.async copies 4, 8 or 16 bytes");
+    if constexpr (BYTES == 16) cp_async_16_stream(dst_smem, src, pol);
+    else if constexpr (BYTES == 8) cp_async_8_stream(dst_smem, src, pol);
+    else cp_async_4_stream(dst_smem, src, pol);
+}
+// one point (x1, x2) in the element type of X: the column sweep's ring holds the points as they are stored
+template <class T> struct Pair;
+template <> struct Pair<double> { using type = double2; };
+template <> struct Pair<float> { using type = float2; };
+__device__ __forceinline__ double2 to_double2(const double2 p) { return p; }
+__device__ __forceinline__ double2 to_double2(const float2 p) { return make_double2(p.x, p.y); }
+template <int K, class TX, class TY>
+constexpr size_t cols_smem() {
+    return sizeof(double) * 3 * kColsWarps * 32 * (3 * (size_t)K + 2)                                   // sums, factors, per-row table
+           + (size_t)kColsWarps * ColsRing<K>::kRows * 32 * (sizeof(typename Pair<TX>::type) + sizeof(TY));   // the ring
+}
 
-template <int K>
+template <int K, class TX, class TY>
 __global__ void __launch_bounds__(kColsWarps * 32, 1)
-accum_2d_cols_kernel(const double* __restrict__ X, const double* __restrict__ y, int64_t n,
+accum_2d_cols_kernel(const TX* __restrict__ X, const TY* __restrict__ y, int64_t n,
                      const double* __restrict__ knots1, int nk1, const double* __restrict__ knots2, int nk2,
                      double* __restrict__ cellmom, double* __restrict__ scal, const ProbeResult* __restrict__ probe,
                      int hint_n2, int tasks_per_warp) {
@@ -654,10 +692,11 @@ accum_2d_cols_kernel(const double* __restrict__ X, const double* __restrict__ y,
     double (*s_S)[32][NS] = reinterpret_cast<double (*)[32][NS]>(raster_smem);
     double (*s_B)[32][NS] = reinterpret_cast<double (*)[32][NS]>(raster_smem + sizeof(double) * kWarps * 32 * NS);
     double (*s_T)[32][NS] = reinterpret_cast<double (*)[32][NS]>(raster_smem + 2 * sizeof(double) * kWarps * 32 * NS);
-    // per warp: ring of kColsRing rows, [row][lane] double2 of X then [row][lane] double of y
+    // per warp: ring of kColsRing rows, [row][lane] point of X then [row][lane] y, in their element types
+    using PX = typename Pair<TX>::type;
     unsigned char* ring_base = raster_smem + 3 * sizeof(double) * kWarps * 32 * NS;
-    double2* ringX = reinterpret_cast<double2*>(ring_base) + (size_t)(threadIdx.x >> 5) * kColsRing * 32;
-    double* ringY = reinterpret_cast<double*>(ring_base + sizeof(double2) * kWarps * kColsRing * 32) + (size_t)(threadIdx.x >> 5) * kColsRing * 32;
+    PX* ringX = reinterpret_cast<PX*>(ring_base) + (size_t)(threadIdx.x >> 5) * kColsRing * 32;
+    TY* ringY = reinterpret_cast<TY*>(ring_base + sizeof(PX) * kWarps * kColsRing * 32) + (size_t)(threadIdx.x >> 5) * kColsRing * 32;
     __shared__ __align__(16) long long s_bits[kWarps][32];     // x1 bit pattern of each table row
     __shared__ __align__(16) int s_cell[kWarps][32];           // its knot interval
     // per group of four table rows: sum over the rows of the Gram factors beta_p(t1) (the same for every column, so on a
@@ -697,7 +736,7 @@ accum_2d_cols_kernel(const double* __restrict__ X, const double* __restrict__ y,
     if (seg_len < 64) seg_len = 64;
     n_seg = (n1 + seg_len - 1) / seg_len;
     const int64_t n_tasks = n_strips * n_seg;
-    const double2* __restrict__ X2 = reinterpret_cast<const double2*>(X);
+    const PX* __restrict__ X2 = reinterpret_cast<const PX*>(X);
 
     double s[NB], sy[NY];
     double su[NB];                       // warp-uniform part of the dim-1 Gram sums (fast path); a lane's sum is s + su
@@ -784,16 +823,16 @@ accum_2d_cols_kernel(const double* __restrict__ X, const double* __restrict__ y,
         // ---- the column walk, pipelined kColsRing rows deep through the shared-memory ring -------------------------
         const int64_t rows_total = r_end - r_begin;
         const int64_t n_groups = (rows_total + 3) >> 2;               // groups of four rows (the last may be ragged)
-        const double2* xq = X2 + r_begin * n2 + colc;                 // next row to request: += n2 per row
-        const double* yq = y + r_begin * n2 + colc;
+        const PX* xq = X2 + r_begin * n2 + colc;                      // next row to request: += n2 per row
+        const TY* yq = y + r_begin * n2 + colc;
         int to_request = (int)rows_total;                             // rows not requested yet (a segment is < 2^31 rows)
         int wslot = 0;                                                // ring slot of the next request (32-bit, no modulo)
         auto request_group = [&]() {                                  // one commit group = up to four rows
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
                 if (to_request > 0) {
-                    cp_async_16_stream(smem_u32(ringX + wslot * 32 + lane), xq, stream_policy);
-                    cp_async_8_stream(smem_u32(ringY + wslot * 32 + lane), yq, stream_policy);
+                    cp_async_stream<sizeof(PX)>(smem_u32(ringX + wslot * 32 + lane), xq, stream_policy);
+                    cp_async_stream<sizeof(TY)>(smem_u32(ringY + wslot * 32 + lane), yq, stream_policy);
                     xq += n2;
                     yq += n2;
                     --to_request;
@@ -807,7 +846,7 @@ accum_2d_cols_kernel(const double* __restrict__ X, const double* __restrict__ y,
         for (int g = 0; g < kGroupsInFlight; ++g) request_group();
         int rslot = 0;                                                // ring slot of the next row to consume
         // x1 of table row `lane` of the next 32-row block, requested one block ahead so that its DRAM latency is hidden
-        double x1_next = (r_begin + lane < r_end) ? __ldg(X + 2 * ((r_begin + lane) * n2 + strip * 32)) : 0.0;
+        double x1_next = (r_begin + lane < r_end) ? ldg_d(X + 2 * ((r_begin + lane) * n2 + strip * 32)) : 0.0;
 
         for (int64_t r0 = r_begin; r0 < r_end; r0 += 32) {
             // ---- dim-1 factors of rows r0 .. r0+31: lane l does row r0 + l ---------------------------------------------
@@ -815,7 +854,7 @@ accum_2d_cols_kernel(const double* __restrict__ X, const double* __restrict__ y,
             {
                 const int64_t r = r0 + lane;
                 const double x1 = x1_next;
-                if (r + 32 < r_end) x1_next = __ldg(X + 2 * ((r + 32) * n2 + strip * 32));
+                if (r + 32 < r_end) x1_next = ldg_d(X + 2 * ((r + 32) * n2 + strip * 32));
                 if (r < r_end) {
                     if (!it.inside(x1)) it.set(mesh1s, locate_interval(mesh1s, x1, PlainLoader2()), PlainLoader2());
                     double tp[2 * K + 1], up[2 * K + 1];
@@ -849,8 +888,8 @@ accum_2d_cols_kernel(const double* __restrict__ X, const double* __restrict__ y,
                 double cy[4];
 #pragma unroll
                 for (int u = 0; u < 4; ++u) {
-                    cx[u] = ringX[(rslot + u) * 32 + lane];           // groups never straddle the end of the ring
-                    cy[u] = ringY[(rslot + u) * 32 + lane];
+                    cx[u] = to_double2(ringX[(rslot + u) * 32 + lane]);   // groups never straddle the end of the ring
+                    cy[u] = (double)ringY[(rslot + u) * 32 + lane];
                 }
                 rslot = rslot + 4 == kColsRing ? 0 : rslot + 4;
                 request_group();
@@ -912,13 +951,16 @@ accum_2d_cols_kernel(const double* __restrict__ X, const double* __restrict__ y,
 //   separable raster : additionally x2 of 1024 sampled points equals x2 of the same column in the first row
 //   x1-run  : at least three quarters of 4096 sampled points share x1 with their successor
 //   general : everything else
-__global__ void __launch_bounds__(1024) accum_2d_probe_kernel(const double* __restrict__ X, const double* __restrict__ y,
+// (Bit patterns are compared on the values converted to double: the conversion from float is exact and one-to-one, so that
+// is the comparison in the source type.)
+template <class TX, class TY>
+__global__ void __launch_bounds__(1024) accum_2d_probe_kernel(const TX* __restrict__ X, const TY* __restrict__ y,
                                                               int64_t n, ProbeResult* __restrict__ out) {
     // 1024 threads, every thread's samples issued back to back: the probe costs a handful of DRAM round trips
     __shared__ int s_cnt[32];
     __shared__ long long s_first;
     const int tid = threadIdx.x;
-    auto x1bits = [&](int64_t i) { return __double_as_longlong(__ldg(X + 2 * i)); };
+    auto x1bits = [&](int64_t i) { return __double_as_longlong(ldg_d(X + 2 * i)); };
     // fraction of points equal to their successor (4 samples per thread)
     const int n_probe = (int)(n - 1 < 4096 ? n - 1 : 4096);
     int hits = 0;
@@ -971,8 +1013,8 @@ __global__ void __launch_bounds__(1024) accum_2d_probe_kernel(const double* __re
         const long long a = x1bits(r * n2), e = x1bits(r * n2 + n2 - 1), pz = r > 0 ? x1bits(r * n2 - 1) : ~a;
         const int64_t rs = n1 > 1 ? 1 + (int64_t)((double)tid * (double)(n1 - 2) / 1023.0 + 0.5) : 0;
         const int64_t c = (int64_t)(((unsigned long long)tid * 2654435761ull) % (unsigned long long)n2);
-        const long long s0 = __double_as_longlong(__ldg(X + 2 * c + 1));
-        const long long s1 = rs < n1 ? __double_as_longlong(__ldg(X + 2 * (rs * n2 + c) + 1)) : s0;
+        const long long s0 = __double_as_longlong(ldg_d(X + 2 * c + 1));
+        const long long s1 = rs < n1 ? __double_as_longlong(ldg_d(X + 2 * (rs * n2 + c) + 1)) : s0;
         raster = !__syncthreads_or(a != e || a == pz);
         separable = !__syncthreads_or(s0 != s1) && raster;
     }
@@ -1420,9 +1462,10 @@ template <int K> struct Units2 {
     static constexpr int EX = NV * GL + 2;                                // doubles of one group's exchange area (+2: groups land on different banks)
 };
 
+template <class TX, class TY>
 struct Points2D {
-    const double* X;
-    const double* y;
+    const TX* X;
+    const TY* y;
     const double* knots1;
     int n_knots1;
     int ipb;            // dim-1 knot intervals per bucket
@@ -1436,10 +1479,10 @@ struct Points2D {
         const int hi = n_knots1 - 2;
         return g < 0.0 ? 0 : (g > (double)hi ? hi : (int)g);
     }
-    __device__ __forceinline__ int bucket(int64_t i) const { return guess(__ldg(X + 2 * i)) / ipb; }
+    __device__ __forceinline__ int bucket(int64_t i) const { return guess(ldg_d(X + 2 * i)) / ipb; }
     __device__ __forceinline__ void load(int64_t i, double (&v)[3]) const {
-        const double2 p = __ldg(reinterpret_cast<const double2*>(X) + i);
-        v[0] = p.x; v[1] = p.y; v[2] = __ldg(y + i);
+        const double2 p = ldg_point(X, i);
+        v[0] = p.x; v[1] = p.y; v[2] = ldg_d(y + i);
     }
     __device__ __forceinline__ int bucket_of(const double (&v)[3]) const { return guess(v[0]) / ipb; }
 };
@@ -1697,15 +1740,16 @@ static size_t accum_2d_units_smem(int nb1, int nc2, int nk2) {
 
 // Fraction of sampled neighbours (point i, point i+1) that lie more than one cell apart in either dimension: ~0 for
 // raster / run-ordered input, ~1 for shuffled input.
-__global__ void __launch_bounds__(256) order_probe_2d_kernel(const double* __restrict__ X, int64_t n, const double* __restrict__ knots1,
+template <class TX>
+__global__ void __launch_bounds__(256) order_probe_2d_kernel(const TX* __restrict__ X, int64_t n, const double* __restrict__ knots1,
                                                              int nk1, const double* __restrict__ knots2, int nk2, int samples,
                                                              double* __restrict__ out) {
     const Mesh mesh1 = load_mesh2(knots1, nk1), mesh2 = load_mesh2(knots2, nk2);
     int jumps = 0;
     for (int s = threadIdx.x; s < samples; s += blockDim.x) {
         const int64_t i = (int64_t)((double)s * (double)(n - 1) / (double)samples);
-        const int a1 = locate_interval(mesh1, __ldg(X + 2 * i), LdgLoader2()), b1 = locate_interval(mesh1, __ldg(X + 2 * i + 2), LdgLoader2());
-        const int a2 = locate_interval(mesh2, __ldg(X + 2 * i + 1), LdgLoader2()), b2 = locate_interval(mesh2, __ldg(X + 2 * i + 3), LdgLoader2());
+        const int a1 = locate_interval(mesh1, ldg_d(X + 2 * i), LdgLoader2()), b1 = locate_interval(mesh1, ldg_d(X + 2 * i + 2), LdgLoader2());
+        const int a2 = locate_interval(mesh2, ldg_d(X + 2 * i + 1), LdgLoader2()), b2 = locate_interval(mesh2, ldg_d(X + 2 * i + 3), LdgLoader2());
         const int d1 = a1 > b1 ? a1 - b1 : b1 - a1, d2 = a2 > b2 ? a2 - b2 : b2 - a2;
         // (a raster row end — x1 moves on by at most one interval, x2 jumps back — is not a sign of disorder)
         jumps += (d1 > 1 || (d1 == 0 && d2 > 1)) ? 1 : 0;
@@ -1728,8 +1772,8 @@ static int launch_accum_2d_units(const PartWork& w, int64_t n, const double* k1,
     return kOk;
 }
 
-template <int K, int P0, int P1, bool WITH_Y>
-static int launch_accum_part(const double* X, const double* y, int64_t n, const double* k1, int nk1, const double* k2,
+template <int K, int P0, int P1, bool WITH_Y, class TX, class TY>
+static int launch_accum_part(const TX* X, const TY* y, int64_t n, const double* k1, int nk1, const double* k2,
                              int nk2, double* cellmom, double* scal, const int* select, cudaStream_t st) {
     const int64_t want = (n + 511) / 512;          // at least ~2 points per thread; at most one CTA per SM
     const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>(want, sm_count2()));
@@ -1738,46 +1782,40 @@ static int launch_accum_part(const double* X, const double* y, int64_t n, const 
     return kOk;
 }
 
-template <int K>
-static int launch_accum_2d(const double* X, const double* y, int64_t n, const double* k1, int nk1, const double* k2,
-                           int nk2, double* cellmom, double* scal, const int* select, cudaStream_t st);
-
-#define ASVGP_ACC2D(K_, ...)                                                                                          \
-    template <>                                                                                                       \
-    int launch_accum_2d<K_>(const double* X, const double* y, int64_t n, const double* k1, int nk1, const double* k2, \
-                            int nk2, double* cellmom, double* scal, const int* select, cudaStream_t st) {             \
-        int rc = kOk;                                                                                                 \
-        __VA_ARGS__                                                                                                   \
-        return rc;                                                                                                    \
-    }
-#define PART(K_, P0_, P1_, Y_) \
-    if (rc == kOk) rc = launch_accum_part<K_, P0_, P1_, Y_>(X, y, n, k1, nk1, k2, nk2, cellmom, scal, select, st);
+#define PART(P0_, P1_, Y_) \
+    if (rc == kOk) rc = launch_accum_part<K, P0_, P1_, Y_>(X, y, n, k1, nk1, k2, nk2, cellmom, scal, select, st);
 // moment index ranges per launch: <= ~70 register-resident sums per thread
-ASVGP_ACC2D(1, PART(1, 0, 3, true))
-ASVGP_ACC2D(2, PART(2, 0, 5, true))
-ASVGP_ACC2D(3, PART(3, 0, 7, true))
-ASVGP_ACC2D(4, PART(4, 0, 5, true) PART(4, 5, 9, false))
-ASVGP_ACC2D(5, PART(5, 0, 3, true) PART(5, 3, 8, false) PART(5, 8, 11, false))
-ASVGP_ACC2D(6, PART(6, 0, 2, true) PART(6, 2, 6, false) PART(6, 6, 10, false) PART(6, 10, 13, false))
+template <int K, class TX, class TY>
+static int launch_accum_2d(const TX* X, const TY* y, int64_t n, const double* k1, int nk1, const double* k2,
+                           int nk2, double* cellmom, double* scal, const int* select, cudaStream_t st) {
+    int rc = kOk;
+    if constexpr (K == 1) { PART(0, 3, true) }
+    else if constexpr (K == 2) { PART(0, 5, true) }
+    else if constexpr (K == 3) { PART(0, 7, true) }
+    else if constexpr (K == 4) { PART(0, 5, true) PART(5, 9, false) }
+    else if constexpr (K == 5) { PART(0, 3, true) PART(3, 8, false) PART(8, 11, false) }
+    else { PART(0, 2, true) PART(2, 6, false) PART(6, 10, false) PART(10, 13, false) }
+    return rc;
+}
+#undef PART
 
-template <int K>
-static int launch_cols(const double* X, const double* y, int64_t n, const double* k1, int nk1, const double* k2, int nk2,
+template <int K, class TX, class TY>
+static int launch_cols(const TX* X, const TY* y, int64_t n, const double* k1, int nk1, const double* k2, int nk2,
                        double* cellmom, double* scal, const ProbeResult* probe, int hint_n2, cudaStream_t st) {
-    const size_t smem_cols = sizeof(double) * 3 * kColsWarps * 32 * (3 * (size_t)K + 2)     // sums, factors, per-row table
-                             + (size_t)kColsWarps * ColsRing<K>::kRows * 32 * 24;            // the ring
-    ASVGP_CUDA_OK(cudaFuncSetAttribute(accum_2d_cols_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_cols));
+    constexpr size_t smem_cols = cols_smem<K, TX, TY>();
+    ASVGP_CUDA_OK(cudaFuncSetAttribute(accum_2d_cols_kernel<K, TX, TY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_cols));
     const int tpw = 8;             // row segments per warp (tools/accum_sweep.py: 0.603 ms at 4, 0.581 at 8, 0.587 at 16, 0.651 at 32)
-    accum_2d_cols_kernel<K><<<sm_count2(), kColsWarps * 32, smem_cols, st>>>(X, y, n, k1, nk1, k2, nk2, cellmom, scal, probe, hint_n2, tpw); ASVGP_LAUNCHED();
+    accum_2d_cols_kernel<K, TX, TY><<<sm_count2(), kColsWarps * 32, smem_cols, st>>>(X, y, n, k1, nk1, k2, nk2, cellmom, scal, probe, hint_n2, tpw); ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     return kOk;
 }
 
-template <int K>
-static int launch_raster(const double* X, const double* y, int64_t n, const double* k1, int nk1, const double* k2, int nk2,
+template <int K, class TX, class TY>
+static int launch_raster(const TX* X, const TY* y, int64_t n, const double* k1, int nk1, const double* k2, int nk2,
                          double* cellmom, double* scal, const ProbeResult* probe, int blocks, size_t smem,
                          cudaStream_t st) {
-    ASVGP_CUDA_OK(cudaFuncSetAttribute(accum_2d_raster_kernel<K, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ASVGP_CUDA_OK(cudaFuncSetAttribute(accum_2d_raster_kernel<K, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ASVGP_CUDA_OK(cudaFuncSetAttribute(accum_2d_raster_kernel<K, true, TX, TY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ASVGP_CUDA_OK(cudaFuncSetAttribute(accum_2d_raster_kernel<K, false, TX, TY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     accum_2d_raster_kernel<K, true><<<blocks, kRasterWarps * 32, smem, st>>>(X, y, n, k1, nk1, k2, nk2, cellmom, scal, probe); ASVGP_LAUNCHED();
     accum_2d_raster_kernel<K, false><<<blocks, kRasterWarps * 32, smem, st>>>(X, y, n, k1, nk1, k2, nk2, cellmom, scal, probe); ASVGP_LAUNCHED();
     return launch_cols<K>(X, y, n, k1, nk1, k2, nk2, cellmom, scal, probe, 0, st);
@@ -1806,14 +1844,9 @@ extern "C" int64_t asvgp_accum_2d_moment_doubles(int n_knots1, int n_knots2, int
     return per * (n_knots1 - 1) * (n_knots2 - 1) + 1;          // + 1: path-selection slot of asvgp_accum_2d
 }
 
-extern "C" int asvgp_accum_2d(const double* X, const double* y, int64_t n, const double* mesh1, int n_knots1,
-                              const double* mesh2, int n_knots2, int order, double* cellmom, double* scal,
-                              void* stream) {
-    ASVGP_REQUIRE(n >= 0 && n_knots1 >= 2 && n_knots2 >= 2, "accum_2d: n=%lld knots=%d,%d", (long long)n, n_knots1, n_knots2);
-    ASVGP_REQUIRE((reinterpret_cast<uintptr_t>(X) & 15u) == 0 && (reinterpret_cast<uintptr_t>(y) & 15u) == 0,
-                  "accum_2d: X and y must be 16-byte aligned");
-    if (n == 0) return kOk;
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
+template <class TX, class TY>
+static int accum_2d_impl(const TX* X, const TY* y, int64_t n, const double* mesh1, int n_knots1, const double* mesh2,
+                         int n_knots2, int order, double* cellmom, double* scal, cudaStream_t st) {
     // Path selection without a host round trip: a one-CTA probe classifies the input (raster / x1-runs / general) into
     // the trailing slot of the moment table (asvgp_accum_2d_moment_doubles reserves it); every candidate kernel is
     // launched and those that are not selected return at once.
@@ -1835,9 +1868,33 @@ extern "C" int asvgp_accum_2d(const double* X, const double* y, int64_t n, const
     return kOk;
 }
 
-extern "C" int asvgp_accum_2d_raster(const double* X, const double* y, int64_t n, int64_t row_len, const double* mesh1,
-                                     int n_knots1, const double* mesh2, int n_knots2, int order, double* cellmom,
-                                     double* scal, void* stream) {
+extern "C" int asvgp_accum_2d_typed(const void* X, int x_type, const void* y, int y_type, int64_t n, const double* mesh1,
+                                    int n_knots1, const double* mesh2, int n_knots2, int order, double* cellmom, double* scal,
+                                    void* stream) {
+    ASVGP_REQUIRE_TYPES("accum_2d", x_type, y_type);
+    ASVGP_REQUIRE(n >= 0 && n_knots1 >= 2 && n_knots2 >= 2, "accum_2d: n=%lld knots=%d,%d", (long long)n, n_knots1, n_knots2);
+    ASVGP_REQUIRE((reinterpret_cast<uintptr_t>(X) & 15u) == 0 && (reinterpret_cast<uintptr_t>(y) & 15u) == 0,
+                  "accum_2d: X and y must be 16-byte aligned");
+    if (n == 0) return kOk;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    return with_elem_types(x_type, y_type, [&](auto tx, auto ty) -> int {
+        using TX = typename decltype(tx)::type;
+        using TY = typename decltype(ty)::type;
+        return accum_2d_impl(static_cast<const TX*>(X), static_cast<const TY*>(y), n, mesh1, n_knots1, mesh2, n_knots2, order,
+                             cellmom, scal, st);
+    });
+}
+
+extern "C" int asvgp_accum_2d(const double* X, const double* y, int64_t n, const double* mesh1, int n_knots1,
+                              const double* mesh2, int n_knots2, int order, double* cellmom, double* scal,
+                              void* stream) {
+    return asvgp_accum_2d_typed(X, ASVGP_F64, y, ASVGP_F64, n, mesh1, n_knots1, mesh2, n_knots2, order, cellmom, scal, stream);
+}
+
+extern "C" int asvgp_accum_2d_raster_typed(const void* X, int x_type, const void* y, int y_type, int64_t n, int64_t row_len,
+                                           const double* mesh1, int n_knots1, const double* mesh2, int n_knots2, int order,
+                                           double* cellmom, double* scal, void* stream) {
+    ASVGP_REQUIRE_TYPES("accum_2d_raster", x_type, y_type);
     ASVGP_REQUIRE(n >= 0 && n_knots1 >= 2 && n_knots2 >= 2, "accum_2d_raster: n=%lld knots=%d,%d", (long long)n, n_knots1, n_knots2);
     ASVGP_REQUIRE(row_len > 0 && row_len <= 0x7fffffff && n % row_len == 0, "accum_2d_raster: n=%lld is not a whole number of rows of %lld points",
                   (long long)n, (long long)row_len);
@@ -1845,28 +1902,50 @@ extern "C" int asvgp_accum_2d_raster(const double* X, const double* y, int64_t n
                   "accum_2d_raster: X and y must be 16-byte aligned");
     if (n == 0) return kOk;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    ASVGP_DISPATCH_ORDER(order, { if (int rc = launch_cols<K>(X, y, n, mesh1, n_knots1, mesh2, n_knots2, cellmom, scal, nullptr, (int)row_len, st)) return rc; });
-    return kOk;
+    return with_elem_types(x_type, y_type, [&](auto tx, auto ty) -> int {
+        using TX = typename decltype(tx)::type;
+        using TY = typename decltype(ty)::type;
+        const TX* Xt = static_cast<const TX*>(X);
+        const TY* yt = static_cast<const TY*>(y);
+        ASVGP_DISPATCH_ORDER(order, { if (int rc = launch_cols<K>(Xt, yt, n, mesh1, n_knots1, mesh2, n_knots2, cellmom, scal, nullptr, (int)row_len, st)) return rc; });
+        return kOk;
+    });
+}
+
+extern "C" int asvgp_accum_2d_raster(const double* X, const double* y, int64_t n, int64_t row_len, const double* mesh1,
+                                     int n_knots1, const double* mesh2, int n_knots2, int order, double* cellmom,
+                                     double* scal, void* stream) {
+    return asvgp_accum_2d_raster_typed(X, ASVGP_F64, y, ASVGP_F64, n, row_len, mesh1, n_knots1, mesh2, n_knots2, order, cellmom,
+                                       scal, stream);
 }
 
 extern "C" int64_t asvgp_accum_2d_binned_work_bytes(int64_t n) { return PartWork::bytes(n < 0 ? 0 : n, 3); }
 
-extern "C" int asvgp_order_probe_2d(const double* X, int64_t n, const double* mesh1, int n_knots1, const double* mesh2,
-                                    int n_knots2, double* out, void* stream) {
+extern "C" int asvgp_order_probe_2d_typed(const void* X, int x_type, int64_t n, const double* mesh1, int n_knots1,
+                                          const double* mesh2, int n_knots2, double* out, void* stream) {
+    ASVGP_REQUIRE(valid_elem_type(x_type), "order_probe_2d: element type %d (0 = float64, 1 = float32)", x_type);
     ASVGP_REQUIRE(n >= 0 && n_knots1 >= 2 && n_knots2 >= 2 && out != nullptr, "order_probe_2d: n=%lld knots=%d,%d",
                   (long long)n, n_knots1, n_knots2);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     ASVGP_CUDA_OK(cudaMemsetAsync(out, 0, sizeof(double), st));
     if (n < 2) return kOk;
     const int samples = (int)std::min<int64_t>(n - 1, 4096);
-    order_probe_2d_kernel<<<1, 256, 0, st>>>(X, n, mesh1, n_knots1, mesh2, n_knots2, samples, out); ASVGP_LAUNCHED();
+    if (x_type == ASVGP_F32) order_probe_2d_kernel<<<1, 256, 0, st>>>(static_cast<const float*>(X), n, mesh1, n_knots1, mesh2, n_knots2, samples, out);
+    else order_probe_2d_kernel<<<1, 256, 0, st>>>(static_cast<const double*>(X), n, mesh1, n_knots1, mesh2, n_knots2, samples, out);
+    ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     return kOk;
 }
 
-extern "C" int asvgp_accum_2d_binned(const double* X, const double* y, int64_t n, const double* mesh1, int n_knots1,
-                                     const double* mesh2, int n_knots2, int order, double* cellmom, double* scal,
-                                     void* work, int64_t work_bytes, void* stream) {
+extern "C" int asvgp_order_probe_2d(const double* X, int64_t n, const double* mesh1, int n_knots1, const double* mesh2,
+                                    int n_knots2, double* out, void* stream) {
+    return asvgp_order_probe_2d_typed(X, ASVGP_F64, n, mesh1, n_knots1, mesh2, n_knots2, out, stream);
+}
+
+extern "C" int asvgp_accum_2d_binned_typed(const void* X, int x_type, const void* y, int y_type, int64_t n, const double* mesh1,
+                                           int n_knots1, const double* mesh2, int n_knots2, int order, double* cellmom,
+                                           double* scal, void* work, int64_t work_bytes, void* stream) {
+    ASVGP_REQUIRE_TYPES("accum_2d_binned", x_type, y_type);
     ASVGP_REQUIRE(n >= 0 && n_knots1 >= 2 && n_knots2 >= 2, "accum_2d_binned: n=%lld knots=%d,%d", (long long)n, n_knots1, n_knots2);
     ASVGP_REQUIRE(order >= 1 && order <= kMaxOrder, "accum_2d_binned: spline order %d not in 1..6", order);
     ASVGP_REQUIRE((reinterpret_cast<uintptr_t>(X) & 15u) == 0, "accum_2d_binned: X must be 16-byte aligned");
@@ -1876,20 +1955,34 @@ extern "C" int asvgp_accum_2d_binned(const double* X, const double* y, int64_t n
     ASVGP_DISPATCH_ORDER(order, (smem_units = accum_2d_units_smem<K>(ipb + 2 * kUnitMargin2, nc2, n_knots2)));
     // too many cells per bucket for the shared-memory sort: the streaming kernels handle any order
     if ((int64_t)(ipb + 2 * kUnitMargin2) * nc2 > kUnitMaxBins || smem_units > 227 * 1024)
-        return asvgp_accum_2d(X, y, n, mesh1, n_knots1, mesh2, n_knots2, order, cellmom, scal, stream);
+        return asvgp_accum_2d_typed(X, x_type, y, y_type, n, mesh1, n_knots1, mesh2, n_knots2, order, cellmom, scal, stream);
     ASVGP_REQUIRE(work != nullptr && work_bytes >= PartWork::bytes(n, 3), "accum_2d_binned: work_bytes=%lld < %lld",
                   (long long)work_bytes, (long long)PartWork::bytes(n, 3));
     if (n == 0) return kOk;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const PartWork w = PartWork::carve(work);
     ASVGP_CUDA_OK(cudaMemsetAsync(w.count, 0, kPartBuckets * sizeof(u64), st));
-    Points2D src;
-    src.X = X; src.y = y; src.knots1 = mesh1; src.n_knots1 = n_knots1; src.ipb = ipb;
     const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>((n + kPartTile - 1) / kPartTile, (int64_t)sm_count2() * 2));
-    ASVGP_CUDA_OK((launch_partition<Points2D, 3>(src, n, w, kUnitPoints2, blocks, st)));
+    // the partition reads the points in their own types and writes float64 records: the units kernel is type-free
+    const int prc = with_elem_types(x_type, y_type, [&](auto tx, auto ty) -> int {
+        using TX = typename decltype(tx)::type;
+        using TY = typename decltype(ty)::type;
+        Points2D<TX, TY> src;
+        src.X = static_cast<const TX*>(X); src.y = static_cast<const TY*>(y); src.knots1 = mesh1; src.n_knots1 = n_knots1; src.ipb = ipb;
+        ASVGP_CUDA_OK((launch_partition<Points2D<TX, TY>, 3>(src, n, w, kUnitPoints2, blocks, st)));
+        return kOk;
+    });
+    if (prc != kOk) return prc;
     ASVGP_DISPATCH_ORDER(order, { if (int rc = launch_accum_2d_units<K>(w, n, mesh1, n_knots1, mesh2, n_knots2, ipb, cellmom, scal, st)) return rc; });
     ASVGP_CUDA_OK(cudaGetLastError());
     return kOk;
+}
+
+extern "C" int asvgp_accum_2d_binned(const double* X, const double* y, int64_t n, const double* mesh1, int n_knots1,
+                                     const double* mesh2, int n_knots2, int order, double* cellmom, double* scal,
+                                     void* work, int64_t work_bytes, void* stream) {
+    return asvgp_accum_2d_binned_typed(X, ASVGP_F64, y, ASVGP_F64, n, mesh1, n_knots1, mesh2, n_knots2, order, cellmom, scal, work,
+                                       work_bytes, stream);
 }
 
 extern "C" int asvgp_expand_moments_2d(const double* cellmom, const double* Cprod, const double* Dy, int n_knots1,

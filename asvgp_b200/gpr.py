@@ -68,7 +68,11 @@ def _to_numpy(a):
 
 
 class GPR_1d(_ModelBase):
-    """Collapsed-bound sparse GP regression in 1-D with B-spline inducing features (reference gpr.py:18-136)."""
+    """Collapsed-bound sparse GP regression in 1-D with B-spline inducing features (reference gpr.py:18-136).
+
+    data = (X[n, 1], y[n] or y[n, D]) as CUDA tensors or host arrays; X and y may each be float32 or float64 and are read
+    as they are (the accumulate converts every value to float64 in registers, so the model equals the one built from the
+    float64-converted data up to summation order).  Everything after the O(N) pass is float64."""
 
     def __init__(self, data, kernel, basis, distributed="auto", check_inputs=True, chunks=0):
         # Check inputs (reference gpr.py:22-26)
@@ -262,7 +266,9 @@ class GPR_kron(_ModelBase):
 
     def __init__(self, data, kernels, bases, distributed="auto", check_inputs=True, method=None, raster_shape=None):
         """raster_shape=(n1, n2): the caller's statement that X is np.meshgrid(x1, x2, indexing="ij") flattened (x1 slow),
-        the eNATL60-shaped input — skips the on-device input classification (a wrong statement is slow, never wrong)."""
+        the eNATL60-shaped input — skips the on-device input classification (a wrong statement is slow, never wrong).
+        X[n, 2] and y may each be float32 or float64 (CUDA tensors or host arrays) and are read as they are; the model
+        equals the one built from the float64-converted data up to summation order."""
         X, y = data
         self.X, self.y = X, y
         self.n = X.shape[0]

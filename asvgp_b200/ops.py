@@ -9,6 +9,9 @@ import torch
 from . import _lib
 
 F64 = torch.float64
+F32 = torch.float32
+# element-type codes of the typed entry points (ASVGP_F64 / ASVGP_F32 in include/asvgp_b200.h)
+ELEM_TYPES = {F64: 0, F32: 1}
 
 
 _HAVE_CUDA = None
@@ -28,19 +31,42 @@ def device():
     return d
 
 
+def _as_tensor(a):
+    """numpy / torch / DLPack object -> torch tensor (no copy where the source allows, dtype and device unchanged)."""
+    if isinstance(a, torch.Tensor):
+        return a
+    if isinstance(a, np.ndarray):
+        return torch.from_numpy(np.ascontiguousarray(a))
+    if hasattr(a, "__dlpack__"):
+        return torch.from_dlpack(a)
+    return torch.as_tensor(np.asarray(a))
+
+
 def to_device(a, dtype=F64):
     """numpy / torch / DLPack object -> contiguous CUDA tensor of `dtype` on the current device."""
-    if isinstance(a, torch.Tensor):
-        if a.is_cuda and a.dtype == dtype and a.is_contiguous() and a.device.index == torch.cuda.current_device():
-            return a                            # the hot path's inputs are already where they belong
-        t = a
-    elif isinstance(a, np.ndarray):
-        t = torch.from_numpy(np.ascontiguousarray(a))
-    elif hasattr(a, "__dlpack__"):
-        t = torch.from_dlpack(a)
-    else:
-        t = torch.as_tensor(np.asarray(a))
-    return t.to(device=device(), dtype=dtype).contiguous()
+    if isinstance(a, torch.Tensor) and a.is_cuda and a.dtype == dtype and a.is_contiguous() and \
+            a.device.index == torch.cuda.current_device():
+        return a                                # the hot path's inputs are already where they belong
+    return _as_tensor(a).to(device=device(), dtype=dtype).contiguous()
+
+
+def point_dtype(dtype):
+    """The dtype training points are read in: float32 and float64 as they are, anything else converted to float64."""
+    return dtype if dtype in ELEM_TYPES else F64
+
+
+def points_to_device(a):
+    """Training points (x, X or y) -> (contiguous CUDA tensor, element-type code).  float32 / float64 data keep their
+    dtype, so the accumulate kernels read it without a widened copy (they convert each value in registers, exactly)."""
+    t = _as_tensor(a)
+    t = to_device(t, dtype=point_dtype(t.dtype))
+    return t, ELEM_TYPES[t.dtype]
+
+
+def points_to_host(a):
+    """Host-resident training points -> CPU tensor of their point dtype (no copy for float32 / float64 data)."""
+    t = a if isinstance(a, torch.Tensor) else torch.as_tensor(np.asarray(a))
+    return t.to(dtype=point_dtype(t.dtype))
 
 
 def _p(t):
@@ -84,10 +110,11 @@ BINNED_JUMP_FRACTION = 0.05
 
 def order_probe_1d(x, basis):
     """Fraction of sampled neighbour pairs of x that lie more than one knot interval apart (one small D2H read)."""
-    x = to_device(x).reshape(-1)
+    x, xt = points_to_device(x)
+    x = x.reshape(-1)
     mesh = device_mesh(basis)
     out = torch.empty(1, dtype=F64, device=x.device)
-    _lib.call("asvgp_order_probe_1d", _p(x), x.numel(), _p(mesh), mesh.numel(), _p(out), _stream())
+    _lib.call("asvgp_order_probe_1d_typed", _p(x), xt, x.numel(), _p(mesh), mesh.numel(), _p(out), _stream())
     return float(out.item())
 
 
@@ -96,9 +123,11 @@ def accum_1d(x, y, basis, acc=None, binned=False):
     packed accumulator [G_band | b | sum(y^2) | count] (allocated zeroed if None).  Reference gpr.py:39-44.
     binned: False = streaming kernel (any order is exact; fast when consecutive points share knot intervals),
     True = bucket-partition first (inputs in no particular order), "auto" = sample the order on the device and choose
-    (one host synchronisation)."""
-    x = to_device(x).reshape(-1)
-    y = to_device(y).reshape(-1)
+    (one host synchronisation).  x and y may each be float32 or float64 and are read as they are (other dtypes are
+    converted to float64); the sums are float64 and equal those of the float64-converted points up to summation order."""
+    x, xt = points_to_device(x)
+    y, yt = points_to_device(y)
+    x, y = x.reshape(-1), y.reshape(-1)
     if x.numel() != y.numel():
         raise ValueError("x and y must have the same number of points")
     mesh = device_mesh(basis)
@@ -109,10 +138,11 @@ def accum_1d(x, y, basis, acc=None, binned=False):
     if binned:
         nbytes = _lib.load().asvgp_accum_1d_binned_work_bytes(x.numel())
         work = torch.empty(nbytes, dtype=torch.uint8, device=x.device)
-        _lib.call("asvgp_accum_1d_binned", _p(x), _p(y), x.numel(), _p(mesh), mesh.numel(), basis.order, _p(acc),
-                  _p(work), nbytes, _stream())
+        _lib.call("asvgp_accum_1d_binned_typed", _p(x), xt, _p(y), yt, x.numel(), _p(mesh), mesh.numel(), basis.order,
+                  _p(acc), _p(work), nbytes, _stream())
         return acc
-    _lib.call("asvgp_accum_1d", _p(x), _p(y), x.numel(), _p(mesh), mesh.numel(), basis.order, _p(acc), _stream())
+    _lib.call("asvgp_accum_1d_typed", _p(x), xt, _p(y), yt, x.numel(), _p(mesh), mesh.numel(), basis.order, _p(acc),
+              _stream())
     return acc
 
 
@@ -281,13 +311,14 @@ def posterior_1d(Kuu, acc, basis, sigma2, chunks=0):
 _STAGING = {}
 
 
-def _staging(dev, chunk):
-    key = (dev, chunk)
+def _staging(dev, key, nbytes):
+    """Double-buffered pinned and device staging areas of `nbytes` bytes each, cached per (device, key)."""
+    key = (dev,) + key
     st = _STAGING.get(key)
     if st is None:
         st = dict(
-            host=[torch.empty((2, chunk), dtype=F64).pin_memory() for _ in range(2)],
-            dev=[torch.empty((2, chunk), dtype=F64, device=dev) for _ in range(2)],
+            host=[torch.empty(nbytes, dtype=torch.uint8).pin_memory() for _ in range(2)],
+            dev=[torch.empty(nbytes, dtype=torch.uint8, device=dev) for _ in range(2)],
             copy_stream=torch.cuda.Stream(device=dev),
             filled=[torch.cuda.Event() for _ in range(2)],
             drained=[torch.cuda.Event() for _ in range(2)],
@@ -297,13 +328,29 @@ def _staging(dev, chunk):
     return st
 
 
+def _split_staging(buf, parts):
+    """Typed views of consecutive regions of a uint8 staging buffer: parts = [(dtype, count), ...], every region starting
+    at a 32-byte boundary (the kernels' vector loads)."""
+    out, off = [], 0
+    for dtype, count in parts:
+        nb = count * dtype.itemsize
+        out.append(buf[off: off + nb].view(dtype))
+        off += -(-nb // 32) * 32
+    return out
+
+
+def _staging_bytes(parts):
+    return sum(-(-count * dtype.itemsize // 32) * 32 for dtype, count in parts)
+
+
 def accum_1d_host(x, y, basis, acc=None, chunk=1 << 23):
     """accum_1d for HOST arrays (numpy or CPU tensors): the points are streamed to the GPU in `chunk`-point pieces,
     host->pinned staging (unless already pinned), async H2D on a copy stream, double-buffered against the accumulate
-    kernel — the device never holds more than two chunks."""
+    kernel — the device never holds more than two chunks.  float32 / float64 arrays are staged and sent in their own dtype
+    (float32 halves the PCIe bytes); other dtypes are converted to float64."""
     dev = device()
-    xt = torch.as_tensor(np.asarray(x) if not isinstance(x, torch.Tensor) else x, dtype=F64).reshape(-1)
-    yt = torch.as_tensor(np.asarray(y) if not isinstance(y, torch.Tensor) else y, dtype=F64).reshape(-1)
+    xt = points_to_host(x).reshape(-1)
+    yt = points_to_host(y).reshape(-1)
     n = xt.numel()
     if yt.numel() != n:
         raise ValueError("x and y must have the same number of points")
@@ -313,7 +360,9 @@ def accum_1d_host(x, y, basis, acc=None, chunk=1 << 23):
     if n == 0:
         return acc
     chunk = min(chunk, n + (n & 1))
-    st = _staging(dev, chunk)
+    parts = [(xt.dtype, chunk), (yt.dtype, chunk)]
+    st = _staging(dev, ("1d", chunk, xt.dtype, yt.dtype), _staging_bytes(parts))
+    xc, yc = ELEM_TYPES[xt.dtype], ELEM_TYPES[yt.dtype]
     pinned = xt.is_pinned() and yt.is_pinned()
     main = torch.cuda.current_stream()
     cs = st["copy_stream"]
@@ -321,24 +370,25 @@ def accum_1d_host(x, y, basis, acc=None, chunk=1 << 23):
     for c in range(n_chunks):
         lo, hi = c * chunk, min((c + 1) * chunk, n)
         s = c & 1
-        dbuf = st["dev"][s]
-        # the kernel that last read dbuf (two chunks ago, or the previous CALL: the staging buffers are cached and
+        dx, dy = _split_staging(st["dev"][s], parts)
+        # the kernel that last read this buffer (two chunks ago, or the previous CALL: the staging buffers are cached and
         # shared between calls) has finished; waiting on a never-recorded event is a no-op
         cs.wait_event(st["drained"][s])
         with torch.cuda.stream(cs):
             if pinned:
-                dbuf[0, : hi - lo].copy_(xt[lo:hi], non_blocking=True)
-                dbuf[1, : hi - lo].copy_(yt[lo:hi], non_blocking=True)
+                dx[: hi - lo].copy_(xt[lo:hi], non_blocking=True)
+                dy[: hi - lo].copy_(yt[lo:hi], non_blocking=True)
             else:
-                hbuf = st["host"][s]
+                hx, hy = _split_staging(st["host"][s], parts)
                 st["staged"][s].synchronize()          # previous H2D out of this pinned buffer (also a previous call's) is done
-                hbuf[0, : hi - lo].copy_(xt[lo:hi])
-                hbuf[1, : hi - lo].copy_(yt[lo:hi])
-                dbuf[:, : hi - lo].copy_(hbuf[:, : hi - lo], non_blocking=True)
+                hx[: hi - lo].copy_(xt[lo:hi])
+                hy[: hi - lo].copy_(yt[lo:hi])
+                dx[: hi - lo].copy_(hx[: hi - lo], non_blocking=True)
+                dy[: hi - lo].copy_(hy[: hi - lo], non_blocking=True)
                 st["staged"][s].record(cs)
             st["filled"][s].record(cs)
         main.wait_event(st["filled"][s])
-        _lib.call("asvgp_accum_1d", _p(dbuf[0]), _p(dbuf[1]), hi - lo, _p(mesh), mesh.numel(), basis.order, _p(acc),
+        _lib.call("asvgp_accum_1d_typed", _p(dx), xc, _p(dy), yc, hi - lo, _p(mesh), mesh.numel(), basis.order, _p(acc),
                   ctypes.c_void_p(main.cuda_stream))
         st["drained"][s].record(main)
     return acc
@@ -381,10 +431,11 @@ def moment_table_2d(bases):
 
 def order_probe_2d(X, bases):
     """Fraction of sampled neighbour pairs of X[n,2] that lie more than one cell apart (one small D2H read)."""
-    X = to_device(X)
+    X, xt = points_to_device(X)
     mesh1, mesh2 = device_mesh(bases[0]), device_mesh(bases[1])
     out = torch.empty(1, dtype=F64, device=X.device)
-    _lib.call("asvgp_order_probe_2d", _p(X), X.shape[0], _p(mesh1), mesh1.numel(), _p(mesh2), mesh2.numel(), _p(out), _stream())
+    _lib.call("asvgp_order_probe_2d_typed", _p(X), xt, X.shape[0], _p(mesh1), mesh1.numel(), _p(mesh2), mesh2.numel(), _p(out),
+              _stream())
     return float(out.item())
 
 
@@ -392,30 +443,32 @@ def accum_2d(X, y, bases, cellmom, scal, binned=False, raster_row_len=None):
     """Adds the per-cell moments of the points (X[n,2], y[n]) into `cellmom` and (sum y^2, n) into `scal`
     (reference gpr.py:268-274 without materialising the Khatri-Rao Kuf).  binned: as accum_1d.
     raster_row_len: the caller's statement that X is a flattened raster (meshgrid, x1 slow) with rows of that many points
-    — skips the on-device classification (asvgp_accum_2d_raster); a wrong statement is slow, never wrong."""
+    — skips the on-device classification (asvgp_accum_2d_raster); a wrong statement is slow, never wrong.
+    X and y may each be float32 or float64 and are read as they are (other dtypes are converted to float64)."""
     k, _, _ = _check_bases_2d(bases)
-    X = to_device(X)
-    y = to_device(y).reshape(-1)
+    X, xt = points_to_device(X)
+    y, yt = points_to_device(y)
+    y = y.reshape(-1)
     if X.dim() != 2 or X.shape[1] != 2 or X.shape[0] != y.numel():
         raise ValueError("X must be [n, 2] and y [n]")
-    if X.data_ptr() % 16:            # the kernel reads one point (16 B) / two targets per load
+    if X.data_ptr() % 16:            # the kernel reads one point / two targets per load (a clone keeps the dtype)
         X = X.clone()
     if y.data_ptr() % 16:
         y = y.clone()
     mesh1, mesh2 = device_mesh(bases[0]), device_mesh(bases[1])
     if raster_row_len:
-        _lib.call("asvgp_accum_2d_raster", _p(X), _p(y), X.shape[0], int(raster_row_len), _p(mesh1), mesh1.numel(), _p(mesh2),
-                  mesh2.numel(), k, _p(cellmom), _p(scal), _stream())
+        _lib.call("asvgp_accum_2d_raster_typed", _p(X), xt, _p(y), yt, X.shape[0], int(raster_row_len), _p(mesh1),
+                  mesh1.numel(), _p(mesh2), mesh2.numel(), k, _p(cellmom), _p(scal), _stream())
         return cellmom, scal
     if binned == "auto":
         binned = X.shape[0] >= BINNED_MIN_POINTS and order_probe_2d(X, bases) > BINNED_JUMP_FRACTION
     if binned:
         nbytes = _lib.load().asvgp_accum_2d_binned_work_bytes(X.shape[0])
         work = torch.empty(nbytes, dtype=torch.uint8, device=X.device)
-        _lib.call("asvgp_accum_2d_binned", _p(X), _p(y), X.shape[0], _p(mesh1), mesh1.numel(), _p(mesh2), mesh2.numel(), k,
-                  _p(cellmom), _p(scal), _p(work), nbytes, _stream())
+        _lib.call("asvgp_accum_2d_binned_typed", _p(X), xt, _p(y), yt, X.shape[0], _p(mesh1), mesh1.numel(), _p(mesh2),
+                  mesh2.numel(), k, _p(cellmom), _p(scal), _p(work), nbytes, _stream())
         return cellmom, scal
-    _lib.call("asvgp_accum_2d", _p(X), _p(y), X.shape[0], _p(mesh1), mesh1.numel(), _p(mesh2), mesh2.numel(), k,
+    _lib.call("asvgp_accum_2d_typed", _p(X), xt, _p(y), yt, X.shape[0], _p(mesh1), mesh1.numel(), _p(mesh2), mesh2.numel(), k,
               _p(cellmom), _p(scal), _stream())
     return cellmom, scal
 
@@ -447,10 +500,11 @@ def expand_moments_2d(cellmom, bases, acc):
 
 def accum_2d_host(X, y, bases, cellmom, scal, chunk=1 << 22, raster_row_len=None):
     """accum_2d for HOST arrays: streamed through pinned staging buffers, double-buffered against the kernel.
-    raster_row_len: as accum_2d (the chunks are then whole rows)."""
+    raster_row_len: as accum_2d (the chunks are then whole rows).  float32 / float64 arrays are staged and sent in their own
+    dtype; other dtypes are converted to float64."""
     dev = device()
-    Xt = torch.as_tensor(np.asarray(X) if not isinstance(X, torch.Tensor) else X, dtype=F64)
-    yt = torch.as_tensor(np.asarray(y) if not isinstance(y, torch.Tensor) else y, dtype=F64).reshape(-1)
+    Xt = points_to_host(X)
+    yt = points_to_host(y).reshape(-1)
     n = Xt.shape[0]
     if Xt.dim() != 2 or Xt.shape[1] != 2 or yt.numel() != n:
         raise ValueError("X must be [n, 2] and y [n]")
@@ -466,42 +520,36 @@ def accum_2d_host(X, y, bases, cellmom, scal, chunk=1 << 22, raster_row_len=None
         if chunk & 1:
             chunk *= 2
     chunk = min(chunk, n + (n & 1))
-    key = (dev, "2d", chunk)
-    st = _STAGING.get(key)
-    if st is None:
-        st = dict(host=[torch.empty(3 * chunk, dtype=F64).pin_memory() for _ in range(2)],
-                  dev=[torch.empty(3 * chunk, dtype=F64, device=dev) for _ in range(2)],
-                  copy_stream=torch.cuda.Stream(device=dev),
-                  filled=[torch.cuda.Event() for _ in range(2)], drained=[torch.cuda.Event() for _ in range(2)],
-                  staged=[torch.cuda.Event() for _ in range(2)])
-        _STAGING[key] = st
+    parts = [(Xt.dtype, 2 * chunk), (yt.dtype, chunk)]
+    st = _staging(dev, ("2d", chunk, Xt.dtype, yt.dtype), _staging_bytes(parts))
+    xc, yc = ELEM_TYPES[Xt.dtype], ELEM_TYPES[yt.dtype]
     pinned = Xt.is_pinned() and yt.is_pinned()
     main, cs = torch.cuda.current_stream(), st["copy_stream"]
     for c in range(-(-n // chunk)):
         lo, hi = c * chunk, min((c + 1) * chunk, n)
         cnt, s = hi - lo, c & 1
-        dbuf = st["dev"][s]
-        dX, dy = dbuf[: 2 * cnt].view(cnt, 2), dbuf[2 * chunk: 2 * chunk + cnt]
+        dXf, dyf = _split_staging(st["dev"][s], parts)
+        dX, dy = dXf[: 2 * cnt].view(cnt, 2), dyf[:cnt]
         cs.wait_event(st["drained"][s])                # also covers the previous call (cached, shared staging buffers)
         with torch.cuda.stream(cs):
             if pinned:
                 dX.copy_(Xt[lo:hi], non_blocking=True)
                 dy.copy_(yt[lo:hi], non_blocking=True)
             else:
-                hbuf = st["host"][s]
+                hXf, hyf = _split_staging(st["host"][s], parts)
                 st["staged"][s].synchronize()
-                hbuf[: 2 * cnt].view(cnt, 2).copy_(Xt[lo:hi])
-                hbuf[2 * chunk: 2 * chunk + cnt].copy_(yt[lo:hi])
-                dbuf[: 2 * cnt].copy_(hbuf[: 2 * cnt], non_blocking=True)
-                dy.copy_(hbuf[2 * chunk: 2 * chunk + cnt], non_blocking=True)
+                hXf[: 2 * cnt].view(cnt, 2).copy_(Xt[lo:hi])
+                hyf[:cnt].copy_(yt[lo:hi])
+                dXf[: 2 * cnt].copy_(hXf[: 2 * cnt], non_blocking=True)
+                dy.copy_(hyf[:cnt], non_blocking=True)
                 st["staged"][s].record(cs)
             st["filled"][s].record(cs)
         main.wait_event(st["filled"][s])
         if raster_row_len:
-            _lib.call("asvgp_accum_2d_raster", _p(dX), _p(dy), cnt, int(raster_row_len), _p(mesh1), mesh1.numel(), _p(mesh2),
-                      mesh2.numel(), k, _p(cellmom), _p(scal), ctypes.c_void_p(main.cuda_stream))
+            _lib.call("asvgp_accum_2d_raster_typed", _p(dX), xc, _p(dy), yc, cnt, int(raster_row_len), _p(mesh1), mesh1.numel(),
+                      _p(mesh2), mesh2.numel(), k, _p(cellmom), _p(scal), ctypes.c_void_p(main.cuda_stream))
         else:
-            _lib.call("asvgp_accum_2d", _p(dX), _p(dy), cnt, _p(mesh1), mesh1.numel(), _p(mesh2), mesh2.numel(), k,
+            _lib.call("asvgp_accum_2d_typed", _p(dX), xc, _p(dy), yc, cnt, _p(mesh1), mesh1.numel(), _p(mesh2), mesh2.numel(), k,
                       _p(cellmom), _p(scal), ctypes.c_void_p(main.cuda_stream))
         st["drained"][s].record(main)
     return cellmom, scal

@@ -76,6 +76,23 @@ ASVGP_API int asvgp_accum_1d_binned(const double* x, const double* y, int64_t n,
                                     int order, double* acc, void* work, int64_t work_bytes, void* stream);
 ASVGP_API int asvgp_order_probe_1d(const double* x, int64_t n, const double* mesh, int n_knots, double* out, void* stream);
 
+/* ---- element types of the training points ------------------------------------------------------------------------------
+ * The *_typed twins below read x / X and y as float64 or float32, each independently (x_type, y_type: ASVGP_F64 or
+ * ASVGP_F32).  A float32 value converts to float64 exactly, so the kernels convert every loaded value in registers and the
+ * results equal those for the same points converted to float64 first, up to summation order; the accumulators stay
+ * float64.  float32 halves the bytes the O(N) pass reads and needs no widened copy of the data.  The untyped functions are
+ * these with ASVGP_F64 for both arrays.  An unknown type code returns an error before any CUDA call.  Alignment rules are
+ * those of the untyped functions; binned scratch records stay float64 (the *_work_bytes queries do not depend on the
+ * types). */
+#define ASVGP_F64 0
+#define ASVGP_F32 1
+ASVGP_API int asvgp_accum_1d_typed(const void* x, int x_type, const void* y, int y_type, int64_t n, const double* mesh,
+                                   int n_knots, int order, double* acc, void* stream);
+ASVGP_API int asvgp_accum_1d_binned_typed(const void* x, int x_type, const void* y, int y_type, int64_t n, const double* mesh,
+                                          int n_knots, int order, double* acc, void* work, int64_t work_bytes, void* stream);
+ASVGP_API int asvgp_order_probe_1d_typed(const void* x, int x_type, int64_t n, const double* mesh, int n_knots, double* out,
+                                         void* stream);
+
 /* ---- a10: 1-D posterior mean / variance over test points ----------------------------------------------------------------
  * Replaces GPR_1d.predict_f (gpr.py:91-136): mean[i] = sum_r w_r alpha[idx+r],
  * var[i] = variance + sum_{r,s} w_r w_s S[idx+r, idx+s] with S = band(P^-1) - band(Kuu^-1) (lower band, (order+1) x M). */
@@ -182,6 +199,19 @@ ASVGP_API int asvgp_accum_2d_binned(const double* X, const double* y, int64_t n,
                                     void* work, int64_t work_bytes, void* stream);
 ASVGP_API int asvgp_order_probe_2d(const double* X, int64_t n, const double* mesh1, int n_knots1, const double* mesh2,
                                    int n_knots2, double* out, void* stream);
+
+/* Typed twins of the four entry points above (element types as for asvgp_accum_1d_typed; X [n, 2] has one type). */
+ASVGP_API int asvgp_accum_2d_typed(const void* X, int x_type, const void* y, int y_type, int64_t n, const double* mesh1,
+                                   int n_knots1, const double* mesh2, int n_knots2, int order, double* cellmom, double* scal,
+                                   void* stream);
+ASVGP_API int asvgp_accum_2d_raster_typed(const void* X, int x_type, const void* y, int y_type, int64_t n, int64_t row_len,
+                                          const double* mesh1, int n_knots1, const double* mesh2, int n_knots2, int order,
+                                          double* cellmom, double* scal, void* stream);
+ASVGP_API int asvgp_accum_2d_binned_typed(const void* X, int x_type, const void* y, int y_type, int64_t n, const double* mesh1,
+                                          int n_knots1, const double* mesh2, int n_knots2, int order, double* cellmom,
+                                          double* scal, void* work, int64_t work_bytes, void* stream);
+ASVGP_API int asvgp_order_probe_2d_typed(const void* X, int x_type, int64_t n, const double* mesh1, int n_knots1,
+                                         const double* mesh2, int n_knots2, double* out, void* stream);
 
 /* Expands the moment table into the Gram stencil Gs[(o+1)(2o+1) x M] and the projection b[M] (both must be zeroed by
  * the caller).  Cprod[(o+1)(o+1)(2o+1)], Dy[(o+1)(o+1)]: exact Bernstein-type expansion tables (host-computed). */
