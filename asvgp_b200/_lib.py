@@ -45,6 +45,9 @@ SIGNATURES = {
     "asvgp_expand_moments_2d": [_vp, _vp, _vp, _c_int, _c_int, _c_int, _vp, _vp, _vp],
     "asvgp_kron_factor": [_vp, _vp, _vp, _c_int, _c_int, _c_int, _c_dbl, _vp, _vp, _vp, _vp],
     "asvgp_kron_selinv": [_vp, _c_int, _c_int, _c_int, _vp, _vp, _vp, _vp, _vp],
+    "asvgp_kron_doubles_multi": [_c_int, _c_int, _c_int, _c_int, _vp],
+    "asvgp_kron_factor_multi": [_vp, _vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_dbl, _vp, _vp, _vp, _vp],
+    "asvgp_kron_selinv_multi": [_vp, _c_int, _c_int, _c_int, _c_int, _vp, _vp, _vp, _vp, _vp],
     "asvgp_kronband_factor": [_vp, _vp, _vp, _c_int, _c_int, _c_int, _c_dbl, _vp, _vp, _vp, _vp],
     "asvgp_kronband_selinv": [_vp, _c_int, _c_int, _c_int, _vp, _vp, _vp, _vp, _vp],
     "asvgp_kron_terms": [_vp] * 11 + [_c_int, _c_int, _c_int, _vp, _vp],
@@ -52,6 +55,9 @@ SIGNATURES = {
     "asvgp_allreduce_oneshot": [_vp, _vp, _c_int, _c_int, _c_i64, _c_i64, ctypes.c_uint, _c_int, _vp, _vp, _vp],
     "asvgp_dense_factor": [_vp, _c_int, _vp, _vp, _vp, _vp],
     "asvgp_dense_selinv": [_vp, _c_int, _vp, _vp, _vp, _vp, _vp],
+    "asvgp_dense_doubles_multi": [_c_int, _c_int, _vp],
+    "asvgp_dense_factor_multi": [_vp, _c_int, _c_int, _vp, _vp, _vp, _vp],
+    "asvgp_dense_selinv_multi": [_vp, _c_int, _c_int, _vp, _vp, _vp, _vp, _vp],
     "asvgp_accum_cross": [_vp, _vp, _c_i64, _c_i64, _vp, _c_int, _vp, _c_int, _c_int, _vp, _vp],
     "asvgp_additive_put_band": [_vp, _c_int, _c_int, _c_int, _c_int, _c_dbl, _c_int, _vp, _vp],
     "asvgp_additive_put_cross": [_vp, _c_int, _c_int, _c_int, _c_int, _c_int, _vp, _vp],
@@ -79,6 +85,7 @@ VALUE_FUNCTIONS = {
     "asvgp_dense_sig_doubles": (_c_i64, [_c_int]),
     "asvgp_dense_work_doubles": (_c_i64, [_c_int]),
     "asvgp_kron_plan_info": (_c_i64, [_c_int, _c_int, _c_int, _vp, _vp, _c_i64]),
+    "asvgp_kron_plan_info_multi": (_c_i64, [_c_int, _c_int, _c_int, _c_int, _vp, _vp, _c_i64]),
     "asvgp_kronband_band_doubles": (_c_i64, [_c_int, _c_int, _c_int]),
     "asvgp_kronband_work_doubles": (_c_i64, [_c_int, _c_int, _c_int]),
     "asvgp_kronband_sig_doubles": (_c_i64, [_c_int, _c_int, _c_int]),

@@ -26,6 +26,15 @@
 // 1e-6 fraction of sqrt(P^-1_ii P^-1_jj) (Cauchy-Schwarz), so subtracting it costs no digits.  No separate triangular
 // solves, no separate chains.
 //
+// Several right-hand sides (multi-output targets, the *_multi entry points).  B = [b_1 ... b_D] rides along as D rhs nodes
+// with ids M ... M+D-1, the last D boundary unknowns of every front; the root's boundary is exactly these D ids (one tile).
+// The factorised matrix is A' = [[P, B], [B^T, 0]]: eliminating the grid unknowns leaves the root update block -B^T P^-1 B,
+// whose diagonal is -Q_d, Q_d = b_d^T P^-1 b_d.  Seeding the selected inverse with Sigma'(rhs, rhs) = tau I_D gives
+// Sigma'(s, rhs_d) = -tau x_d, x_d = P^-1 b_d, and Sigma' = P^-1 + tau sum_d x_d x_d^T on the grid, so the stencil of P^-1
+// and the dense A^-1 are Sigma' - tau sum_d x_d x_d^T.  tau = 2^-20 / (1 + sum_d Q_d) (today's tau for D = 1) keeps the
+// correction below 2^-20 sqrt(P^-1_ii P^-1_jj): |x_d,i| <= sqrt(P^-1_ii Q_d) by Cauchy-Schwarz.  One factorisation and one
+// selected inverse serve every column; with D = 1 the plan and every operation are those of the single-rhs functions.
+//
 // Kernels, per tree level (bottom-up for the factorisation, top-down for the selected inverse):
 //   nd_assemble_kernel   (once) entries of P and the right-hand-side row into every front
 //   nd_factor_kernel     persistent tile DAG over all tiles of all fronts of the level: left-looking updates on the fp64
@@ -34,7 +43,7 @@
 //   nd_ypass_kernel      (once) L(R,C) -> Y(R,C)^T = (L(R,C) L(C,C)^-1)^T, Sigma(C,C) seeded with L(C,C)^-T L(C,C)^-1
 //   nd_gather_kernel     Sigma on the boundary of a front from its parent's Sigma
 //   nd_selinv_kernel     persistent tile DAG: blocked Takahashi recursion inside every front of the level
-//   nd_scalars_kernel / nd_x_kernel / nd_stencil_kernel   log|P|, ||y||^2, x, stencil entries of P^-1
+//   nd_scalars_kernel / nd_x_kernel / nd_stencil_kernel   log|P|, ||y_d||^2, x_d, stencil entries of P^-1
 #include <cstdlib>
 #include <map>
 #include <mutex>
@@ -52,8 +61,8 @@ namespace asvgp {
 struct FrontDesc {                 // device-visible
     long long tile_base;           // first tile of this front in the tile pools (in tiles)
     int nT, nsT;                   // block rows in total, separator block columns
-    int ns, nb;                    // separator / boundary unknowns (unpadded; the rhs node is the last boundary unknown)
-    int idx_off;                   // into idx[]: nT * 64 node ids, -1 = padding, M = rhs node
+    int ns, nb;                    // separator / boundary unknowns (unpadded; the n_rhs rhs nodes are the last boundary unknowns)
+    int idx_off;                   // into idx[]: nT * 64 node ids, -1 = padding, M + d = rhs node of column d
     int pmap_off;                  // into pmap[]: (nT - nsT) * 64 positions in the parent's padded list (-1 = none)
     int parent;
     int child[2];
@@ -122,7 +131,7 @@ static int nd_rec(std::vector<NdFrontHost>& F, int r0, int r1, int c0, int c1, i
 }
 
 struct NdPlan {
-    int m1 = 0, m2 = 0, K = 0, M = 0;
+    int m1 = 0, m2 = 0, K = 0, M = 0, R = 1;     // R: right-hand sides (rhs nodes M ... M+R-1)
     int n_fronts = 0, n_levels = 0, root = -1;
     long long n_tiles = 0;         // tiles per pool
     int n_linv = 0, n_cnt = 0;
@@ -130,21 +139,21 @@ struct NdPlan {
     std::vector<int> idx, pmap, cpos;
     std::vector<std::vector<int4>> factor_tasks, selinv_tasks, gather_tasks;    // per level
     std::vector<int4> ypass_tasks, all_tasks;
-    std::vector<long long> doff, xoff, sigoff;
-    long long quad_off = 0, tau_off = 0;           // L-pool offset of the root's update entry (rhs, rhs); sig-pool offset of Sigma'(rhs, rhs)
+    std::vector<long long> doff, xoff, sigoff;     // xoff[d * M + j]: Sigma'(rhs_d, j)
+    std::vector<long long> quad_off;               // [R]: L-pool offsets of the root's update entries (rhs_d, rhs_d)
     // device copies
     FrontDesc* d_fronts = nullptr;
     int *d_idx = nullptr, *d_pmap = nullptr, *d_cpos = nullptr;
     std::vector<int4*> d_factor_tasks, d_selinv_tasks, d_gather_tasks;
     int4 *d_ypass_tasks = nullptr, *d_all_tasks = nullptr;
-    long long *d_doff = nullptr, *d_xoff = nullptr, *d_sigoff = nullptr;
+    long long *d_doff = nullptr, *d_xoff = nullptr, *d_sigoff = nullptr, *d_quad_off = nullptr;
 };
 
 constexpr int kNdScalarBlocks = 64;   // slices of the log-determinant sum
 constexpr int kNdLeaf = 12;        // regions whose sides are both <= this many grid lines are eliminated as one front
 
-static void nd_build(NdPlan& P, int m1, int m2, int K) {
-    P.m1 = m1; P.m2 = m2; P.K = K; P.M = m1 * m2;
+static void nd_build(NdPlan& P, int m1, int m2, int K, int R) {
+    P.m1 = m1; P.m2 = m2; P.K = K; P.M = m1 * m2; P.R = R;
     const int M = P.M, RHS = M;
     std::vector<NdFrontHost> F;
     int leaf = kNdLeaf;
@@ -166,7 +175,7 @@ static void nd_build(NdPlan& P, int m1, int m2, int K) {
                 const int s1 = g / m2, s2 = g % m2;
                 if (s1 >= f.r0 - K && s1 <= f.r1 - 1 + K && s2 >= f.c0 - K && s2 <= f.c1 - 1 + K) f.bnd.push_back(g);
             }
-        f.bnd.push_back(RHS);
+        for (int d = 0; d < R; ++d) f.bnd.push_back(RHS + d);
         P.n_levels = std::max(P.n_levels, f.level + 1);
     }
     P.fronts.resize(P.n_fronts);
@@ -245,17 +254,19 @@ static void nd_build(NdPlan& P, int m1, int m2, int K) {
     auto elem = [&](const FrontDesc& d, int prow, int pcol) {       // element (prow, pcol), prow >= pcol, of the front's lower triangle
         return front_tile(d, prow / NB, pcol / NB) * TILE_P + (long long)(pcol % NB) * LDT + prow % NB;
     };
-    P.doff.resize(M); P.xoff.resize(M);
+    P.doff.resize(M); P.xoff.resize((size_t)R * M);
     for (int j = 0; j < M; ++j) {
         const FrontDesc& d = P.fronts[owner[j]];
         P.doff[j] = elem(d, opos[j], opos[j]);
-        P.xoff[j] = elem(d, d.nsT * NB + d.nb - 1, opos[j]);
+        for (int c = 0; c < R; ++c) P.xoff[(size_t)c * M + j] = elem(d, d.nsT * NB + d.nb - R + c, opos[j]);
     }
     {
         const FrontDesc& r = P.fronts[P.root];
-        const int p = r.nsT * NB + r.nb - 1;
-        P.quad_off = elem(r, p, p);
-        P.tau_off = P.quad_off;
+        P.quad_off.resize(R);
+        for (int c = 0; c < R; ++c) {
+            const int p = r.nsT * NB + r.nb - R + c;
+            P.quad_off[c] = elem(r, p, p);
+        }
     }
     if (dense) return;             // the dense extraction kernel computes its offsets itself (one front)
     const int NS = 2 * K + 1, n_e = (K + 1) * NS;
@@ -294,29 +305,29 @@ static int nd_upload(T** dst, const std::vector<T>& src) {
 }
 
 static std::mutex g_plan_mutex;
-static std::map<std::tuple<int, int, int, int>, NdPlan*> g_plans;     // (device or -1 for host-only, m1, m2, order)
+static std::map<std::tuple<int, int, int, int, int>, NdPlan*> g_plans;     // (device or -1 for host-only, m1, m2, order, n_rhs)
 
 // host-only plan (sizes, diagnostics); no CUDA calls
-static const NdPlan* nd_plan_host(int m1, int m2, int K) {
+static const NdPlan* nd_plan_host(int m1, int m2, int K, int R = 1) {
     std::lock_guard<std::mutex> lock(g_plan_mutex);
-    auto key = std::make_tuple(-1, m1, m2, K);
+    auto key = std::make_tuple(-1, m1, m2, K, R);
     auto it = g_plans.find(key);
     if (it != g_plans.end()) return it->second;
     NdPlan* P = new NdPlan();
-    nd_build(*P, m1, m2, K);
+    nd_build(*P, m1, m2, K, R);
     g_plans[key] = P;
     return P;
 }
 
-static int nd_plan_device(int m1, int m2, int K, const NdPlan** out) {
+static int nd_plan_device(int m1, int m2, int K, int R, const NdPlan** out) {
     int dev = 0;
     ASVGP_CUDA_OK(cudaGetDevice(&dev));
     std::lock_guard<std::mutex> lock(g_plan_mutex);
-    auto key = std::make_tuple(dev, m1, m2, K);
+    auto key = std::make_tuple(dev, m1, m2, K, R);
     auto it = g_plans.find(key);
     if (it != g_plans.end()) { *out = it->second; return kOk; }
     NdPlan* P = new NdPlan();
-    nd_build(*P, m1, m2, K);
+    nd_build(*P, m1, m2, K, R);
     if (int rc = nd_upload(&P->d_fronts, P->fronts)) return rc;
     if (int rc = nd_upload(&P->d_idx, P->idx)) return rc;
     if (int rc = nd_upload(&P->d_pmap, P->pmap)) return rc;
@@ -332,6 +343,7 @@ static int nd_plan_device(int m1, int m2, int K, const NdPlan** out) {
     if (int rc = nd_upload(&P->d_doff, P->doff)) return rc;
     if (int rc = nd_upload(&P->d_xoff, P->xoff)) return rc;
     if (int rc = nd_upload(&P->d_sigoff, P->sigoff)) return rc;
+    if (int rc = nd_upload(&P->d_quad_off, P->quad_off)) return rc;
     g_plans[key] = P;
     *out = P;
     return kOk;
@@ -377,9 +389,13 @@ __device__ __forceinline__ double nd_band_sym(const double* B, int m, int K, int
     return d <= K ? __ldg(B + (long long)d * m + (i < j ? i : j)) : 0.0;
 }
 
-// A'(gi, gj): gi, gj grid unknowns or the rhs node (id M).  Same roundings as the reference's `Kuu + KufKfu / sigma2`.
+// A'(gi, gj): gi, gj grid unknowns or rhs nodes (id M + d: A'(g, rhs_d) = b[d M + g], A'(rhs_d, rhs_e) = 0).  Same roundings as
+// the reference's `Kuu + KufKfu / sigma2`.
 __device__ __forceinline__ double nd_entry(const NdAssembleArgs& a, int gi, int gj) {
-    if (gi == a.M || gj == a.M) return (gi == gj) ? 0.0 : __ldg(a.b + (gi == a.M ? gj : gi));
+    if (gi >= a.M || gj >= a.M) {
+        if (gi >= a.M && gj >= a.M) return 0.0;
+        return gi >= a.M ? __ldg(a.b + (long long)(gi - a.M) * a.M + gj) : __ldg(a.b + (long long)(gj - a.M) * a.M + gi);
+    }
     if (a.dense != nullptr) return __ldg(a.dense + (long long)max(gi, gj) * a.M + min(gi, gj));
     const int i1 = gi / a.m2, i2 = gi % a.m2, j1 = gj / a.m2, j2 = gj % a.m2;
     int d1 = i1 - j1, d2 = i2 - j2;
@@ -560,9 +576,11 @@ __global__ void __launch_bounds__(kTdThreads, 2) nd_factor_kernel(NdFactorArgs a
 }
 
 // log|P| = 2 sum log L_jj (deterministic: fixed slices, tree reductions, the last block to finish adds the slices in order),
-// ||y||^2 = -(root update entry (rhs, rhs)), info, and tau
+// ||y_d||^2 = -(root update entry (rhs_d, rhs_d)), info, and tau.  scal_out[0] = log|P|, scal_out[q_slot + d] = ||y_d||^2,
+// scal_out[info_slot] = info.
 __global__ void __launch_bounds__(256) nd_scalars_kernel(const long long* __restrict__ doff, int M, const double* __restrict__ Lpool,
-                                                         long long quad_off, int* __restrict__ ready, long long n_tiles,
+                                                         const long long* __restrict__ quad_off, int R, int q_slot, int info_slot,
+                                                         int* __restrict__ ready, long long n_tiles,
                                                          double* __restrict__ scal_out, double* __restrict__ scal_keep) {
     __shared__ double s[256];
     __shared__ bool last;
@@ -585,13 +603,17 @@ __global__ void __launch_bounds__(256) nd_scalars_kernel(const long long* __rest
     if (threadIdx.x == 0) {
         double tot = 0.0;
         for (int bk = 0; bk < (int)gridDim.x; ++bk) tot += __ldcg(scal_keep + 8 + bk);
-        const double quad = -__ldcg(Lpool + quad_off);
         const int aborted = ready[n_tiles], bad = ready[n_tiles + 1];
         scal_out[0] = 2.0 * tot;
-        scal_out[1] = quad;
-        scal_out[2] = aborted ? -1.0 : (bad != kNoBadPivot ? (double)bad : 0.0);
+        double quad = 0.0;
+        for (int d = 0; d < R; ++d) {
+            const double q = -__ldcg(Lpool + quad_off[d]);
+            scal_out[q_slot + d] = q;
+            quad = d == 0 ? q : quad + q;
+        }
+        scal_out[info_slot] = aborted ? -1.0 : (bad != kNoBadPivot ? (double)bad : 0.0);
         scal_keep[0] = quad;
-        scal_keep[1] = 9.5367431640625e-07 / (1.0 + quad);        // tau = 2^-20 / (1 + ||y||^2)
+        scal_keep[1] = 9.5367431640625e-07 / (1.0 + quad);        // tau = 2^-20 / (1 + sum_d ||y_d||^2)
     }
 }
 
@@ -632,13 +654,14 @@ __global__ void __launch_bounds__(kTdThreads) nd_ypass_kernel(const FrontDesc* _
     }
 }
 
-// Sigma on the boundary block of every front of a level, from the parent's Sigma (the root's boundary is the rhs node
-// alone: Sigma'(rhs, rhs) = tau).  Lower tiles and their transposes.
+// Sigma on the boundary block of every front of a level, from the parent's Sigma (the root's boundary is the rhs nodes
+// alone: Sigma'(rhs, rhs) = tau I).  Lower tiles and their transposes.
 struct NdGatherArgs {
     const FrontDesc* fronts; const int4* tasks; int n_tasks;
     const int* pmap;
     double *sig_lower, *sig_upper;
     const double* scal_keep;        // [1] = tau
+    int n_rhs;
 };
 __global__ void __launch_bounds__(256) nd_gather_kernel(NdGatherArgs a) {
     __shared__ double s_t[NB][NB + 1];
@@ -650,14 +673,14 @@ __global__ void __launch_bounds__(256) nd_gather_kernel(NdGatherArgs a) {
         const int* pm = a.pmap + f.pmap_off;
         FrontDesc p;
         if (f.parent >= 0) p = a.fronts[f.parent];
-        const int rhs_pos = f.nb - 1;                                    // boundary-local position of the rhs node
+        const int rhs_pos = f.nb - a.n_rhs;                              // boundary-local position of the first rhs node
         __syncthreads();
         for (int e = threadIdx.x; e < TILE; e += blockDim.x) {
             const int r = e % NB, c = e / NB;
             const int I = (R - f.nsT) * NB + r, J = (C - f.nsT) * NB + c;
             double v = 0.0;
             if (f.parent < 0) {
-                v = (I == rhs_pos && J == rhs_pos) ? a.scal_keep[1] : 0.0;
+                v = (I == J && I >= rhs_pos && I < f.nb) ? a.scal_keep[1] : 0.0;
             } else {
                 int pa = pm[I], pb = pm[J];
                 if (pa >= 0 && pb >= 0) {
@@ -796,18 +819,26 @@ __global__ void __launch_bounds__(kTdThreads, 2) nd_selinv_kernel(NdSelArgs a) {
     }
 }
 
-// x_j = -Sigma'(rhs, j) / tau
-__global__ void __launch_bounds__(256) nd_x_kernel(const long long* __restrict__ xoff, int M, const double* __restrict__ sig_lower,
+// x[d M + j] = x_d,j = -Sigma'(rhs_d, j) / tau  (t < R M)
+__global__ void __launch_bounds__(256) nd_x_kernel(const long long* __restrict__ xoff, int RM, const double* __restrict__ sig_lower,
                                                    const double* __restrict__ scal_keep, const int* __restrict__ abort_flag,
                                                    double* __restrict__ x) {
     const double inv_tau = -1.0 / scal_keep[1];
     const bool aborted = *abort_flag != 0;
-    for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < M; j += gridDim.x * blockDim.x)
+    for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < RM; j += gridDim.x * blockDim.x)
         x[j] = aborted ? nan("") : __ldcg(sig_lower + xoff[j]) * inv_tau;
 }
 
-// stencil entries of P^-1 = Sigma' - tau x x^T
-__global__ void __launch_bounds__(256) nd_stencil_kernel(const long long* __restrict__ sigoff, int m1, int m2, int K,
+// tau sum_d x_d,i x_d,j for R > 1 right-hand sides
+__device__ __forceinline__ double nd_rank_correction(const double* __restrict__ x, long long M, int R, double tau, long long i,
+                                                     long long j) {
+    double c = tau * x[i] * x[j];
+    for (int d = 1; d < R; ++d) c += tau * x[d * M + i] * x[d * M + j];
+    return c;
+}
+
+// stencil entries of P^-1 = Sigma' - tau sum_d x_d x_d^T
+__global__ void __launch_bounds__(256) nd_stencil_kernel(const long long* __restrict__ sigoff, int m1, int m2, int K, int R,
                                                          const double* __restrict__ sig_lower, const double* __restrict__ x,
                                                          const double* __restrict__ scal_keep, const int* __restrict__ abort_flag,
                                                          double* __restrict__ out) {
@@ -829,7 +860,8 @@ __global__ void __launch_bounds__(256) nd_stencil_kernel(const long long* __rest
             const int ee = (int)(t / M);
             const long long j = t % M;
             const long long i = j + (long long)(ee / NS) * m2 + (ee % NS - K);
-            v -= tau * x[i] * x[j];
+            if (R == 1) v -= tau * x[i] * x[j];          // the single-rhs expression as it was (same contraction, same bits)
+            else v -= nd_rank_correction(x, M, R, tau, i, j);
         }
         out[t] = aborted ? nan("") : v;
     }
@@ -877,13 +909,47 @@ extern "C" int64_t asvgp_kron_rhs_doubles(int m1, int m2, int order) {
     return (int64_t)m1 * m2;
 }
 
+#define ND_CHECK_RHS(name)                                                                                               \
+    ASVGP_REQUIRE(n_rhs >= 1 && n_rhs <= ASVGP_MAX_RHS, name ": n_rhs=%d (1 ... %d right-hand sides)", n_rhs, ASVGP_MAX_RHS)
+
+static void nd_sizes(const NdPlan& P, int64_t* h_sizes) {
+    const NdLayout L = nd_layout(P);
+    h_sizes[0] = L.band_total; h_sizes[1] = L.sig_total; h_sizes[2] = L.work_total; h_sizes[3] = (int64_t)P.M * P.R;
+}
+
+extern "C" int asvgp_kron_doubles_multi(int m1, int m2, int order, int n_rhs, int64_t* h_sizes) {
+    ND_CHECK_ARGS("kron_doubles_multi");
+    ND_CHECK_RHS("kron_doubles_multi");
+    nd_sizes(*nd_plan_host(m1, m2, order, n_rhs), h_sizes);
+    return kOk;
+}
+
 // Diagnostics / tests: out[0..7] = fronts, levels, tiles per pool, separator block columns, sum of separator sizes along the
 // longest root-to-leaf path (the dependency chain, in columns), the same in block columns, largest front (unknowns), flops.
-// idx_out (may be NULL): for every front, level, ns, nb, then the ns + nb node ids (rhs node = m1*m2); returns the number of
-// ints that takes.
+// idx_out (may be NULL): for every front, level, ns, nb, then the ns + nb node ids (rhs nodes = m1*m2 ... m1*m2+n_rhs-1);
+// returns the number of ints that takes.
+static int64_t nd_plan_info(int m1, int m2, int order, int n_rhs, double* out, int32_t* idx_out, int64_t idx_capacity);
+
 extern "C" int64_t asvgp_kron_plan_info(int m1, int m2, int order, double* out, int32_t* idx_out, int64_t idx_capacity) {
     if (m1 <= 0 || m2 <= 0 || order < 1 || order > kMaxOrder) return -1;
-    const NdPlan& P = *nd_plan_host(m1, m2, order);
+    return nd_plan_info(m1, m2, order, 1, out, idx_out, idx_capacity);
+}
+
+extern "C" int64_t asvgp_kron_plan_info_multi(int m1, int m2, int order, int n_rhs, double* out, int32_t* idx_out,
+                                              int64_t idx_capacity) {
+    if (m1 <= 0 || m2 <= 0 || order < 1 || order > kMaxOrder) {
+        set_last_error("kron_plan_info_multi: m=%d,%d order=%d", m1, m2, order);
+        return -1;
+    }
+    if (n_rhs < 1 || n_rhs > ASVGP_MAX_RHS) {
+        set_last_error("kron_plan_info_multi: n_rhs=%d (1 ... %d right-hand sides)", n_rhs, ASVGP_MAX_RHS);
+        return -1;
+    }
+    return nd_plan_info(m1, m2, order, n_rhs, out, idx_out, idx_capacity);
+}
+
+static int64_t nd_plan_info(int m1, int m2, int order, int n_rhs, double* out, int32_t* idx_out, int64_t idx_capacity) {
+    const NdPlan& P = *nd_plan_host(m1, m2, order, n_rhs);
     std::vector<long long> chain(P.n_fronts, 0), chainT(P.n_fronts, 0);
     double flops = 0.0;
     long long best = 0, bestT = 0;
@@ -913,8 +979,10 @@ extern "C" int64_t asvgp_kron_plan_info(int m1, int m2, int order, double* out, 
     return need;
 }
 
+
 // ---- shared bodies of the Kronecker and the dense entry points -----------------------------------------------------------------
-static int nd_factor_run(const NdPlan& P, NdAssembleArgs aa, double* band, double* scal, cudaStream_t st) {
+// multi = false: scal = { log|P|, Q, info } (single-rhs layout); true: scal = { log|P|, info, Q_1 ... Q_R }
+static int nd_factor_run(const NdPlan& P, NdAssembleArgs aa, double* band, double* scal, bool multi, cudaStream_t st) {
     const NdLayout lay = nd_layout(P);
     int* flags = reinterpret_cast<int*>(band + lay.flags);
     ASVGP_CUDA_OK(cudaMemsetAsync(flags, 0, (size_t)lay.n_flag_ints * sizeof(int), st));
@@ -928,12 +996,13 @@ static int nd_factor_run(const NdPlan& P, NdAssembleArgs aa, double* band, doubl
         NdFactorArgs fa{P.d_fronts, P.d_factor_tasks[lev], n_tasks, P.d_idx, P.d_pmap, band, band + lay.linv, flags, P.n_tiles};
         if (int rc = nd_launch_persistent(nd_factor_kernel, &fa, n_tasks, st)) return rc;
     }
-    nd_scalars_kernel<<<kNdScalarBlocks, 256, 0, st>>>(P.d_doff, P.M, band, P.quad_off, flags, P.n_tiles, scal, band + lay.scal); ASVGP_LAUNCHED();
+    nd_scalars_kernel<<<kNdScalarBlocks, 256, 0, st>>>(P.d_doff, P.M, band, P.d_quad_off, P.R, multi ? 2 : 1, multi ? 1 : 2, flags,
+                                                       P.n_tiles, scal, band + lay.scal); ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     return kOk;
 }
 
-// selected inverse of every front + x = P^-1 b; returns the abort flag's address for the extraction kernels
+// selected inverse of every front + x_d = P^-1 b_d; returns the abort flag's address for the extraction kernels
 static int nd_selinv_run(const NdPlan& P, double* band, double* sig_band, double* x_out, double* work, cudaStream_t st,
                          const int** abort_flag_out) {
     const NdLayout lay = nd_layout(P);
@@ -949,7 +1018,7 @@ static int nd_selinv_run(const NdPlan& P, double* band, double* sig_band, double
     ASVGP_CUDA_OK(cudaGetLastError());
     for (int lev = 0; lev < P.n_levels; ++lev) {
         const int n_g = (int)P.gather_tasks[lev].size();
-        NdGatherArgs ga{P.d_fronts, P.d_gather_tasks[lev], n_g, P.d_pmap, sigL, sigU, band + lay.scal};
+        NdGatherArgs ga{P.d_fronts, P.d_gather_tasks[lev], n_g, P.d_pmap, sigL, sigU, band + lay.scal, P.R};
         nd_gather_kernel<<<std::min(n_g, 148 * 8), 256, 0, st>>>(ga); ASVGP_LAUNCHED();
         ASVGP_CUDA_OK(cudaGetLastError());
         const int n_s = (int)P.selinv_tasks[lev].size();
@@ -958,9 +1027,37 @@ static int nd_selinv_run(const NdPlan& P, double* band, double* sig_band, double
         if (int rc = nd_launch_persistent(nd_selinv_kernel, &sa, n_s, st)) return rc;
     }
     const int* abort_flag = flags + P.n_tiles + P.n_cnt;
-    nd_x_kernel<<<(P.M + 255) / 256, 256, 0, st>>>(P.d_xoff, P.M, sigL, band + lay.scal, abort_flag, x_out); ASVGP_LAUNCHED();
+    const int RM = P.M * P.R;
+    nd_x_kernel<<<(RM + 255) / 256, 256, 0, st>>>(P.d_xoff, RM, sigL, band + lay.scal, abort_flag, x_out); ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     *abort_flag_out = abort_flag;
+    return kOk;
+}
+
+static int nd_kron_factor(const double* K1, const double* K2, const double* Gs, int m1, int m2, int order, int n_rhs, double sigma2,
+                          double* band, double* rhs_io, double* scal, bool multi, void* stream) {
+    const NdPlan* Pp = nullptr;
+    if (int rc = nd_plan_device(m1, m2, order, n_rhs, &Pp)) return rc;
+    NdAssembleArgs aa{};
+    aa.K1 = K1; aa.K2 = K2; aa.Gs = Gs; aa.b = rhs_io; aa.sigma2 = sigma2; aa.m1 = m1; aa.m2 = m2; aa.K = order; aa.dense = nullptr;
+    return nd_factor_run(*Pp, aa, band, scal, multi, static_cast<cudaStream_t>(stream));
+}
+
+static int nd_kron_selinv(double* band, int m1, int m2, int order, int n_rhs, double* sig_band, double* x_io, double* sigma_stencil,
+                          double* work, void* stream) {
+    const NdPlan* Pp = nullptr;
+    if (int rc = nd_plan_device(m1, m2, order, n_rhs, &Pp)) return rc;
+    const NdPlan& P = *Pp;
+    const NdLayout lay = nd_layout(P);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int* abort_flag = nullptr;
+    if (int rc = nd_selinv_run(P, band, sig_band, x_io, work, st, &abort_flag)) return rc;
+    const int64_t total = (int64_t)P.M * (order + 1) * (2 * order + 1);
+    nd_stencil_kernel<<<(int)std::min<int64_t>((total + 255) / 256, 148 * 16), 256, 0, st>>>(P.d_sigoff, m1, m2, order, P.R, sig_band,
+                                                                                          x_io, band + lay.scal, abort_flag,
+                                                                                          sigma_stencil);
+    ASVGP_LAUNCHED();
+    ASVGP_CUDA_OK(cudaGetLastError());
     return kOk;
 }
 
@@ -970,11 +1067,7 @@ extern "C" int asvgp_kron_factor(const double* K1, const double* K2, const doubl
                                  double sigma2, double* band, double* rhs_io, double* scal, void* stream) {
     ND_CHECK_ARGS("kron_factor");
     ASVGP_REQUIRE(sigma2 > 0.0, "kron_factor: sigma2=%g", sigma2);
-    const NdPlan* Pp = nullptr;
-    if (int rc = nd_plan_device(m1, m2, order, &Pp)) return rc;
-    NdAssembleArgs aa{};
-    aa.K1 = K1; aa.K2 = K2; aa.Gs = Gs; aa.b = rhs_io; aa.sigma2 = sigma2; aa.m1 = m1; aa.m2 = m2; aa.K = order; aa.dense = nullptr;
-    return nd_factor_run(*Pp, aa, band, scal, static_cast<cudaStream_t>(stream));
+    return nd_kron_factor(K1, K2, Gs, m1, m2, order, 1, sigma2, band, rhs_io, scal, false, stream);
 }
 
 // From the factor (consumed: its off-diagonal tiles become Y^T): sigma_stencil[(order+1)(2 order+1) x M] = entries of P^-1
@@ -983,19 +1076,23 @@ extern "C" int asvgp_kron_factor(const double* K1, const double* K2, const doubl
 extern "C" int asvgp_kron_selinv(double* band, int m1, int m2, int order, double* sig_band, double* x_io,
                                  double* sigma_stencil, double* work, void* stream) {
     ND_CHECK_ARGS("kron_selinv");
-    const NdPlan* Pp = nullptr;
-    if (int rc = nd_plan_device(m1, m2, order, &Pp)) return rc;
-    const NdPlan& P = *Pp;
-    const NdLayout lay = nd_layout(P);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const int* abort_flag = nullptr;
-    if (int rc = nd_selinv_run(P, band, sig_band, x_io, work, st, &abort_flag)) return rc;
-    const int64_t total = (int64_t)P.M * (order + 1) * (2 * order + 1);
-    nd_stencil_kernel<<<(int)std::min<int64_t>((total + 255) / 256, 148 * 16), 256, 0, st>>>(P.d_sigoff, m1, m2, order, sig_band, x_io,
-                                                                                          band + lay.scal, abort_flag, sigma_stencil);
-    ASVGP_LAUNCHED();
-    ASVGP_CUDA_OK(cudaGetLastError());
-    return kOk;
+    return nd_kron_selinv(band, m1, m2, order, 1, sig_band, x_io, sigma_stencil, work, stream);
+}
+
+// n_rhs right-hand sides: rhs_io[n_rhs x M] (column d at d M), scal[2 + n_rhs] = { log|P|, info, ||L^-1 b_d||^2 ... }
+extern "C" int asvgp_kron_factor_multi(const double* K1, const double* K2, const double* Gs, int m1, int m2, int order, int n_rhs,
+                                       double sigma2, double* band, double* rhs_io, double* scal, void* stream) {
+    ND_CHECK_ARGS("kron_factor_multi");
+    ND_CHECK_RHS("kron_factor_multi");
+    ASVGP_REQUIRE(sigma2 > 0.0, "kron_factor_multi: sigma2=%g", sigma2);
+    return nd_kron_factor(K1, K2, Gs, m1, m2, order, n_rhs, sigma2, band, rhs_io, scal, true, stream);
+}
+
+extern "C" int asvgp_kron_selinv_multi(double* band, int m1, int m2, int order, int n_rhs, double* sig_band, double* x_io,
+                                       double* sigma_stencil, double* work, void* stream) {
+    ND_CHECK_ARGS("kron_selinv_multi");
+    ND_CHECK_RHS("kron_selinv_multi");
+    return nd_kron_selinv(band, m1, m2, order, n_rhs, sig_band, x_io, sigma_stencil, work, stream);
 }
 
 // ---- dense symmetric positive definite matrices on the same kernels (one front) -----------------------------------------------------
@@ -1014,20 +1111,42 @@ extern "C" int64_t asvgp_dense_work_doubles(int n) {
     return nd_layout(*nd_plan_host(n, 1, -1)).work_total;
 }
 
+#define ND_CHECK_DENSE(name) ASVGP_REQUIRE(n > 0 && n <= 32768, name ": n=%d", n)
+
+extern "C" int asvgp_dense_doubles_multi(int n, int n_rhs, int64_t* h_sizes) {
+    ND_CHECK_DENSE("dense_doubles_multi");
+    ND_CHECK_RHS("dense_doubles_multi");
+    nd_sizes(*nd_plan_host(n, 1, -1, n_rhs), h_sizes);
+    return kOk;
+}
+
+static int nd_dense_factor(const double* A, int n, int n_rhs, const double* rhs, double* band, double* scal, bool multi, void* stream) {
+    const NdPlan* Pp = nullptr;
+    if (int rc = nd_plan_device(n, 1, -1, n_rhs, &Pp)) return rc;
+    NdAssembleArgs aa{};
+    aa.b = rhs; aa.sigma2 = 1.0; aa.m1 = n; aa.m2 = 1; aa.K = 0; aa.dense = A;
+    return nd_factor_run(*Pp, aa, band, scal, multi, static_cast<cudaStream_t>(stream));
+}
+
 // A: n x n row-major (lower triangle read), rhs[n].  scal[3] = log|A|, rhs^T A^-1 rhs, info (0 ok, j+1 = row of the first
 // non-positive pivot, -1 internal time-out).
 extern "C" int asvgp_dense_factor(const double* A, int n, const double* rhs, double* band, double* scal, void* stream) {
-    ASVGP_REQUIRE(n > 0 && n <= 32768, "dense_factor: n=%d", n);
-    const NdPlan* Pp = nullptr;
-    if (int rc = nd_plan_device(n, 1, -1, &Pp)) return rc;
-    NdAssembleArgs aa{};
-    aa.b = rhs; aa.sigma2 = 1.0; aa.m1 = n; aa.m2 = 1; aa.K = 0; aa.dense = A;
-    return nd_factor_run(*Pp, aa, band, scal, static_cast<cudaStream_t>(stream));
+    ND_CHECK_DENSE("dense_factor");
+    return nd_dense_factor(A, n, 1, rhs, band, scal, false, stream);
+}
+
+// rhs[n_rhs x n] (column d at d n); scal[2 + n_rhs] = { log|A|, info, rhs_d^T A^-1 rhs_d ... }
+extern "C" int asvgp_dense_factor_multi(const double* A, int n, int n_rhs, const double* rhs, double* band, double* scal,
+                                        void* stream) {
+    ND_CHECK_DENSE("dense_factor_multi");
+    ND_CHECK_RHS("dense_factor_multi");
+    return nd_dense_factor(A, n, n_rhs, rhs, band, scal, true, stream);
 }
 
 namespace asvgp {
-// inv[i * n + j] = Sigma'(i, j) - tau x_i x_j for the single front of a dense plan (diagonal tiles averaged with their mirror)
-__global__ void __launch_bounds__(256) nd_dense_extract_kernel(FrontDesc f, int n, const double* __restrict__ sig_lower,
+// inv[i * n + j] = Sigma'(i, j) - tau sum_d x_d,i x_d,j for the single front of a dense plan (diagonal tiles averaged with their
+// mirror)
+__global__ void __launch_bounds__(256) nd_dense_extract_kernel(FrontDesc f, int n, int R, const double* __restrict__ sig_lower,
                                                                const double* __restrict__ x, const double* __restrict__ scal_keep,
                                                                const int* __restrict__ abort_flag, double* __restrict__ inv) {
     const double tau = scal_keep[1];
@@ -1039,25 +1158,39 @@ __global__ void __launch_bounds__(256) nd_dense_extract_kernel(FrontDesc f, int 
         const double* tile = sig_lower + front_tile(f, hi / NB, lo / NB) * TILE_P;
         double v = __ldcg(tile + (lo % NB) * LDT + hi % NB);
         if (hi / NB == lo / NB) v = 0.5 * (v + __ldcg(tile + (hi % NB) * LDT + lo % NB));
-        inv[t] = aborted ? nan("") : v - tau * x[i] * x[j];
+        if (R == 1) inv[t] = aborted ? nan("") : v - tau * x[i] * x[j];       // the single-rhs expression as it was
+        else inv[t] = aborted ? nan("") : v - nd_rank_correction(x, n, R, tau, i, j);
     }
 }
 }  // namespace asvgp
 
-// band is CONSUMED.  x_out[n] = A^-1 rhs, inv_out[n x n] = A^-1 (full symmetric, row-major).
-extern "C" int asvgp_dense_selinv(double* band, int n, double* sig_band, double* x_out, double* inv_out, double* work, void* stream) {
-    ASVGP_REQUIRE(n > 0 && n <= 32768, "dense_selinv: n=%d", n);
+static int nd_dense_selinv(double* band, int n, int n_rhs, double* sig_band, double* x_out, double* inv_out, double* work,
+                           void* stream) {
     const NdPlan* Pp = nullptr;
-    if (int rc = nd_plan_device(n, 1, -1, &Pp)) return rc;
+    if (int rc = nd_plan_device(n, 1, -1, n_rhs, &Pp)) return rc;
     const NdPlan& P = *Pp;
     const NdLayout lay = nd_layout(P);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int* abort_flag = nullptr;
     if (int rc = nd_selinv_run(P, band, sig_band, x_out, work, st, &abort_flag)) return rc;
     const int64_t total = (int64_t)n * n;
-    nd_dense_extract_kernel<<<(int)std::min<int64_t>((total + 255) / 256, 148 * 16), 256, 0, st>>>(P.fronts[0], n, sig_band, x_out,
+    nd_dense_extract_kernel<<<(int)std::min<int64_t>((total + 255) / 256, 148 * 16), 256, 0, st>>>(P.fronts[0], n, P.R, sig_band, x_out,
                                                                                                  band + lay.scal, abort_flag, inv_out);
     ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     return kOk;
+}
+
+// band is CONSUMED.  x_out[n] = A^-1 rhs, inv_out[n x n] = A^-1 (full symmetric, row-major).
+extern "C" int asvgp_dense_selinv(double* band, int n, double* sig_band, double* x_out, double* inv_out, double* work, void* stream) {
+    ND_CHECK_DENSE("dense_selinv");
+    return nd_dense_selinv(band, n, 1, sig_band, x_out, inv_out, work, stream);
+}
+
+// x_out[n_rhs x n]: x_out[d n + i] = (A^-1 rhs_d)_i
+extern "C" int asvgp_dense_selinv_multi(double* band, int n, int n_rhs, double* sig_band, double* x_out, double* inv_out,
+                                        double* work, void* stream) {
+    ND_CHECK_DENSE("dense_selinv_multi");
+    ND_CHECK_RHS("dense_selinv_multi");
+    return nd_dense_selinv(band, n, n_rhs, sig_band, x_out, inv_out, work, stream);
 }

@@ -248,6 +248,30 @@ class GPR_1d(_ModelBase):
         return mean.cpu().numpy(), var.cpu().numpy()
 
 
+def _kron_column_bound(N, s2, v, m1, m2, sc1, sc2, logdetP, Q, yy, T, want_grad):
+    """ELBO of the Kronecker model for one output column and, with want_grad, its derivatives [v1, l1, v2, l2, sigma2];
+    sc_i = {log|K_i|, dlog|K_i|, ...}, T = the 11 slots of asvgp_kron_terms.  Returns (elbo, grads or None, log|Kuu|)."""
+    M = m1 * m2
+    logdetK = m2 * sc1[0] + m1 * sc2[0]                       # log|K1 (x) K2|
+    tr = T[8]
+    v12 = v[0] * v[1]
+    elbo = (-0.5 * N * np.log(2 * np.pi * s2) - 0.5 * logdetP + 0.5 * logdetK - 0.5 * yy / s2
+            + 0.5 * Q / s2**2 - 0.5 * N * v12 / s2 + 0.5 * tr / s2)
+    if not want_grad:
+        return elbo, None, logdetK
+    trPG, trPdK1, trPdK2, trPK = T[0:4]
+    xGx, xdK1x, xdK2x, xKx = T[4:8]
+    d_l1 = -0.5 * trPdK1 + 0.5 * m2 * sc1[1] - 0.5 * xdK1x / s2**2 + 0.5 * T[9] / s2
+    d_l2 = -0.5 * trPdK2 + 0.5 * m1 * sc2[1] - 0.5 * xdK2x / s2**2 + 0.5 * T[10] / s2
+    # Kuu is proportional to 1 / (v1 v2): dKuu/dv_i = -Kuu / v_i
+    common = 0.5 * trPK - 0.5 * M + 0.5 * xKx / s2**2 + 0.5 * tr / s2
+    d_v1 = common / v[0] - 0.5 * N * v[1] / s2
+    d_v2 = common / v[1] - 0.5 * N * v[0] / s2
+    d_s2 = (-0.5 * N / s2 + 0.5 * trPG / s2**2 + 0.5 * yy / s2**2 + 0.5 * xGx / s2**4 - Q / s2**3
+            + 0.5 * N * v12 / s2**2 - 0.5 * tr / s2**2)
+    return elbo, np.array([d_v1, d_l1, d_v2, d_l2, d_s2]), logdetK
+
+
 class GPR_kron(_ModelBase):
     """Collapsed-bound sparse GP regression on 2-D inputs with Kronecker-structured B-spline inducing features
     (reference gpr.py:239-359).  Same constructor, attributes and methods; what differs is only *how*:
@@ -264,11 +288,16 @@ class GPR_kron(_ModelBase):
         [G stencil | Kuf_y | sum y^2 | N] is all-reduced once, the factorisation is replicated.
     """
 
+    n_outputs = 1           # output columns (y[N, D]); class defaults for objects assembled without the constructor
+    _extra = None
+
     def __init__(self, data, kernels, bases, distributed="auto", check_inputs=True, method=None, raster_shape=None):
         """raster_shape=(n1, n2): the caller's statement that X is np.meshgrid(x1, x2, indexing="ij") flattened (x1 slow),
         the eNATL60-shaped input — skips the on-device input classification (a wrong statement is slow, never wrong).
         X[n, 2] and y may each be float32 or float64 (CUDA tensors or host arrays) and are read as they are; the model
-        equals the one built from the float64-converted data up to summation order."""
+        equals the one built from the float64-converted data up to summation order.
+        y[n, D] (D <= ops.MAX_RHS, method "nd"): D output columns on the same points share one factorisation of P per step;
+        the bound is the reference's multi-output bound (as GPR_1d), predict_f returns means (n*, D) and variances (n*, 1)."""
         X, y = data
         self.X, self.y = X, y
         self.n = X.shape[0]
@@ -279,7 +308,11 @@ class GPR_kron(_ModelBase):
         assert len(kernels) == len(bases) == self.d
         if y.ndim == 1:
             y = y.reshape(-1, 1)
-        assert y.shape[1] == 1
+        n_out = self.n_outputs = int(y.shape[1])
+        if not 1 <= n_out <= ops.MAX_RHS:
+            raise ValueError("GPR_kron takes 1 ... %d output columns, got %d" % (ops.MAX_RHS, n_out))
+        if n_out > 1 and (method or ops.KRON_METHOD) != "nd":
+            raise NotImplementedError("several output columns need method='nd' (the scalar-band method takes one column)")
         self._kinds = [kernel_kind(k) for k in kernels]
         if self.d != 2:
             raise NotImplementedError("GPR_kron is implemented for d = 2 (as reference utils.py:57)")
@@ -305,32 +338,77 @@ class GPR_kron(_ModelBase):
 
         # Precompute static quantities (reference gpr.py:268-274): one fused pass over this rank's points
         dev = ops.device()
-        self._acc = torch.zeros(ops.accum_size_2d(self.bases), dtype=torch.float64, device=dev)
-        _, _, scal = ops.split_accum_2d(self._acc, self.bases)
-        cellmom = ops.moment_table_2d(self.bases)
         if raster_shape is not None:
             assert int(raster_shape[0]) * int(raster_shape[1]) == self.n, "raster_shape does not match the number of points"
-        if isinstance(X, torch.Tensor) and X.is_cuda:
-            if raster_shape is not None:
-                ops.accum_2d(X, y.reshape(-1), self.bases, cellmom, scal, raster_row_len=int(raster_shape[1]))
+        row_len = None if raster_shape is None else int(raster_shape[1])
+        if n_out == 1:
+            self._acc = torch.zeros(ops.accum_size_2d(self.bases), dtype=torch.float64, device=dev)
+            _, _, scal = ops.split_accum_2d(self._acc, self.bases)
+            cellmom = ops.moment_table_2d(self.bases)
+            if isinstance(X, torch.Tensor) and X.is_cuda:
+                if raster_shape is not None:
+                    ops.accum_2d(X, y.reshape(-1), self.bases, cellmom, scal, raster_row_len=row_len)
+                else:
+                    ops.accum_2d(X, y.reshape(-1), self.bases, cellmom, scal, binned="auto")
             else:
-                ops.accum_2d(X, y.reshape(-1), self.bases, cellmom, scal, binned="auto")
+                ops.accum_2d_host(X, y, self.bases, cellmom, scal, raster_row_len=row_len)
+            ops.expand_moments_2d(cellmom, self.bases, self._acc)
+            del cellmom
+            self._distributed = _dist.is_distributed(distributed)
+            if self._distributed:
+                _dist.allreduce_packed(self._acc)
+            self._extra = None
         else:
-            ops.accum_2d_host(X, y, self.bases, cellmom, scal,
-                              raster_row_len=None if raster_shape is None else int(raster_shape[1]))
-        ops.expand_moments_2d(cellmom, self.bases, self._acc)
-        del cellmom
-        self._distributed = _dist.is_distributed(distributed)
-        if self._distributed:
-            _dist.allreduce_packed(self._acc)
+            self._accumulate_columns(X, y, dev, row_len)
+            self._distributed = _dist.is_distributed(distributed)
+            if self._distributed:               # ONE collective over the packed accumulator and the other columns' [b_d | sum y_d^2 | N]
+                _dist.allreduce_packed(self._packed)
         self._Gs, self._b, self._scal = ops.split_accum_2d(self._acc, self.bases)
         self._host = None
+
+    def _accumulate_columns(self, X, y, dev, row_len):
+        """O(N) pass for D > 1 output columns: column 0 gives G, b_1 and its scalars exactly as a single-column model; every
+        further column is accumulated into a scratch moment table of its own, of which only b_d and (sum y_d^2, N) are kept.
+        All of it lives in one packed buffer [accumulator | (b_d, sum y_d^2, N) for d = 2 ... D] (one all-reduce)."""
+        n_out, M = self.n_outputs, self.bases[0].m * self.bases[1].m
+        na = ops.accum_size_2d(self.bases)
+        self._packed = torch.zeros(na + (n_out - 1) * (M + 2), dtype=torch.float64, device=dev)
+        self._acc = self._packed[:na]
+        self._extra = self._packed[na:].view(n_out - 1, M + 2)
+        accs = [self._acc] + [torch.zeros(na, dtype=torch.float64, device=dev) for _ in range(n_out - 1)]
+        scals = [ops.split_accum_2d(a, self.bases)[2] for a in accs]
+        cellmoms = [ops.moment_table_2d(self.bases) for _ in range(n_out)]
+        if isinstance(X, torch.Tensor) and X.is_cuda:
+            binned = False if row_len else ops.choose_binned_2d(X, self.bases)     # the order of X is probed once
+            for d in range(n_out):
+                yd = y[:, d].contiguous()
+                ops.accum_2d(X, yd, self.bases, cellmoms[d], scals[d], binned=binned, raster_row_len=row_len)
+        else:                   # host data: each chunk of X is staged and sent once for all columns
+            ops.accum_2d_host(X, y, self.bases, cellmoms, scals, raster_row_len=row_len)
+        for d in range(n_out):
+            ops.expand_moments_2d(cellmoms[d], self.bases, accs[d])
+            if d:
+                _, b_d, sc_d = ops.split_accum_2d(accs[d], self.bases)
+                self._extra[d - 1, :M].copy_(b_d)
+                self._extra[d - 1, M:].copy_(sc_d)
 
     # -- the reference's cached attributes (host copies, fetched lazily) --------------------------------------
     def _host_stats(self):
         if self._host is None:
-            self._host = (self._Gs.cpu().numpy(), self._b.cpu().numpy().reshape(-1, 1), self._scal.cpu().numpy())
+            b, scal = self._b.cpu().numpy().reshape(-1, 1), self._scal.cpu().numpy()
+            if self._extra is not None:         # (M, D) and the sum of y^2 over all columns (reference gpr.py:274, 78-79)
+                extra = self._extra.cpu().numpy()
+                M = b.shape[0]
+                b = np.concatenate([b, extra[:, :M].T], 1)
+                scal = scal.copy()
+                scal[0] = scal[0] + extra[:, M].sum()
+            self._host = (self._Gs.cpu().numpy(), b, scal)
         return self._host
+
+    def _rhs(self):
+        """Kuf_y of every output column as one device tensor [D, M] (D > 1 only)."""
+        M = self._b.numel()
+        return torch.cat([self._b.view(1, M), self._extra[:, :M]], 0)
 
     @property
     def Kuf_y(self):
@@ -395,44 +473,58 @@ class GPR_kron(_ModelBase):
         s2 = hyper_value(self.likelihood.variance)
         v = [hyper_value(k.variance) for k in self.kernels]
         m1, m2 = self.bases[0].m, self.bases[1].m
-        ws = ops.kron_workspace(m1, m2, self.order, getattr(self, "_method", None))
+        D = self.n_outputs
+        ws = ops.kron_workspace(m1, m2, self.order, getattr(self, "_method", None), n_rhs=D)
         Ks, dKs, Ss, dSs, scals = self._factors(want_grad, defer=True)
-        ops.kron_factor(Ks[0], Ks[1], self._acc, self.bases, s2, ws)
+        ops.kron_factor(Ks[0], Ks[1], self._acc, self.bases, s2, ws, b=self._rhs() if D > 1 else None)
         if want_grad:
             SigP, x = ops.kron_selinv(self.bases, ws)
         else:
             ws.sigma_stencil.zero_()
-            SigP, x = ws.sigma_stencil, ws.rhs[: ws.M]            # x unused for the value (multiplied by nothing read)
+            SigP, x = ws.sigma_stencil, ws.rhs[: ws.M * D].view(D, ws.M).squeeze(0)   # x unused for the value
         self._join()
-        ops.kron_terms(SigP, self._acc, x, Ks[0], dKs[0], Ks[1], dKs[1], Ss[0], dSs[0], Ss[1], dSs[1], self.bases,
-                       ws.terms)
-        packed = torch.cat([scals[0], scals[1], ws.scal, ws.terms, self._scal]).cpu().numpy()   # one D2H read
-        sc1, sc2, scP, T, (yy, N) = packed[0:4], packed[4:8], packed[8:11], packed[11:22], packed[22:24]
-        info = scP[2] or sc1[2] or sc2[2]
-        if info != 0:
-            raise np.linalg.LinAlgError("Cholesky failed: non-positive pivot %d" % int(info))
-        M = m1 * m2
-        logdetK = m2 * sc1[0] + m1 * sc2[0]                       # log|K1 (x) K2|
-        logdetP, Q, tr = scP[0], scP[1], T[8]
-        v12 = v[0] * v[1]
-        elbo = (-0.5 * N * np.log(2 * np.pi * s2) - 0.5 * logdetP + 0.5 * logdetK - 0.5 * yy / s2
-                + 0.5 * Q / s2**2 - 0.5 * N * v12 / s2 + 0.5 * tr / s2)
-        self.last_terms = dict(log_det_Kuu=logdetK, log_det_P=logdetP, quad=Q, trace=tr)
+        if D == 1:
+            ops.kron_terms(SigP, self._acc, x, Ks[0], dKs[0], Ks[1], dKs[1], Ss[0], dSs[0], Ss[1], dSs[1], self.bases,
+                           ws.terms)
+            packed = torch.cat([scals[0], scals[1], ws.scal, ws.terms, self._scal]).cpu().numpy()   # one D2H read
+            sc1, sc2, scP, T, (yy, N) = packed[0:4], packed[4:8], packed[8:11], packed[11:22], packed[22:24]
+            info = scP[2] or sc1[2] or sc2[2]
+            if info != 0:
+                raise np.linalg.LinAlgError("Cholesky failed: non-positive pivot %d" % int(info))
+            elbo, g, logdetK = _kron_column_bound(N, s2, v, m1, m2, sc1, sc2, scP[0], scP[1], yy, T, want_grad)
+            self.last_terms = dict(log_det_Kuu=logdetK, log_det_P=scP[0], quad=scP[1], trace=T[8])
+        else:
+            # one factorisation, the xT Op x terms per column (slots 0..3 and 8..10 are the same in every column)
+            for d in range(D):
+                ops.kron_terms(SigP, self._acc, x[d], Ks[0], dKs[0], Ks[1], dKs[1], Ss[0], dSs[0], Ss[1], dSs[1], self.bases,
+                               ws.terms[d])
+            packed = torch.cat([scals[0], scals[1], ws.scal, ws.terms.reshape(-1), self._scal,
+                                self._extra[:, -2]]).cpu().numpy()
+            sc1, sc2, p = packed[0:4], packed[4:8], 8
+            logdetP, info, Qs = packed[p], packed[p + 1], packed[p + 2: p + 2 + D]; p += 2 + D
+            Ts = packed[p: p + 11 * D].reshape(D, 11); p += 11 * D
+            N = packed[p + 1]
+            yys = np.concatenate([[packed[p]], packed[p + 2: p + 1 + D]])
+            info = info or sc1[2] or sc2[2]
+            if info != 0:
+                raise np.linalg.LinAlgError("Cholesky failed: non-positive pivot %d" % int(info))
+            cols = [_kron_column_bound(N, s2, v, m1, m2, sc1, sc2, logdetP, Qs[d], yys[d], Ts[d], want_grad) for d in range(D)]
+            logdetK, tr = cols[0][2], Ts[0][8]
+            # -N v1 v2 / 2 s2 + trace / 2 s2 count once (reference gpr.py:81-87), not once per column: take D - 1 copies of
+            # T = (-N v1 v2 + tr) / (2 s2) out again.  tr is proportional to v1 v2 (S_i = K_i^-1 is proportional to v_i).
+            T0 = 0.5 * (-N * v[0] * v[1] + tr) / s2
+            elbo = sum(c[0] for c in cols) - (D - 1) * T0
+            g = None
+            if want_grad:
+                dT = np.array([0.5 * (-N * v[1] + tr / v[0]) / s2, 0.5 * Ts[0][9] / s2,
+                               0.5 * (-N * v[0] + tr / v[1]) / s2, 0.5 * Ts[0][10] / s2, -T0 / s2])
+                g = np.sum([c[1] for c in cols], 0) - (D - 1) * dT
+            self.last_terms = dict(log_det_Kuu=logdetK, log_det_P=logdetP, quad=float(np.sum(Qs)), trace=tr)
         if not want_grad:
             return float(elbo), None
-        trPG, trPdK1, trPdK2, trPK = T[0:4]
-        xGx, xdK1x, xdK2x, xKx = T[4:8]
-        d_l1 = -0.5 * trPdK1 + 0.5 * m2 * sc1[1] - 0.5 * xdK1x / s2**2 + 0.5 * T[9] / s2
-        d_l2 = -0.5 * trPdK2 + 0.5 * m1 * sc2[1] - 0.5 * xdK2x / s2**2 + 0.5 * T[10] / s2
-        # Kuu is proportional to 1 / (v1 v2): dKuu/dv_i = -Kuu / v_i
-        common = 0.5 * trPK - 0.5 * M + 0.5 * xKx / s2**2 + 0.5 * tr / s2
-        d_v1 = common / v[0] - 0.5 * N * v[1] / s2
-        d_v2 = common / v[1] - 0.5 * N * v[0] / s2
-        d_s2 = (-0.5 * N / s2 + 0.5 * trPG / s2**2 + 0.5 * yy / s2**2 + 0.5 * xGx / s2**4 - Q / s2**3
-                + 0.5 * N * v12 / s2**2 - 0.5 * tr / s2**2)
-        grads = _grad_dict([(self.kernels[0].variance, d_v1), (self.kernels[0].lengthscales, d_l1),
-                            (self.kernels[1].variance, d_v2), (self.kernels[1].lengthscales, d_l2),
-                            (self.likelihood.variance, d_s2)])
+        grads = _grad_dict([(self.kernels[0].variance, g[0]), (self.kernels[0].lengthscales, g[1]),
+                            (self.kernels[1].variance, g[2]), (self.kernels[1].lengthscales, g[3]),
+                            (self.likelihood.variance, g[4])])
         return float(elbo), grads
 
     def elbo_and_grad(self):
@@ -448,14 +540,15 @@ class GPR_kron(_ModelBase):
 
     # -- prediction ----------------------------------------------------------------------------------------------
     def posterior_weights(self):
-        """(alpha, SigP stencil, S1, S2) on the device: alpha = P^-1 Kuf_y / sigma2, SigP = stencil entries of P^-1,
-        S_i = band(K_i^-1)."""
+        """(alpha, SigP stencil, S1, S2) on the device: alpha = P^-1 Kuf_y / sigma2 ([D, M] for D > 1 output columns),
+        SigP = stencil entries of P^-1, S_i = band(K_i^-1)."""
         s2 = hyper_value(self.likelihood.variance)
-        ws = ops.kron_workspace(self.bases[0].m, self.bases[1].m, self.order, getattr(self, "_method", None))
+        D = self.n_outputs
+        ws = ops.kron_workspace(self.bases[0].m, self.bases[1].m, self.order, getattr(self, "_method", None), n_rhs=D)
         Ks, _, Ss, _, scals = self._factors(False)
-        ops.kron_factor(Ks[0], Ks[1], self._acc, self.bases, s2, ws)
+        ops.kron_factor(Ks[0], Ks[1], self._acc, self.bases, s2, ws, b=self._rhs() if D > 1 else None)
         SigP, x = ops.kron_selinv(self.bases, ws)
-        info = torch.stack([ws.scal[2], scals[0][2], scals[1][2]])
+        info = torch.stack([ws.scal[2 if D == 1 else 1], scals[0][2], scals[1][2]])
         return x / s2, SigP, Ss[0], Ss[1], info
 
     def _hyper_state(self):
@@ -469,23 +562,31 @@ class GPR_kron(_ModelBase):
         cached = getattr(self, "_table", None)
         if cached is None or cached[0] != state:
             alpha, SigP, S1, S2, info = self.posterior_weights()
-            table = ops.predict_2d_prepare(self.bases, alpha, SigP, S1, S2)
+            if self.n_outputs == 1:
+                table = ops.predict_2d_prepare(self.bases, alpha, SigP, S1, S2)
+            else:                   # one table per output column (the variance part is the same in all of them)
+                table = [ops.predict_2d_prepare(self.bases, a_d, SigP, S1, S2) for a_d in alpha]
             if info.any().item():
                 raise np.linalg.LinAlgError("Cholesky failed in predict_f")
             self._table = cached = (state, table)
         return cached[1]
 
     def predict_f(self, Xnew, full_cov=False, full_output_cov=False, raster_shape=None):
-        """Posterior mean and variance at Xnew[n*, 2], each (n*, 1) (reference gpr.py:310-334).  raster_shape: as in the
+        """Posterior mean (n*, D) and variance (n*, 1) at Xnew[n*, 2] (reference gpr.py:310-334).  raster_shape: as in the
         constructor, for gridded test points."""
         assert not full_output_cov
         if full_cov:
             raise NotImplementedError
         table = self.posterior_table()
         prior = hyper_value(self.kernels[0].variance) * hyper_value(self.kernels[1].variance)
-        mean, var = ops.predict_2d_apply(Xnew, self.bases, table, prior,
-                                         raster_row_len=None if raster_shape is None else int(raster_shape[1]))
-        mean, var = mean.view(-1, 1), var.view(-1, 1)
+        row_len = None if raster_shape is None else int(raster_shape[1])
+        if self.n_outputs == 1:
+            mean, var = ops.predict_2d_apply(Xnew, self.bases, table, prior, raster_row_len=row_len)
+        else:
+            Xs = ops.to_device(Xnew)
+            cols = [ops.predict_2d_apply(Xs, self.bases, t, prior, raster_row_len=row_len) for t in table]
+            mean, var = torch.stack([c[0] for c in cols], 1), cols[0][1]
+        mean, var = mean.reshape(mean.shape[0], -1), var.view(-1, 1)
         if isinstance(Xnew, torch.Tensor) and Xnew.is_cuda:
             return mean, var
         return mean.cpu().numpy(), var.cpu().numpy()
@@ -493,6 +594,26 @@ class GPR_kron(_ModelBase):
     def predict_f_sparse(self, Xnew, full_cov=False, full_output_cov=False):
         """Same numbers as predict_f (reference gpr.py:336-359 is its CHOLMOD twin)."""
         return self.predict_f(Xnew, full_cov=full_cov, full_output_cov=full_output_cov)
+
+
+def _additive_column_bound(N, s2, v, vsum, ms, sc, logdetP, logdetK, trace, trn, Q, yy, T, dn, want_grad):
+    """ELBO of the additive model for one output column and, with want_grad, its derivatives [v_1, l_1, ..., v_D, l_D,
+    sigma2]; T[i] = asvgp_additive_terms of P^-1 and this column's x, dn = asvgp_dense_terms.  Returns (elbo, grads or None)."""
+    elbo = (-0.5 * N * np.log(2 * np.pi * s2) - 0.5 * logdetP + 0.5 * logdetK - 0.5 * yy / s2
+            + 0.5 * Q / s2**2 - 0.5 * N * vsum / s2 + 0.5 * trace / s2)
+    if not want_grad:
+        return elbo, None
+    g = []
+    for i, m in enumerate(ms):
+        trPK, trPdK, xKx, xdKx = T[i]
+        d_l = -0.5 * trPdK + 0.5 * sc[i, 1] - 0.5 * xdKx / s2**2 + 0.5 * trn[i, 1] / s2
+        # K_d is proportional to 1 / v_d: dK_d/dv_d = -K_d / v_d, trace(K_d^-1 G_dd) is proportional to v_d
+        d_v = (0.5 * trPK - 0.5 * m + 0.5 * xKx / s2**2 + 0.5 * trn[i, 0] / s2) / v[i] - 0.5 * N / s2
+        g += [d_v, d_l]
+    trPG, xGx = dn
+    d_s2 = (-0.5 * N / s2 + 0.5 * trPG / s2**2 + 0.5 * yy / s2**2 + 0.5 * xGx / s2**4 - Q / s2**3
+            + 0.5 * N * vsum / s2**2 - 0.5 * trace / s2**2)
+    return elbo, np.array(g + [d_s2])
 
 
 class GPR_additive(_ModelBase):
@@ -510,6 +631,9 @@ class GPR_additive(_ModelBase):
       * `elbo_and_grad()` returns the 2 D + 1 derivatives with the bound (TF reverse mode in the reference).
     """
 
+    n_outputs = 1
+    _B = None
+
     def __init__(self, data, kernels, bases, distributed="auto", check_inputs=True):
         X, y = data
         self.X, self.y = X, y
@@ -520,7 +644,9 @@ class GPR_additive(_ModelBase):
         assert len(kernels) == len(bases) == self.d
         if y.ndim == 1:
             y = y.reshape(-1, 1)
-        assert y.shape[1] == 1
+        n_out = self.n_outputs = int(y.shape[1])
+        if not 1 <= n_out <= ops.MAX_RHS:
+            raise ValueError("GPR_additive takes 1 ... %d output columns, got %d" % (ops.MAX_RHS, n_out))
         self._kinds = [kernel_kind(k) for k in kernels]
         if self.d > 8:
             raise NotImplementedError("GPR_additive is implemented for at most 8 input dimensions")
@@ -545,17 +671,21 @@ class GPR_additive(_ModelBase):
 
         # Precompute static quantities (reference gpr.py:169-176): D banded passes + D (D - 1) / 2 cross passes
         Xd = ops.to_device(X)
-        yd = ops.to_device(y).reshape(-1)
+        yall = ops.to_device(y)
+        yd = yall[:, 0].contiguous() if n_out > 1 else yall.reshape(-1)
         self._offsets = np.concatenate([[0], np.cumsum([b.m for b in self.bases])]).astype(int)
         self.M = int(self._offsets[-1])
         self._accs = [ops.accum_1d(Xd[:, i].contiguous(), yd, self.bases[i], binned="auto") for i in range(self.d)]
+        # further output columns: Kuf_y and sum(y^2) per (dimension, column); G comes from column 0 only
+        self._col_accs = [[ops.accum_1d(Xd[:, i].contiguous(), yall[:, c].contiguous(), self.bases[i], binned="auto")
+                           for i in range(self.d)] for c in range(1, n_out)]
         self._cross = {}
         for i in range(self.d):
             for j in range(i + 1, self.d):
                 self._cross[(i, j)] = ops.accum_cross(Xd, i, j, self.bases[i], self.bases[j])
         self._distributed = _dist.is_distributed(distributed)
         if self._distributed:
-            for acc in self._accs:
+            for acc in self._accs + [a for col in self._col_accs for a in col]:
                 _dist.allreduce_packed(acc)
             for c in self._cross.values():
                 _dist.allreduce_packed(c)
@@ -571,13 +701,31 @@ class GPR_additive(_ModelBase):
             ops._lib.call("asvgp_additive_put_cross", ops._p(c), self.bases[i].m, self.bases[j].m, int(self._offsets[i]),
                           int(self._offsets[j]), self.M, ops._p(self._G), ops._stream())
         self._scal = ops.split_accum_1d(self._accs[0], self.bases[0])[2]          # {sum y^2, N}: the same in every dimension
+        self._B, self._yy = None, None
+        if n_out > 1:               # right-hand sides [D, M] and sum(y_d^2) per column
+            self._B = torch.empty((n_out, self.M), dtype=torch.float64, device=Xd.device)
+            self._B[0].copy_(self._b)
+            self._yy = torch.empty(n_out, dtype=torch.float64, device=Xd.device)
+            self._yy[0:1].copy_(self._scal[0:1])
+            for c, accs in enumerate(self._col_accs, start=1):
+                for i, (acc, basis) in enumerate(zip(accs, self.bases)):
+                    _, bi, scal = ops.split_accum_1d(acc, basis)
+                    o = int(self._offsets[i])
+                    self._B[c, o: o + basis.m].copy_(bi)
+                self._yy[c: c + 1].copy_(ops.split_accum_1d(accs[0], self.bases[0])[2][0:1])
+        del self._col_accs
         self._P = torch.empty_like(self._G)
         self._host = None
 
     # -- the reference's cached attributes ------------------------------------------------------------------------------------
     def _host_stats(self):
         if self._host is None:
-            self._host = (self._G.cpu().numpy(), self._b.cpu().numpy().reshape(-1, 1), self._scal.cpu().numpy())
+            if self._B is None:
+                self._host = (self._G.cpu().numpy(), self._b.cpu().numpy().reshape(-1, 1), self._scal.cpu().numpy())
+            else:                   # Kuf_y (M, D); tr_yTy sums over the columns (reference gpr.py:78-79)
+                scal = self._scal.cpu().numpy().copy()
+                scal[0] = float(self._yy.sum().item())
+                self._host = (self._G.cpu().numpy(), self._B.cpu().numpy().T.copy(), scal)
         return self._host
 
     @property
@@ -630,8 +778,8 @@ class GPR_additive(_ModelBase):
         for i, basis in enumerate(self.bases):
             ops._lib.call("asvgp_additive_put_band", ops._p(Ks[i]), basis.m, basis.order, int(self._offsets[i]), self.M, 1.0, 1,
                           ops._p(self._P), ops._stream())
-        ws = ops.dense_workspace(self.M)
-        ops.dense_factor(self._P, self._b, ws)
+        ws = ops.dense_workspace(self.M, self.n_outputs)
+        ops.dense_factor(self._P, self._b if self._B is None else self._B, ws)
         x, Pinv = ops.dense_selinv(ws) if want_inverse else (None, None)
         for s in side:
             main.wait_stream(s)
@@ -641,12 +789,13 @@ class GPR_additive(_ModelBase):
         s2 = hyper_value(self.likelihood.variance)
         v = [hyper_value(k.variance) for k in self.kernels]
         Ks, dKs, Ss, dSs, scals, ws, x, Pinv = self._factor(want_grad)
-        D = self.d
+        D, R = self.d, self.n_outputs
         dev = self._G.device
+        xs = [x] if R == 1 else (list(x) if x is not None else [None] * R)
         # trace(Kuu^-1 KufKfu) and its lengthscale derivatives: per dimension, on the bands
         tr = torch.zeros((D, 4), dtype=torch.float64, device=dev)         # sum S_d .* G_dd, sum dS_d .* G_dd, -, -
-        terms = torch.zeros((D, 4), dtype=torch.float64, device=dev)
-        dense = torch.zeros(2, dtype=torch.float64, device=dev)
+        terms = torch.zeros((R, D, 4), dtype=torch.float64, device=dev)  # per output column: the x-dependent terms
+        dense = torch.zeros((R, 2), dtype=torch.float64, device=dev)
         zero_x = torch.zeros(self.M, dtype=torch.float64, device=dev)
         for i, basis in enumerate(self.bases):
             o = int(self._offsets[i])
@@ -654,39 +803,53 @@ class GPR_additive(_ModelBase):
             ops._lib.call("asvgp_additive_terms", ops._p(self._G), ops._p(zero_x), self.M, o, basis.m, basis.order, ops._p(Ss[i]),
                           ops._p(dSs[i]), ops._p(tr[i]), ops._stream())
             if want_grad:
-                ops._lib.call("asvgp_additive_terms", ops._p(Pinv), ops._p(x), self.M, o, basis.m, basis.order, ops._p(Ks[i]),
-                              ops._p(dKs[i]), ops._p(terms[i]), ops._stream())
+                for c in range(R):
+                    ops._lib.call("asvgp_additive_terms", ops._p(Pinv), ops._p(xs[c]), self.M, o, basis.m, basis.order,
+                                  ops._p(Ks[i]), ops._p(dKs[i]), ops._p(terms[c, i]), ops._stream())
         if want_grad:
-            ops._lib.call("asvgp_dense_terms", ops._p(Pinv), ops._p(self._G), ops._p(x), self.M, ops._p(dense), ops._stream())
-        packed = torch.cat([torch.stack(scals).reshape(-1), ws.scal, tr.reshape(-1), terms.reshape(-1), dense, self._scal]).cpu().numpy()
+            for c in range(R):
+                ops._lib.call("asvgp_dense_terms", ops._p(Pinv), ops._p(self._G), ops._p(xs[c]), self.M, ops._p(dense[c]),
+                              ops._stream())
+        yy_cols = self._scal[0:1] if R == 1 else self._yy
+        packed = torch.cat([torch.stack(scals).reshape(-1), ws.scal, tr.reshape(-1), terms.reshape(-1), dense.reshape(-1),
+                            self._scal, yy_cols]).cpu().numpy()
         sc = packed[: 4 * D].reshape(D, 4); p = 4 * D
-        scP = packed[p: p + 3]; p += 3
+        scP = packed[p: p + ws.scal.numel()]; p += ws.scal.numel()
         trn = packed[p: p + 4 * D].reshape(D, 4); p += 4 * D
-        T = packed[p: p + 4 * D].reshape(D, 4); p += 4 * D
-        trPG, xGx = packed[p: p + 2]; p += 2
-        yy, N = packed[p: p + 2]
-        info = scP[2] or next((s[2] for s in sc if s[2] != 0), 0.0)
+        T = packed[p: p + 4 * D * R].reshape(R, D, 4); p += 4 * D * R
+        dn = packed[p: p + 2 * R].reshape(R, 2); p += 2 * R
+        N = packed[p + 1]; p += 2
+        yys = packed[p: p + R]
+        # scal layouts of asvgp_dense_factor (one rhs) and asvgp_dense_factor_multi
+        logdetP, infoP, Qs = (scP[0], scP[2], scP[1:2]) if R == 1 else (scP[0], scP[1], scP[2:])
+        info = infoP or next((s[2] for s in sc if s[2] != 0), 0.0)
         if info != 0:
             raise np.linalg.LinAlgError("Cholesky failed: non-positive pivot %d" % int(info))
         logdetK = float(sc[:, 0].sum())
-        logdetP, Q = scP[0], scP[1]
         trace = float(trn[:, 0].sum())
         vsum = float(np.sum(v))
-        elbo = (-0.5 * N * np.log(2 * np.pi * s2) - 0.5 * logdetP + 0.5 * logdetK - 0.5 * yy / s2
-                + 0.5 * Q / s2**2 - 0.5 * N * vsum / s2 + 0.5 * trace / s2)
-        self.last_terms = dict(log_det_Kuu=logdetK, log_det_P=logdetP, quad=Q, trace=trace)
+        ms = [basis.m for basis in self.bases]
+        cols = [_additive_column_bound(N, s2, v, vsum, ms, sc, logdetP, logdetK, trace, trn, Qs[c], yys[c], T[c], dn[c],
+                                       want_grad) for c in range(R)]
+        self.last_terms = dict(log_det_Kuu=logdetK, log_det_P=logdetP, quad=float(np.sum(Qs)) if R > 1 else Qs[0], trace=trace)
+        if R == 1:
+            elbo, g = cols[0]
+        else:
+            # -N sum(v) / 2 s2 + trace / 2 s2 count once (reference gpr.py:81-87), not once per column: take R - 1 copies of
+            # T = (-N sum(v) + trace) / (2 s2) out again.  trace(K_d^-1 G_dd) is proportional to v_d.
+            T0 = 0.5 * (-N * vsum + trace) / s2
+            elbo = sum(c[0] for c in cols) - (R - 1) * T0
+            if want_grad:
+                dT = []
+                for i in range(D):
+                    dT += [0.5 * (-N + trn[i, 0] / v[i]) / s2, 0.5 * trn[i, 1] / s2]
+                g = np.sum([c[1] for c in cols], 0) - (R - 1) * np.array(dT + [-T0 / s2])
         if not want_grad:
             return float(elbo), None
         pairs = []
-        for i, (kern, basis) in enumerate(zip(self.kernels, self.bases)):
-            trPK, trPdK, xKx, xdKx = T[i]
-            d_l = -0.5 * trPdK + 0.5 * sc[i, 1] - 0.5 * xdKx / s2**2 + 0.5 * trn[i, 1] / s2
-            # K_d is proportional to 1 / v_d: dK_d/dv_d = -K_d / v_d, trace(K_d^-1 G_dd) is proportional to v_d
-            d_v = (0.5 * trPK - 0.5 * basis.m + 0.5 * xKx / s2**2 + 0.5 * trn[i, 0] / s2) / v[i] - 0.5 * N / s2
-            pairs += [(kern.variance, d_v), (kern.lengthscales, d_l)]
-        d_s2 = (-0.5 * N / s2 + 0.5 * trPG / s2**2 + 0.5 * yy / s2**2 + 0.5 * xGx / s2**4 - Q / s2**3
-                + 0.5 * N * vsum / s2**2 - 0.5 * trace / s2**2)
-        pairs.append((self.likelihood.variance, d_s2))
+        for i, kern in enumerate(self.kernels):
+            pairs += [(kern.variance, g[2 * i]), (kern.lengthscales, g[2 * i + 1])]
+        pairs.append((self.likelihood.variance, g[2 * D]))
         return float(elbo), _grad_dict(pairs)
 
     def elbo_and_grad(self):
@@ -701,13 +864,13 @@ class GPR_additive(_ModelBase):
 
     # -- prediction -----------------------------------------------------------------------------------------------------------------
     def predict_f(self, Xnew, full_cov=False, full_output_cov=False):
-        """Posterior mean and variance at Xnew[n*, D], each (n*, 1) (reference gpr.py:212-236)."""
+        """Posterior mean (n*, R) and variance (n*, 1) at Xnew[n*, D] for R output columns (reference gpr.py:212-236)."""
         assert not full_output_cov
         if full_cov:
             raise NotImplementedError
         s2 = hyper_value(self.likelihood.variance)
         Ks, dKs, Ss, dSs, scals, ws, x, Pinv = self._factor(True)
-        info = torch.stack([ws.scal[2]] + [s[2] for s in scals])
+        info = torch.stack([ws.scal[2 if self.n_outputs == 1 else 1]] + [s[2] for s in scals])
         Xs = ops.to_device(Xnew)
         assert Xs.dim() == 2 and Xs.shape[1] == self.d
         n = Xs.shape[0]
@@ -720,15 +883,18 @@ class GPR_additive(_ModelBase):
             koff += nk
         meta = torch.tensor(meta, dtype=torch.int32, device=dev)
         S_all = torch.cat([S.reshape(-1) for S in Ss])
-        alpha = x / s2
-        mean = torch.empty(n, dtype=torch.float64, device=dev)
-        var = torch.empty(n, dtype=torch.float64, device=dev)
+        alphas = x / s2
         prior = float(sum(hyper_value(k.variance) for k in self.kernels))
-        ops._lib.call("asvgp_predict_additive", ops._p(Xs), n, self.d, ops._p(meshes), ops._p(meta), self.M, self.order, ops._p(alpha),
-                      ops._p(Pinv), ops._p(S_all), prior, ops._p(mean), ops._p(var), ops._stream())
+        cols = []
+        for alpha in ([alphas] if self.n_outputs == 1 else list(alphas)):       # one pass per output column
+            mean = torch.empty(n, dtype=torch.float64, device=dev)
+            var = torch.empty(n, dtype=torch.float64, device=dev)
+            ops._lib.call("asvgp_predict_additive", ops._p(Xs), n, self.d, ops._p(meshes), ops._p(meta), self.M, self.order,
+                          ops._p(alpha), ops._p(Pinv), ops._p(S_all), prior, ops._p(mean), ops._p(var), ops._stream())
+            cols.append((mean, var))
         if info.any().item():
             raise np.linalg.LinAlgError("Cholesky failed in predict_f")
-        mean, var = mean.view(-1, 1), var.view(-1, 1)
+        mean, var = torch.stack([c[0] for c in cols], 1), cols[0][1].view(-1, 1)
         if isinstance(Xnew, torch.Tensor) and Xnew.is_cuda:
             return mean, var
         return mean.cpu().numpy(), var.cpu().numpy()

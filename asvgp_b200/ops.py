@@ -439,6 +439,12 @@ def order_probe_2d(X, bases):
     return float(out.item())
 
 
+def choose_binned_2d(X, bases):
+    """accum_2d's binned="auto" choice for the device points X[n, 2] (one order probe, one host synchronisation): callers
+    that accumulate several target columns over the same X probe once and pass the answer to every call."""
+    return X.shape[0] >= BINNED_MIN_POINTS and order_probe_2d(X, bases) > BINNED_JUMP_FRACTION
+
+
 def accum_2d(X, y, bases, cellmom, scal, binned=False, raster_row_len=None):
     """Adds the per-cell moments of the points (X[n,2], y[n]) into `cellmom` and (sum y^2, n) into `scal`
     (reference gpr.py:268-274 without materialising the Khatri-Rao Kuf).  binned: as accum_1d.
@@ -461,7 +467,7 @@ def accum_2d(X, y, bases, cellmom, scal, binned=False, raster_row_len=None):
                   mesh1.numel(), _p(mesh2), mesh2.numel(), k, _p(cellmom), _p(scal), _stream())
         return cellmom, scal
     if binned == "auto":
-        binned = X.shape[0] >= BINNED_MIN_POINTS and order_probe_2d(X, bases) > BINNED_JUMP_FRACTION
+        binned = choose_binned_2d(X, bases)
     if binned:
         nbytes = _lib.load().asvgp_accum_2d_binned_work_bytes(X.shape[0])
         work = torch.empty(nbytes, dtype=torch.uint8, device=X.device)
@@ -501,13 +507,20 @@ def expand_moments_2d(cellmom, bases, acc):
 def accum_2d_host(X, y, bases, cellmom, scal, chunk=1 << 22, raster_row_len=None):
     """accum_2d for HOST arrays: streamed through pinned staging buffers, double-buffered against the kernel.
     raster_row_len: as accum_2d (the chunks are then whole rows).  float32 / float64 arrays are staged and sent in their own
-    dtype; other dtypes are converted to float64."""
+    dtype; other dtypes are converted to float64.
+    Several target columns: y [n, D] with D moment tables and scalar pairs (cellmom, scal: sequences of D) — every chunk of X
+    crosses PCIe once and the accumulate runs once per column on it."""
     dev = device()
     Xt = points_to_host(X)
-    yt = points_to_host(y).reshape(-1)
+    yt = points_to_host(y)
+    multi = isinstance(cellmom, (list, tuple))
+    ycols = [yt[:, d] for d in range(yt.shape[1])] if multi else [yt.reshape(-1)]
+    cellmoms, scals = (list(cellmom), list(scal)) if multi else ([cellmom], [scal])
     n = Xt.shape[0]
-    if Xt.dim() != 2 or Xt.shape[1] != 2 or yt.numel() != n:
-        raise ValueError("X must be [n, 2] and y [n]")
+    if Xt.dim() != 2 or Xt.shape[1] != 2 or any(c.numel() != n for c in ycols):
+        raise ValueError("X must be [n, 2] and y [n] (or [n, D] with D moment tables)")
+    if not (len(ycols) == len(cellmoms) == len(scals)):
+        raise ValueError("one moment table and one scalar pair per target column")
     Xt = Xt.contiguous()
     if n == 0:
         return cellmom, scal
@@ -520,37 +533,43 @@ def accum_2d_host(X, y, bases, cellmom, scal, chunk=1 << 22, raster_row_len=None
         if chunk & 1:
             chunk *= 2
     chunk = min(chunk, n + (n & 1))
-    parts = [(Xt.dtype, 2 * chunk), (yt.dtype, chunk)]
-    st = _staging(dev, ("2d", chunk, Xt.dtype, yt.dtype), _staging_bytes(parts))
+    n_cols = len(ycols)
+    parts = [(Xt.dtype, 2 * chunk)] + [(yt.dtype, chunk)] * n_cols
+    key = ("2d", chunk, Xt.dtype, yt.dtype) if not multi else ("2d", chunk, Xt.dtype, yt.dtype, n_cols)
+    st = _staging(dev, key, _staging_bytes(parts))
     xc, yc = ELEM_TYPES[Xt.dtype], ELEM_TYPES[yt.dtype]
-    pinned = Xt.is_pinned() and yt.is_pinned()
+    pinned = Xt.is_pinned() and all(c.is_pinned() and c.is_contiguous() for c in ycols)
     main, cs = torch.cuda.current_stream(), st["copy_stream"]
     for c in range(-(-n // chunk)):
         lo, hi = c * chunk, min((c + 1) * chunk, n)
         cnt, s = hi - lo, c & 1
-        dXf, dyf = _split_staging(st["dev"][s], parts)
-        dX, dy = dXf[: 2 * cnt].view(cnt, 2), dyf[:cnt]
+        dXf, *dyfs = _split_staging(st["dev"][s], parts)
+        dX, dys = dXf[: 2 * cnt].view(cnt, 2), [dyf[:cnt] for dyf in dyfs]
         cs.wait_event(st["drained"][s])                # also covers the previous call (cached, shared staging buffers)
         with torch.cuda.stream(cs):
             if pinned:
                 dX.copy_(Xt[lo:hi], non_blocking=True)
-                dy.copy_(yt[lo:hi], non_blocking=True)
+                for dy, yc_host in zip(dys, ycols):
+                    dy.copy_(yc_host[lo:hi], non_blocking=True)
             else:
-                hXf, hyf = _split_staging(st["host"][s], parts)
+                hXf, *hyfs = _split_staging(st["host"][s], parts)
                 st["staged"][s].synchronize()
                 hXf[: 2 * cnt].view(cnt, 2).copy_(Xt[lo:hi])
-                hyf[:cnt].copy_(yt[lo:hi])
+                for hyf, yc_host in zip(hyfs, ycols):
+                    hyf[:cnt].copy_(yc_host[lo:hi])
                 dXf[: 2 * cnt].copy_(hXf[: 2 * cnt], non_blocking=True)
-                dy.copy_(hyf[:cnt], non_blocking=True)
+                for dy, hyf in zip(dys, hyfs):
+                    dy.copy_(hyf[:cnt], non_blocking=True)
                 st["staged"][s].record(cs)
             st["filled"][s].record(cs)
         main.wait_event(st["filled"][s])
-        if raster_row_len:
-            _lib.call("asvgp_accum_2d_raster_typed", _p(dX), xc, _p(dy), yc, cnt, int(raster_row_len), _p(mesh1), mesh1.numel(),
-                      _p(mesh2), mesh2.numel(), k, _p(cellmom), _p(scal), ctypes.c_void_p(main.cuda_stream))
-        else:
-            _lib.call("asvgp_accum_2d_typed", _p(dX), xc, _p(dy), yc, cnt, _p(mesh1), mesh1.numel(), _p(mesh2), mesh2.numel(), k,
-                      _p(cellmom), _p(scal), ctypes.c_void_p(main.cuda_stream))
+        for dy, cm, sc in zip(dys, cellmoms, scals):
+            if raster_row_len:
+                _lib.call("asvgp_accum_2d_raster_typed", _p(dX), xc, _p(dy), yc, cnt, int(raster_row_len), _p(mesh1),
+                          mesh1.numel(), _p(mesh2), mesh2.numel(), k, _p(cm), _p(sc), ctypes.c_void_p(main.cuda_stream))
+            else:
+                _lib.call("asvgp_accum_2d_typed", _p(dX), xc, _p(dy), yc, cnt, _p(mesh1), mesh1.numel(), _p(mesh2), mesh2.numel(),
+                          k, _p(cm), _p(sc), ctypes.c_void_p(main.cuda_stream))
         st["drained"][s].record(main)
     return cellmom, scal
 
@@ -583,55 +602,80 @@ KRON_METHODS = ("nd", "band")
 KRON_METHOD = "nd"        # default factorisation of the 2-D model: nested-dissection fronts; "band" = tile DAG over the scalar band
 
 
-class KronWorkspace:
-    """Device buffers of the factorisation of P = K1 (x) K2 + G / sigma2 (cached per (device, m1, m2, k, method))."""
+MAX_RHS = 32       # ASVGP_MAX_RHS of include/asvgp_b200.h: right-hand sides (output columns) per factorisation
 
-    def __init__(self, m1, m2, order, method="nd"):
+
+def _check_n_rhs(n_rhs):
+    n_rhs = int(n_rhs)
+    if not 1 <= n_rhs <= MAX_RHS:
+        raise ValueError("n_rhs must lie in [1, %d], got %d" % (MAX_RHS, n_rhs))
+    return n_rhs
+
+
+class KronWorkspace:
+    """Device buffers of the factorisation of P = K1 (x) K2 + G / sigma2 (cached per (device, m1, m2, k, method, n_rhs)).
+    n_rhs > 1: one factorisation for n_rhs right-hand sides (asvgp_kron_*_multi; rhs is [n_rhs * M], scal
+    {log|P|, info, Q_1 ... Q_n_rhs}, terms [n_rhs, 11]); n_rhs = 1 is the single-rhs layout of asvgp_kron_factor."""
+
+    def __init__(self, m1, m2, order, method="nd", n_rhs=1):
         lib = _lib.load()
         dev = device()
         if method not in KRON_METHODS:
             raise ValueError("method must be one of %r" % (KRON_METHODS,))
-        self.m1, self.m2, self.order, self.method = m1, m2, order, method
+        n_rhs = _check_n_rhs(n_rhs)
+        if n_rhs > 1 and method != "nd":
+            raise NotImplementedError("several right-hand sides need method='nd' (the scalar-band method takes one)")
+        self.m1, self.m2, self.order, self.method, self.n_rhs = m1, m2, order, method, n_rhs
         self.M = m1 * m2
         self.prefix = "asvgp_kron_" if method == "nd" else "asvgp_kronband_"
-        nb, nw, ns, nr = (getattr(lib, self.prefix + q)(m1, m2, order) for q in ("band_doubles", "work_doubles", "sig_doubles", "rhs_doubles"))
-        if min(nb, nw, ns, nr) < 0:
-            raise _lib.AsvgpNativeError("kron workspace query rejected m=%d,%d order=%d" % (m1, m2, order))
+        if n_rhs == 1:
+            nb, nw, ns, nr = (getattr(lib, self.prefix + q)(m1, m2, order) for q in ("band_doubles", "work_doubles", "sig_doubles", "rhs_doubles"))
+            if min(nb, nw, ns, nr) < 0:
+                raise _lib.AsvgpNativeError("kron workspace query rejected m=%d,%d order=%d" % (m1, m2, order))
+        else:
+            sizes = (ctypes.c_int64 * 4)()
+            _lib.call("asvgp_kron_doubles_multi", m1, m2, order, n_rhs, ctypes.cast(sizes, ctypes.c_void_p))
+            nb, ns, nw, nr = sizes
         self.band = torch.empty(nb, dtype=F64, device=dev)
         self.sig_band = None                     # allocated on first selected inverse
         self.n_sig = ns
         self.work = torch.empty(nw, dtype=F64, device=dev)
         self.rhs = torch.zeros(nr, dtype=F64, device=dev)
-        self.scal = torch.zeros(3, dtype=F64, device=dev)
+        self.scal = torch.zeros(3 if n_rhs == 1 else 2 + n_rhs, dtype=F64, device=dev)
         self.sigma_stencil = torch.zeros((stencil_rows(order), self.M), dtype=F64, device=dev)
-        self.terms = torch.zeros(11, dtype=F64, device=dev)
+        self.terms = torch.zeros(11 if n_rhs == 1 else (n_rhs, 11), dtype=F64, device=dev)
 
 
 _KRON_WS = {}
 
 
-def kron_workspace(m1, m2, order, method=None):
+def kron_workspace(m1, m2, order, method=None, n_rhs=1):
     method = method or KRON_METHOD
-    key = (device(), m1, m2, order, method)
+    key = (device(), m1, m2, order, method, int(n_rhs))
     ws = _KRON_WS.get(key)
     if ws is None:
-        ws = _KRON_WS[key] = KronWorkspace(m1, m2, order, method)
+        ws = _KRON_WS[key] = KronWorkspace(m1, m2, order, method, n_rhs)
     return ws
 
 
-def kron_plan_info(m1, m2, order, with_fronts=False):
+def kron_plan_info(m1, m2, order, with_fronts=False, n_rhs=None):
     """Shape of the nested-dissection elimination tree (host-side query, no GPU needed): dict of counts and, with
-    `with_fronts`, the list of fronts as (level, separator ids, boundary ids); id m1*m2 is the right-hand-side row."""
+    `with_fronts`, the list of fronts as (level, separator ids, boundary ids); id m1*m2 is the right-hand-side row
+    (n_rhs given: ids m1*m2 ... m1*m2 + n_rhs - 1 are the rows of the n_rhs right-hand sides)."""
     lib = _lib.load()
     out = (ctypes.c_double * 8)()
-    need = lib.asvgp_kron_plan_info(m1, m2, order, ctypes.cast(out, ctypes.c_void_p), None, 0)
+    if n_rhs is None:
+        query = lambda o, buf, cap: lib.asvgp_kron_plan_info(m1, m2, order, o, buf, cap)   # noqa: E731
+    else:
+        query = lambda o, buf, cap: lib.asvgp_kron_plan_info_multi(m1, m2, order, int(n_rhs), o, buf, cap)   # noqa: E731
+    need = query(ctypes.cast(out, ctypes.c_void_p), None, 0)
     if need < 0:
-        raise _lib.AsvgpNativeError("kron_plan_info rejected m=%d,%d order=%d" % (m1, m2, order))
+        raise _lib.AsvgpNativeError("kron_plan_info rejected m=%d,%d order=%d n_rhs=%s" % (m1, m2, order, n_rhs))
     info = dict(zip(("fronts", "levels", "tiles", "separator_block_columns", "chain_columns", "chain_block_columns",
                      "largest_front", "flops"), [float(v) for v in out]))
     if with_fronts:
         buf = np.zeros(need, dtype=np.int32)
-        lib.asvgp_kron_plan_info(m1, m2, order, None, buf.ctypes.data_as(ctypes.c_void_p), need)
+        query(None, buf.ctypes.data_as(ctypes.c_void_p), need)
         fronts, w = [], 0
         while w < need:
             level, ns, nb = (int(v) for v in buf[w:w + 3])
@@ -641,26 +685,41 @@ def kron_plan_info(m1, m2, order, with_fronts=False):
     return info
 
 
-def kron_factor(K1, K2, acc, bases, sigma2, ws):
-    """Factorisation of P and forward substitution of Kuf_y; ws.scal = {log|P|, ||L^-1 b||^2, info}."""
+def kron_factor(K1, K2, acc, bases, sigma2, ws, b=None):
+    """Factorisation of P and forward substitution of Kuf_y; ws.scal = {log|P|, ||L^-1 b||^2, info}.
+    b: right-hand sides [D, M] (D = ws.n_rhs; default: the projection in acc, D = 1).  With D > 1 one factorisation
+    serves all columns and ws.scal = {log|P|, info, ||L^-1 b_1||^2, ..., ||L^-1 b_D||^2}."""
     k, m1, m2 = _check_bases_2d(bases)
-    Gs, b, _ = split_accum_2d(acc, bases)
+    Gs, b_acc, _ = split_accum_2d(acc, bases)
+    if b is None:
+        b = b_acc
+    if b.numel() != ws.n_rhs * ws.M:
+        raise ValueError("b must hold n_rhs = %d columns of %d entries" % (ws.n_rhs, ws.M))
     if ws.method == "band":
         ws.rhs.zero_()
-    ws.rhs[: ws.M].copy_(b)
-    _lib.call(ws.prefix + "factor", _p(K1), _p(K2), _p(Gs), m1, m2, k, float(sigma2), _p(ws.band), _p(ws.rhs),
-              _p(ws.scal), _stream())
+    ws.rhs[: ws.n_rhs * ws.M].view_as(b).copy_(b)
+    if ws.n_rhs == 1:
+        _lib.call(ws.prefix + "factor", _p(K1), _p(K2), _p(Gs), m1, m2, k, float(sigma2), _p(ws.band), _p(ws.rhs),
+                  _p(ws.scal), _stream())
+    else:
+        _lib.call("asvgp_kron_factor_multi", _p(K1), _p(K2), _p(Gs), m1, m2, k, ws.n_rhs, float(sigma2), _p(ws.band),
+                  _p(ws.rhs), _p(ws.scal), _stream())
     return ws
 
 
 def kron_selinv(bases, ws):
-    """Selected inverse of P on the stencil pattern (ws.sigma_stencil) and x = P^-1 Kuf_y (ws.rhs[:M])."""
+    """Selected inverse of P on the stencil pattern (ws.sigma_stencil) and x = P^-1 Kuf_y (ws.rhs[:M]; [D, M] for a
+    workspace of D > 1 right-hand sides)."""
     k, m1, m2 = _check_bases_2d(bases)
     if ws.sig_band is None:
         ws.sig_band = torch.empty(ws.n_sig, dtype=F64, device=ws.band.device)
-    _lib.call(ws.prefix + "selinv", _p(ws.band), m1, m2, k, _p(ws.sig_band), _p(ws.rhs), _p(ws.sigma_stencil),
+    if ws.n_rhs == 1:
+        _lib.call(ws.prefix + "selinv", _p(ws.band), m1, m2, k, _p(ws.sig_band), _p(ws.rhs), _p(ws.sigma_stencil),
+                  _p(ws.work), _stream())
+        return ws.sigma_stencil, ws.rhs[: ws.M]
+    _lib.call("asvgp_kron_selinv_multi", _p(ws.band), m1, m2, k, ws.n_rhs, _p(ws.sig_band), _p(ws.rhs), _p(ws.sigma_stencil),
               _p(ws.work), _stream())
-    return ws.sigma_stencil, ws.rhs[: ws.M]
+    return ws.sigma_stencil, ws.rhs.view(ws.n_rhs, ws.M)
 
 
 def kron_terms(SigP, acc, x, K1, dK1, K2, dK2, S1, dS1, S2, dS2, bases, out):
@@ -727,43 +786,61 @@ _PREDICT_WORK = {}
 # dense SPD matrices (one front of the nested-dissection kernels) and the additive model's operators
 # =====================================================================================================================
 class DenseWorkspace:
-    """Device buffers of asvgp_dense_factor / asvgp_dense_selinv for n x n matrices (cached per (device, n))."""
+    """Device buffers of asvgp_dense_factor / asvgp_dense_selinv for n x n matrices (cached per (device, n, n_rhs)).
+    n_rhs > 1: asvgp_dense_*_multi, x is [n_rhs, n] and scal {log|A|, info, rhs_1^T A^-1 rhs_1, ...}."""
 
-    def __init__(self, n):
+    def __init__(self, n, n_rhs=1):
         lib = _lib.load()
         dev = device()
-        nb, ns, nw = lib.asvgp_dense_band_doubles(n), lib.asvgp_dense_sig_doubles(n), lib.asvgp_dense_work_doubles(n)
-        if min(nb, ns, nw) < 0:
-            raise _lib.AsvgpNativeError("dense workspace query rejected n=%d" % n)
-        self.n = n
+        n_rhs = _check_n_rhs(n_rhs)
+        if n_rhs == 1:
+            nb, ns, nw = lib.asvgp_dense_band_doubles(n), lib.asvgp_dense_sig_doubles(n), lib.asvgp_dense_work_doubles(n)
+            if min(nb, ns, nw) < 0:
+                raise _lib.AsvgpNativeError("dense workspace query rejected n=%d" % n)
+        else:
+            sizes = (ctypes.c_int64 * 4)()
+            _lib.call("asvgp_dense_doubles_multi", n, n_rhs, ctypes.cast(sizes, ctypes.c_void_p))
+            nb, ns, nw, _ = sizes
+        self.n, self.n_rhs = n, n_rhs
         self.band = torch.empty(nb, dtype=F64, device=dev)
         self.sig_band = torch.empty(ns, dtype=F64, device=dev)
         self.work = torch.empty(nw, dtype=F64, device=dev)
-        self.scal = torch.zeros(3, dtype=F64, device=dev)
-        self.x = torch.empty(n, dtype=F64, device=dev)
+        self.scal = torch.zeros(3 if n_rhs == 1 else 2 + n_rhs, dtype=F64, device=dev)
+        self.x = torch.empty(n if n_rhs == 1 else (n_rhs, n), dtype=F64, device=dev)
         self.inv = torch.empty((n, n), dtype=F64, device=dev)
 
 
 _DENSE_WS = {}
 
 
-def dense_workspace(n):
-    key = (device(), n)
+def dense_workspace(n, n_rhs=1):
+    key = (device(), n, int(n_rhs))
     ws = _DENSE_WS.get(key)
     if ws is None:
-        ws = _DENSE_WS[key] = DenseWorkspace(n)
+        ws = _DENSE_WS[key] = DenseWorkspace(n, n_rhs)
     return ws
 
 
 def dense_factor(A, rhs, ws):
-    """Cholesky of the dense SPD matrix A (lower triangle read); ws.scal = {log|A|, rhs^T A^-1 rhs, info}."""
-    _lib.call("asvgp_dense_factor", _p(A), ws.n, _p(rhs), _p(ws.band), _p(ws.scal), _stream())
+    """Cholesky of the dense SPD matrix A (lower triangle read); ws.scal = {log|A|, rhs^T A^-1 rhs, info}.  rhs may be
+    [D, n] for a workspace of D = ws.n_rhs > 1 right-hand sides: ws.scal = {log|A|, info, rhs_1^T A^-1 rhs_1, ...}."""
+    if rhs.numel() != ws.n_rhs * ws.n:
+        raise ValueError("rhs must hold n_rhs = %d columns of %d entries" % (ws.n_rhs, ws.n))
+    rhs = rhs.contiguous()
+    if ws.n_rhs == 1:
+        _lib.call("asvgp_dense_factor", _p(A), ws.n, _p(rhs), _p(ws.band), _p(ws.scal), _stream())
+    else:
+        _lib.call("asvgp_dense_factor_multi", _p(A), ws.n, ws.n_rhs, _p(rhs), _p(ws.band), _p(ws.scal), _stream())
     return ws
 
 
 def dense_selinv(ws):
-    """(A^-1 rhs, A^-1) from the factor held in ws (consumed)."""
-    _lib.call("asvgp_dense_selinv", _p(ws.band), ws.n, _p(ws.sig_band), _p(ws.x), _p(ws.inv), _p(ws.work), _stream())
+    """(A^-1 rhs, A^-1) from the factor held in ws (consumed); A^-1 rhs is [D, n] for D = ws.n_rhs > 1."""
+    if ws.n_rhs == 1:
+        _lib.call("asvgp_dense_selinv", _p(ws.band), ws.n, _p(ws.sig_band), _p(ws.x), _p(ws.inv), _p(ws.work), _stream())
+    else:
+        _lib.call("asvgp_dense_selinv_multi", _p(ws.band), ws.n, ws.n_rhs, _p(ws.sig_band), _p(ws.x), _p(ws.inv), _p(ws.work),
+                  _stream())
     return ws.x, ws.inv
 
 

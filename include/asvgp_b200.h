@@ -246,6 +246,28 @@ ASVGP_API int asvgp_kron_factor(const double* K1, const double* K2, const double
 ASVGP_API int asvgp_kron_selinv(double* band, int m1, int m2, int order, double* sig_band, double* x_io,
                                 double* sigma_stencil, double* work, void* stream);
 
+/* ---- several right-hand sides (multi-output targets y[N, D]) -----------------------------------------------------------------
+ * P does not depend on y: one factorisation and one selected inverse serve D = n_rhs columns b_d = Kuf y_d, which ride along
+ * as D extra boundary unknowns of every front (the root's boundary is exactly these D, one 64-wide tile).
+ *   rhs_io[n_rhs x M]: column d at d*M (input of the factor; the selected inverse overwrites it with x_d = P^-1 b_d, same layout);
+ *   scal[2 + n_rhs] = { log|P|, info, ||L^-1 b_1||^2, ..., ||L^-1 b_D||^2 } (info as for asvgp_kron_factor);
+ *   sigma_stencil: entries of P^-1 in stencil layout, as for asvgp_kron_selinv.
+ * asvgp_kron_doubles_multi: h_sizes[4] (HOST) = { band, sig, work, rhs } doubles of the buffers for this n_rhs.
+ * asvgp_kron_plan_info_multi: asvgp_kron_plan_info for this n_rhs (rhs nodes m1*m2 ... m1*m2 + n_rhs - 1, the last n_rhs
+ *   boundary ids of every front); -1 (with asvgp_last_error set) for invalid arguments.
+ * The dense twins take rhs[n_rhs x n] and return x_out[n_rhs x n] and scal in the same layouts.
+ * n_rhs lies in [1, ASVGP_MAX_RHS]: every front's boundary grows by n_rhs - 1 rows, and 32 keeps that growth within half a
+ * 64-wide tile block (and the root's boundary within one tile); anything else is rejected before any CUDA call.  With
+ * n_rhs = 1 every _multi function runs the plan and the arithmetic of its single-rhs counterpart, bit for bit. */
+#define ASVGP_MAX_RHS 32
+ASVGP_API int asvgp_kron_doubles_multi(int m1, int m2, int order, int n_rhs, int64_t* h_sizes);
+ASVGP_API int64_t asvgp_kron_plan_info_multi(int m1, int m2, int order, int n_rhs, double* out, int32_t* idx_out,
+                                             int64_t idx_capacity);
+ASVGP_API int asvgp_kron_factor_multi(const double* K1, const double* K2, const double* Gs, int m1, int m2, int order, int n_rhs,
+                                      double sigma2, double* band, double* rhs_io, double* scal, void* stream);
+ASVGP_API int asvgp_kron_selinv_multi(double* band, int m1, int m2, int order, int n_rhs, double* sig_band, double* x_io,
+                                      double* sigma_stencil, double* work, void* stream);
+
 /* asvgp_kronband_*: the same two operations on the scalar band of P in the natural order (bandwidth order*(m2+1), gpr.py:262)
  * as one tile DAG over the band (csrc/tiledag_2d.cu) — a single chain over all m1 m2 columns, 10x slower at 200 x 200; kept
  * as an independent second implementation (the tests compare the two).  Same arguments, except that rhs_io has
@@ -312,6 +334,13 @@ ASVGP_API int64_t asvgp_dense_work_doubles(int n);
 ASVGP_API int asvgp_dense_factor(const double* A, int n, const double* rhs, double* band, double* scal, void* stream);
 ASVGP_API int asvgp_dense_selinv(double* band, int n, double* sig_band, double* x_out, double* inv_out, double* work,
                                  void* stream);
+/* n_rhs right-hand sides (layouts as for asvgp_kron_factor_multi): rhs[n_rhs x n], scal[2 + n_rhs] = { log|A|, info,
+ * rhs_d^T A^-1 rhs_d ... }, x_out[n_rhs x n]; h_sizes[4] (HOST) = { band, sig, work, rhs } doubles. */
+ASVGP_API int asvgp_dense_doubles_multi(int n, int n_rhs, int64_t* h_sizes);
+ASVGP_API int asvgp_dense_factor_multi(const double* A, int n, int n_rhs, const double* rhs, double* band, double* scal,
+                                       void* stream);
+ASVGP_API int asvgp_dense_selinv_multi(double* band, int n, int n_rhs, double* sig_band, double* x_out, double* inv_out,
+                                       double* work, void* stream);
 
 /* ---- GPR_additive (gpr.py:139-236): sum of 1-D models, Kuf = stacked per-dimension features ------------------------------------------
  * asvgp_accum_cross: C[m_a x m_b] += Kuf_a Kuf_b^T for two dimensions of the same points (xa[i * stride], xb[i * stride]) — the
