@@ -29,6 +29,8 @@ SIGNATURES = {
     "asvgp_debug_poison_smem": [_vp],
     "asvgp_kuu_chain_1d": [_vp, _vp, _c_int, _c_int, _c_int, _vp, _vp, _c_i64, _vp, _vp],
     "asvgp_elbo_grad_1d_prepared": [_vp, _vp, _vp, _vp, _c_int, _c_int, _c_dbl, _c_dbl, _c_int, _vp, _vp, _c_i64, _vp, _c_int, _vp],
+    "asvgp_kuu_assemble_batched": [_vp, _c_int, _c_int, _vp, _vp, _c_int, _c_int, _vp, _vp, _vp],
+    "asvgp_elbo_grad_1d_batched": [_vp, _vp, _vp, _c_int, _c_int, _c_int, _c_int, _vp, _vp, _c_int, _vp, _vp, _c_i64, _vp],
     "asvgp_posterior_1d": [_vp, _vp, _c_int, _c_int, _c_dbl, _c_int, _vp, _vp, _vp, _vp, _c_i64, _vp],
     "asvgp_band_inverse_1d": [_vp, _vp, _c_int, _c_int, _c_int, _vp, _vp, _vp, _vp, _c_i64, _vp],
     "asvgp_accum_2d": [_vp, _vp, _c_i64, _vp, _c_int, _vp, _c_int, _c_int, _vp, _vp, _vp],
@@ -73,6 +75,7 @@ SIGNATURES = {
 VALUE_FUNCTIONS = {
     "asvgp_launch_count": (_c_i64, []),
     "asvgp_workspace_bytes_1d": (_c_i64, [_c_int, _c_int, _c_int]),
+    "asvgp_workspace_bytes_1d_batched": (_c_i64, [_c_int, _c_int, _c_int, _c_int, _c_int]),
     "asvgp_kuu_state_doubles": (_c_i64, [_c_int, _c_int]),
     "asvgp_accum_1d_binned_work_bytes": (_c_i64, [_c_i64]),
     "asvgp_accum_2d_binned_work_bytes": (_c_i64, [_c_i64]),
@@ -125,6 +128,9 @@ def load():
     _lib = lib
     return lib
 
+
+MAX_BATCH = 64              # ASVGP_MAX_BATCH / ASVGP_MAX_BATCH_COLUMNS in include/asvgp_b200.h
+MAX_BATCH_COLUMNS = 64
 
 _POISON_EVERY_CALL = os.environ.get("ASVGP_POISON_SMEM") is not None      # test aid: NaN-fill shared memory before EVERY native call
 

@@ -4,6 +4,7 @@
 //   asvgp_kuu_assemble   <- SplineFeatures1D.make_Kuu                    (reference asvgp/inducing_features.py:12-44)
 //   asvgp_elbo_grad_1d   <- GPR_1d.elbo + its TF-autodiff gradient       (reference asvgp/gpr.py:49-89, example.py:31-32)
 //   asvgp_posterior_1d   <- the factorisations/solves of GPR_1d.predict_f (reference asvgp/gpr.py:96-108)
+//   asvgp_kuu_assemble_batched, asvgp_elbo_grad_1d_batched: the first two for B hyper-parameter settings at once
 //
 // Design (DESIGN.md §4.2).  The work is O(M k^2) flops — nothing — but a length-M dependency chain of
 // sqrt/div/FMA.  Each "chain" (one SPD banded matrix) runs in ONE CTA through the partitioned engine of
@@ -42,9 +43,16 @@ struct KuuTerms {
     double dcoef[kMaxTerms];
 };
 
-__global__ void __launch_bounds__(256) kuu_assemble_kernel(const double* __restrict__ tables, KuuTerms terms,
-                                                           int64_t band_elems, double* __restrict__ Kuu,
-                                                           double* __restrict__ dKuu) {
+// One coefficient set per slot of a batch (asvgp_kuu_assemble_batched): ~12 KB of kernel parameters at ASVGP_MAX_BATCH.
+struct KuuTermsBatch {
+    int n_terms;
+    double coef[ASVGP_MAX_BATCH][kMaxTerms];
+    double dcoef[ASVGP_MAX_BATCH][kMaxTerms];
+};
+
+__device__ __forceinline__ void kuu_assemble_band(const double* __restrict__ tables, int n_terms, const double* coef,
+                                                  const double* dcoef, int64_t band_elems, double* __restrict__ Kuu,
+                                                  double* __restrict__ dKuu) {
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < band_elems;
          i += (int64_t)gridDim.x * blockDim.x) {
         // The reference's own operation order (inducing_features.py:17-44: every term `coefficient * table` rounded, then
@@ -52,14 +60,29 @@ __global__ void __launch_bounds__(256) kuu_assemble_kernel(const double* __restr
         // relative per ulp of Kuu (cond(Kuu) ~ 6e4 against 1 / sigma2), so the assembly should round where the
         // reference's does.
         double v = 0.0, dv = 0.0;
-        for (int t = 0; t < terms.n_terms; ++t) {
+        for (int t = 0; t < n_terms; ++t) {
             const double s = __ldg(tables + (int64_t)t * band_elems + i);
-            v = __dadd_rn(v, __dmul_rn(terms.coef[t], s));
-            dv = __dadd_rn(dv, __dmul_rn(terms.dcoef[t], s));
+            v = __dadd_rn(v, __dmul_rn(coef[t], s));
+            dv = __dadd_rn(dv, __dmul_rn(dcoef[t], s));
         }
         Kuu[i] = v;
         if (dKuu != nullptr) dKuu[i] = dv;
     }
+}
+
+__global__ void __launch_bounds__(256) kuu_assemble_kernel(const double* __restrict__ tables, const __grid_constant__ KuuTerms terms,
+                                                           int64_t band_elems, double* __restrict__ Kuu,
+                                                           double* __restrict__ dKuu) {
+    kuu_assemble_band(tables, terms.n_terms, terms.coef, terms.dcoef, band_elems, Kuu, dKuu);
+}
+
+// slot = blockIdx.y: the band of slot b is Kuu[b] of [B, k+1, M], entry for entry the operations of kuu_assemble_kernel
+__global__ void __launch_bounds__(256) kuu_assemble_batched_kernel(const double* __restrict__ tables, const __grid_constant__ KuuTermsBatch terms,
+                                                                   int64_t band_elems, double* __restrict__ Kuu,
+                                                                   double* __restrict__ dKuu) {
+    const int b = blockIdx.y;
+    kuu_assemble_band(tables, terms.n_terms, terms.coef[b], terms.dcoef[b], band_elems, Kuu + b * band_elems,
+                      dKuu != nullptr ? dKuu + b * band_elems : nullptr);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -187,6 +210,22 @@ __device__ __forceinline__ void trace_partial(const double* __restrict__ kstate,
     }
 }
 
+// Entry e of one chain's row table (layout above).
+template <class T, int K>
+__device__ __forceinline__ T chain_rows_entry(const ChunkLayout& lay, const ChainSpec<T>& sp, unsigned e) {
+    const unsigned n_rho = chain_n_rho(lay, K), P = lay.P;
+    const unsigned q = e / P;
+    const int p = (int)(e - q * P);
+    const int g0 = P > 1 ? lay.start(p) : 0;
+    if (q < n_rho * (K + 1)) {
+        const int rho = (int)(q / (K + 1)), bidx = (int)(q - (unsigned)rho * (K + 1));
+        const int row = g0 + rho, col = row - K + bidx;
+        return sp.A(K - bidx, col);
+    }
+    const int rho = (int)(q - n_rho * (K + 1));
+    return sp.rhs(g0 + rho);
+}
+
 template <class T, int K, int NCHAINS>
 __global__ void __launch_bounds__(256) chain_rows_kernel(ChunkLayout lay, ChainSpec<T> s0, ChainSpec<T> s1, ChainSpec<T> s2, ChainSpec<T> s3,
                                                          T* __restrict__ out, unsigned* __restrict__ zero_me = nullptr,
@@ -197,7 +236,6 @@ __global__ void __launch_bounds__(256) chain_rows_kernel(ChunkLayout lay, ChainS
         trace_partial(trace.kstate, trace.G, trace.M, trace.K, (int)blockIdx.x - trace.first_block, trace.tr_part);
         return;
     }
-    const unsigned n_rho = chain_n_rho(lay, K), P = lay.P;
     const unsigned per_chain = (unsigned)chain_rows_count<T, K>(lay);          // 32-bit index arithmetic (the launchers check the range)
     const unsigned total = per_chain * NCHAINS;
     const unsigned n_row_blocks = trace.kstate != nullptr ? (unsigned)trace.first_block : gridDim.x;
@@ -205,18 +243,39 @@ __global__ void __launch_bounds__(256) chain_rows_kernel(ChunkLayout lay, ChainS
         const unsigned chain = t / per_chain;
         const unsigned e = t - chain * per_chain;
         const ChainSpec<T>& sp = chain == 0 ? s0 : (chain == 1 ? s1 : (chain == 2 ? s2 : s3));
-        const unsigned q = e / P;
-        const int p = (int)(e - q * P);
-        const int g0 = P > 1 ? lay.start(p) : 0;
-        if (q < n_rho * (K + 1)) {
-            const int rho = (int)(q / (K + 1)), bidx = (int)(q - (unsigned)rho * (K + 1));
-            const int row = g0 + rho, col = row - K + bidx;
-            out[t] = sp.A(K - bidx, col);
-        } else {
-            const int rho = (int)(q - n_rho * (K + 1));
-            out[t] = sp.rhs(g0 + rho);
-        }
+        out[t] = chain_rows_entry<T, K>(lay, sp, e);
     }
+}
+
+// Row tables of a batch (asvgp_elbo_grad_1d_batched): blockIdx.z = slot b, blockIdx.y = chain c of the slot — 0 the Kuu
+// chain of Kuu[b], 2d+1 / 2d+2 the P chains (d/dl, d/dsigma2) of output column d — each table built with the matrix and
+// right-hand-side functors of the single call (launch_kuu_chain, launch_pchains), so every entry has the same bits.
+struct BatchRowsArgs {
+    const double* Kuu; const double* dKuu;          // [B][K+1][M]
+    const double* acc; size_t acc_stride;           // column d's packed accumulator at acc + d * acc_stride
+    unsigned* counters; size_t counter_stride;      // finalize arrival counter of (b, d) at counters + (b * D + d) * counter_stride
+    double inv_s2[ASVGP_MAX_BATCH], tan_s2[ASVGP_MAX_BATCH];   // 1 / sigma2 and -1 / sigma2^2 per slot (rounded on the host as there)
+};
+template <int K>
+__global__ void __launch_bounds__(256) batch_rows_kernel(ChunkLayout lay, const __grid_constant__ BatchRowsArgs a, Dual<1>* __restrict__ out) {
+    using T = Dual<1>;
+    pdl_launch_dependents();
+    const int M = lay.M, b = blockIdx.z, c = blockIdx.y, n_chains = gridDim.y;
+    const size_t band = (size_t)(K + 1) * M;
+    const double* Kuu = a.Kuu + b * band;
+    const double* dKuu = a.dKuu + b * band;
+    ChainSpec<T> sp{BandMat<T>{Kuu, dKuu, nullptr, 0.0, 0.0, 1, M}, VecRhs<T>{Kuu, M, 0}};
+    if (c > 0) {
+        const int d = (c - 1) >> 1;
+        const double* G = a.acc + d * a.acc_stride;
+        sp = (c & 1) ? ChainSpec<T>{BandMat<T>{Kuu, dKuu, G, a.inv_s2[b], 0.0, 1, M}, VecRhs<T>{G + band, M, 1}}
+                     : ChainSpec<T>{BandMat<T>{Kuu, dKuu, G, a.inv_s2[b], a.tan_s2[b], 0, M}, VecRhs<T>{G + band, M, 1}};
+        if ((c & 1) && blockIdx.x == 0 && threadIdx.x == 0) a.counters[((size_t)b * (n_chains >> 1) + d) * a.counter_stride] = 0u;
+    }
+    const unsigned per_chain = (unsigned)chain_rows_count<T, K>(lay);
+    T* tab = out + ((size_t)b * n_chains + c) * per_chain;
+    for (unsigned e = blockIdx.x * blockDim.x + threadIdx.x; e < per_chain; e += gridDim.x * blockDim.x)
+        tab[e] = chain_rows_entry<T, K>(lay, sp, e);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -414,40 +473,60 @@ __device__ __forceinline__ void run_chain_cluster(const ChunkLayout& lay, const 
 //   P chains   (chains 1, 2: [P, d/dl], [P, d/dsigma2], forward only) need G and b;
 //   finalize   trace(Kuu^-1 G) = sum band(Kuu^-1) .* band(G) (off-diagonals twice, reference gpr.py:60-70) as a fixed-order
 //              dot product of the stored inverse band with G, then the bound and its derivatives.
+// per-launch record area: [2][16] chain records, the finalize kernel's arrival counter (double slot 32), the [kTraceBlocks][2]
+// trace partials (from slot 64); one per output column of every slot in a batch
+constexpr size_t kPartialBytes = 2048, kPartialDoubles = kPartialBytes / sizeof(double);
+
+// Chains of every slot of a batch (blockIdx.y; one slot outside asvgp_elbo_grad_1d_batched) in one launch.  Chain c of a slot is
+// 0: the Kuu chain;  2d+1: P of output column d with tangent d/dl;  2d+2: the same P with tangent d/dsigma2.
+// A launch runs chains first_chain .. first_chain + n_chains - 1 of each slot, launched chain i = slot * n_chains + (c - first_chain).
 template <int K>
 struct ElboArgs {
     ChunkLayout lay;
-    int first_chain;                        // 0: the Kuu chain alone;  1: the two P chains
-    ColumnStore<Dual<1>, K, true> cols[2];  // per launched chain
-    double* partial[2];                     // per launched chain [16]: logdet, dlogdet, quad, dquad, -, -, info, -, clocks[4]
-    const Dual<1>* rows;                    // lane-interleaved row tables of the launched chains (chain_rows_kernel)
-    Dual<1>* kinv;                          // Kuu chain: where band(Kuu^-1) goes, (K+1) x M
+    int first_chain, n_chains;
+    char* cols; size_t cols_bytes;          // launched chain i's column store at cols + i * cols_bytes
+    const Dual<1>* rows;                    // and its lane-interleaved row table at rows + i * chain_rows_count
+    Dual<1>* red_scratch;                   // and its reduced-solution scratch at red_scratch + i * red_scratch_count (clusters)
+    double* kstate; size_t kstate_stride;   // slot's Kuu state: the Kuu chain's [16] record, then band(Kuu^-1) (K+1) x M duals
+    double* partial; size_t partial_stride; // slot's P-chain records ([16]: logdet, dlogdet, quad, dquad, -, -, info, -, clocks[4]):
+                                            // column d at partial + slot * partial_stride + d * kPartialDoubles, + 16 for d/dsigma2
+    __device__ __forceinline__ int launched(int slot, int c) const { return slot * n_chains + c; }
+    __device__ __forceinline__ double* record(int slot, int chain) const {
+        if (chain == 0) return kstate + slot * kstate_stride;
+        return partial + slot * partial_stride + ((chain - 1) >> 1) * kPartialDoubles + 16 * ((chain - 1) & 1);
+    }
+    __device__ __forceinline__ Dual<1>* kinv(int slot) const { return reinterpret_cast<Dual<1>*>(kstate + slot * kstate_stride + 16); }
 };
+template <class T, int K>
+__device__ __forceinline__ ColumnStore<T, K, true> launched_cols(const ChunkLayout& lay, char* cols, size_t cols_bytes, int i) {
+    return ColumnStore<T, K, true>{reinterpret_cast<T*>(cols + (size_t)i * cols_bytes), lay.max_size(), lay.P};
+}
 
 template <int K>
 __global__ void __launch_bounds__(kChainThreads) elbo_chains_kernel(ElboArgs<K> a) {
     using T = Dual<1>;
     extern __shared__ __align__(16) char smem[];
-    const int slot = blockIdx.x, chain = a.first_chain + slot, p = threadIdx.x;
+    const int slot = blockIdx.y, chain = a.first_chain + blockIdx.x, li = a.launched(slot, blockIdx.x), p = threadIdx.x;
     const ChunkLayout lay = a.lay;
     const int M = lay.M;
     __shared__ ChainTotals<T, K> tot;
     __shared__ long long clk[4];
-    double* out = a.partial[slot];
+    double* out = a.record(slot, chain);
+    const ColumnStore<T, K, true> cols = launched_cols<T, K>(lay, a.cols, a.cols_bytes, li);
     pdl_launch_dependents();
     pdl_wait();                              // the row tables are complete
 
     const int n_rho = chain_n_rho(lay, K), g0 = lay.P > 1 ? lay.start(p < lay.P ? p : 0) : 0, pp = p < lay.P ? p : 0;
-    const T* tab = a.rows + (size_t)slot * chain_rows_count<T, K>(lay);
+    const T* tab = a.rows + (size_t)li * chain_rows_count<T, K>(lay);
     const RowsMat<T, K> A{tab, g0, lay.P, pp, n_rho};
     const RowsRhs<T> rhs{tab + (size_t)n_rho * (K + 1) * lay.P, g0, lay.P, pp, n_rho};
     if (chain == 0) {
-        BandSink<T> sink{a.kinv, M};
-        run_chain<T, K, true, false, true>(lay, a.cols[slot], smem, A, rhs, static_cast<T*>(nullptr), sink, &tot, clk);
+        BandSink<T> sink{a.kinv(slot), M};
+        run_chain<T, K, true, false, true>(lay, cols, smem, A, rhs, static_cast<T*>(nullptr), sink, &tot, clk);
     } else {
-        // chain 1: P with tangent d/dl;  chain 2: P with tangent d/dsigma2 (tables built by the launcher)
+        // P with tangent d/dl or d/dsigma2 (tables built by the launcher)
         BandSink<T> no_sink{nullptr, M};
-        run_chain<T, K, false, false, false>(lay, a.cols[slot], smem, A, rhs, static_cast<T*>(nullptr), no_sink, &tot, clk);
+        run_chain<T, K, false, false, false>(lay, cols, smem, A, rhs, static_cast<T*>(nullptr), no_sink, &tot, clk);
     }
     if (p == 0) {
         out[0] = tot.logdet.v; out[1] = tot.logdet.d[0];
@@ -461,28 +540,30 @@ __global__ void __launch_bounds__(kChainThreads) elbo_chains_kernel(ElboArgs<K> 
 
 // Cluster version (M large): launched chain `slot` runs on cluster `slot` of NCTA CTAs with 128 * NCTA chunks.
 template <int K, int NCTA>
-__global__ void __cluster_dims__(NCTA, 1, 1) __launch_bounds__(kChainThreads) elbo_chains_cluster_kernel(ElboArgs<K> a, Dual<1>* red_scratch) {
+__global__ void __cluster_dims__(NCTA, 1, 1) __launch_bounds__(kChainThreads) elbo_chains_cluster_kernel(ElboArgs<K> a) {
     using T = Dual<1>;
     extern __shared__ __align__(16) char smem[];
-    const int slot = blockIdx.x / NCTA, chain = a.first_chain + slot, rank = blockIdx.x % NCTA, tid = threadIdx.x;
+    const int slot = blockIdx.y, c = blockIdx.x / NCTA, chain = a.first_chain + c, li = a.launched(slot, c);
+    const int rank = blockIdx.x % NCTA, tid = threadIdx.x;
     const ChunkLayout lay = a.lay;
     __shared__ ChainTotals<T, K> tot;
     __shared__ long long clk[4];
-    double* out = a.partial[slot];
+    double* out = a.record(slot, chain);
+    const ColumnStore<T, K, true> cols = launched_cols<T, K>(lay, a.cols, a.cols_bytes, li);
     pdl_launch_dependents();
     pdl_wait();                              // the row tables are complete
     const int n_rho = chain_n_rho(lay, K);
-    const T* tab = a.rows + (size_t)slot * chain_rows_count<T, K>(lay);
-    T* scratch = red_scratch + (size_t)slot * ((size_t)(2 * K + 1) * lay.n_reduced() + 8);
+    const T* tab = a.rows + (size_t)li * chain_rows_count<T, K>(lay);
+    T* scratch = a.red_scratch + (size_t)li * ((size_t)(2 * K + 1) * lay.n_reduced() + 8);
     auto g0_of = [&](int lane) { return lay.P > 1 ? lay.start(lane) : 0; };
     auto make_A = [&](int lane) { return RowsMat<T, K>{tab, g0_of(lane), lay.P, lane, n_rho}; };
     auto make_rhs = [&](int lane) { return RowsRhs<T>{tab + (size_t)n_rho * (K + 1) * lay.P, g0_of(lane), lay.P, lane, n_rho}; };
     if (chain == 0) {
-        auto make_sink = [&](int) { return BandSink<T>{a.kinv, lay.M}; };
-        run_chain_cluster<T, K, true, false, true>(lay, a.cols[slot], smem, scratch, make_A, make_rhs, make_sink, static_cast<T*>(nullptr), &tot, clk);
+        auto make_sink = [&](int) { return BandSink<T>{a.kinv(slot), lay.M}; };
+        run_chain_cluster<T, K, true, false, true>(lay, cols, smem, scratch, make_A, make_rhs, make_sink, static_cast<T*>(nullptr), &tot, clk);
     } else {
         auto make_sink = [&](int) { return BandSink<T>{nullptr, lay.M}; };
-        run_chain_cluster<T, K, false, false, false>(lay, a.cols[slot], smem, scratch, make_A, make_rhs, make_sink, static_cast<T*>(nullptr), &tot, clk);
+        run_chain_cluster<T, K, false, false, false>(lay, cols, smem, scratch, make_A, make_rhs, make_sink, static_cast<T*>(nullptr), &tot, clk);
     }
     if (rank == 0 && tid == 0) {
         out[0] = tot.logdet.v; out[1] = tot.logdet.d[0];
@@ -501,18 +582,19 @@ __global__ void __cluster_dims__(NCTA, 1, 1) __launch_bounds__(kChainThreads) el
 //   dlog|P|/dv = -M/v - (s2/v) dlog|P|/ds2,   dQ/dv = Q/v - (s2/v) dQ/ds2,   dlog|Kuu|/dv = -M/v,   dtr/dv = tr/v.
 // trace_done = 0: launched with kTraceBlocks CTAs that compute the trace partials first (trace_partial); the CTA that arrives
 // last combines.  trace_done = 1: the partials are there already (the P chains' chain_rows_kernel hosted the trace CTAs), one CTA.
-__global__ void __launch_bounds__(kTraceThreads) elbo_finalize_kernel(const double* __restrict__ kstate, double* __restrict__ partial,
-                                                                      const double* __restrict__ G, const double* __restrict__ scal,
-                                                                      int M, int K, double variance, double sigma2, int trace_done,
-                                                                      double* __restrict__ out) {
+// One bound: `block` is this CTA's trace share (trace_done = 0, kTraceBlocks CTAs per bound), the sums are the same whichever
+// CTA arrives last.
+__device__ __forceinline__ void elbo_finalize(const double* __restrict__ kstate, double* __restrict__ partial,
+                                              const double* __restrict__ G, const double* __restrict__ scal,
+                                              int M, int K, double variance, double sigma2, int trace_done, int block,
+                                              double* __restrict__ out) {
     double* tr_part = partial + 64;                                     // [kTraceBlocks][2]
-    unsigned* counter = reinterpret_cast<unsigned*>(partial + 32);      // zeroed by the P chains' chain_rows_kernel
-    pdl_wait();                                                         // the P chains are complete
+    unsigned* counter = reinterpret_cast<unsigned*>(partial + 32);      // zeroed by the P chains' row-table kernel
     if (!trace_done) {
-        trace_partial(kstate, G, M, K, (int)blockIdx.x, tr_part);
+        trace_partial(kstate, G, M, K, block, tr_part);
         if (threadIdx.x != 0) return;
         __threadfence();
-        if (atomicAdd(counter, 1u) != gridDim.x - 1) return;
+        if (atomicAdd(counter, 1u) != kTraceBlocks - 1) return;
         __threadfence();
     } else if (threadIdx.x != 0) {
         return;
@@ -547,6 +629,30 @@ __global__ void __launch_bounds__(kTraceThreads) elbo_finalize_kernel(const doub
     out[9] = cK[8]; out[10] = cK[9]; out[11] = cK[10]; out[12] = cK[11];
     out[13] = cL[8]; out[14] = cL[9];
     out[15] = dtr_dl;             // d trace(Kuu^-1 G) / d lengthscale (multi-output bound: trace terms count once)
+}
+
+__global__ void __launch_bounds__(kTraceThreads) elbo_finalize_kernel(const double* __restrict__ kstate, double* __restrict__ partial,
+                                                                      const double* __restrict__ G, const double* __restrict__ scal,
+                                                                      int M, int K, double variance, double sigma2, int trace_done,
+                                                                      double* __restrict__ out) {
+    pdl_wait();                                                         // the P chains are complete
+    elbo_finalize(kstate, partial, G, scal, M, K, variance, sigma2, trace_done, (int)blockIdx.x, out);
+}
+
+// The bounds of a batch: blockIdx.z = slot b, blockIdx.y = output column d, kTraceBlocks CTAs each; out[b][d][16].
+struct BatchFinalizeArgs {
+    const double* kstate; size_t kstate_stride;
+    double* partial; size_t partial_stride;          // as ElboArgs
+    const double* acc; size_t acc_stride;
+    double variance[ASVGP_MAX_BATCH], sigma2[ASVGP_MAX_BATCH];
+};
+__global__ void __launch_bounds__(kTraceThreads) elbo_finalize_batched_kernel(const __grid_constant__ BatchFinalizeArgs a, int M, int K,
+                                                                              double* __restrict__ out) {
+    pdl_wait();                                                         // every chain of the batch is complete
+    const int b = blockIdx.z, d = blockIdx.y, D = gridDim.y;
+    const double* G = a.acc + d * a.acc_stride;
+    elbo_finalize(a.kstate + b * a.kstate_stride, a.partial + b * a.partial_stride + d * kPartialDoubles, G, G + (size_t)(K + 2) * M,
+                  M, K, a.variance[b], a.sigma2[b], 0, (int)blockIdx.x, out + ((size_t)b * D + d) * 16);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -666,9 +772,9 @@ static size_t align256(size_t n) { return (n + 255) & ~(size_t)255; }
 // park in pdl_wait() until that grid has completed and flushed), which takes the launch latency and the cluster's
 // co-scheduling off the chain of three dependent launches (row tables -> chains -> bound).
 template <class... KArgs, class... Args>
-static cudaError_t launch_dependent(void (*kernel)(KArgs...), int grid, int block, size_t smem, cudaStream_t st, bool pdl, Args... args) {
+static cudaError_t launch_dependent(void (*kernel)(KArgs...), dim3 grid, int block, size_t smem, cudaStream_t st, bool pdl, Args... args) {
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(block); cfg.dynamicSmemBytes = smem; cfg.stream = st;
+    cfg.gridDim = grid; cfg.blockDim = dim3(block); cfg.dynamicSmemBytes = smem; cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
@@ -685,8 +791,6 @@ static cudaError_t allow_smem(Kernel kernel, size_t smem) {
     if (e == cudaSuccess) { allowed = smem; which = reinterpret_cast<const void*>(kernel); }
     return e;
 }
-// per-launch record area: [2][16] chain records, the finalize kernel's arrival counter (double slot 32), the [kTraceBlocks][2] trace partials (from slot 64)
-constexpr size_t kPartialBytes = 2048;
 template <int K>
 static size_t red_scratch_count(const ChunkLayout& lay) { return (size_t)(2 * K + 1) * lay.n_reduced() + 8; }     // per chain (clustered layout)
 // workspace of one launch of n_chains chains: column stores, [n_chains][16] partials, row tables, reduced-solution scratch
@@ -706,31 +810,62 @@ static size_t posterior_work_bytes(const ChunkLayout& lay) {
            + 256 + (((size_t)lay.M * sizeof(double) + 255) & ~(size_t)255) + 2 * chain_rows_count<double, K>(lay) * sizeof(double) + 256;
 }
 
+// The chain kernel of `a` for `n_slots` slots (blockIdx.y): one CTA per chain, or a cluster of lay.P / 128 CTAs
+// (pick_layout_elbo).  smem_floor: see launch_chain_group.
+template <int K>
+static int launch_chains(const ElboArgs<K>& a, int n_slots, size_t smem_floor, bool pdl, cudaStream_t st) {
+    using T = Dual<1>;
+    const ChunkLayout& lay = a.lay;
+    const int n_cta = (lay.P + kChainThreads - 1) / kChainThreads;          // > 1: clustered layout
+    if (n_cta > 1) {
+        const size_t smem = std::max(ChainSmall<T, K>::bytes(kChainThreads + 1), smem_floor);
+        const dim3 grid(a.n_chains * n_cta, n_slots);
+        if (n_cta == 2) {
+            ASVGP_CUDA_OK(allow_smem(elbo_chains_cluster_kernel<K, 2>, smem));
+            ASVGP_CUDA_OK(launch_dependent(elbo_chains_cluster_kernel<K, 2>, grid, kChainThreads, smem, st, pdl, a));
+        } else if (n_cta == 8) {
+            ASVGP_CUDA_OK(allow_smem(elbo_chains_cluster_kernel<K, 8>, smem));
+            ASVGP_CUDA_OK(launch_dependent(elbo_chains_cluster_kernel<K, 8>, grid, kChainThreads, smem, st, pdl, a));
+        } else {
+            ASVGP_CUDA_OK(allow_smem(elbo_chains_cluster_kernel<K, 4>, smem));
+            ASVGP_CUDA_OK(launch_dependent(elbo_chains_cluster_kernel<K, 4>, grid, kChainThreads, smem, st, pdl, a));
+        }
+    } else {
+        const size_t smem = std::max(ChainSmall<T, K>::bytes(lay.P), smem_floor);
+        ASVGP_CUDA_OK(allow_smem(elbo_chains_kernel<K>, smem));
+        ASVGP_CUDA_OK(launch_dependent(elbo_chains_kernel<K>, dim3(a.n_chains, n_slots), kChainThreads, smem, st, pdl, a));
+    }
+    ASVGP_LAUNCHED();
+    ASVGP_CUDA_OK(cudaGetLastError());
+    return kOk;
+}
+
 // Row tables + chain kernel of `n_chains` chains starting at chain `first_chain` (0: Kuu; 1, 2: P with d/dl, d/dsigma2).
-// `partial0` overrides where the first chain's 16-slot record goes (the Kuu state's header); returns the partials in work.
+// `kstate` receives the Kuu chain's record and band(Kuu^-1); returns the P chains' partials in work.
 template <int K>
 static int launch_chain_group(const ChunkLayout& lay, int first_chain, int n_chains, const ChainSpec<Dual<1>>& s0,
-                              const ChainSpec<Dual<1>>& s1, double* partial0, Dual<1>* kinv, char* work, double** partials_out,
+                              const ChainSpec<Dual<1>>& s1, double* kstate, char* work, double** partials_out,
                               cudaEvent_t gate, TraceJob trace, cudaStream_t st) {
     using T = Dual<1>;
     ElboArgs<K> a;
     a.lay = lay;
     a.first_chain = first_chain;
-    a.kinv = kinv;
+    a.n_chains = n_chains;
     char* p = work;
-    for (int c = 0; c < 2; ++c) {
-        a.cols[c] = ChainPlan<T, K>::carve(lay, c < n_chains ? p : work);
-        if (c < n_chains) p += ChainPlan<T, K>::bytes(lay);
-    }
+    a.cols = p;
+    a.cols_bytes = ChainPlan<T, K>::bytes(lay);
+    p += n_chains * a.cols_bytes;
     double* partial = reinterpret_cast<double*>(p);
     p += kPartialBytes;
-    a.partial[0] = partial0 != nullptr ? partial0 : partial;
-    a.partial[1] = partial + 16;
+    a.kstate = kstate;
+    a.kstate_stride = 0;
+    a.partial = partial;
+    a.partial_stride = 0;
     if (partials_out != nullptr) *partials_out = partial;
     T* rows = reinterpret_cast<T*>(p);
     p += align256(n_chains * chain_rows_count<T, K>(lay) * sizeof(T));
     a.rows = rows;
-    T* scratch = reinterpret_cast<T*>(p);
+    a.red_scratch = reinterpret_cast<T*>(p);
     const size_t total = n_chains * chain_rows_count<T, K>(lay);
     ASVGP_REQUIRE(total < ((size_t)1 << 31), "banded chains: %zu row-table entries exceed the 32-bit index range", total);
     const int grid = (int)std::min<size_t>((total + 255) / 256, 148 * 8);
@@ -745,32 +880,12 @@ static int launch_chain_group(const ChunkLayout& lay, int first_chain, int n_cha
     ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     if (gate != nullptr) ASVGP_CUDA_OK(cudaEventRecord(gate, st));          // "the chain kernel is next in line"
-    const int n_cta = (lay.P + kChainThreads - 1) / kChainThreads;          // > 1: clustered layout (pick_layout_elbo)
-    const bool pdl = gate == nullptr;        // an event record between the two launches rules the early launch out
     // A gated chain runs BESIDE a streaming kernel whose CTAs all carry the same share of the work: one of them landing on a
     // chain SM (shared issue slots, the L1 invalidation of every cluster barrier) becomes the straggler the whole kernel waits
     // for (+12 % on the accumulate, measured).  Asking for all of the SM's shared memory keeps the chain's SMs to itself.
     const size_t smem_floor = gate != nullptr ? (size_t)(227 * 1024 - 2048) : 0;
-    if (n_cta > 1) {
-        const size_t smem = std::max(ChainSmall<T, K>::bytes(kChainThreads + 1), smem_floor);
-        if (n_cta == 2) {
-            ASVGP_CUDA_OK(allow_smem(elbo_chains_cluster_kernel<K, 2>, smem));
-            ASVGP_CUDA_OK(launch_dependent(elbo_chains_cluster_kernel<K, 2>, n_chains * 2, kChainThreads, smem, st, pdl, a, scratch));
-        } else if (n_cta == 8) {
-            ASVGP_CUDA_OK(allow_smem(elbo_chains_cluster_kernel<K, 8>, smem));
-            ASVGP_CUDA_OK(launch_dependent(elbo_chains_cluster_kernel<K, 8>, n_chains * 8, kChainThreads, smem, st, pdl, a, scratch));
-        } else {
-            ASVGP_CUDA_OK(allow_smem(elbo_chains_cluster_kernel<K, 4>, smem));
-            ASVGP_CUDA_OK(launch_dependent(elbo_chains_cluster_kernel<K, 4>, n_chains * 4, kChainThreads, smem, st, pdl, a, scratch));
-        }
-    } else {
-        const size_t smem = std::max(ChainSmall<T, K>::bytes(lay.P), smem_floor);
-        ASVGP_CUDA_OK(allow_smem(elbo_chains_kernel<K>, smem));
-        ASVGP_CUDA_OK(launch_dependent(elbo_chains_kernel<K>, n_chains, kChainThreads, smem, st, pdl, a));
-    }
-    ASVGP_LAUNCHED();
-    ASVGP_CUDA_OK(cudaGetLastError());
-    return kOk;
+    // an event record between the two launches rules the early launch out
+    return launch_chains<K>(a, 1, smem_floor, gate == nullptr, st);
 }
 
 // The Kuu chain: log|Kuu|, its d/dl and band(Kuu^-1) with tangent into `kstate` ([16] record + (K+1) x M duals).
@@ -780,8 +895,7 @@ static int launch_kuu_chain(const ChunkLayout& lay, const double* Kuu, const dou
     using T = Dual<1>;
     const int M = lay.M;
     ChainSpec<T> s0{BandMat<T>{Kuu, dKuu, nullptr, 0.0, 0.0, 1, M}, VecRhs<T>{Kuu, M, 0}};
-    return launch_chain_group<K>(lay, 0, 1, s0, s0, kstate, reinterpret_cast<T*>(kstate + 16), work, nullptr, gate,
-                                 TraceJob{nullptr, nullptr, nullptr, 0, 0, 0}, st);
+    return launch_chain_group<K>(lay, 0, 1, s0, s0, kstate, work, nullptr, gate, TraceJob{nullptr, nullptr, nullptr, 0, 0, 0}, st);
 }
 
 // The two P chains and the bound, given the Kuu state.
@@ -801,7 +915,7 @@ static int launch_pchains(const ChunkLayout& lay, const double* kstate, const do
     // join_late = 1: the Kuu chain may still be running beside us — join only where its state is first read, after the P chains.
     if (!join_late && kuu_ready != nullptr) ASVGP_CUDA_OK(cudaStreamWaitEvent(st, kuu_ready, 0));
     const TraceJob trace{join_late ? nullptr : kstate, G, nullptr, M, K, 0};
-    if (int rc = launch_chain_group<K>(lay, 1, 2, s1, s2, nullptr, nullptr, work, &partial, nullptr, trace, st)) return rc;
+    if (int rc = launch_chain_group<K>(lay, 1, 2, s1, s2, nullptr, work, &partial, nullptr, trace, st)) return rc;
     if (join_late && kuu_ready != nullptr) ASVGP_CUDA_OK(cudaStreamWaitEvent(st, kuu_ready, 0));
     const bool pdl = !(join_late && kuu_ready != nullptr);       // nothing between the chain kernel and this launch
     ASVGP_CUDA_OK(launch_dependent(elbo_finalize_kernel, join_late ? kTraceBlocks : 1, kTraceThreads, 0, st, pdl, kstate, partial, G,
@@ -818,6 +932,73 @@ static int launch_elbo(const ChunkLayout& lay, const double* Kuu, const double* 
     char* pwork = work + chains_work_bytes<K>(lay, 1) + align256(kuu_state_doubles(lay.M, K) * sizeof(double));
     if (int rc = launch_kuu_chain<K>(lay, Kuu, dKuu, kstate, work, nullptr, st)) return rc;
     return launch_pchains<K>(lay, kstate, Kuu, dKuu, acc, variance, sigma2, out, pwork, nullptr, 0, st);
+}
+
+// Workspace of a batch of B slots with D output columns: per chain (B (1 + 2D) of them) a column store, a row table and
+// reduced-solution scratch; per slot a Kuu state; per (slot, column) a record area.
+template <int K>
+struct BatchPlan {
+    size_t cols_bytes, rows_off, scratch_off, kstate_off, kstate_stride, partial_off, total;
+    BatchPlan(const ChunkLayout& lay, int B, int D) {
+        const size_t n = (size_t)B * (1 + 2 * D);
+        cols_bytes = ChainPlan<Dual<1>, K>::bytes(lay);
+        rows_off = n * cols_bytes;
+        scratch_off = rows_off + align256(n * chain_rows_count<Dual<1>, K>(lay) * sizeof(Dual<1>));
+        kstate_off = scratch_off + align256(n * red_scratch_count<K>(lay) * sizeof(Dual<1>));
+        kstate_stride = align256(kuu_state_doubles(lay.M, K) * sizeof(double)) / sizeof(double);
+        partial_off = kstate_off + (size_t)B * kstate_stride * sizeof(double);
+        total = partial_off + (size_t)B * D * kPartialBytes;
+    }
+};
+
+// B bounds with D output columns each in three launches: the row tables of every chain, every chain (the Kuu chains beside the
+// P chains: these read Kuu, not the Kuu state), the trace and the bound of every (slot, column).  Each chain, trace share and
+// bound runs the code of the single call on its own workspace, so slot b's bits depend neither on B nor on the other slots.
+template <int K>
+static int launch_elbo_batched(const ChunkLayout& lay, int B, int D, const double* Kuu, const double* dKuu, const double* acc,
+                               const double* h_variance, const double* h_sigma2, double* out, char* work, cudaStream_t st) {
+    using T = Dual<1>;
+    const BatchPlan<K> plan(lay, B, D);
+    const int M = lay.M;
+    const size_t acc_stride = (size_t)(K + 2) * M + 2;
+    const size_t per_chain = chain_rows_count<T, K>(lay);
+    ASVGP_REQUIRE(per_chain < ((size_t)1 << 31), "banded chains: %zu row-table entries exceed the 32-bit index range", per_chain);
+    ElboArgs<K> a;
+    a.lay = lay;
+    a.first_chain = 0;
+    a.n_chains = 1 + 2 * D;
+    a.cols = work;
+    a.cols_bytes = plan.cols_bytes;
+    a.rows = reinterpret_cast<T*>(work + plan.rows_off);
+    a.red_scratch = reinterpret_cast<T*>(work + plan.scratch_off);
+    a.kstate = reinterpret_cast<double*>(work + plan.kstate_off);
+    a.kstate_stride = plan.kstate_stride;
+    a.partial = reinterpret_cast<double*>(work + plan.partial_off);
+    a.partial_stride = (size_t)D * kPartialDoubles;
+
+    BatchRowsArgs r;
+    r.Kuu = Kuu; r.dKuu = dKuu; r.acc = acc; r.acc_stride = acc_stride;
+    r.counters = reinterpret_cast<unsigned*>(a.partial + 32);
+    r.counter_stride = kPartialBytes / sizeof(unsigned);
+    for (int b = 0; b < B; ++b) {
+        const double inv_s2 = 1.0 / h_sigma2[b];       // as launch_pchains
+        r.inv_s2[b] = inv_s2;
+        r.tan_s2[b] = -inv_s2 * inv_s2;
+    }
+    const int n_tables = a.n_chains * B;
+    const int gx = (int)std::min<size_t>((per_chain + 255) / 256, std::max(1, 148 * 8 / n_tables));
+    batch_rows_kernel<K><<<dim3(gx, a.n_chains, B), 256, 0, st>>>(lay, r, reinterpret_cast<T*>(work + plan.rows_off)); ASVGP_LAUNCHED();
+    ASVGP_CUDA_OK(cudaGetLastError());
+    if (int rc = launch_chains<K>(a, B, 0, true, st)) return rc;
+    BatchFinalizeArgs f;
+    f.kstate = a.kstate; f.kstate_stride = a.kstate_stride;
+    f.partial = a.partial; f.partial_stride = a.partial_stride;
+    f.acc = acc; f.acc_stride = acc_stride;
+    for (int b = 0; b < B; ++b) { f.variance[b] = h_variance[b]; f.sigma2[b] = h_sigma2[b]; }
+    ASVGP_CUDA_OK(launch_dependent(elbo_finalize_batched_kernel, dim3(kTraceBlocks, D, B), kTraceThreads, 0, st, true, f, M, K, out));
+    ASVGP_LAUNCHED();
+    ASVGP_CUDA_OK(cudaGetLastError());
+    return kOk;
 }
 
 template <int K>
@@ -927,18 +1108,47 @@ extern "C" int asvgp_kuu_assemble(const double* tables, int n_terms, const doubl
     return kOk;
 }
 
-extern "C" int64_t asvgp_workspace_bytes_1d(int M, int order, int chunks) {
-    if (M <= 0 || order < 1 || order > kMaxOrder) return -1;
+extern "C" int asvgp_kuu_assemble_batched(const double* tables, int n_terms, int B, const double* h_coef, const double* h_dcoef,
+                                          int M, int order, double* Kuu, double* dKuu, void* stream) {
+    ASVGP_REQUIRE(n_terms >= 1 && n_terms <= kMaxTerms, "kuu_assemble_batched: n_terms=%d not in 1..%d", n_terms, kMaxTerms);
+    ASVGP_REQUIRE(B >= 1 && B <= ASVGP_MAX_BATCH, "kuu_assemble_batched: B=%d not in 1..%d", B, ASVGP_MAX_BATCH);
+    ASVGP_REQUIRE(M > 0 && order >= 1 && order <= kMaxOrder, "kuu_assemble_batched: M=%d order=%d", M, order);
+    ASVGP_REQUIRE(h_coef != nullptr, "kuu_assemble_batched: h_coef is NULL");
+    KuuTermsBatch t;
+    t.n_terms = n_terms;
+    for (int b = 0; b < B; ++b)
+        for (int i = 0; i < n_terms; ++i) {
+            t.coef[b][i] = h_coef[b * n_terms + i];
+            t.dcoef[b][i] = h_dcoef ? h_dcoef[b * n_terms + i] : 0.0;
+        }
+    const int64_t elems = (int64_t)(order + 1) * M;
+    const dim3 grid((unsigned)((elems + 255) / 256), B);
+    kuu_assemble_batched_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(tables, t, elems, Kuu, dKuu); ASVGP_LAUNCHED();
+    ASVGP_CUDA_OK(cudaGetLastError());
+    return kOk;
+}
+
+// Every layout pick_layout_elbo may choose for (M, order, chunks) (ASVGP_CHAIN_CTAS can change it between calls); cand[0] is
+// the single-CTA layout of pick_layout.
+static int elbo_layout_candidates(int M, int order, int chunks, ChunkLayout cand[4]) {
     const ChunkLayout lay = pick_layout(M, order, chunks > kChainThreads ? 0 : chunks);
-    // the ELBO chains may run on a clustered layout (pick_layout_elbo; ASVGP_CHAIN_CTAS): size for every candidate
-    ChunkLayout cand[4] = {lay, lay, lay, lay};
-    int n_cand = 1;
+    int n_cand = 0;
+    cand[n_cand++] = lay;
     if ((chunks == 0 || chunks == 2 * kChainThreads || chunks == 4 * kChainThreads || chunks == 8 * kChainThreads) && lay.P >= kChainThreads) {
         const int P = M / (2 * (order + 1) + 1);
         if (P >= 2 * kChainThreads) cand[n_cand++] = make_layout(M, order, 2 * kChainThreads);
         if (P >= 4 * kChainThreads) cand[n_cand++] = make_layout(M, order, 4 * kChainThreads);
         if (P >= 8 * kChainThreads) cand[n_cand++] = make_layout(M, order, 8 * kChainThreads);
     }
+    return n_cand;
+}
+
+extern "C" int64_t asvgp_workspace_bytes_1d(int M, int order, int chunks) {
+    if (M <= 0 || order < 1 || order > kMaxOrder) return -1;
+    // the ELBO chains may run on a clustered layout (pick_layout_elbo; ASVGP_CHAIN_CTAS): size for every candidate
+    ChunkLayout cand[4];
+    const int n_cand = elbo_layout_candidates(M, order, chunks, cand);
+    const ChunkLayout lay = cand[0];
     size_t e = 0, p = 0;
     for (int c = 0; c < n_cand; ++c) {
         size_t ec = 0;
@@ -955,6 +1165,26 @@ extern "C" int64_t asvgp_workspace_bytes_1d(int M, int order, int chunks) {
     return (int64_t)(e > p ? e : p);
 }
 
+extern "C" int64_t asvgp_workspace_bytes_1d_batched(int M, int order, int chunks, int B, int D) {
+    if (M <= 0 || order < 1 || order > kMaxOrder || B < 1 || B > ASVGP_MAX_BATCH || D < 1 || D > ASVGP_MAX_BATCH_COLUMNS) return -1;
+    ChunkLayout cand[4];
+    const int n_cand = elbo_layout_candidates(M, order, chunks, cand);
+    size_t e = 0;
+    for (int c = 0; c < n_cand; ++c) {
+        size_t ec = 0;
+        switch (order) {
+            case 1: ec = BatchPlan<1>(cand[c], B, D).total; break;
+            case 2: ec = BatchPlan<2>(cand[c], B, D).total; break;
+            case 3: ec = BatchPlan<3>(cand[c], B, D).total; break;
+            case 4: ec = BatchPlan<4>(cand[c], B, D).total; break;
+            case 5: ec = BatchPlan<5>(cand[c], B, D).total; break;
+            case 6: ec = BatchPlan<6>(cand[c], B, D).total; break;
+        }
+        e = ec > e ? ec : e;
+    }
+    return (int64_t)e;
+}
+
 extern "C" int asvgp_elbo_grad_1d(const double* Kuu, const double* dKuu, const double* acc, int M, int order,
                                   double variance, double sigma2, int chunks, double* out, void* work,
                                   int64_t work_bytes, void* stream) {
@@ -965,6 +1195,24 @@ extern "C" int asvgp_elbo_grad_1d(const double* Kuu, const double* dKuu, const d
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     ASVGP_DISPATCH_ORDER(order, { if (int rc = launch_elbo<K>(lay, Kuu, dKuu, acc, variance, sigma2, out,
                                                               static_cast<char*>(work), st)) return rc; });
+    return kOk;
+}
+
+extern "C" int asvgp_elbo_grad_1d_batched(const double* Kuu, const double* dKuu, const double* acc, int M, int order, int B, int D,
+                                          const double* h_variance, const double* h_sigma2, int chunks, double* out, void* work,
+                                          int64_t work_bytes, void* stream) {
+    ASVGP_REQUIRE(M > 2 * order && order >= 1 && order <= kMaxOrder, "elbo_grad_1d_batched: M=%d order=%d", M, order);
+    ASVGP_REQUIRE(B >= 1 && B <= ASVGP_MAX_BATCH, "elbo_grad_1d_batched: B=%d not in 1..%d", B, ASVGP_MAX_BATCH);
+    ASVGP_REQUIRE(D >= 1 && D <= ASVGP_MAX_BATCH_COLUMNS, "elbo_grad_1d_batched: D=%d not in 1..%d", D, ASVGP_MAX_BATCH_COLUMNS);
+    ASVGP_REQUIRE(h_variance != nullptr && h_sigma2 != nullptr, "elbo_grad_1d_batched: h_variance / h_sigma2 is NULL");
+    for (int b = 0; b < B; ++b)
+        ASVGP_REQUIRE(h_variance[b] > 0.0 && h_sigma2[b] > 0.0, "elbo_grad_1d_batched: slot %d: variance=%g sigma2=%g must be positive",
+                      b, h_variance[b], h_sigma2[b]);
+    ASVGP_REQUIRE(work_bytes >= asvgp_workspace_bytes_1d_batched(M, order, chunks, B, D), "elbo_grad_1d_batched: workspace too small");
+    const ChunkLayout lay = pick_layout_elbo(M, order, chunks);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    ASVGP_DISPATCH_ORDER(order, { if (int rc = launch_elbo_batched<K>(lay, B, D, Kuu, dKuu, acc, h_variance, h_sigma2, out,
+                                                                      static_cast<char*>(work), st)) return rc; });
     return kOk;
 }
 

@@ -14,6 +14,7 @@ What differs from the reference is only *how*:
 import numpy as np
 import torch
 
+from . import _lib
 from . import dist as _dist
 from . import ops
 from .inducing_features import SplineFeatures1D
@@ -73,6 +74,9 @@ class GPR_1d(_ModelBase):
     data = (X[n, 1], y[n] or y[n, D]) as CUDA tensors or host arrays; X and y may each be float32 or float64 and are read
     as they are (the accumulate converts every value to float64 in registers, so the model equals the one built from the
     float64-converted data up to summation order).  Everything after the O(N) pass is float64."""
+
+    _acc_batch = None       # the accumulators as one [D, L] tensor (training_loss_and_gradients_batch), built on first use
+    _n_host = None
 
     def __init__(self, data, kernel, basis, distributed="auto", check_inputs=True, chunks=0):
         # Check inputs (reference gpr.py:22-26)
@@ -176,17 +180,17 @@ class GPR_1d(_ModelBase):
             ops.elbo_grad_1d(Kuu, dKuu, acc, self.basis, var, s2, chunks=self._chunks, out=out, kuu=kuu, join_late=True)
         return self._out
 
-    def _combine_outputs(self):
-        """Bound for D output columns from the D single-column evaluations.  The reference scales the log-dets by
-        D and sums the data-fit terms over columns, but counts -sum(K_diag)/2s2 + trace/2s2 ONCE (gpr.py:81-87);
-        summing the columns counts it D times, so D - 1 copies of T = (-N v + trace)/(2 s2) are taken out again:
-        dT/dv = (-N + trace/v)/(2 s2) (trace is linear in v), dT/dl = (dtrace/dl)/(2 s2), dT/ds2 = -T/s2."""
-        outs = torch.stack(self._outs).cpu().numpy()
+    @staticmethod
+    def _combine_columns(outs, v, s2, n):
+        """Bound for D output columns from the D single-column evaluations outs[D, 16] at variance v, sigma2 s2 and n data
+        points (v, s2, n are only read for D > 1).  The reference scales the log-dets by D and sums the data-fit terms over
+        columns, but counts -sum(K_diag)/2s2 + trace/2s2 ONCE (gpr.py:81-87); summing the columns counts it D times, so
+        D - 1 copies of T = (-N v + trace)/(2 s2) are taken out again: dT/dv = (-N + trace/v)/(2 s2) (trace is linear in
+        v), dT/dl = (dtrace/dl)/(2 s2), dT/ds2 = -T/s2."""
         out = outs[0].copy()
-        extra = len(self._outs) - 1
+        extra = len(outs) - 1
         if extra:
-            v, s2 = hyper_value(self.kernel.variance), hyper_value(self.likelihood.variance)
-            n, tr, dtr_dl = float(self._scal[1].item()), out[7], out[15]
+            tr, dtr_dl = out[7], out[15]
             T = 0.5 * (-n * v + tr) / s2
             out[0:4] = outs[:, 0:4].sum(0) - extra * np.array([T, 0.5 * (-n + tr / v) / s2, 0.5 * dtr_dl / s2, -T / s2])
             out[6] = outs[:, 6].sum()
@@ -194,16 +198,64 @@ class GPR_1d(_ModelBase):
             out[8] = bad[0] if bad.size else 0.0
         return out
 
+    def _combine_outputs(self):
+        outs = torch.stack(self._outs).cpu().numpy()
+        if len(outs) == 1:
+            return self._combine_columns(outs, None, None, None)
+        v, s2 = hyper_value(self.kernel.variance), hyper_value(self.likelihood.variance)
+        return self._combine_columns(outs, v, s2, float(self._scal[1].item()))
+
+    def _grads(self, out):
+        return _grad_dict([(self.kernel.variance, out[1]), (self.kernel.lengthscales, out[2]),
+                           (self.likelihood.variance, out[3])])
+
     def elbo_and_grad(self):
         """ELBO (reference gpr.py:49-89) and {id(param): dELBO/dparam} for variance, lengthscales, sigma^2."""
         self._launch_elbo()
         out = self._combine_outputs()
         if out[8] != 0:
             raise np.linalg.LinAlgError("banded Cholesky failed: non-positive pivot %d" % int(out[8]))
-        grads = _grad_dict([(self.kernel.variance, out[1]), (self.kernel.lengthscales, out[2]),
-                            (self.likelihood.variance, out[3])])
+        grads = self._grads(out)
         self.last_terms = dict(log_det_Kuu=out[4], log_det_P=out[5], quad=out[6], trace=out[7])
         return float(out[0]), grads
+
+    def training_loss_and_gradients_batch(self, U):
+        """training_loss_and_gradients at B settings at once, without changing the model's parameters.
+
+        U[B, 3]: unconstrained values in the order of `trainable_variables` (1 <= B <= 64).  Returns (loss[B], grad[B, 3],
+        info[B]); row b equals training_loss_and_gradients() with the parameters set to U[b], bit for bit.  A setting whose
+        banded Cholesky fails gets loss = +inf, NaN gradients and its first failing pivot in info (nothing is raised).  All
+        settings share the accumulators and run as one batch of chains on the GPU (asvgp_elbo_grad_1d_batched); the results
+        come back in one device-to-host copy."""
+        params = self.trainable_variables
+        U = np.asarray(U, dtype=np.float64)
+        if U.ndim != 2 or U.shape[1] != len(params):
+            raise ValueError("U must be [B, %d] (unconstrained values of trainable_variables), got shape %s"
+                             % (len(params), U.shape))
+        if not 1 <= U.shape[0] <= _lib.MAX_BATCH:
+            raise ValueError("U has %d rows; a batch holds 1..%d settings" % (U.shape[0], _lib.MAX_BATCH))
+        if not np.isfinite(U).all():
+            raise ValueError("U must be finite")
+        vals = np.array([[p.value_at(float(u)) for p, u in zip(params, row)] for row in U])
+        var, ell, s2 = vals[:, 0], vals[:, 1], vals[:, 2]
+        Kuu, dKuu = self.inducing_features.make_Kuu_device_batched(self.kernel, ell, var, want_grad=True)
+        if self._acc_batch is None:
+            self._acc_batch = self._acc.view(1, -1) if len(self._accs) == 1 else torch.stack(self._accs)
+        D = len(self._accs)
+        if D > 1 and self._n_host is None:
+            self._n_host = float(self._scal[1].item())
+        outs = ops.elbo_grad_1d_batched(Kuu, dKuu, self._acc_batch, self.basis, var, s2, chunks=self._chunks).cpu().numpy()
+        B = U.shape[0]
+        loss, grad, info = np.empty(B), np.empty((B, len(params))), np.zeros(B, dtype=np.int64)
+        for b in range(B):
+            out = self._combine_columns(outs[b], var[b], s2[b], self._n_host)
+            if out[8] != 0:
+                loss[b], grad[b], info[b] = np.inf, np.nan, int(out[8])
+                continue
+            grads = self._grads(out)
+            loss[b] = -float(out[0])
+            grad[b] = [-(grads[id(p)] * p.dvalue_dunconstrained_at(float(u))) for p, u in zip(params, U[b])]
+        return loss, grad, info
 
     def elbo(self):
         """Variational bound on the log marginal likelihood (reference gpr.py:49-89)."""

@@ -40,9 +40,11 @@ class SplineFeatures1D:
         self.kernel = kernel
         self.basis = basis
 
-    def _terms(self, kernel):
+    def _terms(self, kernel, ell=None, var=None):
         kind = kernel_kind(kernel)
-        terms = kuu_terms(kind, hyper_value(kernel.lengthscales), hyper_value(kernel.variance))
+        if ell is None:
+            ell, var = hyper_value(kernel.lengthscales), hyper_value(kernel.variance)
+        terms = kuu_terms(kind, ell, var)
         missing = [n for n, _, _ in terms if not hasattr(self.basis, n)]
         if missing:
             raise AttributeError("B%dSpline has no table %s needed by %s (as in the reference)"
@@ -54,6 +56,14 @@ class SplineFeatures1D:
         terms = self._terms(kernel)
         return ops.kuu_assemble(self.basis, [t[0] for t in terms], [t[1] for t in terms], [t[2] for t in terms],
                                 want_grad=want_grad)
+
+    def make_Kuu_device_batched(self, kernel, lengthscales, variances, want_grad=True):
+        """make_Kuu_device of `kernel`'s family at B (lengthscale, variance) settings: bands [B, k+1, m], slot b equal to
+        make_Kuu_device at that setting (asvgp_kuu_assemble_batched)."""
+        sets = [self._terms(kernel, ell, var) for ell, var in zip(lengthscales, variances)]
+        names = [t[0] for t in sets[0]]
+        return ops.kuu_assemble_batched(self.basis, names, [[t[1] for t in s] for s in sets], [[t[2] for t in s] for s in sets],
+                                        want_grad=want_grad)
 
     def make_Kuu(self, kernel):
         """Banded Kuu, (k+1) x m lower band, as the reference returns it (inducing_features.py:12-44)."""

@@ -34,10 +34,17 @@ class Parameter:
 
     @property
     def value(self):
-        return self.lower + _softplus(self.unconstrained)
+        return self.value_at(self.unconstrained)
 
     def dvalue_dunconstrained(self):
-        u = self.unconstrained
+        return self.dvalue_dunconstrained_at(self.unconstrained)
+
+    def value_at(self, u):
+        """The value at unconstrained value `u` (the parameter itself is not changed)."""
+        return self.lower + _softplus(u)
+
+    @staticmethod
+    def dvalue_dunconstrained_at(u):
         return 1.0 / (1.0 + math.exp(-u))
 
     def numpy(self):

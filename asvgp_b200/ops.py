@@ -213,6 +213,62 @@ def kuu_assemble(basis, names, coef, dcoef=None, want_grad=True):
     return Kuu, dKuu
 
 
+def kuu_assemble_batched(basis, names, coefs, dcoefs=None, want_grad=True):
+    """kuu_assemble for B coefficient sets, the rows of coefs / dcoefs [B, len(names)]: (Kuu, dKuu) as [B, k+1, m] CUDA
+    bands; slot b equals kuu_assemble(basis, names, coefs[b], dcoefs[b]) bit for bit."""
+    tables = device_tables(basis, names)
+    k, m, n = basis.order, basis.m, len(names)
+    coefs = np.ascontiguousarray(coefs, dtype=np.float64)
+    dcoefs = np.zeros_like(coefs) if dcoefs is None else np.ascontiguousarray(dcoefs, dtype=np.float64)
+    if coefs.ndim != 2 or coefs.shape[1] != n or dcoefs.shape != coefs.shape:
+        raise ValueError("coefs / dcoefs must be [B, %d], got %s / %s" % (n, coefs.shape, dcoefs.shape))
+    B = coefs.shape[0]
+    Kuu = torch.empty((B, k + 1, m), dtype=F64, device=tables.device)
+    dKuu = torch.empty_like(Kuu) if want_grad else None
+    _lib.call("asvgp_kuu_assemble_batched", _p(tables), n, B, ctypes.c_void_p(coefs.ctypes.data),
+              ctypes.c_void_p(dcoefs.ctypes.data), m, k, _p(Kuu), _p(dKuu), _stream())
+    return Kuu, dKuu
+
+
+def workspace_1d_batched(m, order, chunks, B, D):
+    """Scratch tensor for elbo_grad_1d_batched (cached per (device, m, order, chunks, B, D))."""
+    dev = device()
+    key = (dev, m, order, chunks, "batched", B, D)
+    ws = _WORKSPACES.get(key)
+    if ws is None:
+        nbytes = _lib.load().asvgp_workspace_bytes_1d_batched(m, order, chunks, B, D)
+        if nbytes < 0:
+            raise _lib.AsvgpNativeError("asvgp_workspace_bytes_1d_batched rejected m=%d order=%d B=%d D=%d" % (m, order, B, D))
+        ws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+        _WORKSPACES[key] = ws
+    return ws
+
+
+def elbo_grad_1d_batched(Kuu, dKuu, accs, basis, variances, sigma2s, chunks=0, out=None):
+    """B settings of the bound in one stream of launches: Kuu, dKuu [B, k+1, m] (kuu_assemble_batched), accs [D, L] (D
+    packed accumulators, or one [L]), variances / sigma2s [B] on the host.  Returns out [B, D, 16] on the device; out[b, d]
+    equals elbo_grad_1d of slot b and column d bit for bit in slots 0..8 and 15 (see include/asvgp_b200.h)."""
+    k, m = basis.order, basis.m
+    accs = accs.reshape(1, -1) if accs.dim() == 1 else accs
+    variances = np.ascontiguousarray(variances, dtype=np.float64).reshape(-1)
+    sigma2s = np.ascontiguousarray(sigma2s, dtype=np.float64).reshape(-1)
+    B, D = variances.size, accs.shape[0]
+    if sigma2s.size != B or tuple(Kuu.shape) != (B, k + 1, m) or tuple(dKuu.shape) != (B, k + 1, m):
+        raise ValueError("elbo_grad_1d_batched: %d variances, %d sigma2s, Kuu %s, dKuu %s" % (B, sigma2s.size, tuple(Kuu.shape),
+                                                                                            tuple(dKuu.shape)))
+    if accs.shape[1] != accum_size_1d(basis) or not accs.is_contiguous():
+        raise ValueError("elbo_grad_1d_batched: accs must be contiguous [D, %d]" % accum_size_1d(basis))
+    if not 1 <= B <= _lib.MAX_BATCH or not 1 <= D <= _lib.MAX_BATCH_COLUMNS:
+        raise ValueError("elbo_grad_1d_batched: B=%d not in 1..%d or D=%d not in 1..%d"
+                         % (B, _lib.MAX_BATCH, D, _lib.MAX_BATCH_COLUMNS))
+    ws = workspace_1d_batched(m, k, int(chunks), B, D)
+    if out is None:
+        out = torch.empty((B, D, 16), dtype=F64, device=accs.device)
+    _lib.call("asvgp_elbo_grad_1d_batched", _p(Kuu), _p(dKuu), _p(accs), m, k, B, D, ctypes.c_void_p(variances.ctypes.data),
+              ctypes.c_void_p(sigma2s.ctypes.data), int(chunks), _p(out), _p(ws), ws.numel(), _stream())
+    return out
+
+
 class KuuChain:
     """Handle of a Kuu chain in flight on the side stream (kuu_chain_1d): its state buffer, the event that marks it
     complete, and the operands it reads (kept alive until the bound has consumed the state)."""

@@ -146,6 +146,31 @@ ASVGP_API int asvgp_elbo_grad_1d_prepared(const double* kuu_state, const double*
                                           int M, int order, double variance, double sigma2, int chunks, double* out,
                                           void* work, int64_t work_bytes, void* kuu_ready_event, int join_late, void* stream);
 
+/* ---- batched hyper-parameter evaluation -----------------------------------------------------------------------------------
+ * B settings (v_b, l_b, sigma2_b) of the bound over the same data, in one stream of launches (a multi-start optimiser, a
+ * lengthscale scan).  The data term does not depend on the hyper-parameters, so all slots share the accumulators.
+ *
+ * asvgp_kuu_assemble_batched: asvgp_kuu_assemble for B coefficient sets.  h_coef / h_dcoef are HOST arrays [B][n_terms]
+ * (h_dcoef may be NULL: zeros); Kuu and dKuu (may be NULL) are [B][order+1][M].  Slot b's band equals asvgp_kuu_assemble with
+ * row b of the coefficients bit for bit.
+ *
+ * asvgp_elbo_grad_1d_batched: `acc` holds D packed accumulators of asvgp_accum_1d, one per output column, contiguous
+ * ([D][(order+2) M + 2]); Kuu / dKuu are [B][order+1][M]; h_variance / h_sigma2 are HOST arrays [B].  out[B][D][16] (device)
+ * has the 16 slots of asvgp_elbo_grad_1d.  For the same `chunks`, out[b][d][0..8] and [15] equal asvgp_elbo_grad_1d on
+ * (Kuu[b], dKuu[b], accumulator d, v_b, sigma2_b) bit for bit, whatever B, the other slots and the position of b in the batch;
+ * [9..14] are that evaluation's own clock diagnostics.  A slot whose factorisation fails reports its pivot in its own info
+ * slot and leaves the others untouched.  B outside 1..ASVGP_MAX_BATCH, D outside 1..ASVGP_MAX_BATCH_COLUMNS, a
+ * non-positive v_b or sigma2_b and a workspace smaller than asvgp_workspace_bytes_1d_batched(M, order, chunks, B, D) bytes
+ * are rejected before any CUDA call (the query returns -1 for arguments out of range). */
+#define ASVGP_MAX_BATCH 64
+#define ASVGP_MAX_BATCH_COLUMNS 64
+ASVGP_API int asvgp_kuu_assemble_batched(const double* tables, int n_terms, int B, const double* h_coef, const double* h_dcoef,
+                                         int M, int order, double* Kuu, double* dKuu, void* stream);
+ASVGP_API int64_t asvgp_workspace_bytes_1d_batched(int M, int order, int chunks, int B, int D);
+ASVGP_API int asvgp_elbo_grad_1d_batched(const double* Kuu, const double* dKuu, const double* acc, int M, int order, int B, int D,
+                                         const double* h_variance, const double* h_sigma2, int chunks, double* out, void* work,
+                                         int64_t work_bytes, void* stream);
+
 /* ---- a10 (factorisation half): posterior weights -------------------------------------------------------------------------
  * Replaces the CHOLMOD factorisations and solves of GPR_1d.predict_f (gpr.py:96-108):
  * alpha = P^-1 Kuf_y / sigma2 and S = band(P^-1) - band(Kuu^-1), P = Kuu + G / sigma2.  info[2] (device): failing
