@@ -32,6 +32,11 @@ SIGNATURES = {
     "asvgp_kuu_assemble_batched": [_vp, _c_int, _c_int, _vp, _vp, _c_int, _c_int, _vp, _vp, _vp],
     "asvgp_elbo_grad_1d_batched": [_vp, _vp, _vp, _c_int, _c_int, _c_int, _c_int, _vp, _vp, _c_int, _vp, _vp, _c_i64, _vp],
     "asvgp_posterior_1d": [_vp, _vp, _c_int, _c_int, _c_dbl, _c_int, _vp, _vp, _vp, _vp, _c_i64, _vp],
+    "asvgp_accum_1d_segmented_typed": [_vp, _c_int, _vp, _c_int, _c_i64, _vp, _c_int, _vp, _c_int, _c_int, _vp, _vp],
+    "asvgp_elbo_grad_1d_batched_rows": [_vp, _vp, _vp, _c_int, _vp, _c_int, _c_int, _c_int, _c_int, _vp, _vp, _c_int, _vp, _vp,
+                                        _c_i64, _vp],
+    "asvgp_posterior_1d_batched": [_vp, _vp, _c_int, _vp, _c_int, _c_int, _c_int, _vp, _c_int, _vp, _vp, _vp, _vp, _c_i64, _vp],
+    "asvgp_predict_1d_segmented": [_vp, _c_i64, _vp, _c_int, _vp, _c_int, _c_int, _vp, _vp, _vp, _vp, _vp, _vp],
     "asvgp_band_inverse_1d": [_vp, _vp, _c_int, _c_int, _c_int, _vp, _vp, _vp, _vp, _c_i64, _vp],
     "asvgp_accum_2d": [_vp, _vp, _c_i64, _vp, _c_int, _vp, _c_int, _c_int, _vp, _vp, _vp],
     "asvgp_accum_2d_raster": [_vp, _vp, _c_i64, _c_i64, _vp, _c_int, _vp, _c_int, _c_int, _vp, _vp, _vp],
@@ -76,6 +81,7 @@ VALUE_FUNCTIONS = {
     "asvgp_launch_count": (_c_i64, []),
     "asvgp_workspace_bytes_1d": (_c_i64, [_c_int, _c_int, _c_int]),
     "asvgp_workspace_bytes_1d_batched": (_c_i64, [_c_int, _c_int, _c_int, _c_int, _c_int]),
+    "asvgp_workspace_bytes_posterior_1d_batched": (_c_i64, [_c_int, _c_int, _c_int, _c_int]),
     "asvgp_kuu_state_doubles": (_c_i64, [_c_int, _c_int]),
     "asvgp_accum_1d_binned_work_bytes": (_c_i64, [_c_i64]),
     "asvgp_accum_2d_binned_work_bytes": (_c_i64, [_c_i64]),

@@ -247,12 +247,13 @@ __global__ void __launch_bounds__(256) chain_rows_kernel(ChunkLayout lay, ChainS
     }
 }
 
-// Row tables of a batch (asvgp_elbo_grad_1d_batched): blockIdx.z = slot b, blockIdx.y = chain c of the slot — 0 the Kuu
+// Row tables of a batch (asvgp_elbo_grad_1d_batched_rows): blockIdx.z = slot b, blockIdx.y = chain c of the slot — 0 the Kuu
 // chain of Kuu[b], 2d+1 / 2d+2 the P chains (d/dl, d/dsigma2) of output column d — each table built with the matrix and
 // right-hand-side functors of the single call (launch_kuu_chain, launch_pchains), so every entry has the same bits.
 struct BatchRowsArgs {
     const double* Kuu; const double* dKuu;          // [B][K+1][M]
-    const double* acc; size_t acc_stride;           // column d's packed accumulator at acc + d * acc_stride
+    const double* acc; size_t acc_stride;           // slot b, column d: packed accumulator at acc + (row[b] * D + d) * acc_stride
+    int64_t row[ASVGP_MAX_BATCH];
     unsigned* counters; size_t counter_stride;      // finalize arrival counter of (b, d) at counters + (b * D + d) * counter_stride
     double inv_s2[ASVGP_MAX_BATCH], tan_s2[ASVGP_MAX_BATCH];   // 1 / sigma2 and -1 / sigma2^2 per slot (rounded on the host as there)
 };
@@ -267,7 +268,7 @@ __global__ void __launch_bounds__(256) batch_rows_kernel(ChunkLayout lay, const 
     ChainSpec<T> sp{BandMat<T>{Kuu, dKuu, nullptr, 0.0, 0.0, 1, M}, VecRhs<T>{Kuu, M, 0}};
     if (c > 0) {
         const int d = (c - 1) >> 1;
-        const double* G = a.acc + d * a.acc_stride;
+        const double* G = a.acc + (a.row[b] * (n_chains >> 1) + d) * a.acc_stride;
         sp = (c & 1) ? ChainSpec<T>{BandMat<T>{Kuu, dKuu, G, a.inv_s2[b], 0.0, 1, M}, VecRhs<T>{G + band, M, 1}}
                      : ChainSpec<T>{BandMat<T>{Kuu, dKuu, G, a.inv_s2[b], a.tan_s2[b], 0, M}, VecRhs<T>{G + band, M, 1}};
         if ((c & 1) && blockIdx.x == 0 && threadIdx.x == 0) a.counters[((size_t)b * (n_chains >> 1) + d) * a.counter_stride] = 0u;
@@ -643,14 +644,15 @@ __global__ void __launch_bounds__(kTraceThreads) elbo_finalize_kernel(const doub
 struct BatchFinalizeArgs {
     const double* kstate; size_t kstate_stride;
     double* partial; size_t partial_stride;          // as ElboArgs
-    const double* acc; size_t acc_stride;
+    const double* acc; size_t acc_stride;            // as BatchRowsArgs
+    int64_t row[ASVGP_MAX_BATCH];
     double variance[ASVGP_MAX_BATCH], sigma2[ASVGP_MAX_BATCH];
 };
 __global__ void __launch_bounds__(kTraceThreads) elbo_finalize_batched_kernel(const __grid_constant__ BatchFinalizeArgs a, int M, int K,
                                                                               double* __restrict__ out) {
     pdl_wait();                                                         // every chain of the batch is complete
     const int b = blockIdx.z, d = blockIdx.y, D = gridDim.y;
-    const double* G = a.acc + d * a.acc_stride;
+    const double* G = a.acc + (a.row[b] * D + d) * a.acc_stride;
     elbo_finalize(a.kstate + b * a.kstate_stride, a.partial + b * a.partial_stride + d * kPartialDoubles, G, G + (size_t)(K + 2) * M,
                   M, K, a.variance[b], a.sigma2[b], 0, (int)blockIdx.x, out + ((size_t)b * D + d) * 16);
 }
@@ -658,41 +660,72 @@ __global__ void __launch_bounds__(kTraceThreads) elbo_finalize_batched_kernel(co
 // ------------------------------------------------------------------------------------------------------------------
 // posterior weights
 // ------------------------------------------------------------------------------------------------------------------
+// Posteriors of a batch of B slots (one slot for asvgp_posterior_1d): slot b factorises Kuu[b] and P_b = Kuu[b] + G / sigma2_b with
+// G, b from accumulator row[b].  Chain c of slot b (0: Kuu, Takahashi;  1: P, solve + Takahashi) is CTA (c, b) of one launch.
 template <int K>
 struct PosteriorArgs {
     ChunkLayout lay;
-    ColumnStore<double, K, true> cols[2];
-    const double* Kuu; const double* G; const double* b;
-    double sigma2;
-    double* sigK; double* sigP; double* x;       // (K+1) x M, (K+1) x M, M
-    double* info;                                // [2]
-    const double* rows;                          // lane-interleaved row tables of the two chains
+    char* cols; size_t cols_bytes;               // chain (b, c)'s column store at cols + (2 b + c) * cols_bytes
+    const double* rows;                          // and its lane-interleaved row table at rows + (2 b + c) * chain_rows_count
+    double* sigK; double* sigP; size_t band_stride;     // slot b's (K+1) x M bands at sigK / sigP + b * band_stride
+    double* x; size_t x_stride;                  // slot b's P^-1 b at x + b * x_stride
+    double* info;                                // [B][2]
 };
+
+// Per-slot operands of the row tables and of the combine kernel, as kernel parameters.
+struct PosteriorBatchArgs {
+    const double* Kuu;                           // [B][K+1][M]
+    const double* acc; size_t acc_stride;        // slot b's packed accumulator at acc + row[b] * acc_stride
+    int64_t row[ASVGP_MAX_BATCH];
+    double inv_s2[ASVGP_MAX_BATCH];              // 1 / sigma2_b, rounded on the host
+};
+
+// blockIdx.z = slot, blockIdx.y = chain: the tables of chain_rows_kernel for the single call's two chain specifications.
+template <int K>
+__global__ void __launch_bounds__(256) posterior_rows_kernel(ChunkLayout lay, const __grid_constant__ PosteriorBatchArgs a,
+                                                             double* __restrict__ out) {
+    using T = double;
+    const int M = lay.M, b = blockIdx.z, c = blockIdx.y;
+    const size_t band = (size_t)(K + 1) * M;
+    const double* Kuu = a.Kuu + b * band;
+    const double* G = a.acc + a.row[b] * a.acc_stride;
+    const ChainSpec<T> sp = c == 0 ? ChainSpec<T>{BandMat<T>{Kuu, nullptr, nullptr, 0.0, 0.0, 0, M}, VecRhs<T>{Kuu, M, 0}}
+                                   : ChainSpec<T>{BandMat<T>{Kuu, nullptr, G, a.inv_s2[b], 0.0, 0, M}, VecRhs<T>{G + band, M, 1}};
+    const unsigned per_chain = (unsigned)chain_rows_count<T, K>(lay);
+    T* tab = out + ((size_t)b * 2 + c) * per_chain;
+    for (unsigned e = blockIdx.x * blockDim.x + threadIdx.x; e < per_chain; e += gridDim.x * blockDim.x)
+        tab[e] = chain_rows_entry<T, K>(lay, sp, e);
+}
 
 template <int K>
 __global__ void __launch_bounds__(kChainThreads) posterior_chains_kernel(PosteriorArgs<K> a) {
     using T = double;
     extern __shared__ __align__(16) char smem[];
-    const int chain = blockIdx.x, p = threadIdx.x;
+    const int chain = blockIdx.x, slot = blockIdx.y, li = 2 * slot + chain, p = threadIdx.x;
     const ChunkLayout lay = a.lay;
-    const int M = lay.M;
     __shared__ ChainTotals<T, K> tot;
-    (void)M;
+    const ColumnStore<T, K, true> cols = launched_cols<T, K>(lay, a.cols, a.cols_bytes, li);
     const int n_rho = chain_n_rho(lay, K), g0 = lay.P > 1 ? lay.start(p < lay.P ? p : 0) : 0, pp = p < lay.P ? p : 0;
-    const T* tab = a.rows + (size_t)chain * chain_rows_count<T, K>(lay);
+    const T* tab = a.rows + (size_t)li * chain_rows_count<T, K>(lay);
     const RowsMat<T, K> A{tab, g0, lay.P, pp, n_rho};
     const RowsRhs<T> rhs{tab + (size_t)n_rho * (K + 1) * lay.P, g0, lay.P, pp, n_rho};
-    BandSink<T> sinkK{a.sigK, lay.M}, sinkP{a.sigP, lay.M};
-    if (chain == 0) run_chain<T, K, true, false, true>(lay, a.cols[0], smem, A, rhs, static_cast<T*>(nullptr), sinkK, &tot, nullptr);
-    else run_chain<T, K, true, true, true>(lay, a.cols[1], smem, A, rhs, a.x, sinkP, &tot, nullptr);
-    if (p == 0) a.info[chain] = (double)tot.info;
+    BandSink<T> sinkK{a.sigK + slot * a.band_stride, lay.M}, sinkP{a.sigP + slot * a.band_stride, lay.M};
+    if (chain == 0) run_chain<T, K, true, false, true>(lay, cols, smem, A, rhs, static_cast<T*>(nullptr), sinkK, &tot, nullptr);
+    else run_chain<T, K, true, true, true>(lay, cols, smem, A, rhs, a.x + slot * a.x_stride, sinkP, &tot, nullptr);
+    if (p == 0) a.info[li] = (double)tot.info;
 }
 
+// blockIdx.y = slot: S = band(P^-1) - band(Kuu^-1), alpha = P^-1 b / sigma2
 __global__ void __launch_bounds__(256) posterior_combine_kernel(const double* __restrict__ sigK,
-                                                                const double* __restrict__ sigP,
-                                                                const double* __restrict__ x, double inv_s2, int M,
+                                                                const double* __restrict__ sigP, size_t band_stride,
+                                                                const double* __restrict__ x, size_t x_stride,
+                                                                const __grid_constant__ PosteriorBatchArgs a, int M,
                                                                 int band_elems, double* __restrict__ alpha,
                                                                 double* __restrict__ S) {
+    const int b = blockIdx.y;
+    const double inv_s2 = a.inv_s2[b];
+    sigK += b * band_stride; sigP += b * band_stride; x += b * x_stride;
+    alpha += (size_t)b * M; S += (size_t)b * band_elems;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < band_elems; i += gridDim.x * blockDim.x) {
         S[i] = sigP[i] - sigK[i];
         if (i < M) alpha[i] = x[i] * inv_s2;
@@ -956,7 +989,7 @@ struct BatchPlan {
 // bound runs the code of the single call on its own workspace, so slot b's bits depend neither on B nor on the other slots.
 template <int K>
 static int launch_elbo_batched(const ChunkLayout& lay, int B, int D, const double* Kuu, const double* dKuu, const double* acc,
-                               const double* h_variance, const double* h_sigma2, double* out, char* work, cudaStream_t st) {
+                               const int64_t* h_row, const double* h_variance, const double* h_sigma2, double* out, char* work, cudaStream_t st) {
     using T = Dual<1>;
     const BatchPlan<K> plan(lay, B, D);
     const int M = lay.M;
@@ -982,6 +1015,7 @@ static int launch_elbo_batched(const ChunkLayout& lay, int B, int D, const doubl
     r.counter_stride = kPartialBytes / sizeof(unsigned);
     for (int b = 0; b < B; ++b) {
         const double inv_s2 = 1.0 / h_sigma2[b];       // as launch_pchains
+        r.row[b] = h_row[b];
         r.inv_s2[b] = inv_s2;
         r.tan_s2[b] = -inv_s2 * inv_s2;
     }
@@ -994,47 +1028,62 @@ static int launch_elbo_batched(const ChunkLayout& lay, int B, int D, const doubl
     f.kstate = a.kstate; f.kstate_stride = a.kstate_stride;
     f.partial = a.partial; f.partial_stride = a.partial_stride;
     f.acc = acc; f.acc_stride = acc_stride;
-    for (int b = 0; b < B; ++b) { f.variance[b] = h_variance[b]; f.sigma2[b] = h_sigma2[b]; }
+    for (int b = 0; b < B; ++b) { f.row[b] = h_row[b]; f.variance[b] = h_variance[b]; f.sigma2[b] = h_sigma2[b]; }
     ASVGP_CUDA_OK(launch_dependent(elbo_finalize_batched_kernel, dim3(kTraceBlocks, D, B), kTraceThreads, 0, st, true, f, M, K, out));
     ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     return kOk;
 }
 
+// Workspace of a batch of B posteriors: per chain (2B) a column store and a row table; per slot the two bands and P^-1 b.
 template <int K>
-static int launch_posterior(const ChunkLayout& lay, const double* Kuu, const double* acc, double sigma2,
-                            double* alpha, double* S, double* info, char* work, cudaStream_t st) {
+struct PosteriorPlan {
+    size_t cols_bytes, band_stride, x_stride, sig_off, x_off, rows_off, total;
+    PosteriorPlan(const ChunkLayout& lay, int B) {
+        cols_bytes = ChainPlan<double, K>::bytes(lay);
+        band_stride = align256((size_t)(K + 1) * lay.M * sizeof(double)) / sizeof(double);
+        x_stride = align256((size_t)lay.M * sizeof(double)) / sizeof(double);
+        sig_off = (size_t)2 * B * cols_bytes;                                   // sigK of every slot, then sigP of every slot
+        x_off = sig_off + (size_t)2 * B * band_stride * sizeof(double);
+        rows_off = x_off + (size_t)B * x_stride * sizeof(double);
+        total = rows_off + (size_t)2 * B * chain_rows_count<double, K>(lay) * sizeof(double);
+    }
+};
+
+// B posteriors in three launches (row tables, chains, combine); each chain runs the single call's code on its own workspace.
+template <int K>
+static int launch_posterior_batched(const ChunkLayout& lay, int B, const double* Kuu, const double* acc, const int64_t* h_row,
+                                    const double* h_sigma2, double* alpha, double* S, double* info, char* work, cudaStream_t st) {
+    using T = double;
+    const PosteriorPlan<K> plan(lay, B);
+    const int M = lay.M;
+    const size_t per_chain = chain_rows_count<T, K>(lay);
+    ASVGP_REQUIRE(per_chain < ((size_t)1 << 31), "banded chains: %zu row-table entries exceed the 32-bit index range", per_chain);
     PosteriorArgs<K> a;
     a.lay = lay;
-    char* p = work;
-    for (int c = 0; c < 2; ++c) { a.cols[c] = ChainPlan<double, K>::carve(lay, p); p += ChainPlan<double, K>::bytes(lay); }
-    const int M = lay.M;
-    const size_t band_bytes = (((size_t)(K + 1) * M * sizeof(double)) + 255) & ~(size_t)255;
-    a.sigK = reinterpret_cast<double*>(p); p += band_bytes;
-    a.sigP = reinterpret_cast<double*>(p); p += band_bytes;
-    a.x = reinterpret_cast<double*>(p);
-    p += ((size_t)M * sizeof(double) + 255) & ~(size_t)255;
-    a.Kuu = Kuu; a.G = acc; a.b = acc + (size_t)(K + 1) * M;
-    a.sigma2 = sigma2;
+    a.cols = work;
+    a.cols_bytes = plan.cols_bytes;
+    a.rows = reinterpret_cast<T*>(work + plan.rows_off);
+    a.sigK = reinterpret_cast<double*>(work + plan.sig_off);
+    a.sigP = a.sigK + (size_t)B * plan.band_stride;
+    a.band_stride = plan.band_stride;
+    a.x = reinterpret_cast<double*>(work + plan.x_off);
+    a.x_stride = plan.x_stride;
     a.info = info;
-    {
-        using T = double;
-        T* rows = reinterpret_cast<T*>(p);
-        a.rows = rows;
-        ChainSpec<T> s0{BandMat<T>{Kuu, nullptr, nullptr, 0.0, 0.0, 0, M}, VecRhs<T>{Kuu, M, 0}};
-        ChainSpec<T> s1{BandMat<T>{Kuu, nullptr, a.G, 1.0 / sigma2, 0.0, 0, M}, VecRhs<T>{a.b, M, 1}};
-        const size_t total = 2 * chain_rows_count<T, K>(lay);
-        chain_rows_kernel<T, K, 2><<<(int)std::min<size_t>((total + 255) / 256, 148 * 8), 256, 0, st>>>(lay, s0, s1, s1, s1, rows); ASVGP_LAUNCHED();
-        ASVGP_CUDA_OK(cudaGetLastError());
-    }
-    ASVGP_CUDA_OK(cudaMemsetAsync(a.sigK, 0, 2 * band_bytes, st));
+    PosteriorBatchArgs r;
+    r.Kuu = Kuu; r.acc = acc; r.acc_stride = (size_t)(K + 2) * M + 2;
+    for (int b = 0; b < B; ++b) { r.row[b] = h_row[b]; r.inv_s2[b] = 1.0 / h_sigma2[b]; }
+    const int gx = (int)std::min<size_t>((per_chain + 255) / 256, std::max(1, 148 * 8 / (2 * B)));
+    posterior_rows_kernel<K><<<dim3(gx, 2, B), 256, 0, st>>>(lay, r, reinterpret_cast<T*>(work + plan.rows_off)); ASVGP_LAUNCHED();
+    ASVGP_CUDA_OK(cudaGetLastError());
+    ASVGP_CUDA_OK(cudaMemsetAsync(a.sigK, 0, (size_t)2 * B * plan.band_stride * sizeof(double), st));
     const size_t smem = ChainSmall<double, K>::bytes(lay.P);
     ASVGP_CUDA_OK(cudaFuncSetAttribute(posterior_chains_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    posterior_chains_kernel<K><<<2, kChainThreads, smem, st>>>(a); ASVGP_LAUNCHED();
+    posterior_chains_kernel<K><<<dim3(2, B), kChainThreads, smem, st>>>(a); ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     const int band_elems = (K + 1) * M;
-    posterior_combine_kernel<<<(band_elems + 255) / 256, 256, 0, st>>>(a.sigK, a.sigP, a.x, 1.0 / sigma2, M, band_elems,
-                                                                      alpha, S); ASVGP_LAUNCHED();
+    posterior_combine_kernel<<<dim3((band_elems + 255) / 256, B), 256, 0, st>>>(a.sigK, a.sigP, plan.band_stride, a.x, plan.x_stride, r, M,
+                                                                               band_elems, alpha, S); ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     return kOk;
 }
@@ -1198,22 +1247,34 @@ extern "C" int asvgp_elbo_grad_1d(const double* Kuu, const double* dKuu, const d
     return kOk;
 }
 
-extern "C" int asvgp_elbo_grad_1d_batched(const double* Kuu, const double* dKuu, const double* acc, int M, int order, int B, int D,
-                                          const double* h_variance, const double* h_sigma2, int chunks, double* out, void* work,
-                                          int64_t work_bytes, void* stream) {
+extern "C" int asvgp_elbo_grad_1d_batched_rows(const double* Kuu, const double* dKuu, const double* acc, int R, const int64_t* h_row,
+                                               int M, int order, int B, int D, const double* h_variance, const double* h_sigma2,
+                                               int chunks, double* out, void* work, int64_t work_bytes, void* stream) {
     ASVGP_REQUIRE(M > 2 * order && order >= 1 && order <= kMaxOrder, "elbo_grad_1d_batched: M=%d order=%d", M, order);
     ASVGP_REQUIRE(B >= 1 && B <= ASVGP_MAX_BATCH, "elbo_grad_1d_batched: B=%d not in 1..%d", B, ASVGP_MAX_BATCH);
     ASVGP_REQUIRE(D >= 1 && D <= ASVGP_MAX_BATCH_COLUMNS, "elbo_grad_1d_batched: D=%d not in 1..%d", D, ASVGP_MAX_BATCH_COLUMNS);
     ASVGP_REQUIRE(h_variance != nullptr && h_sigma2 != nullptr, "elbo_grad_1d_batched: h_variance / h_sigma2 is NULL");
+    ASVGP_REQUIRE(R >= 1 && h_row != nullptr, "elbo_grad_1d_batched: R=%d must be at least 1 and h_row not NULL", R);
+    for (int b = 0; b < B; ++b)
+        ASVGP_REQUIRE(h_row[b] >= 0 && h_row[b] < R, "elbo_grad_1d_batched: slot %d: row %lld not in 0..%d", b, (long long)h_row[b], R - 1);
     for (int b = 0; b < B; ++b)
         ASVGP_REQUIRE(h_variance[b] > 0.0 && h_sigma2[b] > 0.0, "elbo_grad_1d_batched: slot %d: variance=%g sigma2=%g must be positive",
                       b, h_variance[b], h_sigma2[b]);
     ASVGP_REQUIRE(work_bytes >= asvgp_workspace_bytes_1d_batched(M, order, chunks, B, D), "elbo_grad_1d_batched: workspace too small");
     const ChunkLayout lay = pick_layout_elbo(M, order, chunks);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    ASVGP_DISPATCH_ORDER(order, { if (int rc = launch_elbo_batched<K>(lay, B, D, Kuu, dKuu, acc, h_variance, h_sigma2, out,
+    ASVGP_DISPATCH_ORDER(order, { if (int rc = launch_elbo_batched<K>(lay, B, D, Kuu, dKuu, acc, h_row, h_variance, h_sigma2, out,
                                                                       static_cast<char*>(work), st)) return rc; });
     return kOk;
+}
+
+static const int64_t kRowZero[ASVGP_MAX_BATCH] = {};
+
+extern "C" int asvgp_elbo_grad_1d_batched(const double* Kuu, const double* dKuu, const double* acc, int M, int order, int B, int D,
+                                          const double* h_variance, const double* h_sigma2, int chunks, double* out, void* work,
+                                          int64_t work_bytes, void* stream) {
+    return asvgp_elbo_grad_1d_batched_rows(Kuu, dKuu, acc, 1, kRowZero, M, order, B, D, h_variance, h_sigma2, chunks, out, work,
+                                           work_bytes, stream);
 }
 
 extern "C" int64_t asvgp_kuu_state_doubles(int M, int order) {
@@ -1253,8 +1314,35 @@ extern "C" int asvgp_posterior_1d(const double* Kuu, const double* acc, int M, i
     ASVGP_REQUIRE(work_bytes >= asvgp_workspace_bytes_1d(M, order, chunks), "posterior_1d: workspace too small");
     const ChunkLayout lay = pick_layout(M, order, chunks);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    ASVGP_DISPATCH_ORDER(order, { if (int rc = launch_posterior<K>(lay, Kuu, acc, sigma2, alpha, S_band, info,
-                                                                   static_cast<char*>(work), st)) return rc; });
+    ASVGP_DISPATCH_ORDER(order, { if (int rc = launch_posterior_batched<K>(lay, 1, Kuu, acc, kRowZero, &sigma2, alpha, S_band, info,
+                                                                           static_cast<char*>(work), st)) return rc; });
+    return kOk;
+}
+
+extern "C" int64_t asvgp_workspace_bytes_posterior_1d_batched(int M, int order, int chunks, int B) {
+    if (M <= 0 || order < 1 || order > kMaxOrder || B < 1 || B > ASVGP_MAX_BATCH) return -1;
+    const ChunkLayout lay = pick_layout(M, order, chunks);
+    size_t bytes = 0;
+    ASVGP_DISPATCH_ORDER(order, bytes = PosteriorPlan<K>(lay, B).total);
+    return (int64_t)bytes;
+}
+
+extern "C" int asvgp_posterior_1d_batched(const double* Kuu, const double* acc, int R, const int64_t* h_row, int M, int order, int B,
+                                          const double* h_sigma2, int chunks, double* alpha, double* S_band, double* info, void* work,
+                                          int64_t work_bytes, void* stream) {
+    ASVGP_REQUIRE(M > 2 * order && order >= 1 && order <= kMaxOrder, "posterior_1d_batched: M=%d order=%d", M, order);
+    ASVGP_REQUIRE(B >= 1 && B <= ASVGP_MAX_BATCH, "posterior_1d_batched: B=%d not in 1..%d", B, ASVGP_MAX_BATCH);
+    ASVGP_REQUIRE(h_sigma2 != nullptr, "posterior_1d_batched: h_sigma2 is NULL");
+    ASVGP_REQUIRE(R >= 1 && h_row != nullptr, "posterior_1d_batched: R=%d must be at least 1 and h_row not NULL", R);
+    for (int b = 0; b < B; ++b) {
+        ASVGP_REQUIRE(h_row[b] >= 0 && h_row[b] < R, "posterior_1d_batched: slot %d: row %lld not in 0..%d", b, (long long)h_row[b], R - 1);
+        ASVGP_REQUIRE(h_sigma2[b] > 0.0, "posterior_1d_batched: slot %d: sigma2=%g must be positive", b, h_sigma2[b]);
+    }
+    ASVGP_REQUIRE(work_bytes >= asvgp_workspace_bytes_posterior_1d_batched(M, order, chunks, B), "posterior_1d_batched: workspace too small");
+    const ChunkLayout lay = pick_layout(M, order, chunks);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    ASVGP_DISPATCH_ORDER(order, { if (int rc = launch_posterior_batched<K>(lay, B, Kuu, acc, h_row, h_sigma2, alpha, S_band, info,
+                                                                           static_cast<char*>(work), st)) return rc; });
     return kOk;
 }
 

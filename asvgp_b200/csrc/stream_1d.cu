@@ -245,6 +245,72 @@ __device__ __forceinline__ void ldg_stream_vec(const float* p, float (&v)[VEC], 
 template <int VEC, class TX, class TY>
 constexpr int accum_unroll() { return VEC == 4 ? (sizeof(TX) == sizeof(TY) ? 6 : 4) : kAccumUnroll; }
 
+// The U slots of one warp tile: VEC points per slot from 16-byte aligned addresses (VEC > 1) or scalar loads (VEC = 1).
+template <int U, int VEC, class TX, class TY>
+__device__ __forceinline__ void load_tile(const TX* __restrict__ x, const TY* __restrict__ y, int64_t n, int64_t slot0,
+                                          TX (&xs)[U][VEC], TY (&ys)[U][VEC], uint64_t stream_policy) {
+#pragma unroll
+    for (int j = 0; j < U; ++j) {
+        const int64_t slot = slot0 + j * 32;
+        const int64_t p = slot * VEC;
+        if constexpr (VEC > 1) {
+            if (p + VEC - 1 < n) {
+                ldg_stream_vec<VEC>(x + p, xs[j], stream_policy);
+                ldg_stream_vec<VEC>(y + p, ys[j], stream_policy);
+            } else {
+                // the array's tail: entries past n (never added) repeat the slot's first x
+#pragma unroll
+                for (int e = 0; e < VEC; ++e) {
+                    xs[j][e] = (p + e < n) ? __ldg(x + p + e) : (e ? xs[j][0] : (TX)0);
+                    ys[j][e] = (p + e < n) ? __ldg(y + p + e) : (TY)0;
+                }
+            }
+        } else {
+            xs[j][0] = (p < n) ? __ldg(x + p) : (TX)0;
+            ys[j][0] = (p < n) ? __ldg(y + p) : (TY)0;
+        }
+    }
+}
+
+// One slot whose points do not all lie in the warp's interval: the points of `valid` inside it join the register sums, which are
+// flushed; the warp adopts the interval of the highest lane's outside point (at least one lane must have one), and outside
+// points of any other interval go to global memory one by one.
+template <int K, int VEC>
+__device__ __forceinline__ void cross_interval(WarpAccum<K>& wa, const Mesh& mesh, const double (&xd)[VEC], const double (&yd)[VEC],
+                                               const bool (&valid)[VEC], const bool (&in)[VEC], double* __restrict__ G,
+                                               double* __restrict__ b, int M, int lane) {
+    int where[VEC];
+    bool pending = false, added_old = false;
+    int cand = -1;
+#pragma unroll
+    for (int e = 0; e < VEC; ++e) {
+        where[e] = -1;
+        if (valid[e]) {
+            if (in[e]) { wa.add(mesh, xd[e], yd[e]); added_old = true; }
+            else {
+                where[e] = locate_interval(mesh, xd[e], LdgLoader());
+                pending = true;
+                cand = where[e];
+            }
+        }
+    }
+    // (cur == -1 before the first point: nothing accumulated yet, nothing to flush)
+    wa.dirty = wa.dirty || __any_sync(0xffffffffu, added_old);
+    wa.flush(G, b, M, lane);
+    const unsigned pend = __ballot_sync(0xffffffffu, pending);   // non-zero here
+    const int src = 31 - __clz(pend);
+    wa.set_interval(mesh, __shfl_sync(0xffffffffu, cand, src));
+    bool added = false;
+#pragma unroll
+    for (int e = 0; e < VEC; ++e) {
+        if (where[e] >= 0) {
+            if (where[e] == wa.cur) { wa.add(mesh, xd[e], yd[e]); added = true; }
+            else scatter_point<K>(mesh, where[e], xd[e], yd[e], G, b, M);
+        }
+    }
+    wa.dirty = __any_sync(0xffffffffu, added);
+}
+
 // x and y hold float64 or float32 (TX, TY); the values stay in their own type until they are used and are converted to
 // double there (exact).  VEC = 2: both arrays are float64 and 16-byte aligned and are read as double2; VEC = 4: at least
 // one is float32, both are 16-byte aligned, a slot is 4 points (float4, or 2 x double2); VEC = 1: scalar loads
@@ -377,6 +443,176 @@ accum_1d_kernel(const TX* __restrict__ x, const TY* __restrict__ y, int64_t n,
         atomicAdd(scal, tot);
         if (blockIdx.x == 0) atomicAdd(scal + 1, (double)n);
     }
+}
+
+// Series of point p (0 <= p < offsets[S]): the largest s with offsets[s] <= p, which skips empty series.
+__device__ __forceinline__ int find_series(const int64_t* __restrict__ offsets, int S, int64_t p) {
+    int lo = 0, hi = S - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (__ldg(offsets + mid) <= p) lo = mid;
+        else hi = mid - 1;
+    }
+    return lo;
+}
+
+// S independent series concatenated in (x, y), series s being points offsets[s] .. offsets[s+1] - 1: accum_1d_kernel's tiles and
+// register sums, with one packed accumulator per series (acc + s * ((K+2) M + 2)).  A warp tracks the series of its points
+// (binary search for its first point, the series' end in a register).  A tile that lies inside the series runs accum_1d_kernel's
+// slots after one warp-uniform compare.  A tile in which the series ends is walked slot by slot: a slot that crosses the end
+// flushes the sums and sum(y^2) into that series, moves on to the series of the slot's last point and starts a new interval there;
+// the points of series that lie wholly inside the slot go to their own accumulators one by one.
+template <int K, int VEC, class TX, class TY>
+__global__ void __launch_bounds__(kAccumThreads, 2)
+accum_1d_segmented_kernel(const TX* __restrict__ x, const TY* __restrict__ y, int64_t n, const int64_t* __restrict__ offsets, int S,
+                          const double* __restrict__ knots, int n_knots, int M, double* __restrict__ acc) {
+    constexpr int U = accum_unroll<VEC, TX, TY>();
+    const Mesh mesh = load_mesh(knots, n_knots);
+    const int lane = threadIdx.x & 31;
+    const int warp = threadIdx.x >> 5;
+    constexpr int kWarps = kAccumThreads / 32;
+    const int64_t L = (int64_t)(K + 2) * M + 2;
+
+    const int64_t n_slots = (n + VEC - 1) / VEC;
+    const int64_t tile = 32 * U;
+    const int64_t n_tiles = (n_slots + tile - 1) / tile;
+    const int64_t tiles_per_cta = (n_tiles + gridDim.x - 1) / gridDim.x;
+    const int64_t t_begin = blockIdx.x * tiles_per_cta;
+    const int64_t t_end = imin64(t_begin + tiles_per_cta, n_tiles);
+    const int64_t my_tiles = t_end > t_begin ? t_end - t_begin : 0;
+    const int64_t per_warp = (my_tiles + kWarps - 1) / kWarps;
+    const int64_t w_begin = t_begin + warp * per_warp;
+    const int64_t w_end = imin64(w_begin + per_warp, t_end);
+
+    WarpAccum<K> wa;
+    wa.clear();
+    wa.cur = -1;
+    wa.u = 0.0;
+    wa.lo = INFINITY;
+    wa.hi = -INFINITY;
+    double yy = 0.0;
+    const uint64_t stream_policy = evict_first_policy();
+
+    int seg = -1;
+    int64_t seg_end = 0;
+    double* G = acc;
+    if (w_begin < w_end) {
+        seg = find_series(offsets, S, w_begin * tile * VEC);
+        seg_end = __ldg(offsets + seg + 1);
+        G = acc + seg * L;
+    }
+
+    for (int64_t tl = w_begin; tl < w_end; ++tl) {
+        TX xs[U][VEC];
+        TY ys[U][VEC];
+        const int64_t slot0 = tl * tile + lane;
+        load_tile<U, VEC>(x, y, n, slot0, xs, ys, stream_policy);
+        if (imin64((tl + 1) * tile * VEC, n) <= seg_end) {
+            // the tile lies inside the warp's series: accum_1d_kernel's slots
+#pragma unroll
+            for (int j = 0; j < U; ++j) {
+                const int64_t p = (slot0 + j * 32) * VEC;
+                double xd[VEC], yd[VEC];
+#pragma unroll
+                for (int e = 0; e < VEC; ++e) { xd[e] = (double)xs[j][e]; yd[e] = (double)ys[j][e]; }
+                bool valid[VEC], in[VEC];
+                bool all_in = true;
+#pragma unroll
+                for (int e = 0; e < VEC; ++e) {
+                    valid[e] = (p + e) < n;
+                    in[e] = wa.inside(xd[e]);
+                    all_in = all_in && (in[e] || !valid[e]);
+                    if (valid[e]) yy = fma(yd[e], yd[e], yy);
+                }
+                if (__all_sync(0xffffffffu, all_in)) {
+#pragma unroll
+                    for (int e = 0; e < VEC; ++e)
+                        if (valid[e]) wa.add(mesh, xd[e], yd[e]);
+                    wa.dirty = true;
+                } else {
+                    cross_interval<K, VEC>(wa, mesh, xd, yd, valid, in, G, G + (K + 1) * M, M, lane);
+                }
+            }
+            continue;
+        }
+        // a series ends inside the tile: slot by slot, not unrolled (one copy of this code), the points read again (cached)
+#pragma unroll 1
+        for (int j = 0; j < U; ++j) {
+            const int64_t p = (slot0 + j * 32) * VEC;
+            const int64_t slot_last = imin64((tl * tile + j * 32 + 32) * VEC, n) - 1;      // warp-uniform
+            double xd[VEC], yd[VEC];
+#pragma unroll
+            for (int e = 0; e < VEC; ++e) {
+                xd[e] = (p + e < n) ? (double)__ldg(x + p + e) : 0.0;
+                yd[e] = (p + e < n) ? (double)__ldg(y + p + e) : 0.0;
+            }
+            bool valid[VEC], in[VEC];
+            bool all_in = true;
+#pragma unroll
+            for (int e = 0; e < VEC; ++e) {
+                valid[e] = (p + e) < seg_end;
+                in[e] = wa.inside(xd[e]);
+                all_in = all_in && (in[e] || !valid[e]);
+                if (valid[e]) yy = fma(yd[e], yd[e], yy);
+            }
+            if (slot_last < seg_end) {
+                if (__all_sync(0xffffffffu, all_in)) {
+#pragma unroll
+                    for (int e = 0; e < VEC; ++e)
+                        if (valid[e]) wa.add(mesh, xd[e], yd[e]);
+                    wa.dirty = true;
+                } else {
+                    cross_interval<K, VEC>(wa, mesh, xd, yd, valid, in, G, G + (K + 1) * M, M, lane);
+                }
+                continue;
+            }
+            // the series ends in this slot: its points here join the sums (or, outside the interval, go one by one)
+            bool added_old = false;
+#pragma unroll
+            for (int e = 0; e < VEC; ++e) {
+                if (valid[e]) {
+                    if (in[e]) { wa.add(mesh, xd[e], yd[e]); added_old = true; }
+                    else scatter_point<K>(mesh, locate_interval(mesh, xd[e], LdgLoader()), xd[e], yd[e], G, G + (K + 1) * M, M);
+                }
+            }
+            wa.dirty = wa.dirty || __any_sync(0xffffffffu, added_old);
+            wa.flush(G, G + (K + 1) * M, M, lane);
+            yy = warp_sum(yy);
+            if (lane == 0) atomicAdd(G + (K + 2) * M, yy);
+            yy = 0.0;
+            // next series: that of the slot's last point (empty series are skipped by the search)
+            const int64_t old_end = seg_end;
+            seg = find_series(offsets, S, slot_last);
+            const int64_t seg_begin = __ldg(offsets + seg);
+            seg_end = __ldg(offsets + seg + 1);
+            G = acc + seg * L;
+            wa.cur = -1;
+            wa.lo = INFINITY;
+            wa.hi = -INFINITY;
+            bool mine[VEC], none[VEC];
+#pragma unroll
+            for (int e = 0; e < VEC; ++e) {
+                const int64_t q = p + e;
+                mine[e] = q >= seg_begin && q < n;
+                none[e] = false;
+                if (mine[e]) yy = fma(yd[e], yd[e], yy);
+                if (q >= old_end && q < seg_begin) {         // a series that lies wholly inside this slot
+                    double* Gs = acc + find_series(offsets, S, q) * L;
+                    scatter_point<K>(mesh, locate_interval(mesh, xd[e], LdgLoader()), xd[e], yd[e], Gs, Gs + (K + 1) * M, M);
+                    atomicAdd(Gs + (K + 2) * M, yd[e] * yd[e]);
+                }
+            }
+            // the lane holding the slot's last point has a point of the new series
+            cross_interval<K, VEC>(wa, mesh, xd, yd, mine, none, G, G + (K + 1) * M, M, lane);
+        }
+    }
+    wa.flush(G, G + (K + 1) * M, M, lane);
+    if (seg >= 0) {
+        yy = warp_sum(yy);
+        if (lane == 0) atomicAdd(G + (K + 2) * M, yy);
+    }
+    for (int64_t s = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; s < S; s += (int64_t)gridDim.x * blockDim.x)
+        acc[s * L + L - 1] += (double)(__ldg(offsets + s + 1) - __ldg(offsets + s));
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -563,21 +799,25 @@ __global__ void __launch_bounds__(256) order_probe_1d_kernel(const TX* __restric
 // instructions) and no gathers; lanes take consecutive pairs of points, loads and stores are fully coalesced 128-bit
 // accesses.  A lane whose points jump between intervals (unordered test sets) evaluates pieces and window entries
 // directly instead of refreshing its cache every time.  24 B of traffic per point.
-template <int K, int U, bool PREFETCH, int MINB>
-__global__ void __launch_bounds__(256, MINB) predict_1d_kernel(const double* __restrict__ xs, int64_t n, const double* __restrict__ knots,
-                                                         int n_knots, int M,
-                                                         const double* __restrict__ alpha,
-                                                         const double* __restrict__ S, double variance,
-                                                         double* __restrict__ mean, double* __restrict__ var) {
-    const Mesh mesh = load_mesh(knots, n_knots);
-    const MomentCoef<K>& mc = g_moment_coef<K>;
-    const bool vec = ((reinterpret_cast<uintptr_t>(xs) | reinterpret_cast<uintptr_t>(mean) | reinterpret_cast<uintptr_t>(var)) & 15u) == 0;
-
+// One lane's evaluator of the posterior (alpha, S, variance) with its interval cache; start() forgets the cache.
+template <int K>
+struct PredictPoint {
+    const double* alpha;
+    const double* S;
+    double variance;
+    int M;
     double cm[K + 1], cv[2 * K + 1];     // mean / variance polynomials (ascending powers of tau) of the cached interval
-    int cur = -1, since_refresh = 1 << 20;
-    double u = 0.0, lo = INFINITY, hi = -INFINITY;
+    int cur, since_refresh;
+    double u, lo, hi;
 
-    auto eval = [&](double x, double& mu, double& vv) {
+    __device__ __forceinline__ void start(const double* alpha_, const double* S_, double variance_, int M_) {
+        alpha = alpha_; S = S_; variance = variance_; M = M_;
+        cur = -1; since_refresh = 1 << 20;
+        u = 0.0; lo = INFINITY; hi = -INFINITY;
+    }
+
+    __device__ __forceinline__ void eval(const Mesh& mesh, double x, double& mu, double& vv) {
+        const MomentCoef<K>& mc = g_moment_coef<K>;
         if (x > lo && x <= hi) {
             const double tau = fma(x - u, mesh.inv_delta, -0.5);
             double m = cm[K];
@@ -644,7 +884,20 @@ __global__ void __launch_bounds__(256, MINB) predict_1d_kernel(const double* __r
         }
         mu = m;
         vv = variance + 2.0 * q;
-    };
+    }
+};
+
+template <int K, int U, bool PREFETCH, int MINB>
+__global__ void __launch_bounds__(256, MINB) predict_1d_kernel(const double* __restrict__ xs, int64_t n, const double* __restrict__ knots,
+                                                         int n_knots, int M,
+                                                         const double* __restrict__ alpha,
+                                                         const double* __restrict__ S, double variance,
+                                                         double* __restrict__ mean, double* __restrict__ var) {
+    const Mesh mesh = load_mesh(knots, n_knots);
+    const bool vec = ((reinterpret_cast<uintptr_t>(xs) | reinterpret_cast<uintptr_t>(mean) | reinterpret_cast<uintptr_t>(var)) & 15u) == 0;
+    PredictPoint<K> pp;
+    pp.start(alpha, S, variance, M);
+    auto eval = [&](double x, double& mu, double& vv) { pp.eval(mesh, x, mu, vv); };
 
     if (vec) {
         // every CTA walks its own contiguous range of pairs in tiles of 256 * U, so that for an ordered test set a lane's
@@ -700,6 +953,31 @@ __global__ void __launch_bounds__(256, MINB) predict_1d_kernel(const double* __r
     } else {
         const int64_t stride = (int64_t)gridDim.x * blockDim.x;
         for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += stride) eval(__ldg(xs + i), mean[i], var[i]);
+    }
+}
+
+// predict_1d_kernel's per-point evaluation for S posteriors at once: test points offsets[s] .. offsets[s+1] - 1 belong to series s
+// (alpha + s M, S + s (K+1) M, variance[s]).  Every CTA walks a contiguous range with coalesced scalar accesses; a lane looks its
+// series up again (and forgets its interval cache) whenever its point passes the current series' end.
+template <int K>
+__global__ void __launch_bounds__(256) predict_1d_segmented_kernel(const double* __restrict__ xs, int64_t n,
+                                                                   const int64_t* __restrict__ offsets, int S,
+                                                                   const double* __restrict__ knots, int n_knots, int M,
+                                                                   const double* __restrict__ alpha, const double* __restrict__ Sb,
+                                                                   const double* __restrict__ variance, double* __restrict__ mean,
+                                                                   double* __restrict__ var) {
+    const Mesh mesh = load_mesh(knots, n_knots);
+    const int64_t per_cta = (n + gridDim.x - 1) / gridDim.x;
+    const int64_t c_begin = blockIdx.x * per_cta, c_end = imin64(c_begin + per_cta, n);
+    PredictPoint<K> pp;
+    int64_t seg_end = -1;
+    for (int64_t i = c_begin + threadIdx.x; i < c_end; i += blockDim.x) {
+        if (i >= seg_end) {
+            const int s = find_series(offsets, S, i);
+            seg_end = __ldg(offsets + s + 1);
+            pp.start(alpha + (int64_t)s * M, Sb + (int64_t)s * (K + 1) * M, __ldg(variance + s), M);
+        }
+        pp.eval(mesh, __ldg(xs + i), mean[i], var[i]);
     }
 }
 
@@ -798,6 +1076,40 @@ extern "C" int asvgp_accum_1d(const double* x, const double* y, int64_t n, const
     return asvgp_accum_1d_typed(x, ASVGP_F64, y, ASVGP_F64, n, mesh, n_knots, order, acc, stream);
 }
 
+template <class TX, class TY>
+static int launch_accum_1d_segmented(const TX* x, const TY* y, int64_t n, const int64_t* offsets, int S, const double* mesh,
+                                     int n_knots, int order, double* acc, cudaStream_t st) {
+    const int M = n_knots + order - 1;
+    const bool vec = ((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) & 15u) == 0;
+    constexpr int VV = (sizeof(TX) == 8 && sizeof(TY) == 8) ? 2 : 4;
+    const int64_t per_tile = 32 * (vec ? (int64_t)accum_unroll<VV, TX, TY>() * VV : (int64_t)accum_unroll<1, TX, TY>());
+    const int64_t n_tiles = (n + per_tile - 1) / per_tile;
+    // the grid of launch_accum_1d; at least one CTA, whose grid-stride loop writes the counts
+    const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>((n_tiles + 7) / 8, (int64_t)accum_sm_budget() * 2));
+    if (vec) {
+        ASVGP_DISPATCH_ORDER(order, (accum_1d_segmented_kernel<K, VV, TX, TY><<<blocks, kAccumThreads, 0, st>>>(x, y, n, offsets, S, mesh, n_knots, M, acc))); ASVGP_LAUNCHED();
+    } else {
+        ASVGP_DISPATCH_ORDER(order, (accum_1d_segmented_kernel<K, 1, TX, TY><<<blocks, kAccumThreads, 0, st>>>(x, y, n, offsets, S, mesh, n_knots, M, acc))); ASVGP_LAUNCHED();
+    }
+    ASVGP_CUDA_OK(cudaGetLastError());
+    return kOk;
+}
+
+extern "C" int asvgp_accum_1d_segmented_typed(const void* x, int x_type, const void* y, int y_type, int64_t n, const int64_t* offsets,
+                                              int S, const double* mesh, int n_knots, int order, double* acc, void* stream) {
+    ASVGP_REQUIRE_TYPES("accum_1d_segmented", x_type, y_type);
+    ASVGP_REQUIRE(S >= 1, "accum_1d_segmented: S=%d must be at least 1", S);
+    ASVGP_REQUIRE(n >= 0 && n_knots >= 2, "accum_1d_segmented: n=%lld n_knots=%d", (long long)n, n_knots);
+    ASVGP_REQUIRE(order >= 1 && order <= kMaxOrder, "accum_1d_segmented: spline order %d not in 1..6", order);
+    ASVGP_REQUIRE(offsets != nullptr, "accum_1d_segmented: offsets is NULL");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    return with_elem_types(x_type, y_type, [&](auto tx, auto ty) -> int {
+        using TX = typename decltype(tx)::type;
+        using TY = typename decltype(ty)::type;
+        return launch_accum_1d_segmented(static_cast<const TX*>(x), static_cast<const TY*>(y), n, offsets, S, mesh, n_knots, order, acc, st);
+    });
+}
+
 extern "C" int64_t asvgp_accum_1d_binned_work_bytes(int64_t n) { return PartWork::bytes(n < 0 ? 0 : n, 2); }
 
 extern "C" int asvgp_order_probe_1d_typed(const void* x, int x_type, int64_t n, const double* mesh, int n_knots, double* out,
@@ -886,6 +1198,24 @@ extern "C" int asvgp_predict_1d(const double* xnew, int64_t n, const double* mes
     // (tools/microbench/rw12_bench.cu: 5.4 TB/s) — against 0.69 ms for 4 prefetched pairs at 80+ registers on 4 CTAs per SM.
     const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>((n + 4095) / 4096, (int64_t)sm_count() * 128));
     ASVGP_DISPATCH_ORDER(order, (predict_1d_kernel<K, 2, false, 4><<<blocks, 256, 0, st>>>(xnew, n, mesh, n_knots, M, alpha, S_band, variance, mean, var)));
+    ASVGP_LAUNCHED();
+    ASVGP_CUDA_OK(cudaGetLastError());
+    return kOk;
+}
+
+extern "C" int asvgp_predict_1d_segmented(const double* xnew, int64_t n, const int64_t* offsets_new, int S, const double* mesh,
+                                          int n_knots, int order, const double* alpha, const double* S_band, const double* variance,
+                                          double* mean, double* var, void* stream) {
+    ASVGP_REQUIRE(S >= 1, "predict_1d_segmented: S=%d must be at least 1", S);
+    ASVGP_REQUIRE(n >= 0 && n_knots >= 2, "predict_1d_segmented: n=%lld n_knots=%d", (long long)n, n_knots);
+    ASVGP_REQUIRE(order >= 1 && order <= kMaxOrder, "predict_1d_segmented: spline order %d not in 1..6", order);
+    ASVGP_REQUIRE(offsets_new != nullptr, "predict_1d_segmented: offsets_new is NULL");
+    if (n == 0) return kOk;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int M = n_knots + order - 1;
+    const int blocks = (int)std::max<int64_t>(1, std::min<int64_t>((n + 4095) / 4096, (int64_t)sm_count() * 128));
+    ASVGP_DISPATCH_ORDER(order, (predict_1d_segmented_kernel<K><<<blocks, 256, 0, st>>>(xnew, n, offsets_new, S, mesh, n_knots, M, alpha,
+                                                                                     S_band, variance, mean, var)));
     ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     return kOk;

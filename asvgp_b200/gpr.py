@@ -300,6 +300,154 @@ class GPR_1d(_ModelBase):
         return mean.cpu().numpy(), var.cpu().numpy()
 
 
+class GPR_1d_many:
+    """S independent 1-D regressions (GPR_1d each) that share one B-spline basis and one Matern kind, fitted together.
+
+    data = (X[N, 1], y[N] or y[N, 1]) holds all series concatenated, sorted by series: series s is rows offsets[s] ..
+    offsets[s+1] - 1 (offsets: host array or tensor of S + 1 integers, 0 first, non-decreasing, N last; empty series are
+    allowed).  X and y are CUDA tensors or host arrays (copied to the device once), float32 or float64.  One O(N) pass fills one
+    packed accumulator per series (asvgp_accum_1d_segmented); every later step evaluates up to 64 series per batch of launches,
+    each slot reading its own series' accumulator, with the bits of GPR_1d on that series alone.
+
+    Per-series parameters are the unconstrained array U[S, 3] in the order (variance, lengthscale, sigma2), initialised from the
+    template `kernel` and Gaussian() (or from U0); `variance`, `lengthscales` and `noise_variance` read them back constrained.
+    An empty series has ELBO 0, gradient 0 and predicts the prior."""
+
+    def __init__(self, data, offsets, kernel, basis, check_inputs=True, chunks=0, U0=None):
+        if _dist.is_distributed("auto"):
+            raise NotImplementedError("GPR_1d_many runs on one GPU; torch.distributed is initialised with world size > 1")
+        self._kind = kernel_kind(kernel)
+        X, y = data
+        if X.ndim == 2:
+            assert X.shape[1] == 1
+        if y.ndim == 2 and y.shape[1] != 1:
+            raise NotImplementedError("GPR_1d_many takes one output column per series")
+        n = int(X.shape[0])
+        if int(y.shape[0]) != n:
+            raise ValueError("X and y must have the same number of rows")
+        self._offsets = ops.validate_offsets(offsets, n)
+        self.num_series = S = self._offsets.size - 1
+        self._counts = np.diff(self._offsets)
+        if check_inputs and n:
+            lo, hi = (torch.aminmax(X) if isinstance(X, torch.Tensor) else (X.min(), X.max()))
+            assert float(lo) > basis.a
+            assert float(hi) < basis.b
+        self.kernel = kernel
+        self.basis = basis
+        self.inducing_features = SplineFeatures1D(kernel, basis)
+        self._chunks = chunks
+        # transforms of the three per-series parameters (value_at / dvalue_dunconstrained_at of these templates)
+        self._params = [Parameter(hyper_value(kernel.variance), name="variance"),
+                        Parameter(hyper_value(kernel.lengthscales), name="lengthscales"), Gaussian().variance]
+        if U0 is None:
+            self.U = np.tile([p.unconstrained for p in self._params], (S, 1))
+        else:
+            self.U = np.array(U0, dtype=np.float64)
+            if self.U.shape != (S, 3) or not np.isfinite(self.U).all():
+                raise ValueError("U0 must be finite [%d, 3], got shape %s" % (S, self.U.shape))
+        self._acc = ops.accum_1d_segmented(X.reshape(-1), y.reshape(-1), self._offsets, basis)
+
+    def _values(self, U):
+        return np.array([[p.value_at(float(u)) for p, u in zip(self._params, row)] for row in U]).reshape(-1, 3)
+
+    @property
+    def variance(self):
+        return self._values(self.U)[:, 0]
+
+    @property
+    def lengthscales(self):
+        return self._values(self.U)[:, 1]
+
+    @property
+    def noise_variance(self):
+        return self._values(self.U)[:, 2]
+
+    def _evaluate(self, U, ids):
+        """(loss[n], grad[n, 3], info[n]) of series ids[i] at unconstrained U[i]: -ELBO and its gradient in U, as
+        GPR_1d.training_loss_and_gradients on that series alone.  A failed factorisation gives loss +inf, NaN gradients and its
+        pivot in info; an empty series gives 0, 0."""
+        U = np.asarray(U, dtype=np.float64).reshape(-1, 3)
+        ids = np.asarray(ids, dtype=np.int64).reshape(-1)
+        n = ids.size
+        loss, grad, info = np.zeros(n), np.zeros((n, 3)), np.zeros(n, dtype=np.int64)
+        live = np.flatnonzero(self._counts[ids] > 0)
+        outs = []
+        for c in range(0, live.size, _lib.MAX_BATCH):
+            sel = live[c: c + _lib.MAX_BATCH]
+            vals = self._values(U[sel])
+            Kuu, dKuu = self.inducing_features.make_Kuu_device_batched(self.kernel, vals[:, 1], vals[:, 0], want_grad=True)
+            outs.append(ops.elbo_grad_1d_batched(Kuu, dKuu, self._acc, self.basis, vals[:, 0], vals[:, 2], chunks=self._chunks,
+                                                 rows=ids[sel])[:, 0])
+        if not outs:
+            return loss, grad, info
+        out = torch.cat(outs).cpu().numpy()           # one device-to-host copy per call
+        for i, b in enumerate(live):
+            o = out[i]
+            if o[8] != 0:
+                loss[b], grad[b], info[b] = np.inf, np.nan, int(o[8])
+                continue
+            loss[b] = -float(o[0])
+            grad[b] = [-(o[1 + j] * p.dvalue_dunconstrained_at(float(u))) for j, (p, u) in enumerate(zip(self._params, U[b]))]
+        return loss, grad, info
+
+    def training_loss_and_gradients(self):
+        """(loss[S], grad[S, 3], info[S]) at the current U: -ELBO of every series and its gradient in U."""
+        return self._evaluate(self.U, np.arange(self.num_series))
+
+    def elbo(self):
+        """ELBO of every series [S] (-inf where the factorisation fails)."""
+        return -self.training_loss_and_gradients()[0]
+
+    def optimize(self, method="L-BFGS-B", wave=256, **scipy_kwargs):
+        """One L-BFGS-B (scipy) per series from the current U, in waves of at most `wave` series whose runs advance in lockstep
+        (lockstep_minimize): each round evaluates the running series 64 at a time.  Every run takes the iterates of a serial
+        run on its series.  A failing series ends with fun = +inf and keeps its starting U; the others go on.  Sets U and
+        returns the S results."""
+        from .optimizers import lockstep_minimize
+
+        S = self.num_series
+        results = [None] * S
+        for w0 in range(0, S, int(wave)):
+            ids = np.arange(w0, min(S, w0 + int(wave)))
+            res = lockstep_minimize(lambda Uw, idx, ids=ids: self._evaluate(Uw, ids[idx]), self.U[ids], method=method,
+                                    pass_ids=True, **scipy_kwargs)
+            for s, r in zip(ids, res):
+                results[s] = r
+                if np.isfinite(r.fun):
+                    self.U[s] = r.x
+        return results
+
+    def posterior_weights(self):
+        """(alpha [S, m], S_band [S, k+1, m], info [S, 2]) on the device at the current U (zeros for empty series)."""
+        k, m, S = self.basis.order, self.basis.m, self.num_series
+        dev = self._acc.device
+        alpha = torch.zeros((S, m), dtype=torch.float64, device=dev)
+        S_band = torch.zeros((S, k + 1, m), dtype=torch.float64, device=dev)
+        info = torch.zeros((S, 2), dtype=torch.float64, device=dev)
+        live = np.flatnonzero(self._counts > 0)
+        for c in range(0, live.size, _lib.MAX_BATCH):
+            sel = live[c: c + _lib.MAX_BATCH]
+            vals = self._values(self.U[sel])
+            Kuu, _ = self.inducing_features.make_Kuu_device_batched(self.kernel, vals[:, 1], vals[:, 0], want_grad=False)
+            a, sb, inf = ops.posterior_1d_batched(Kuu, self._acc, self.basis, vals[:, 2], sel, chunks=self._chunks)
+            idx = torch.from_numpy(sel).to(dev)
+            alpha[idx], S_band[idx], info[idx] = a, sb, inf
+        return alpha, S_band, info
+
+    def predict_f(self, Xnew, offsets_new):
+        """Posterior mean (n*, 1) and variance (n*, 1) of every series at its test points: rows offsets_new[s] ..
+        offsets_new[s+1] - 1 of Xnew belong to series s.  numpy in -> numpy out, CUDA tensor in -> CUDA tensors out."""
+        alpha, S_band, info = self.posterior_weights()
+        variances = torch.from_numpy(self.variance).to(alpha.device)
+        mean, var = ops.predict_1d_segmented(ops.to_device(Xnew).reshape(-1), offsets_new, self.basis, alpha, S_band, variances)
+        if info.any().item():
+            raise np.linalg.LinAlgError("banded Cholesky failed in predict_f")
+        mean, var = mean.view(-1, 1), var.view(-1, 1)
+        if isinstance(Xnew, torch.Tensor) and Xnew.is_cuda:
+            return mean, var
+        return mean.cpu().numpy(), var.cpu().numpy()
+
+
 def _kron_column_bound(N, s2, v, m1, m2, sc1, sc2, logdetP, Q, yy, T, want_grad):
     """ELBO of the Kronecker model for one output column and, with want_grad, its derivatives [v1, l1, v2, l2, sigma2];
     sc_i = {log|K_i|, dlog|K_i|, ...}, T = the 11 slots of asvgp_kron_terms.  Returns (elbo, grads or None, log|Kuu|)."""

@@ -146,6 +146,48 @@ def accum_1d(x, y, basis, acc=None, binned=False):
     return acc
 
 
+def validate_offsets(offsets, n, what="offsets"):
+    """Host check of series offsets over n concatenated points: a 1-D integer array [S+1] (numpy, list or tensor on any device),
+    S >= 1, offsets[0] = 0, non-decreasing, offsets[S] = n.  Returns it as a numpy int64 array."""
+    if isinstance(offsets, torch.Tensor):
+        if offsets.dtype.is_floating_point or offsets.dtype.is_complex or offsets.dtype == torch.bool:
+            raise TypeError("%s must hold integers, got %s" % (what, offsets.dtype))
+        offsets = offsets.detach().cpu().numpy()
+    arr = np.asarray(offsets)
+    if arr.dtype.kind not in "iu":
+        raise TypeError("%s must hold integers, got %s" % (what, arr.dtype))
+    if arr.ndim != 1 or arr.size < 2:
+        raise ValueError("%s must be a 1-D array of S + 1 >= 2 entries, got shape %s" % (what, arr.shape))
+    arr = arr.astype(np.int64)
+    if arr[0] != 0 or arr[-1] != n:
+        raise ValueError("%s must start at 0 and end at the number of points %d, got %d ... %d" % (what, n, arr[0], arr[-1]))
+    if (np.diff(arr) < 0).any():
+        raise ValueError("%s must be non-decreasing" % what)
+    return np.ascontiguousarray(arr)
+
+
+def accum_1d_segmented(x, y, offsets, basis, acc=None):
+    """accum_1d for S independent series concatenated in (x, y) (series s = points offsets[s] .. offsets[s+1] - 1, each sorted
+    for speed, any order exact): adds series s into row s of acc [S, L] (allocated zeroed if None) in one launch.  offsets is
+    validated on the host (validate_offsets) and copied to the device; x and y as for accum_1d."""
+    x, xt = points_to_device(x)
+    y, yt = points_to_device(y)
+    x, y = x.reshape(-1), y.reshape(-1)
+    if x.numel() != y.numel():
+        raise ValueError("x and y must have the same number of points")
+    h_off = validate_offsets(offsets, x.numel())
+    S = h_off.size - 1
+    mesh = device_mesh(basis)
+    if acc is None:
+        acc = torch.zeros((S, accum_size_1d(basis)), dtype=F64, device=x.device)
+    elif tuple(acc.shape) != (S, accum_size_1d(basis)) or not acc.is_contiguous():
+        raise ValueError("acc must be contiguous [%d, %d]" % (S, accum_size_1d(basis)))
+    d_off = torch.from_numpy(h_off).to(x.device)
+    _lib.call("asvgp_accum_1d_segmented_typed", _p(x), xt, _p(y), yt, x.numel(), _p(d_off), S, _p(mesh), mesh.numel(), basis.order,
+              _p(acc), _stream())
+    return acc
+
+
 def split_accum_1d(acc, basis):
     """Views (G_band (k+1, M), b (M,), scal (2,)) into the packed accumulator."""
     k, m = basis.order, basis.m
@@ -166,6 +208,29 @@ def predict_1d(xnew, basis, alpha, S_band, variance, mean=None, var=None):
         var = torch.empty(n, dtype=F64, device=x.device)
     _lib.call("asvgp_predict_1d", _p(x), n, _p(mesh), mesh.numel(), basis.order, _p(alpha), _p(S_band),
               float(variance), _p(mean), _p(var), _stream())
+    return mean, var
+
+
+def predict_1d_segmented(xnew, offsets_new, basis, alpha, S_band, variances):
+    """predict_1d for S series in one launch: test points offsets_new[s] .. offsets_new[s+1] - 1 of xnew use alpha [S, m],
+    S_band [S, k+1, m] and variances [S] of series s.  Returns (mean, var) [n*] on the device."""
+    x = to_device(xnew).reshape(-1)
+    n = x.numel()
+    h_off = validate_offsets(offsets_new, n, "offsets_new")
+    S = h_off.size - 1
+    k, m = basis.order, basis.m
+    alpha = to_device(alpha)
+    S_band = to_device(S_band)
+    variances = to_device(variances).reshape(-1)
+    if tuple(alpha.shape) != (S, m) or tuple(S_band.shape) != (S, k + 1, m) or variances.numel() != S:
+        raise ValueError("predict_1d_segmented: alpha %s, S_band %s, %d variances for S = %d series"
+                         % (tuple(alpha.shape), tuple(S_band.shape), variances.numel(), S))
+    mesh = device_mesh(basis)
+    mean = torch.empty(n, dtype=F64, device=x.device)
+    var = torch.empty(n, dtype=F64, device=x.device)
+    d_off = torch.from_numpy(h_off).to(x.device)
+    _lib.call("asvgp_predict_1d_segmented", _p(x), n, _p(d_off), S, _p(mesh), mesh.numel(), k, _p(alpha), _p(S_band), _p(variances),
+              _p(mean), _p(var), _stream())
     return mean, var
 
 
@@ -244,29 +309,70 @@ def workspace_1d_batched(m, order, chunks, B, D):
     return ws
 
 
-def elbo_grad_1d_batched(Kuu, dKuu, accs, basis, variances, sigma2s, chunks=0, out=None):
+def elbo_grad_1d_batched(Kuu, dKuu, accs, basis, variances, sigma2s, chunks=0, out=None, rows=None):
     """B settings of the bound in one stream of launches: Kuu, dKuu [B, k+1, m] (kuu_assemble_batched), accs [D, L] (D
     packed accumulators, or one [L]), variances / sigma2s [B] on the host.  Returns out [B, D, 16] on the device; out[b, d]
-    equals elbo_grad_1d of slot b and column d bit for bit in slots 0..8 and 15 (see include/asvgp_b200.h)."""
+    equals elbo_grad_1d of slot b and column d bit for bit in slots 0..8 and 15 (see include/asvgp_b200.h).
+    rows [B] (host ints): slot b reads accumulator row rows[b] of accs [R, L] (or [R, D, L] with D columns each), e.g. one row
+    per series of accum_1d_segmented; None is the call above."""
     k, m = basis.order, basis.m
-    accs = accs.reshape(1, -1) if accs.dim() == 1 else accs
+    L = accum_size_1d(basis)
     variances = np.ascontiguousarray(variances, dtype=np.float64).reshape(-1)
     sigma2s = np.ascontiguousarray(sigma2s, dtype=np.float64).reshape(-1)
-    B, D = variances.size, accs.shape[0]
+    B = variances.size
+    if rows is None:
+        accs = accs.reshape(1, -1) if accs.dim() == 1 else accs
+        R, D = 1, accs.shape[0]
+        h_rows = np.zeros(B, dtype=np.int64)
+    else:
+        accs = accs.reshape(accs.shape[0], 1, -1) if accs.dim() == 2 else accs
+        R, D = accs.shape[0], accs.shape[1]
+        h_rows = np.ascontiguousarray(rows, dtype=np.int64).reshape(-1)
+        if h_rows.size != B or (B and (h_rows.min() < 0 or h_rows.max() >= R)):
+            raise ValueError("elbo_grad_1d_batched: rows must be %d indices in 0..%d" % (B, R - 1))
     if sigma2s.size != B or tuple(Kuu.shape) != (B, k + 1, m) or tuple(dKuu.shape) != (B, k + 1, m):
         raise ValueError("elbo_grad_1d_batched: %d variances, %d sigma2s, Kuu %s, dKuu %s" % (B, sigma2s.size, tuple(Kuu.shape),
                                                                                             tuple(dKuu.shape)))
-    if accs.shape[1] != accum_size_1d(basis) or not accs.is_contiguous():
-        raise ValueError("elbo_grad_1d_batched: accs must be contiguous [D, %d]" % accum_size_1d(basis))
+    if accs.shape[-1] != L or not accs.is_contiguous():
+        raise ValueError("elbo_grad_1d_batched: accs must be contiguous [D, %d]" % L)
     if not 1 <= B <= _lib.MAX_BATCH or not 1 <= D <= _lib.MAX_BATCH_COLUMNS:
         raise ValueError("elbo_grad_1d_batched: B=%d not in 1..%d or D=%d not in 1..%d"
                          % (B, _lib.MAX_BATCH, D, _lib.MAX_BATCH_COLUMNS))
     ws = workspace_1d_batched(m, k, int(chunks), B, D)
     if out is None:
         out = torch.empty((B, D, 16), dtype=F64, device=accs.device)
-    _lib.call("asvgp_elbo_grad_1d_batched", _p(Kuu), _p(dKuu), _p(accs), m, k, B, D, ctypes.c_void_p(variances.ctypes.data),
-              ctypes.c_void_p(sigma2s.ctypes.data), int(chunks), _p(out), _p(ws), ws.numel(), _stream())
+    _lib.call("asvgp_elbo_grad_1d_batched_rows", _p(Kuu), _p(dKuu), _p(accs), R, ctypes.c_void_p(h_rows.ctypes.data), m, k, B, D,
+              ctypes.c_void_p(variances.ctypes.data), ctypes.c_void_p(sigma2s.ctypes.data), int(chunks), _p(out), _p(ws), ws.numel(),
+              _stream())
     return out
+
+
+def posterior_1d_batched(Kuu, accs, basis, sigma2s, rows, chunks=0):
+    """posterior_1d for B slots: Kuu [B, k+1, m], sigma2s [B] (host), slot b on accumulator row rows[b] of accs [R, L].  Returns
+    (alpha [B, m], S [B, k+1, m], info [B, 2]) on the device; slot b equals posterior_1d on its operands bit for bit."""
+    k, m = basis.order, basis.m
+    sigma2s = np.ascontiguousarray(sigma2s, dtype=np.float64).reshape(-1)
+    h_rows = np.ascontiguousarray(rows, dtype=np.int64).reshape(-1)
+    B, R = sigma2s.size, accs.shape[0]
+    if accs.dim() != 2 or accs.shape[1] != accum_size_1d(basis) or not accs.is_contiguous():
+        raise ValueError("posterior_1d_batched: accs must be contiguous [R, %d]" % accum_size_1d(basis))
+    if not 1 <= B <= _lib.MAX_BATCH or h_rows.size != B or tuple(Kuu.shape) != (B, k + 1, m):
+        raise ValueError("posterior_1d_batched: %d sigma2s (1..%d), %d rows, Kuu %s" % (B, _lib.MAX_BATCH, h_rows.size,
+                                                                                      tuple(Kuu.shape)))
+    dev = device()
+    key = (dev, m, k, int(chunks), "posterior", B)
+    ws = _WORKSPACES.get(key)
+    if ws is None:
+        nbytes = _lib.load().asvgp_workspace_bytes_posterior_1d_batched(m, k, int(chunks), B)
+        if nbytes < 0:
+            raise _lib.AsvgpNativeError("asvgp_workspace_bytes_posterior_1d_batched rejected m=%d order=%d B=%d" % (m, k, B))
+        ws = _WORKSPACES[key] = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+    alpha = torch.empty((B, m), dtype=F64, device=accs.device)
+    S = torch.empty((B, k + 1, m), dtype=F64, device=accs.device)
+    info = torch.zeros((B, 2), dtype=F64, device=accs.device)
+    _lib.call("asvgp_posterior_1d_batched", _p(Kuu), _p(accs), R, ctypes.c_void_p(h_rows.ctypes.data), m, k, B,
+              ctypes.c_void_p(sigma2s.ctypes.data), int(chunks), _p(alpha), _p(S), _p(info), _p(ws), ws.numel(), _stream())
+    return alpha, S, info
 
 
 class KuuChain:

@@ -21,13 +21,15 @@ def _same_on_every_rank(u):
     return t.cpu().numpy()
 
 
-def lockstep_minimize(fun_batch, starts, method="L-BFGS-B", **scipy_kwargs):
+def lockstep_minimize(fun_batch, starts, method="L-BFGS-B", pass_ids=False, **scipy_kwargs):
     """One scipy.optimize.minimize per row of starts[B, n], advanced in lockstep: each run lives in a worker thread whose
     objective posts its point and blocks; once every run still going has posted, fun_batch(U[b', n]) evaluates them all
     at once and returns (loss[b'], grad[b', n], info[b']).  A run sees exactly the values a serial run would, so its iterates
     are those of the serial run from the same start.  Line-search evaluations are simply more rounds; a finished run leaves
     the rounds.  A row with info != 0 raises numpy.linalg.LinAlgError inside that run's objective (as a failing serial
-    evaluation does); the run ends with success=False and fun=+inf while the others go on.  Returns the B results."""
+    evaluation does); the run ends with success=False and fun=+inf while the others go on.  Returns the B results.
+    pass_ids=True: fun_batch(U, ids) also receives the run indices (rows of starts) of the rows of U, for objectives that
+    differ from run to run (one model per run)."""
     starts = np.array(starts, dtype=np.float64, ndmin=2)
     B = starts.shape[0]
     cv = threading.Condition()
@@ -76,7 +78,7 @@ def lockstep_minimize(fun_batch, starts, method="L-BFGS-B", **scipy_kwargs):
         try:
             if error is not None:
                 raise error
-            loss, grad, info = fun_batch(U)
+            loss, grad, info = fun_batch(U, np.array(ids)) if pass_ids else fun_batch(U)
             reply = {b: (float(loss[i]), np.array(grad[i], dtype=np.float64), int(info[i])) for i, b in enumerate(ids)}
         except BaseException as e:      # stop every run, then re-raise
             error = e

@@ -171,6 +171,45 @@ ASVGP_API int asvgp_elbo_grad_1d_batched(const double* Kuu, const double* dKuu, 
                                          const double* h_variance, const double* h_sigma2, int chunks, double* out, void* work,
                                          int64_t work_bytes, void* stream);
 
+/* ---- many independent series on one basis -----------------------------------------------------------------------------------
+ * S series of 1-D data share the basis (mesh, order) but nothing else.  They travel concatenated: x[n], y[n] hold all points,
+ * series s being points offsets[s] .. offsets[s+1] - 1, with offsets[S+1] int64, offsets[0] = 0, non-decreasing and
+ * offsets[S] = n (the library does not check this contract; the Python layer does, on the host).  Empty series are allowed.
+ *
+ * asvgp_accum_1d_segmented_typed: asvgp_accum_1d_typed for every series at once.  acc holds S packed accumulators
+ * ([S][(order+2) M + 2], layout of asvgp_accum_1d); series s's points are added into row s (nothing is zeroed), its count slot
+ * receives offsets[s+1] - offsets[s].  Any order within a series is exact; sorted order is fast, as for asvgp_accum_1d.  x / y
+ * element types as for asvgp_accum_1d_typed.  `offsets` is a DEVICE array.  S < 1 and unknown type codes are rejected before
+ * any CUDA call.
+ *
+ * asvgp_elbo_grad_1d_batched_rows: asvgp_elbo_grad_1d_batched where slot b reads accumulator row h_row[b] of acc[R][D][L]
+ * (column d of slot b at acc + (h_row[b] D + d) L, L = (order+2) M + 2).  h_row is a HOST array [B] of rows in 0..R-1 (repeats
+ * allowed).  out[b][d][0..8] and [15] equal asvgp_elbo_grad_1d on (Kuu[b], dKuu[b], row h_row[b] column d, v_b, sigma2_b) bit for
+ * bit, whatever B, the rows and the other slots.  asvgp_elbo_grad_1d_batched is this call with R = 1 and every row 0.  A row out
+ * of range, a NULL h_row and the range checks of asvgp_elbo_grad_1d_batched are rejected before any CUDA call.
+ *
+ * asvgp_posterior_1d_batched: asvgp_posterior_1d for B slots (Kuu[B][order+1][M], sigma2_b from the HOST array h_sigma2[B],
+ * accumulator row h_row[b] of acc[R][L]); alpha[B][M], S_band[B][order+1][M], info[B][2].  Slot b equals asvgp_posterior_1d on
+ * its operands bit for bit; a failing slot reports its pivot in its own info and leaves the others untouched.  B lies in
+ * 1..ASVGP_MAX_BATCH; the workspace needs asvgp_workspace_bytes_posterior_1d_batched(M, order, chunks, B) bytes (-1 for
+ * arguments out of range).  asvgp_posterior_1d is the one-slot case.
+ *
+ * asvgp_predict_1d_segmented: asvgp_predict_1d per series: test points offsets_new[s] .. offsets_new[s+1] - 1 (DEVICE int64
+ * [S+1], same contract as above) use alpha[s] of [S][M], S_band[s] of [S][order+1][M] and variance[s] of the DEVICE array
+ * variance[S].  The per-point arithmetic is asvgp_predict_1d's. */
+ASVGP_API int asvgp_accum_1d_segmented_typed(const void* x, int x_type, const void* y, int y_type, int64_t n, const int64_t* offsets,
+                                             int S, const double* mesh, int n_knots, int order, double* acc, void* stream);
+ASVGP_API int asvgp_elbo_grad_1d_batched_rows(const double* Kuu, const double* dKuu, const double* acc, int R, const int64_t* h_row,
+                                              int M, int order, int B, int D, const double* h_variance, const double* h_sigma2,
+                                              int chunks, double* out, void* work, int64_t work_bytes, void* stream);
+ASVGP_API int64_t asvgp_workspace_bytes_posterior_1d_batched(int M, int order, int chunks, int B);
+ASVGP_API int asvgp_posterior_1d_batched(const double* Kuu, const double* acc, int R, const int64_t* h_row, int M, int order, int B,
+                                         const double* h_sigma2, int chunks, double* alpha, double* S_band, double* info, void* work,
+                                         int64_t work_bytes, void* stream);
+ASVGP_API int asvgp_predict_1d_segmented(const double* xnew, int64_t n, const int64_t* offsets_new, int S, const double* mesh,
+                                         int n_knots, int order, const double* alpha, const double* S_band, const double* variance,
+                                         double* mean, double* var, void* stream);
+
 /* ---- a10 (factorisation half): posterior weights -------------------------------------------------------------------------
  * Replaces the CHOLMOD factorisations and solves of GPR_1d.predict_f (gpr.py:96-108):
  * alpha = P^-1 Kuf_y / sigma2 and S = band(P^-1) - band(Kuu^-1), P = Kuu + G / sigma2.  info[2] (device): failing
