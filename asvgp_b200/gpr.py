@@ -18,11 +18,40 @@ from . import _lib
 from . import dist as _dist
 from . import ops
 from .inducing_features import SplineFeatures1D
+from .ops import Bound1D
 from .kernels import Gaussian, Parameter, hyper_value, kernel_kind
 
 
 class _ModelBase:
     """The slice of gpflow.models.GPModel + InternalDataTrainingLossMixin the reference's scripts use."""
+
+    _host = None
+
+    def _device_stats(self):
+        """(G, Kuf_y [D, M], sum(y_d^2) [D], N) of the D output columns as device tensors; G is the model's own form of KufKfu."""
+        raise NotImplementedError
+
+    # -- the reference's cached attributes (host copies, fetched lazily) --------------------------------------
+    def _host_stats(self):
+        if self._host is None:
+            G, B, yy, n = (t.cpu().numpy() for t in self._device_stats())
+            self._host = (G, np.ascontiguousarray(B.T), float(yy.sum()), int(n))
+        return self._host
+
+    @property
+    def Kuf_y(self):
+        """(M, D): one column per output column."""
+        return self._host_stats()[1]
+
+    @property
+    def tr_yTy(self):
+        """sum(y^2) over all output columns (reference gpr.py:78-79)."""
+        return self._host_stats()[2]
+
+    @property
+    def num_data(self):
+        """Global number of datapoints (all shards)."""
+        return self._host_stats()[3]
 
     def maximum_log_likelihood_objective(self):
         return self.elbo()
@@ -68,6 +97,65 @@ def _to_numpy(a):
     return a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else a
 
 
+def _like_input(Xnew, mean, var):
+    """(mean, var) as they are for a CUDA tensor Xnew, else as numpy arrays."""
+    if isinstance(Xnew, torch.Tensor) and Xnew.is_cuda:
+        return mean, var
+    return mean.cpu().numpy(), var.cpu().numpy()
+
+
+def _check_domain(X, bases):
+    """Every column i of X[n, d] lies strictly inside the domain of bases[i] (reference gpr.py:22-26); AssertionError if not."""
+    for i, basis in enumerate(bases):
+        col = X[:, i]
+        lo, hi = (torch.aminmax(col) if isinstance(col, torch.Tensor) else (col.min(), col.max()))
+        assert float(lo) > basis.a and float(hi) < basis.b, "inputs must lie strictly inside the basis domain"
+
+
+def _output_columns(y, model, most, error=ValueError):
+    """y[n] or y[n, D] as (y[n, D], D); D outside 1 ... most raises `error`."""
+    if y.ndim == 1:
+        y = y.reshape(-1, 1)
+    D = int(y.shape[1])
+    if not 1 <= D <= most:
+        raise error("%s takes 1 ... %d output columns, got %d" % (model, most, D))
+    return y, D
+
+
+def _combine_columns(values, infos, shared):
+    """The bound of D output columns from their single-column bounds: row values[d] (1 + G entries) holds column d's ELBO and,
+    if G > 0, its G derivatives.  The reference scales the log-dets by D and sums the data-fit terms over the columns, but counts the
+    prior and trace terms T = (-N prior + trace) / (2 sigma2) once, not D times (gpr.py:81-87), so D - 1 copies of T are taken
+    out of the column sums again.  shared() returns [T, dT] (model-specific; read only for D > 1; its first 1 + G entries are
+    used).  The columns are added in order.  Returns (elbo, grad[G], info), info = the first non-zero of `infos` (0.0 if none)."""
+    total = values[0]
+    for row in values[1:]:
+        total = total + row
+    if len(values) > 1:
+        total = total - (len(values) - 1) * shared()[: total.size]
+    info = next((i for i in infos if i != 0), 0.0)
+    return total[0], total[1:], info
+
+
+def _losses(bounds, params, U):
+    """(loss[n], grad[n, G], info[n]) from n combined bounds (elbo, grad[G], info) at the unconstrained points U[n, G] of
+    `params`: loss = -ELBO and its gradient in U.  A failed bound (info != 0) gives loss +inf, NaN gradients and its pivot."""
+    n = len(U)
+    loss, grad, info = np.empty(n), np.empty((n, len(params))), np.zeros(n, dtype=np.int64)
+    for b, ((elbo, g, inf), u) in enumerate(zip(bounds, U)):
+        if inf != 0:
+            loss[b], grad[b], info[b] = np.inf, np.nan, int(inf)
+            continue
+        loss[b] = -float(elbo)
+        grad[b] = [-(g_j * p.dvalue_dunconstrained_at(float(u_j))) for g_j, p, u_j in zip(g, params, u)]
+    return loss, grad, info
+
+
+def _values_at(params, U):
+    """Constrained values [n, len(params)] of params at the unconstrained rows U[n, len(params)]."""
+    return np.array([[p.value_at(float(u)) for p, u in zip(params, row)] for row in U]).reshape(-1, len(params))
+
+
 class GPR_1d(_ModelBase):
     """Collapsed-bound sparse GP regression in 1-D with B-spline inducing features (reference gpr.py:18-136).
 
@@ -89,9 +177,7 @@ class GPR_1d(_ModelBase):
         n_out = int(y.shape[1])
         on_device = isinstance(X, torch.Tensor) and X.is_cuda
         if check_inputs and X.shape[0]:
-            lo, hi = (torch.aminmax(X) if isinstance(X, torch.Tensor) else (X.min(), X.max()))
-            assert float(lo) > basis.a
-            assert float(hi) < basis.b
+            _check_domain(X, [basis])
 
         # Init model (reference gpr.py:29-34)
         self.kernel = kernel
@@ -128,36 +214,16 @@ class GPR_1d(_ModelBase):
                 self._accs = list(stacked.unbind(0))
         self._acc = self._accs[0]
         self._G, self._b, self._scal = ops.split_accum_1d(self._acc, basis)
-        self._host = None
         self._outs = [torch.empty(16, dtype=torch.float64, device=self._acc.device) for _ in self._accs]
         self._out = self._outs[0]
 
-    # -- the reference's cached attributes (host copies, fetched lazily) --------------------------------------
-    def _host_stats(self):
-        if self._host is None:
-            parts = [ops.split_accum_1d(acc, self.basis) for acc in self._accs]
-            b = torch.stack([p[1] for p in parts], 1).cpu().numpy()
-            scal = self._scal.cpu().numpy().copy()
-            scal[0] = float(sum(p[2][0] for p in parts).item())
-            self._host = (self._G.cpu().numpy(), b, scal)
-        return self._host
+    def _device_stats(self):
+        parts = [ops.split_accum_1d(acc, self.basis) for acc in self._accs]
+        return self._G, torch.stack([p[1] for p in parts]), torch.stack([p[2][0] for p in parts]), self._scal[1]
 
     @property
     def KufKfu(self):
         return self._host_stats()[0]
-
-    @property
-    def Kuf_y(self):
-        return self._host_stats()[1]
-
-    @property
-    def tr_yTy(self):
-        return float(self._host_stats()[2][0])
-
-    @property
-    def num_data(self):
-        """Global number of datapoints (all shards)."""
-        return int(self._host_stats()[2][1])
 
     @property
     def KufKfu_sparse(self):
@@ -181,43 +247,28 @@ class GPR_1d(_ModelBase):
         return self._out
 
     @staticmethod
-    def _combine_columns(outs, v, s2, n):
-        """Bound for D output columns from the D single-column evaluations outs[D, 16] at variance v, sigma2 s2 and n data
-        points (v, s2, n are only read for D > 1).  The reference scales the log-dets by D and sums the data-fit terms over
-        columns, but counts -sum(K_diag)/2s2 + trace/2s2 ONCE (gpr.py:81-87); summing the columns counts it D times, so
-        D - 1 copies of T = (-N v + trace)/(2 s2) are taken out again: dT/dv = (-N + trace/v)/(2 s2) (trace is linear in
-        v), dT/dl = (dtrace/dl)/(2 s2), dT/ds2 = -T/s2."""
-        out = outs[0].copy()
-        extra = len(outs) - 1
-        if extra:
-            tr, dtr_dl = out[7], out[15]
-            T = 0.5 * (-n * v + tr) / s2
-            out[0:4] = outs[:, 0:4].sum(0) - extra * np.array([T, 0.5 * (-n + tr / v) / s2, 0.5 * dtr_dl / s2, -T / s2])
-            out[6] = outs[:, 6].sum()
-            bad = outs[:, 8][outs[:, 8] != 0]
-            out[8] = bad[0] if bad.size else 0.0
-        return out
-
-    def _combine_outputs(self):
-        outs = torch.stack(self._outs).cpu().numpy()
-        if len(outs) == 1:
-            return self._combine_columns(outs, None, None, None)
-        v, s2 = hyper_value(self.kernel.variance), hyper_value(self.likelihood.variance)
-        return self._combine_columns(outs, v, s2, float(self._scal[1].item()))
-
-    def _grads(self, out):
-        return _grad_dict([(self.kernel.variance, out[1]), (self.kernel.lengthscales, out[2]),
-                           (self.likelihood.variance, out[3])])
+    def _bound(outs, v, s2, n):
+        """(elbo, grad[3], info) of the D output columns from their rows outs[D, 16] (Bound1D) at variance v and sigma2 s2;
+        n() returns the number of data points (called for D > 1 only).  T = (-N v + trace) / (2 s2) counts once:
+        dT/dv = (-N + trace / v) / (2 s2) (trace is linear in v), dT/dl = (dtrace/dl) / (2 s2), dT/ds2 = -T / s2."""
+        def shared():
+            N, tr = n(), outs[0, Bound1D.TRACE]
+            T = 0.5 * (-N * v + tr) / s2
+            return np.array([T, 0.5 * (-N + tr / v) / s2, 0.5 * outs[0, Bound1D.DTRACE_DL] / s2, -T / s2])
+        return _combine_columns(outs[:, Bound1D.ELBO_GRAD], outs[:, Bound1D.INFO], shared)
 
     def elbo_and_grad(self):
         """ELBO (reference gpr.py:49-89) and {id(param): dELBO/dparam} for variance, lengthscales, sigma^2."""
         self._launch_elbo()
-        out = self._combine_outputs()
-        if out[8] != 0:
-            raise np.linalg.LinAlgError("banded Cholesky failed: non-positive pivot %d" % int(out[8]))
-        grads = self._grads(out)
-        self.last_terms = dict(log_det_Kuu=out[4], log_det_P=out[5], quad=out[6], trace=out[7])
-        return float(out[0]), grads
+        outs = torch.stack(self._outs).cpu().numpy()
+        v, s2 = hyper_value(self.kernel.variance), hyper_value(self.likelihood.variance)
+        elbo, g, info = self._bound(outs, v, s2, lambda: float(self._scal[1].item()))
+        if info != 0:
+            raise np.linalg.LinAlgError("banded Cholesky failed: non-positive pivot %d" % int(info))
+        row = outs[0]
+        self.last_terms = dict(log_det_Kuu=row[Bound1D.LOG_DET_KUU], log_det_P=row[Bound1D.LOG_DET_P],
+                               quad=outs[:, Bound1D.QUAD].sum(), trace=row[Bound1D.TRACE])
+        return float(elbo), _grad_dict(zip(self.trainable_variables, g))
 
     def training_loss_and_gradients_batch(self, U):
         """training_loss_and_gradients at B settings at once, without changing the model's parameters.
@@ -236,26 +287,16 @@ class GPR_1d(_ModelBase):
             raise ValueError("U has %d rows; a batch holds 1..%d settings" % (U.shape[0], _lib.MAX_BATCH))
         if not np.isfinite(U).all():
             raise ValueError("U must be finite")
-        vals = np.array([[p.value_at(float(u)) for p, u in zip(params, row)] for row in U])
+        vals = _values_at(params, U)
         var, ell, s2 = vals[:, 0], vals[:, 1], vals[:, 2]
         Kuu, dKuu = self.inducing_features.make_Kuu_device_batched(self.kernel, ell, var, want_grad=True)
         if self._acc_batch is None:
             self._acc_batch = self._acc.view(1, -1) if len(self._accs) == 1 else torch.stack(self._accs)
-        D = len(self._accs)
-        if D > 1 and self._n_host is None:
+        if len(self._accs) > 1 and self._n_host is None:
             self._n_host = float(self._scal[1].item())
         outs = ops.elbo_grad_1d_batched(Kuu, dKuu, self._acc_batch, self.basis, var, s2, chunks=self._chunks).cpu().numpy()
-        B = U.shape[0]
-        loss, grad, info = np.empty(B), np.empty((B, len(params))), np.zeros(B, dtype=np.int64)
-        for b in range(B):
-            out = self._combine_columns(outs[b], var[b], s2[b], self._n_host)
-            if out[8] != 0:
-                loss[b], grad[b], info[b] = np.inf, np.nan, int(out[8])
-                continue
-            grads = self._grads(out)
-            loss[b] = -float(out[0])
-            grad[b] = [-(grads[id(p)] * p.dvalue_dunconstrained_at(float(u))) for p, u in zip(params, U[b])]
-        return loss, grad, info
+        bounds = [self._bound(outs[b], var[b], s2[b], lambda: self._n_host) for b in range(len(U))]
+        return _losses(bounds, params, U)
 
     def elbo(self):
         """Variational bound on the log marginal likelihood (reference gpr.py:49-89)."""
@@ -294,10 +335,7 @@ class GPR_1d(_ModelBase):
             mean, var = torch.stack([c[0] for c in cols], 1), cols[0][1]
         if info.any().item():
             raise np.linalg.LinAlgError("banded Cholesky failed in predict_f")
-        var = var.view(-1, 1)
-        if isinstance(Xnew, torch.Tensor) and Xnew.is_cuda:
-            return mean, var
-        return mean.cpu().numpy(), var.cpu().numpy()
+        return _like_input(Xnew, mean, var.view(-1, 1))
 
 
 class GPR_1d_many:
@@ -320,8 +358,7 @@ class GPR_1d_many:
         X, y = data
         if X.ndim == 2:
             assert X.shape[1] == 1
-        if y.ndim == 2 and y.shape[1] != 1:
-            raise NotImplementedError("GPR_1d_many takes one output column per series")
+        _output_columns(y, "GPR_1d_many", 1, NotImplementedError)   # one column per series
         n = int(X.shape[0])
         if int(y.shape[0]) != n:
             raise ValueError("X and y must have the same number of rows")
@@ -329,9 +366,7 @@ class GPR_1d_many:
         self.num_series = S = self._offsets.size - 1
         self._counts = np.diff(self._offsets)
         if check_inputs and n:
-            lo, hi = (torch.aminmax(X) if isinstance(X, torch.Tensor) else (X.min(), X.max()))
-            assert float(lo) > basis.a
-            assert float(hi) < basis.b
+            _check_domain(X.reshape(-1, 1), [basis])
         self.kernel = kernel
         self.basis = basis
         self.inducing_features = SplineFeatures1D(kernel, basis)
@@ -347,20 +382,17 @@ class GPR_1d_many:
                 raise ValueError("U0 must be finite [%d, 3], got shape %s" % (S, self.U.shape))
         self._acc = ops.accum_1d_segmented(X.reshape(-1), y.reshape(-1), self._offsets, basis)
 
-    def _values(self, U):
-        return np.array([[p.value_at(float(u)) for p, u in zip(self._params, row)] for row in U]).reshape(-1, 3)
-
     @property
     def variance(self):
-        return self._values(self.U)[:, 0]
+        return _values_at(self._params, self.U)[:, 0]
 
     @property
     def lengthscales(self):
-        return self._values(self.U)[:, 1]
+        return _values_at(self._params, self.U)[:, 1]
 
     @property
     def noise_variance(self):
-        return self._values(self.U)[:, 2]
+        return _values_at(self._params, self.U)[:, 2]
 
     def _evaluate(self, U, ids):
         """(loss[n], grad[n, 3], info[n]) of series ids[i] at unconstrained U[i]: -ELBO and its gradient in U, as
@@ -374,20 +406,15 @@ class GPR_1d_many:
         outs = []
         for c in range(0, live.size, _lib.MAX_BATCH):
             sel = live[c: c + _lib.MAX_BATCH]
-            vals = self._values(U[sel])
+            vals = _values_at(self._params, U[sel])
             Kuu, dKuu = self.inducing_features.make_Kuu_device_batched(self.kernel, vals[:, 1], vals[:, 0], want_grad=True)
             outs.append(ops.elbo_grad_1d_batched(Kuu, dKuu, self._acc, self.basis, vals[:, 0], vals[:, 2], chunks=self._chunks,
                                                  rows=ids[sel])[:, 0])
         if not outs:
             return loss, grad, info
         out = torch.cat(outs).cpu().numpy()           # one device-to-host copy per call
-        for i, b in enumerate(live):
-            o = out[i]
-            if o[8] != 0:
-                loss[b], grad[b], info[b] = np.inf, np.nan, int(o[8])
-                continue
-            loss[b] = -float(o[0])
-            grad[b] = [-(o[1 + j] * p.dvalue_dunconstrained_at(float(u))) for j, (p, u) in enumerate(zip(self._params, U[b]))]
+        bounds = [(o[Bound1D.ELBO], o[Bound1D.GRAD], o[Bound1D.INFO]) for o in out]
+        loss[live], grad[live], info[live] = _losses(bounds, self._params, U[live])
         return loss, grad, info
 
     def training_loss_and_gradients(self):
@@ -427,7 +454,7 @@ class GPR_1d_many:
         live = np.flatnonzero(self._counts > 0)
         for c in range(0, live.size, _lib.MAX_BATCH):
             sel = live[c: c + _lib.MAX_BATCH]
-            vals = self._values(self.U[sel])
+            vals = _values_at(self._params, self.U[sel])
             Kuu, _ = self.inducing_features.make_Kuu_device_batched(self.kernel, vals[:, 1], vals[:, 0], want_grad=False)
             a, sb, inf = ops.posterior_1d_batched(Kuu, self._acc, self.basis, vals[:, 2], sel, chunks=self._chunks)
             idx = torch.from_numpy(sel).to(dev)
@@ -442,15 +469,36 @@ class GPR_1d_many:
         mean, var = ops.predict_1d_segmented(ops.to_device(Xnew).reshape(-1), offsets_new, self.basis, alpha, S_band, variances)
         if info.any().item():
             raise np.linalg.LinAlgError("banded Cholesky failed in predict_f")
-        mean, var = mean.view(-1, 1), var.view(-1, 1)
-        if isinstance(Xnew, torch.Tensor) and Xnew.is_cuda:
-            return mean, var
-        return mean.cpu().numpy(), var.cpu().numpy()
+        return _like_input(Xnew, mean.view(-1, 1), var.view(-1, 1))
+
+
+class _PerDimension(_ModelBase):
+    """What GPR_kron and GPR_additive share: a kernel, a basis and a banded Kuu factor per input dimension."""
+
+    @property
+    def trainable_variables(self):
+        out = []
+        for k in self.kernels:
+            out += [k.variance, k.lengthscales]
+        return _unique(out + [self.likelihood.variance])
+
+    def _factors(self, want_grad, defer=False):
+        """Per-dimension Kuu factors, their lengthscale derivatives, and the bands of their inverses.  The banded
+        inversions run on side streams so that they overlap the factorisation of P; with `defer` the caller joins them
+        itself (`self._join()`) right before it reads the bands."""
+        Ks, dKs = [], []
+        for feat, kern in zip(self.inducing_features, self.kernels):
+            K, dK = feat.make_Kuu_device(kern, want_grad=True)
+            Ks.append(K); dKs.append(dK)
+        Ss, dSs, scals, self._join = ops.band_inverses_beside(Ks, dKs, self.bases)
+        if not defer:
+            self._join()
+        return Ks, dKs, Ss, dSs, scals
 
 
 def _kron_column_bound(N, s2, v, m1, m2, sc1, sc2, logdetP, Q, yy, T, want_grad):
-    """ELBO of the Kronecker model for one output column and, with want_grad, its derivatives [v1, l1, v2, l2, sigma2];
-    sc_i = {log|K_i|, dlog|K_i|, ...}, T = the 11 slots of asvgp_kron_terms.  Returns (elbo, grads or None, log|Kuu|)."""
+    """ELBO of the Kronecker model for one output column and, with want_grad, its derivatives: [elbo] or [elbo, v1, l1, v2,
+    l2, sigma2]; sc_i = {log|K_i|, dlog|K_i|, ...}, T = the 11 slots of asvgp_kron_terms.  Returns (that row, log|Kuu|)."""
     M = m1 * m2
     logdetK = m2 * sc1[0] + m1 * sc2[0]                       # log|K1 (x) K2|
     tr = T[8]
@@ -458,7 +506,7 @@ def _kron_column_bound(N, s2, v, m1, m2, sc1, sc2, logdetP, Q, yy, T, want_grad)
     elbo = (-0.5 * N * np.log(2 * np.pi * s2) - 0.5 * logdetP + 0.5 * logdetK - 0.5 * yy / s2
             + 0.5 * Q / s2**2 - 0.5 * N * v12 / s2 + 0.5 * tr / s2)
     if not want_grad:
-        return elbo, None, logdetK
+        return np.array([elbo]), logdetK
     trPG, trPdK1, trPdK2, trPK = T[0:4]
     xGx, xdK1x, xdK2x, xKx = T[4:8]
     d_l1 = -0.5 * trPdK1 + 0.5 * m2 * sc1[1] - 0.5 * xdK1x / s2**2 + 0.5 * T[9] / s2
@@ -469,10 +517,19 @@ def _kron_column_bound(N, s2, v, m1, m2, sc1, sc2, logdetP, Q, yy, T, want_grad)
     d_v2 = common / v[1] - 0.5 * N * v[0] / s2
     d_s2 = (-0.5 * N / s2 + 0.5 * trPG / s2**2 + 0.5 * yy / s2**2 + 0.5 * xGx / s2**4 - Q / s2**3
             + 0.5 * N * v12 / s2**2 - 0.5 * tr / s2**2)
-    return elbo, np.array([d_v1, d_l1, d_v2, d_l2, d_s2]), logdetK
+    return np.array([elbo, d_v1, d_l1, d_v2, d_l2, d_s2]), logdetK
 
 
-class GPR_kron(_ModelBase):
+def _kron_shared(N, s2, v, T):
+    """The terms -N v1 v2 / (2 s2) + trace / (2 s2) of one column's bound, which count once for all output columns, and
+    their derivatives: [T, v1, l1, v2, l2, sigma2].  trace = T[8] is proportional to v1 v2 (S_i = K_i^-1 is proportional
+    to v_i)."""
+    T0 = 0.5 * (-N * v[0] * v[1] + T[8]) / s2
+    return np.array([T0, 0.5 * (-N * v[1] + T[8] / v[0]) / s2, 0.5 * T[9] / s2, 0.5 * (-N * v[0] + T[8] / v[1]) / s2,
+                     0.5 * T[10] / s2, -T0 / s2])
+
+
+class GPR_kron(_PerDimension):
     """Collapsed-bound sparse GP regression on 2-D inputs with Kronecker-structured B-spline inducing features
     (reference gpr.py:239-359).  Same constructor, attributes and methods; what differs is only *how*:
 
@@ -506,21 +563,15 @@ class GPR_kron(_ModelBase):
 
         # Check dimensionality of inputs / valid kernels (reference gpr.py:247-252)
         assert len(kernels) == len(bases) == self.d
-        if y.ndim == 1:
-            y = y.reshape(-1, 1)
-        n_out = self.n_outputs = int(y.shape[1])
-        if not 1 <= n_out <= ops.MAX_RHS:
-            raise ValueError("GPR_kron takes 1 ... %d output columns, got %d" % (ops.MAX_RHS, n_out))
+        y, n_out = _output_columns(y, "GPR_kron", ops.MAX_RHS)
+        self.n_outputs = n_out
         if n_out > 1 and (method or ops.KRON_METHOD) != "nd":
             raise NotImplementedError("several output columns need method='nd' (the scalar-band method takes one column)")
         self._kinds = [kernel_kind(k) for k in kernels]
         if self.d != 2:
             raise NotImplementedError("GPR_kron is implemented for d = 2 (as reference utils.py:57)")
         if check_inputs and self.n:
-            for i, basis in enumerate(bases):
-                col = X[:, i]
-                lo, hi = (torch.aminmax(col) if isinstance(col, torch.Tensor) else (col.min(), col.max()))
-                assert float(lo) > basis.a and float(hi) < basis.b, "inputs must lie strictly inside the basis domain"
+            _check_domain(X, bases)
 
         self.kernel = kernels[-1]               # the reference hands the last loop kernel to GPModel (SURVEY Q8)
         self.likelihood = Gaussian()
@@ -564,7 +615,6 @@ class GPR_kron(_ModelBase):
             if self._distributed:               # ONE collective over the packed accumulator and the other columns' [b_d | sum y_d^2 | N]
                 _dist.allreduce_packed(self._packed)
         self._Gs, self._b, self._scal = ops.split_accum_2d(self._acc, self.bases)
-        self._host = None
 
     def _accumulate_columns(self, X, y, dev, row_len):
         """O(N) pass for D > 1 output columns: column 0 gives G, b_1 and its scalars exactly as a single-column model; every
@@ -592,35 +642,16 @@ class GPR_kron(_ModelBase):
                 self._extra[d - 1, :M].copy_(b_d)
                 self._extra[d - 1, M:].copy_(sc_d)
 
-    # -- the reference's cached attributes (host copies, fetched lazily) --------------------------------------
-    def _host_stats(self):
-        if self._host is None:
-            b, scal = self._b.cpu().numpy().reshape(-1, 1), self._scal.cpu().numpy()
-            if self._extra is not None:         # (M, D) and the sum of y^2 over all columns (reference gpr.py:274, 78-79)
-                extra = self._extra.cpu().numpy()
-                M = b.shape[0]
-                b = np.concatenate([b, extra[:, :M].T], 1)
-                scal = scal.copy()
-                scal[0] = scal[0] + extra[:, M].sum()
-            self._host = (self._Gs.cpu().numpy(), b, scal)
-        return self._host
-
     def _rhs(self):
-        """Kuf_y of every output column as one device tensor [D, M] (D > 1 only)."""
+        """Kuf_y of every output column as one device tensor [D, M]."""
         M = self._b.numel()
+        if self._extra is None:
+            return self._b.view(1, M)
         return torch.cat([self._b.view(1, M), self._extra[:, :M]], 0)
 
-    @property
-    def Kuf_y(self):
-        return self._host_stats()[1]
-
-    @property
-    def tr_yTy(self):
-        return float(self._host_stats()[2][0])
-
-    @property
-    def num_data(self):
-        return int(self._host_stats()[2][1])
+    def _device_stats(self):
+        yy = self._scal[0:1] if self._extra is None else torch.cat([self._scal[0:1], self._extra[:, -2]])
+        return self._Gs, self._rhs(), yy, self._scal[1]
 
     @property
     def KufKfu_sparse(self):
@@ -635,40 +666,7 @@ class GPR_kron(_ModelBase):
 
         return utils.sparse_to_band(self.KufKfu_sparse, self.bandwidth)
 
-    @property
-    def trainable_variables(self):
-        out = []
-        for k in self.kernels:
-            out += [k.variance, k.lengthscales]
-        return _unique(out + [self.likelihood.variance])
-
     # -- objective ---------------------------------------------------------------------------------------------
-    def _factors(self, want_grad, defer=False):
-        """Per-dimension Kuu factors, their lengthscale derivatives, and the bands of their inverses.  The two banded
-        inversions (one short chain each, ~0.1 ms) run on side streams so that they overlap the factorisation of P;
-        with `defer` the caller joins them itself (`_join`) right before it reads the bands."""
-        main = torch.cuda.current_stream()
-        Ks, dKs, Ss, dSs, scals = [], [], [], [], []
-        for feat, kern in zip(self.inducing_features, self.kernels):
-            K, dK = feat.make_Kuu_device(kern, want_grad=True)
-            Ks.append(K); dKs.append(dK)
-        self._side = ops.side_streams(len(self.bases))
-        for i, (side, basis) in enumerate(zip(self._side, self.bases)):
-            side.wait_stream(main)
-            with torch.cuda.stream(side):
-                S, dS, sc = ops.band_inverse_1d(Ks[i], dKs[i], basis, slot=1 + i)
-            for t in (S, dS, sc):
-                t.record_stream(main)
-            Ss.append(S); dSs.append(dS); scals.append(sc)
-        if not defer:
-            self._join()
-        return Ks, dKs, Ss, dSs, scals
-
-    def _join(self):
-        main = torch.cuda.current_stream()
-        for side in self._side:
-            main.wait_stream(side)
-
     def _evaluate(self, want_grad):
         s2 = hyper_value(self.likelihood.variance)
         v = [hyper_value(k.variance) for k in self.kernels]
@@ -677,49 +675,24 @@ class GPR_kron(_ModelBase):
         ws = ops.kron_workspace(m1, m2, self.order, getattr(self, "_method", None), n_rhs=D)
         Ks, dKs, Ss, dSs, scals = self._factors(want_grad, defer=True)
         ops.kron_factor(Ks[0], Ks[1], self._acc, self.bases, s2, ws, b=self._rhs() if D > 1 else None)
-        if want_grad:
-            SigP, x = ops.kron_selinv(self.bases, ws)
-        else:
-            ws.sigma_stencil.zero_()
-            SigP, x = ws.sigma_stencil, ws.rhs[: ws.M * D].view(D, ws.M).squeeze(0)   # x unused for the value
+        # (x_d, in ws.x_cols, is only read with want_grad: the value needs no selected inverse)
+        SigP = ops.kron_selinv(self.bases, ws)[0] if want_grad else ws.sigma_stencil.zero_()
         self._join()
-        if D == 1:
-            ops.kron_terms(SigP, self._acc, x, Ks[0], dKs[0], Ks[1], dKs[1], Ss[0], dSs[0], Ss[1], dSs[1], self.bases,
-                           ws.terms)
-            packed = torch.cat([scals[0], scals[1], ws.scal, ws.terms, self._scal]).cpu().numpy()   # one D2H read
-            sc1, sc2, scP, T, (yy, N) = packed[0:4], packed[4:8], packed[8:11], packed[11:22], packed[22:24]
-            info = scP[2] or sc1[2] or sc2[2]
-            if info != 0:
-                raise np.linalg.LinAlgError("Cholesky failed: non-positive pivot %d" % int(info))
-            elbo, g, logdetK = _kron_column_bound(N, s2, v, m1, m2, sc1, sc2, scP[0], scP[1], yy, T, want_grad)
-            self.last_terms = dict(log_det_Kuu=logdetK, log_det_P=scP[0], quad=scP[1], trace=T[8])
-        else:
-            # one factorisation, the xT Op x terms per column (slots 0..3 and 8..10 are the same in every column)
-            for d in range(D):
-                ops.kron_terms(SigP, self._acc, x[d], Ks[0], dKs[0], Ks[1], dKs[1], Ss[0], dSs[0], Ss[1], dSs[1], self.bases,
-                               ws.terms[d])
-            packed = torch.cat([scals[0], scals[1], ws.scal, ws.terms.reshape(-1), self._scal,
-                                self._extra[:, -2]]).cpu().numpy()
-            sc1, sc2, p = packed[0:4], packed[4:8], 8
-            logdetP, info, Qs = packed[p], packed[p + 1], packed[p + 2: p + 2 + D]; p += 2 + D
-            Ts = packed[p: p + 11 * D].reshape(D, 11); p += 11 * D
-            N = packed[p + 1]
-            yys = np.concatenate([[packed[p]], packed[p + 2: p + 1 + D]])
-            info = info or sc1[2] or sc2[2]
-            if info != 0:
-                raise np.linalg.LinAlgError("Cholesky failed: non-positive pivot %d" % int(info))
-            cols = [_kron_column_bound(N, s2, v, m1, m2, sc1, sc2, logdetP, Qs[d], yys[d], Ts[d], want_grad) for d in range(D)]
-            logdetK, tr = cols[0][2], Ts[0][8]
-            # -N v1 v2 / 2 s2 + trace / 2 s2 count once (reference gpr.py:81-87), not once per column: take D - 1 copies of
-            # T = (-N v1 v2 + tr) / (2 s2) out again.  tr is proportional to v1 v2 (S_i = K_i^-1 is proportional to v_i).
-            T0 = 0.5 * (-N * v[0] * v[1] + tr) / s2
-            elbo = sum(c[0] for c in cols) - (D - 1) * T0
-            g = None
-            if want_grad:
-                dT = np.array([0.5 * (-N * v[1] + tr / v[0]) / s2, 0.5 * Ts[0][9] / s2,
-                               0.5 * (-N * v[0] + tr / v[1]) / s2, 0.5 * Ts[0][10] / s2, -T0 / s2])
-                g = np.sum([c[1] for c in cols], 0) - (D - 1) * dT
-            self.last_terms = dict(log_det_Kuu=logdetK, log_det_P=logdetP, quad=float(np.sum(Qs)), trace=tr)
+        # one factorisation, the xT Op x terms per column (slots 0..3 and 8..10 are the same in every column)
+        for x_d, terms_d in zip(ws.x_cols, ws.terms_cols):
+            ops.kron_terms(SigP, self._acc, x_d, Ks[0], dKs[0], Ks[1], dKs[1], Ss[0], dSs[0], Ss[1], dSs[1], self.bases, terms_d)
+        yy_rest = [] if self._extra is None else [self._extra[:, -2]]          # sum(y_d^2) of columns 2 ... D
+        packed = torch.cat([scals[0], scals[1], ws.scal, ws.terms_flat, self._scal] + yy_rest).cpu().numpy()   # one D2H read
+        sc1, sc2, p = packed[0:4], packed[4:8], 8 + ws.scal.numel()
+        logdetP, infoP, Qs = ws.unpack_scal(packed[8:p])
+        Ts = packed[p: p + 11 * D].reshape(D, 11); p += 11 * D
+        N = packed[p + 1]
+        yys = [packed[p], *packed[p + 2:]]
+        cols = [_kron_column_bound(N, s2, v, m1, m2, sc1, sc2, logdetP, Qs[d], yys[d], Ts[d], want_grad) for d in range(D)]
+        elbo, g, info = _combine_columns([c[0] for c in cols], [infoP, sc1[2], sc2[2]], lambda: _kron_shared(N, s2, v, Ts[0]))
+        if info != 0:
+            raise np.linalg.LinAlgError("Cholesky failed: non-positive pivot %d" % int(info))
+        self.last_terms = dict(log_det_Kuu=cols[0][1], log_det_P=logdetP, quad=float(Qs.sum()), trace=Ts[0][8])
         if not want_grad:
             return float(elbo), None
         grads = _grad_dict([(self.kernels[0].variance, g[0]), (self.kernels[0].lengthscales, g[1]),
@@ -735,9 +708,6 @@ class GPR_kron(_ModelBase):
         """Variational bound on the log marginal likelihood (reference gpr.py:282-308)."""
         return np.float64(self._evaluate(False)[0])
 
-    def maximum_log_likelihood_objective(self):
-        return self.elbo()
-
     # -- prediction ----------------------------------------------------------------------------------------------
     def posterior_weights(self):
         """(alpha, SigP stencil, S1, S2) on the device: alpha = P^-1 Kuf_y / sigma2 ([D, M] for D > 1 output columns),
@@ -748,7 +718,7 @@ class GPR_kron(_ModelBase):
         Ks, _, Ss, _, scals = self._factors(False)
         ops.kron_factor(Ks[0], Ks[1], self._acc, self.bases, s2, ws, b=self._rhs() if D > 1 else None)
         SigP, x = ops.kron_selinv(self.bases, ws)
-        info = torch.stack([ws.scal[2 if D == 1 else 1], scals[0][2], scals[1][2]])
+        info = torch.stack([ws.info, scals[0][2], scals[1][2]])
         return x / s2, SigP, Ss[0], Ss[1], info
 
     def _hyper_state(self):
@@ -786,10 +756,7 @@ class GPR_kron(_ModelBase):
             Xs = ops.to_device(Xnew)
             cols = [ops.predict_2d_apply(Xs, self.bases, t, prior, raster_row_len=row_len) for t in table]
             mean, var = torch.stack([c[0] for c in cols], 1), cols[0][1]
-        mean, var = mean.reshape(mean.shape[0], -1), var.view(-1, 1)
-        if isinstance(Xnew, torch.Tensor) and Xnew.is_cuda:
-            return mean, var
-        return mean.cpu().numpy(), var.cpu().numpy()
+        return _like_input(Xnew, mean.reshape(mean.shape[0], -1), var.view(-1, 1))
 
     def predict_f_sparse(self, Xnew, full_cov=False, full_output_cov=False):
         """Same numbers as predict_f (reference gpr.py:336-359 is its CHOLMOD twin)."""
@@ -797,13 +764,13 @@ class GPR_kron(_ModelBase):
 
 
 def _additive_column_bound(N, s2, v, vsum, ms, sc, logdetP, logdetK, trace, trn, Q, yy, T, dn, want_grad):
-    """ELBO of the additive model for one output column and, with want_grad, its derivatives [v_1, l_1, ..., v_D, l_D,
-    sigma2]; T[i] = asvgp_additive_terms of P^-1 and this column's x, dn = asvgp_dense_terms.  Returns (elbo, grads or None)."""
+    """ELBO of the additive model for one output column and, with want_grad, its derivatives: [elbo] or [elbo, v_1, l_1, ...,
+    v_D, l_D, sigma2]; T[i] = asvgp_additive_terms of P^-1 and this column's x, dn = asvgp_dense_terms."""
     elbo = (-0.5 * N * np.log(2 * np.pi * s2) - 0.5 * logdetP + 0.5 * logdetK - 0.5 * yy / s2
             + 0.5 * Q / s2**2 - 0.5 * N * vsum / s2 + 0.5 * trace / s2)
     if not want_grad:
-        return elbo, None
-    g = []
+        return np.array([elbo])
+    g = [elbo]
     for i, m in enumerate(ms):
         trPK, trPdK, xKx, xdKx = T[i]
         d_l = -0.5 * trPdK + 0.5 * sc[i, 1] - 0.5 * xdKx / s2**2 + 0.5 * trn[i, 1] / s2
@@ -813,10 +780,20 @@ def _additive_column_bound(N, s2, v, vsum, ms, sc, logdetP, logdetK, trace, trn,
     trPG, xGx = dn
     d_s2 = (-0.5 * N / s2 + 0.5 * trPG / s2**2 + 0.5 * yy / s2**2 + 0.5 * xGx / s2**4 - Q / s2**3
             + 0.5 * N * vsum / s2**2 - 0.5 * trace / s2**2)
-    return elbo, np.array(g + [d_s2])
+    return np.array(g + [d_s2])
 
 
-class GPR_additive(_ModelBase):
+def _additive_shared(N, s2, v, vsum, trace, trn):
+    """The terms -N sum(v) / (2 s2) + trace / (2 s2) of one column's bound, which count once for all output columns, and
+    their derivatives: [T, v_1, l_1, ..., v_D, l_D, sigma2].  trace(K_d^-1 G_dd) = trn[d, 0] is proportional to v_d."""
+    T = 0.5 * (-N * vsum + trace) / s2
+    dT = []
+    for i in range(len(v)):
+        dT += [0.5 * (-N + trn[i, 0] / v[i]) / s2, 0.5 * trn[i, 1] / s2]
+    return np.array([T] + dT + [-T / s2])
+
+
+class GPR_additive(_PerDimension):
     """Collapsed-bound sparse GP regression with an ADDITIVE kernel, f(x) = sum_d f_d(x_d), each f_d on B-spline inducing
     features (reference gpr.py:139-236).  Same constructor, attributes and methods; what differs is only *how*:
 
@@ -842,19 +819,13 @@ class GPR_additive(_ModelBase):
 
         # Check dimensionality of inputs / valid kernels (reference gpr.py:146-152)
         assert len(kernels) == len(bases) == self.d
-        if y.ndim == 1:
-            y = y.reshape(-1, 1)
-        n_out = self.n_outputs = int(y.shape[1])
-        if not 1 <= n_out <= ops.MAX_RHS:
-            raise ValueError("GPR_additive takes 1 ... %d output columns, got %d" % (ops.MAX_RHS, n_out))
+        y, n_out = _output_columns(y, "GPR_additive", ops.MAX_RHS)
+        self.n_outputs = n_out
         self._kinds = [kernel_kind(k) for k in kernels]
         if self.d > 8:
             raise NotImplementedError("GPR_additive is implemented for at most 8 input dimensions")
         if check_inputs and self.n:
-            for i, basis in enumerate(bases):
-                col = X[:, i]
-                lo, hi = (torch.aminmax(col) if isinstance(col, torch.Tensor) else (col.min(), col.max()))
-                assert float(lo) > basis.a and float(hi) < basis.b, "inputs must lie strictly inside the basis domain"
+            _check_domain(X, bases)
 
         self.kernel = kernels[-1]               # as the reference: the last loop kernel goes to GPModel (SURVEY Q8)
         self.likelihood = Gaussian()
@@ -895,11 +866,10 @@ class GPR_additive(_ModelBase):
         for i, (acc, basis) in enumerate(zip(self._accs, self.bases)):
             Gi, bi, scal = ops.split_accum_1d(acc, basis)
             o = int(self._offsets[i])
-            ops._lib.call("asvgp_additive_put_band", ops._p(Gi), basis.m, basis.order, o, self.M, 1.0, 0, ops._p(self._G), ops._stream())
+            ops.additive_put_band(Gi, basis, o, self._G)
             self._b[o: o + basis.m].copy_(bi)
         for (i, j), c in self._cross.items():
-            ops._lib.call("asvgp_additive_put_cross", ops._p(c), self.bases[i].m, self.bases[j].m, int(self._offsets[i]),
-                          int(self._offsets[j]), self.M, ops._p(self._G), ops._stream())
+            ops.additive_put_cross(c, self._offsets[i], self._offsets[j], self._G)
         self._scal = ops.split_accum_1d(self._accs[0], self.bases[0])[2]          # {sum y^2, N}: the same in every dimension
         self._B, self._yy = None, None
         if n_out > 1:               # right-hand sides [D, M] and sum(y_d^2) per column
@@ -915,18 +885,11 @@ class GPR_additive(_ModelBase):
                 self._yy[c: c + 1].copy_(ops.split_accum_1d(accs[0], self.bases[0])[2][0:1])
         del self._col_accs
         self._P = torch.empty_like(self._G)
-        self._host = None
 
-    # -- the reference's cached attributes ------------------------------------------------------------------------------------
-    def _host_stats(self):
-        if self._host is None:
-            if self._B is None:
-                self._host = (self._G.cpu().numpy(), self._b.cpu().numpy().reshape(-1, 1), self._scal.cpu().numpy())
-            else:                   # Kuf_y (M, D); tr_yTy sums over the columns (reference gpr.py:78-79)
-                scal = self._scal.cpu().numpy().copy()
-                scal[0] = float(self._yy.sum().item())
-                self._host = (self._G.cpu().numpy(), self._B.cpu().numpy().T.copy(), scal)
-        return self._host
+    def _device_stats(self):
+        if self._B is None:
+            return self._G, self._b.view(1, -1), self._scal[0:1], self._scal[1]
+        return self._G, self._B, self._yy, self._scal[1]
 
     @property
     def KufKfu(self):
@@ -938,51 +901,18 @@ class GPR_additive(_ModelBase):
 
         return sp.csr_matrix(self.KufKfu)
 
-    @property
-    def Kuf_y(self):
-        return self._host_stats()[1]
-
-    @property
-    def tr_yTy(self):
-        return float(self._host_stats()[2][0])
-
-    @property
-    def num_data(self):
-        return int(self._host_stats()[2][1])
-
-    @property
-    def trainable_variables(self):
-        out = []
-        for k in self.kernels:
-            out += [k.variance, k.lengthscales]
-        return _unique(out + [self.likelihood.variance])
-
     # -- objective ----------------------------------------------------------------------------------------------------------------
     def _factor(self, want_inverse):
         s2 = hyper_value(self.likelihood.variance)
-        main = torch.cuda.current_stream()
-        Ks, dKs, Ss, dSs, scals = [], [], [], [], []
-        for feat, kern in zip(self.inducing_features, self.kernels):
-            K, dK = feat.make_Kuu_device(kern, want_grad=True)
-            Ks.append(K); dKs.append(dK)
-        side = ops.side_streams(self.d)
-        for i, basis in enumerate(self.bases):                 # short banded chains: overlap them with the dense factorisation
-            side[i].wait_stream(main)
-            with torch.cuda.stream(side[i]):
-                S, dS, sc = ops.band_inverse_1d(Ks[i], dKs[i], basis, slot=1 + i)
-            for t in (S, dS, sc):
-                t.record_stream(main)
-            Ss.append(S); dSs.append(dS); scals.append(sc)
+        Ks, dKs, Ss, dSs, scals = self._factors(True, defer=True)   # the short banded chains overlap the dense factorisation
         # P = KufKfu / sigma2 + Kuu  (reference gpr.py:192)
-        ops._lib.call("asvgp_additive_scale", ops._p(self._G), self.M, float(s2), ops._p(self._P), ops._stream())
-        for i, basis in enumerate(self.bases):
-            ops._lib.call("asvgp_additive_put_band", ops._p(Ks[i]), basis.m, basis.order, int(self._offsets[i]), self.M, 1.0, 1,
-                          ops._p(self._P), ops._stream())
+        ops.additive_scale(self._G, s2, self._P)
+        for K, basis, o in zip(Ks, self.bases, self._offsets):
+            ops.additive_put_band(K, basis, o, self._P, add=True)
         ws = ops.dense_workspace(self.M, self.n_outputs)
-        ops.dense_factor(self._P, self._b if self._B is None else self._B, ws)
+        ops.dense_factor(self._P, self._device_stats()[1], ws)
         x, Pinv = ops.dense_selinv(ws) if want_inverse else (None, None)
-        for s in side:
-            main.wait_stream(s)
+        self._join()
         return Ks, dKs, Ss, dSs, scals, ws, x, Pinv
 
     def _evaluate(self, want_grad):
@@ -991,59 +921,41 @@ class GPR_additive(_ModelBase):
         Ks, dKs, Ss, dSs, scals, ws, x, Pinv = self._factor(want_grad)
         D, R = self.d, self.n_outputs
         dev = self._G.device
-        xs = [x] if R == 1 else (list(x) if x is not None else [None] * R)
+        xs = ws.x_cols if want_grad else [None] * R
         # trace(Kuu^-1 KufKfu) and its lengthscale derivatives: per dimension, on the bands
         tr = torch.zeros((D, 4), dtype=torch.float64, device=dev)         # sum S_d .* G_dd, sum dS_d .* G_dd, -, -
         terms = torch.zeros((R, D, 4), dtype=torch.float64, device=dev)  # per output column: the x-dependent terms
         dense = torch.zeros((R, 2), dtype=torch.float64, device=dev)
         zero_x = torch.zeros(self.M, dtype=torch.float64, device=dev)
-        for i, basis in enumerate(self.bases):
-            o = int(self._offsets[i])
+        for i, (basis, o) in enumerate(zip(self.bases, self._offsets)):
             # (the same contraction kernel with S := KufKfu's diagonal block and K := band(K_d^-1))
-            ops._lib.call("asvgp_additive_terms", ops._p(self._G), ops._p(zero_x), self.M, o, basis.m, basis.order, ops._p(Ss[i]),
-                          ops._p(dSs[i]), ops._p(tr[i]), ops._stream())
+            ops.additive_terms(self._G, zero_x, o, basis, Ss[i], dSs[i], tr[i])
             if want_grad:
                 for c in range(R):
-                    ops._lib.call("asvgp_additive_terms", ops._p(Pinv), ops._p(xs[c]), self.M, o, basis.m, basis.order,
-                                  ops._p(Ks[i]), ops._p(dKs[i]), ops._p(terms[c, i]), ops._stream())
+                    ops.additive_terms(Pinv, xs[c], o, basis, Ks[i], dKs[i], terms[c, i])
         if want_grad:
             for c in range(R):
-                ops._lib.call("asvgp_dense_terms", ops._p(Pinv), ops._p(self._G), ops._p(xs[c]), self.M, ops._p(dense[c]),
-                              ops._stream())
-        yy_cols = self._scal[0:1] if R == 1 else self._yy
+                ops.dense_terms(Pinv, self._G, xs[c], dense[c])
         packed = torch.cat([torch.stack(scals).reshape(-1), ws.scal, tr.reshape(-1), terms.reshape(-1), dense.reshape(-1),
-                            self._scal, yy_cols]).cpu().numpy()
+                            self._scal, self._device_stats()[2]]).cpu().numpy()
         sc = packed[: 4 * D].reshape(D, 4); p = 4 * D
-        scP = packed[p: p + ws.scal.numel()]; p += ws.scal.numel()
+        logdetP, infoP, Qs = ws.unpack_scal(packed[p: p + ws.scal.numel()]); p += ws.scal.numel()
         trn = packed[p: p + 4 * D].reshape(D, 4); p += 4 * D
         T = packed[p: p + 4 * D * R].reshape(R, D, 4); p += 4 * D * R
         dn = packed[p: p + 2 * R].reshape(R, 2); p += 2 * R
         N = packed[p + 1]; p += 2
         yys = packed[p: p + R]
-        # scal layouts of asvgp_dense_factor (one rhs) and asvgp_dense_factor_multi
-        logdetP, infoP, Qs = (scP[0], scP[2], scP[1:2]) if R == 1 else (scP[0], scP[1], scP[2:])
-        info = infoP or next((s[2] for s in sc if s[2] != 0), 0.0)
-        if info != 0:
-            raise np.linalg.LinAlgError("Cholesky failed: non-positive pivot %d" % int(info))
         logdetK = float(sc[:, 0].sum())
         trace = float(trn[:, 0].sum())
         vsum = float(np.sum(v))
         ms = [basis.m for basis in self.bases]
         cols = [_additive_column_bound(N, s2, v, vsum, ms, sc, logdetP, logdetK, trace, trn, Qs[c], yys[c], T[c], dn[c],
                                        want_grad) for c in range(R)]
-        self.last_terms = dict(log_det_Kuu=logdetK, log_det_P=logdetP, quad=float(np.sum(Qs)) if R > 1 else Qs[0], trace=trace)
-        if R == 1:
-            elbo, g = cols[0]
-        else:
-            # -N sum(v) / 2 s2 + trace / 2 s2 count once (reference gpr.py:81-87), not once per column: take R - 1 copies of
-            # T = (-N sum(v) + trace) / (2 s2) out again.  trace(K_d^-1 G_dd) is proportional to v_d.
-            T0 = 0.5 * (-N * vsum + trace) / s2
-            elbo = sum(c[0] for c in cols) - (R - 1) * T0
-            if want_grad:
-                dT = []
-                for i in range(D):
-                    dT += [0.5 * (-N + trn[i, 0] / v[i]) / s2, 0.5 * trn[i, 1] / s2]
-                g = np.sum([c[1] for c in cols], 0) - (R - 1) * np.array(dT + [-T0 / s2])
+        elbo, g, info = _combine_columns(cols, [infoP] + list(sc[:, 2]),
+                                         lambda: _additive_shared(N, s2, v, vsum, trace, trn))
+        if info != 0:
+            raise np.linalg.LinAlgError("Cholesky failed: non-positive pivot %d" % int(info))
+        self.last_terms = dict(log_det_Kuu=logdetK, log_det_P=logdetP, quad=float(Qs.sum()), trace=trace)
         if not want_grad:
             return float(elbo), None
         pairs = []
@@ -1059,9 +971,6 @@ class GPR_additive(_ModelBase):
     def elbo(self):
         return np.float64(self._evaluate(False)[0])
 
-    def maximum_log_likelihood_objective(self):
-        return self.elbo()
-
     # -- prediction -----------------------------------------------------------------------------------------------------------------
     def predict_f(self, Xnew, full_cov=False, full_output_cov=False):
         """Posterior mean (n*, R) and variance (n*, 1) at Xnew[n*, D] for R output columns (reference gpr.py:212-236)."""
@@ -1070,31 +979,14 @@ class GPR_additive(_ModelBase):
             raise NotImplementedError
         s2 = hyper_value(self.likelihood.variance)
         Ks, dKs, Ss, dSs, scals, ws, x, Pinv = self._factor(True)
-        info = torch.stack([ws.scal[2 if self.n_outputs == 1 else 1]] + [s[2] for s in scals])
+        info = torch.stack([ws.info] + [s[2] for s in scals])
         Xs = ops.to_device(Xnew)
         assert Xs.dim() == 2 and Xs.shape[1] == self.d
-        n = Xs.shape[0]
-        dev = Xs.device
-        meshes = torch.cat([ops.device_mesh(b) for b in self.bases])
-        meta, koff = [], 0
-        for i, b in enumerate(self.bases):
-            nk = ops.device_mesh(b).numel()
-            meta += [koff, nk, int(self._offsets[i]), b.m]
-            koff += nk
-        meta = torch.tensor(meta, dtype=torch.int32, device=dev)
-        S_all = torch.cat([S.reshape(-1) for S in Ss])
+        prepared = ops.predict_additive_prepare(self.bases, self._offsets, Ss)
         alphas = x / s2
         prior = float(sum(hyper_value(k.variance) for k in self.kernels))
-        cols = []
-        for alpha in ([alphas] if self.n_outputs == 1 else list(alphas)):       # one pass per output column
-            mean = torch.empty(n, dtype=torch.float64, device=dev)
-            var = torch.empty(n, dtype=torch.float64, device=dev)
-            ops._lib.call("asvgp_predict_additive", ops._p(Xs), n, self.d, ops._p(meshes), ops._p(meta), self.M, self.order,
-                          ops._p(alpha), ops._p(Pinv), ops._p(S_all), prior, ops._p(mean), ops._p(var), ops._stream())
-            cols.append((mean, var))
+        cols = [ops.predict_additive(Xs, self.bases, prepared, alpha, Pinv, prior)          # one pass per output column
+                for alpha in alphas.view(self.n_outputs, self.M)]
         if info.any().item():
             raise np.linalg.LinAlgError("Cholesky failed in predict_f")
-        mean, var = torch.stack([c[0] for c in cols], 1), cols[0][1].view(-1, 1)
-        if isinstance(Xnew, torch.Tensor) and Xnew.is_cuda:
-            return mean, var
-        return mean.cpu().numpy(), var.cpu().numpy()
+        return _like_input(Xnew, torch.stack([c[0] for c in cols], 1), cols[0][1].view(-1, 1))

@@ -428,8 +428,18 @@ def kuu_chain_1d(Kuu, dKuu, basis, chunks=0, gate=False, timing=False):
     return handle
 
 
+class Bound1D:
+    """Slots of the 16-double result row of elbo_grad_1d and elbo_grad_1d_batched (asvgp_elbo_grad_1d in
+    include/asvgp_b200.h); slots 9..14 are clock diagnostics."""
+    ELBO = 0
+    GRAD = slice(1, 4)              # dELBO / d(variance, lengthscale, sigma2)
+    ELBO_GRAD = slice(0, 4)
+    LOG_DET_KUU, LOG_DET_P, QUAD, TRACE, INFO = 4, 5, 6, 7, 8      # QUAD = b^T P^-1 b, TRACE = trace(Kuu^-1 G)
+    DTRACE_DL = 15                  # d trace(Kuu^-1 G) / d lengthscale
+
+
 def elbo_grad_1d(Kuu, dKuu, acc, basis, variance, sigma2, chunks=0, out=None, kuu=None, join_late=None):
-    """Launches the ELBO+gradient kernels; returns the 16-slot device result (see include/asvgp_b200.h).  The Kuu chain
+    """Launches the ELBO+gradient kernels; returns the 16-slot device result (Bound1D).  The Kuu chain
     runs on a side stream next to the two P chains (`kuu`: a handle from kuu_chain_1d launched earlier, e.g. before the
     accumulate; shared by the output columns of a multi-output model)."""
     k, m = basis.order, basis.m
@@ -760,6 +770,27 @@ def band_inverse_1d(A, dA, basis, chunks=0, slot=0):
     return sig, dsig, scal
 
 
+def band_inverses_beside(Ks, dKs, bases):
+    """band_inverse_1d of every per-dimension factor (Ks[i], dKs[i]) on a side stream of its own, ordered after the current
+    stream's work so far.  These short chains (~0.1 ms each) then overlap what the caller launches next on the current stream,
+    e.g. the factorisation of P.  Returns (Ss, dSs, scals, join): call join() before the current stream reads any of them."""
+    main = torch.cuda.current_stream()
+    side = side_streams(len(bases))
+    Ss, dSs, scals = [], [], []
+    for i, (stream, basis) in enumerate(zip(side, bases)):
+        stream.wait_stream(main)
+        with torch.cuda.stream(stream):
+            S, dS, sc = band_inverse_1d(Ks[i], dKs[i], basis, slot=1 + i)
+        for t in (S, dS, sc):
+            t.record_stream(main)
+        Ss.append(S); dSs.append(dS); scals.append(sc)
+
+    def join():
+        for stream in side:
+            main.wait_stream(stream)
+    return Ss, dSs, scals, join
+
+
 KRON_METHODS = ("nd", "band")
 KRON_METHOD = "nd"        # default factorisation of the 2-D model: nested-dissection fronts; "band" = tile DAG over the scalar band
 
@@ -774,10 +805,27 @@ def _check_n_rhs(n_rhs):
     return n_rhs
 
 
-class KronWorkspace:
+class _FactorWorkspace:
+    """What the Kronecker and dense factorisations share: the scalars they leave in `scal`, {log|P|, Q, info} for one
+    right-hand side and {log|P|, info, Q_1 ... Q_n_rhs} for n_rhs > 1 (Q_d = rhs_d^T P^-1 rhs_d, info = 0 or the first
+    non-positive pivot).  `info` is a device view of the info slot."""
+
+    def _alloc_scal(self, n_rhs, dev):
+        self.scal = torch.zeros(3 if n_rhs == 1 else 2 + n_rhs, dtype=F64, device=dev)
+        self.info = self.scal[2 if n_rhs == 1 else 1]
+
+    @staticmethod
+    def unpack_scal(scal):
+        """(log|P|, info, Q[n_rhs]) from a host copy of `scal` in either layout (3 entries: one right-hand side)."""
+        if len(scal) == 3:
+            return scal[0], scal[2], scal[1:2]
+        return scal[0], scal[1], scal[2:]
+
+
+class KronWorkspace(_FactorWorkspace):
     """Device buffers of the factorisation of P = K1 (x) K2 + G / sigma2 (cached per (device, m1, m2, k, method, n_rhs)).
-    n_rhs > 1: one factorisation for n_rhs right-hand sides (asvgp_kron_*_multi; rhs is [n_rhs * M], scal
-    {log|P|, info, Q_1 ... Q_n_rhs}, terms [n_rhs, 11]); n_rhs = 1 is the single-rhs layout of asvgp_kron_factor."""
+    n_rhs > 1: one factorisation for n_rhs right-hand sides (asvgp_kron_*_multi; rhs is [n_rhs * M], terms [n_rhs, 11]);
+    n_rhs = 1 is the single-rhs layout of asvgp_kron_factor."""
 
     def __init__(self, m1, m2, order, method="nd", n_rhs=1):
         lib = _lib.load()
@@ -803,9 +851,14 @@ class KronWorkspace:
         self.n_sig = ns
         self.work = torch.empty(nw, dtype=F64, device=dev)
         self.rhs = torch.zeros(nr, dtype=F64, device=dev)
-        self.scal = torch.zeros(3 if n_rhs == 1 else 2 + n_rhs, dtype=F64, device=dev)
+        self._alloc_scal(n_rhs, dev)
         self.sigma_stencil = torch.zeros((stencil_rows(order), self.M), dtype=F64, device=dev)
         self.terms = torch.zeros(11 if n_rhs == 1 else (n_rhs, 11), dtype=F64, device=dev)
+        # per right-hand side d: where kron_selinv leaves x_d and kron_terms writes its 11 slots (views made once: building
+        # them costs host time on every evaluation)
+        self.x_cols = list(self.rhs[: n_rhs * self.M].view(n_rhs, self.M))
+        self.terms_cols = list(self.terms.view(n_rhs, 11))
+        self.terms_flat = self.terms.view(-1)
 
 
 _KRON_WS = {}
@@ -848,9 +901,8 @@ def kron_plan_info(m1, m2, order, with_fronts=False, n_rhs=None):
 
 
 def kron_factor(K1, K2, acc, bases, sigma2, ws, b=None):
-    """Factorisation of P and forward substitution of Kuf_y; ws.scal = {log|P|, ||L^-1 b||^2, info}.
-    b: right-hand sides [D, M] (D = ws.n_rhs; default: the projection in acc, D = 1).  With D > 1 one factorisation
-    serves all columns and ws.scal = {log|P|, info, ||L^-1 b_1||^2, ..., ||L^-1 b_D||^2}."""
+    """Factorisation of P and forward substitution of Kuf_y, the scalars left in ws.scal (_FactorWorkspace).
+    b: right-hand sides [D, M] (D = ws.n_rhs; default: the projection in acc, D = 1), one factorisation for all of them."""
     k, m1, m2 = _check_bases_2d(bases)
     Gs, b_acc, _ = split_accum_2d(acc, bases)
     if b is None:
@@ -947,9 +999,9 @@ _PREDICT_WORK = {}
 # =====================================================================================================================
 # dense SPD matrices (one front of the nested-dissection kernels) and the additive model's operators
 # =====================================================================================================================
-class DenseWorkspace:
+class DenseWorkspace(_FactorWorkspace):
     """Device buffers of asvgp_dense_factor / asvgp_dense_selinv for n x n matrices (cached per (device, n, n_rhs)).
-    n_rhs > 1: asvgp_dense_*_multi, x is [n_rhs, n] and scal {log|A|, info, rhs_1^T A^-1 rhs_1, ...}."""
+    n_rhs > 1: asvgp_dense_*_multi, x is [n_rhs, n]."""
 
     def __init__(self, n, n_rhs=1):
         lib = _lib.load()
@@ -967,8 +1019,9 @@ class DenseWorkspace:
         self.band = torch.empty(nb, dtype=F64, device=dev)
         self.sig_band = torch.empty(ns, dtype=F64, device=dev)
         self.work = torch.empty(nw, dtype=F64, device=dev)
-        self.scal = torch.zeros(3 if n_rhs == 1 else 2 + n_rhs, dtype=F64, device=dev)
+        self._alloc_scal(n_rhs, dev)
         self.x = torch.empty(n if n_rhs == 1 else (n_rhs, n), dtype=F64, device=dev)
+        self.x_cols = list(self.x.view(n_rhs, n))        # x_d of each right-hand side after dense_selinv
         self.inv = torch.empty((n, n), dtype=F64, device=dev)
 
 
@@ -984,8 +1037,8 @@ def dense_workspace(n, n_rhs=1):
 
 
 def dense_factor(A, rhs, ws):
-    """Cholesky of the dense SPD matrix A (lower triangle read); ws.scal = {log|A|, rhs^T A^-1 rhs, info}.  rhs may be
-    [D, n] for a workspace of D = ws.n_rhs > 1 right-hand sides: ws.scal = {log|A|, info, rhs_1^T A^-1 rhs_1, ...}."""
+    """Cholesky of the dense SPD matrix A (lower triangle read), the scalars left in ws.scal (_FactorWorkspace).  rhs may be
+    [D, n] for a workspace of D = ws.n_rhs > 1 right-hand sides."""
     if rhs.numel() != ws.n_rhs * ws.n:
         raise ValueError("rhs must hold n_rhs = %d columns of %d entries" % (ws.n_rhs, ws.n))
     rhs = rhs.contiguous()
@@ -1018,3 +1071,57 @@ def accum_cross(X, da, db, basis_a, basis_b, out=None):
     _lib.call("asvgp_accum_cross", ctypes.c_void_p(X.data_ptr() + 8 * da), ctypes.c_void_p(X.data_ptr() + 8 * db), D, X.shape[0],
               _p(ma), ma.numel(), _p(mb), mb.numel(), basis_a.order, _p(out), _stream())
     return out
+
+
+
+def additive_put_band(band, basis, offset, out, scale=1.0, add=False):
+    """out[o:o+m, o:o+m] = (add: +=) scale * the lower band [k+1, m] of `basis` as a symmetric block, o = offset."""
+    _lib.call("asvgp_additive_put_band", _p(band), basis.m, basis.order, int(offset), out.shape[0], float(scale), int(add), _p(out),
+              _stream())
+
+
+def additive_put_cross(C, offset_a, offset_b, out):
+    """Writes the block C [m_a, m_b] at (offset_a, offset_b) of the dense matrix `out`, and its transpose."""
+    _lib.call("asvgp_additive_put_cross", _p(C), C.shape[0], C.shape[1], int(offset_a), int(offset_b), out.shape[0], _p(out),
+              _stream())
+
+
+def additive_scale(G, sigma2, out):
+    """out = G / sigma2 (dense M x M)."""
+    _lib.call("asvgp_additive_scale", _p(G), G.shape[0], float(sigma2), _p(out), _stream())
+
+
+def additive_terms(S, x, offset, basis, K, dK, out):
+    """out[4] = {sum S_dd .* K, sum S_dd .* dK, x_d^T K x_d, x_d^T dK x_d} for the diagonal block at `offset` of the dense S."""
+    _lib.call("asvgp_additive_terms", _p(S), _p(x), S.shape[0], int(offset), basis.m, basis.order, _p(K), _p(dK), _p(out),
+              _stream())
+
+
+def dense_terms(S, G, x, out):
+    """out[2] = {sum S .* G, x^T G x} (dense M x M)."""
+    _lib.call("asvgp_dense_terms", _p(S), _p(G), _p(x), S.shape[0], _p(out), _stream())
+
+
+def predict_additive_prepare(bases, offsets, S_bands):
+    """(meshes, meta, S_all) of asvgp_predict_additive from the bases, the first basis function offsets[d] of each dimension
+    and the bands S_bands[d] = band(K_d^-1)."""
+    meshes = torch.cat([device_mesh(b) for b in bases])
+    meta, koff = [], 0
+    for b, o in zip(bases, offsets):
+        nk = device_mesh(b).numel()
+        meta += [koff, nk, int(o), b.m]
+        koff += nk
+    meta = torch.tensor(meta, dtype=torch.int32, device=meshes.device)
+    return meshes, meta, torch.cat([S.reshape(-1) for S in S_bands])
+
+
+def predict_additive(X, bases, prepared, alpha, Pinv, prior_var):
+    """Posterior (mean, var) [n] of the additive model at the device points X[n, D] from alpha = P^-1 Kuf_y / sigma2, the dense
+    P^-1 and predict_additive_prepare's operands."""
+    meshes, meta, S_all = prepared
+    n = X.shape[0]
+    mean = torch.empty(n, dtype=F64, device=X.device)
+    var = torch.empty(n, dtype=F64, device=X.device)
+    _lib.call("asvgp_predict_additive", _p(X), n, X.shape[1], _p(meshes), _p(meta), Pinv.shape[0], bases[0].order, _p(alpha),
+              _p(Pinv), _p(S_all), float(prior_var), _p(mean), _p(var), _stream())
+    return mean, var
