@@ -26,7 +26,8 @@ def ops():
     return _ops
 
 
-@pytest.mark.parametrize("m1,m2,k", [(14, 14, 3), (40, 36, 3), (100, 64, 3), (200, 200, 3), (100, 100, 4), (33, 57, 2), (12, 30, 1)])
+@pytest.mark.parametrize("m1,m2,k", [(14, 14, 3), (40, 36, 3), (100, 64, 3), (200, 200, 3), (100, 100, 4), (33, 57, 2), (12, 30, 1),
+                                    (41, 23, 1), (40, 36, 5), (60, 44, 5), (44, 40, 6), (70, 52, 6)])
 def test_cxx_plan_matches_prototype_and_invariants(ops, m1, m2, k):
     info = ops.kron_plan_info(m1, m2, k, with_fronts=True)
     fronts, root = ND.build_tree(m1, m2, k, leaf=12)
@@ -58,7 +59,15 @@ def test_cxx_plan_matches_prototype_and_invariants(ops, m1, m2, k):
         assert int(info["levels"]) == 9 and int(info["chain_columns"]) <= 1760 and int(info["chain_block_columns"]) <= 34
 
 
-@pytest.mark.parametrize("m1,m2,k,kind", [(14, 14, 3, "Matern32"), (40, 36, 3, "Matern32"), (30, 44, 2, "Matern12"), (36, 30, 4, "Matern52")])
+# relative tolerance on x = P^-1 b.  At k = 6 (44 x 40, cond(P) = 8e10) x is only defined to a few 1e-7 of max|x|: moving the
+# band entries of P by one ulp of max|P| (uniform in [-1, 1] ulp, three draws) moves LAPACK's x by 3.5e-7 ... 2.7e-6 of
+# max|x|; the prototype's elimination order lands 1.6e-7 from LAPACK's (iterative refinement in extended precision puts
+# LAPACK itself within 4e-11).  At k <= 5 the same perturbation moves x by <= 1.1e-11.
+X_TOL = {6: 3e-6}
+
+
+@pytest.mark.parametrize("m1,m2,k,kind", [(14, 14, 3, "Matern32"), (40, 36, 3, "Matern32"), (30, 44, 2, "Matern12"), (36, 30, 4, "Matern52"),
+                                         (41, 23, 1, "Matern12"), (40, 36, 5, "Matern52"), (44, 40, 6, "Matern32")])
 def test_prototype_matches_band_oracle(m1, m2, k, kind):
     from asvgp_b200 import utils as U
 
@@ -77,7 +86,7 @@ def test_prototype_matches_band_oracle(m1, m2, k, kind):
     x = sla.cho_solve_banded((cP, True), b)[:, 0]
     assert abs(out["logdet"] - ld) <= 1e-12 * abs(ld)
     assert abs(out["quad"] - b[:, 0] @ x) <= 1e-10 * abs(b[:, 0] @ x)
-    np.testing.assert_allclose(out["x"], x, rtol=0, atol=1e-11 * np.abs(x).max())
+    np.testing.assert_allclose(out["x"], x, rtol=0, atol=X_TOL.get(k, 1e-11) * np.abs(x).max())
     cols = rng.choice(m1 * m2, 10, replace=False)
     want = O.stencil_columns_of_inverse(Ks, G, s2, k, [m1, m2], cols)
     np.testing.assert_allclose(out["sig"][:, cols], want, rtol=0, atol=1e-12 * np.abs(want).max())
