@@ -58,6 +58,11 @@ SIGNATURES = {
     "asvgp_kronband_factor": [_vp, _vp, _vp, _c_int, _c_int, _c_int, _c_dbl, _vp, _vp, _vp, _vp],
     "asvgp_kronband_selinv": [_vp, _c_int, _c_int, _c_int, _vp, _vp, _vp, _vp, _vp],
     "asvgp_kron_terms": [_vp] * 11 + [_c_int, _c_int, _c_int, _vp, _vp],
+    "asvgp_kron_doubles_batched": [_c_int, _c_int, _c_int, _c_int, _c_int, _vp],
+    "asvgp_kron_factor_batched": [_vp, _vp, _vp, _vp, _c_int, _c_int, _c_int, _c_int, _c_int, _vp, _vp, _c_i64, _vp, _vp],
+    "asvgp_kron_selinv_batched": [_vp, _c_int, _c_int, _c_int, _c_int, _c_int, _c_i64, _vp, _c_i64, _vp, _c_i64, _vp, _vp, _vp],
+    "asvgp_band_inverse_1d_batched": [_vp, _vp, _c_int, _c_int, _c_int, _c_int, _vp, _vp, _vp, _vp, _c_i64, _vp],
+    "asvgp_kron_terms_batched": [_vp] * 11 + [_c_int, _c_int, _c_int, _c_int, _c_int, _vp, _vp],
     "asvgp_predict_2d": [_vp, _c_i64, _vp, _c_int, _vp, _c_int, _c_int, _vp, _vp, _vp, _vp, _c_dbl, _vp, _vp, _vp, _vp],
     "asvgp_allreduce_oneshot": [_vp, _vp, _c_int, _c_int, _c_i64, _c_i64, ctypes.c_uint, _c_int, _vp, _vp, _vp],
     "asvgp_dense_factor": [_vp, _c_int, _vp, _vp, _vp, _vp],
@@ -82,6 +87,7 @@ VALUE_FUNCTIONS = {
     "asvgp_workspace_bytes_1d": (_c_i64, [_c_int, _c_int, _c_int]),
     "asvgp_workspace_bytes_1d_batched": (_c_i64, [_c_int, _c_int, _c_int, _c_int, _c_int]),
     "asvgp_workspace_bytes_posterior_1d_batched": (_c_i64, [_c_int, _c_int, _c_int, _c_int]),
+    "asvgp_workspace_bytes_band_inverse_1d_batched": (_c_i64, [_c_int, _c_int, _c_int, _c_int]),
     "asvgp_kuu_state_doubles": (_c_i64, [_c_int, _c_int]),
     "asvgp_accum_1d_binned_work_bytes": (_c_i64, [_c_i64]),
     "asvgp_accum_2d_binned_work_bytes": (_c_i64, [_c_i64]),

@@ -750,7 +750,7 @@ struct BandInvArgs {
 };
 
 template <int K>
-__global__ void __launch_bounds__(kChainThreads) band_inverse_kernel(BandInvArgs<K> a) {
+__device__ __forceinline__ void band_inverse_body(const BandInvArgs<K>& a) {
     using T = Dual<1>;
     extern __shared__ __align__(16) char smem[];
     const int p = threadIdx.x;
@@ -770,6 +770,36 @@ __global__ void __launch_bounds__(kChainThreads) band_inverse_kernel(BandInvArgs
     if (p == 0) {
         a.scal[0] = tot.logdet.v; a.scal[1] = tot.logdet.d[0]; a.scal[2] = (double)tot.info; a.scal[3] = 0.0;
     }
+}
+
+template <int K>
+__global__ void __launch_bounds__(kChainThreads) band_inverse_kernel(BandInvArgs<K> a) {
+    band_inverse_body<K>(a);
+}
+
+// B band inverses of one size in one launch (asvgp_band_inverse_1d_batched): CTA b runs slot b's arguments, so every slot is
+// the single call's chain on its own operands and scratch, bit for bit.  Its row tables come from chain_rows_batched_kernel
+// (blockIdx.y = slot), entry for entry chain_rows_kernel's.
+template <int K>
+struct BandInvBatch {
+    BandInvArgs<K> s[ASVGP_MAX_BATCH];
+};
+template <int K>
+__global__ void __launch_bounds__(kChainThreads) band_inverse_batched_kernel(const __grid_constant__ BandInvBatch<K> b) {
+    band_inverse_body<K>(b.s[blockIdx.x]);
+}
+
+template <class T>
+struct RowsBatch {
+    ChainSpec<T> spec[ASVGP_MAX_BATCH];
+    T* out[ASVGP_MAX_BATCH];
+};
+template <class T, int K>
+__global__ void __launch_bounds__(256) chain_rows_batched_kernel(ChunkLayout lay, const __grid_constant__ RowsBatch<T> r) {
+    const unsigned total = (unsigned)chain_rows_count<T, K>(lay);
+    T* out = r.out[blockIdx.y];
+    for (unsigned t = blockIdx.x * blockDim.x + threadIdx.x; t < total; t += gridDim.x * blockDim.x)
+        out[t] = chain_rows_entry<T, K>(lay, r.spec[blockIdx.y], t);
 }
 
 template <int K>
@@ -801,6 +831,39 @@ static int launch_band_inverse(const ChunkLayout& lay, const double* A, const do
 }
 
 static size_t align256(size_t n) { return (n + 255) & ~(size_t)255; }
+
+// Slot b of a batch: A + b (K+1) M, its scratch at work + b slot_bytes (carved as launch_band_inverse carves it), outputs
+// sig_val / sig_tan + b (K+1) M and scal + 4 b.
+template <int K>
+static int launch_band_inverse_batched(const ChunkLayout& lay, int B, const double* A, const double* dA, double* sig_val,
+                                       double* sig_tan, double* scal, char* work, size_t slot_bytes, cudaStream_t st) {
+    using T = Dual<1>;
+    BandInvBatch<K> bb;
+    RowsBatch<T> rb;
+    const size_t band = (size_t)(K + 1) * lay.M;
+    for (int b = 0; b < B; ++b) {
+        BandInvArgs<K>& a = bb.s[b];
+        a.lay = lay;
+        char* p = work + b * slot_bytes;
+        a.cols = ChainPlan<T, K>::carve(lay, p);
+        p += ChainPlan<T, K>::bytes(lay);
+        a.sig = reinterpret_cast<T*>(p);
+        a.A = A + b * band; a.dA = dA + b * band; a.sig_val = sig_val + b * band; a.sig_tan = sig_tan + b * band; a.scal = scal + 4 * b;
+        p += ((size_t)(K + 1) * lay.M * sizeof(T) + 255) & ~(size_t)255;
+        a.rows = reinterpret_cast<T*>(p);
+        rb.spec[b] = ChainSpec<T>{BandMat<T>{a.A, a.dA, nullptr, 0.0, 0.0, 1, lay.M}, VecRhs<T>{a.A, lay.M, 0}};
+        rb.out[b] = reinterpret_cast<T*>(p);
+        ASVGP_CUDA_OK(cudaMemsetAsync(a.sig, 0, (size_t)(K + 1) * lay.M * sizeof(T), st));
+    }
+    const size_t total = chain_rows_count<T, K>(lay);
+    chain_rows_batched_kernel<T, K><<<dim3((unsigned)((total + 255) / 256), B), 256, 0, st>>>(lay, rb); ASVGP_LAUNCHED();
+    ASVGP_CUDA_OK(cudaGetLastError());
+    const size_t smem = ChainSmall<T, K>::bytes(lay.P);
+    ASVGP_CUDA_OK(cudaFuncSetAttribute(band_inverse_batched_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    band_inverse_batched_kernel<K><<<B, kChainThreads, smem, st>>>(bb); ASVGP_LAUNCHED();
+    ASVGP_CUDA_OK(cudaGetLastError());
+    return kOk;
+}
 // Programmatic dependent launch: the kernel may be scheduled while its predecessor in the stream is still running (its CTAs
 // park in pdl_wait() until that grid has completed and flushed), which takes the launch latency and the cluster's
 // co-scheduling off the chain of three dependent launches (row tables -> chains -> bound).
@@ -1354,5 +1417,32 @@ extern "C" int asvgp_band_inverse_1d(const double* A, const double* dA, int M, i
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     ASVGP_DISPATCH_ORDER(order, { if (int rc = launch_band_inverse<K>(lay, A, dA, sig_val, sig_tan, scal,
                                                                       static_cast<char*>(work), st)) return rc; });
+    return kOk;
+}
+
+// Per-slot scratch of asvgp_band_inverse_1d_batched: asvgp_workspace_bytes_1d rounded up to 256 bytes.
+static int64_t band_inverse_slot_bytes(int M, int order, int chunks) {
+    const int64_t one = asvgp_workspace_bytes_1d(M, order, chunks);
+    return one < 0 ? -1 : (int64_t)align256((size_t)one);
+}
+
+extern "C" int64_t asvgp_workspace_bytes_band_inverse_1d_batched(int M, int order, int chunks, int B) {
+    if (M <= 0 || order < 1 || order > kMaxOrder || B < 1 || B > ASVGP_MAX_BATCH) return -1;
+    return B * band_inverse_slot_bytes(M, order, chunks);
+}
+
+extern "C" int asvgp_band_inverse_1d_batched(const double* A, const double* dA, int M, int order, int chunks, int B, double* sig_val,
+                                             double* sig_tan, double* scal, void* work, int64_t work_bytes, void* stream) {
+    ASVGP_REQUIRE(M > 2 * order && order >= 1 && order <= kMaxOrder, "band_inverse_1d_batched: M=%d order=%d", M, order);
+    ASVGP_REQUIRE(B >= 1 && B <= ASVGP_MAX_BATCH, "band_inverse_1d_batched: B=%d not in 1..%d", B, ASVGP_MAX_BATCH);
+    ASVGP_REQUIRE(A != nullptr && dA != nullptr && sig_val != nullptr && sig_tan != nullptr && scal != nullptr && work != nullptr,
+                  "band_inverse_1d_batched: NULL buffer");
+    ASVGP_REQUIRE(work_bytes >= asvgp_workspace_bytes_band_inverse_1d_batched(M, order, chunks, B),
+                  "band_inverse_1d_batched: workspace too small");
+    const ChunkLayout lay = pick_layout(M, order, chunks);
+    const size_t slot_bytes = (size_t)band_inverse_slot_bytes(M, order, chunks);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    ASVGP_DISPATCH_ORDER(order, { if (int rc = launch_band_inverse_batched<K>(lay, B, A, dA, sig_val, sig_tan, scal,
+                                                                              static_cast<char*>(work), slot_bytes, st)) return rc; });
     return kOk;
 }

@@ -374,14 +374,17 @@ static NdLayout nd_layout(const NdPlan& P) {
 // assembly: entries of P (+ right-hand side row) of every front, one fully parallel launch; the children's update matrices
 // are added by the children's own factorisation tasks (scatter_to_parent)
 // ---------------------------------------------------------------------------------------------------------------------
+// Slot s of a batch (blockIdx.y) assembles K1 + s k1_stride, K2 + s k2_stride and sigma2[s] into Lpool + s band_stride; Gs
+// and b are shared.  The single calls are the one-slot case.
 struct NdAssembleArgs {
     const FrontDesc* fronts; const int4* tasks; int n_tasks;
     const int* idx;
     const double *K1, *K2, *Gs, *b;
-    double sigma2;
     int m1, m2, K, M;
     double* Lpool;
     const double* dense;           // non-null: the matrix itself, M x M row-major (lower triangle read), instead of K1, K2, Gs
+    long long band_stride, k1_stride, k2_stride;
+    double sigma2[ASVGP_MAX_BATCH];
 };
 
 __device__ __forceinline__ double nd_band_sym(const double* B, int m, int K, int i, int j) {
@@ -391,7 +394,7 @@ __device__ __forceinline__ double nd_band_sym(const double* B, int m, int K, int
 
 // A'(gi, gj): gi, gj grid unknowns or rhs nodes (id M + d: A'(g, rhs_d) = b[d M + g], A'(rhs_d, rhs_e) = 0).  Same roundings as
 // the reference's `Kuu + KufKfu / sigma2`.
-__device__ __forceinline__ double nd_entry(const NdAssembleArgs& a, int gi, int gj) {
+__device__ __forceinline__ double nd_entry(const NdAssembleArgs& a, const double* K1, const double* K2, double sigma2, int gi, int gj) {
     if (gi >= a.M || gj >= a.M) {
         if (gi >= a.M && gj >= a.M) return 0.0;
         return gi >= a.M ? __ldg(a.b + (long long)(gi - a.M) * a.M + gj) : __ldg(a.b + (long long)(gj - a.M) * a.M + gi);
@@ -402,17 +405,22 @@ __device__ __forceinline__ double nd_entry(const NdAssembleArgs& a, int gi, int 
     int col = gj;
     if (d1 < 0 || (d1 == 0 && d2 < 0)) { d1 = -d1; d2 = -d2; col = gi; }
     if (d1 > a.K || d2 > a.K || d2 < -a.K) return 0.0;
-    const double kv = __dmul_rn(nd_band_sym(a.K1, a.m1, a.K, i1, j1), nd_band_sym(a.K2, a.m2, a.K, i2, j2));
+    const double kv = __dmul_rn(nd_band_sym(K1, a.m1, a.K, i1, j1), nd_band_sym(K2, a.m2, a.K, i2, j2));
     const double g = __ldg(a.Gs + (long long)(d1 * (2 * a.K + 1) + d2 + a.K) * a.M + col);
-    return __dadd_rn(kv, __ddiv_rn(g, a.sigma2));
+    return __dadd_rn(kv, __ddiv_rn(g, sigma2));
 }
 
-__global__ void __launch_bounds__(256) nd_assemble_kernel(NdAssembleArgs a) {
+__global__ void __launch_bounds__(256) nd_assemble_kernel(const __grid_constant__ NdAssembleArgs a) {
+    const int slot = blockIdx.y;
+    const double* K1 = a.K1 + slot * a.k1_stride;
+    const double* K2 = a.K2 + slot * a.k2_stride;
+    const double sigma2 = a.sigma2[slot];
+    double* Lpool = a.Lpool + slot * a.band_stride;
     for (int t = blockIdx.x; t < a.n_tasks; t += gridDim.x) {
         const int4 tk = a.tasks[t];
         const FrontDesc f = a.fronts[tk.x];
         const int R = tk.y, C = tk.z;
-        double* tile = a.Lpool + front_tile(f, R, C) * TILE_P;
+        double* tile = Lpool + front_tile(f, R, C) * TILE_P;
         const int* idx = a.idx + f.idx_off;
         if (C >= f.nsT && f.child[0] < 0) continue;          // trailing tiles of a leaf front start from zero: never read
         for (int e = threadIdx.x; e < TILE; e += blockDim.x) {
@@ -421,7 +429,7 @@ __global__ void __launch_bounds__(256) nd_assemble_kernel(NdAssembleArgs a) {
             const int gi = idx[I], gj = idx[J];
             double v;
             if (gi < 0 || gj < 0) v = (I == J && C < f.nsT) ? 1.0 : 0.0;
-            else v = (C < f.nsT) ? nd_entry(a, gi, gj) : 0.0;
+            else v = (C < f.nsT) ? nd_entry(a, K1, K2, sigma2, gi, gj) : 0.0;
             tile[c * LDT + r] = v;
         }
     }
@@ -430,20 +438,24 @@ __global__ void __launch_bounds__(256) nd_assemble_kernel(NdAssembleArgs a) {
 // ---------------------------------------------------------------------------------------------------------------------
 // factorisation of all fronts of one level
 // ---------------------------------------------------------------------------------------------------------------------
+// A batch of n_slots settings: combined task t is task t / n_slots of slot t % n_slots (task-major, so every slot keeps its own
+// task order and a task still waits only on tasks dealt before it), and slot s owns the band buffer at s band_stride doubles.
 struct NdFactorArgs {
     const FrontDesc* fronts; const int4* tasks; int n_tasks;
     const int *idx, *pmap;
     double* Lpool; double* linv;
     int* ready;         // [n_tiles] + abort at [n_tiles], first bad pivot (node id + 1) at [n_tiles + 1]
     long long n_tiles;
+    int n_slots;
+    long long band_stride;
 };
 
 // Extend-add, from the child's side: this thread's 4 x 4 block of the update tile (R, C) of front f (R >= C >= nsT) is added
 // into the parent's front (fp64 REDs: the two children of a parent add into the same entries; the parent was assembled before
 // any factorisation kernel ran and is factorised by a later launch).  The parent stores its lower triangle, with FULL diagonal
 // tiles; the child's diagonal update tiles are full too, so only their lower triangle is sent.
-__device__ __forceinline__ void scatter_to_parent(const double (&acc)[4][4], const NdFactorArgs& a, const FrontDesc& f, int R, int C,
-                                                  int tm, int tn) {
+__device__ __forceinline__ void scatter_to_parent(const double (&acc)[4][4], const NdFactorArgs& a, double* Lpool, const FrontDesc& f,
+                                                  int R, int C, int tm, int tn) {
     const FrontDesc p = a.fronts[f.parent];
     const int* pm = a.pmap + f.pmap_off;
     int pr[4], pc[4];
@@ -455,7 +467,7 @@ __device__ __forceinline__ void scatter_to_parent(const double (&acc)[4][4], con
         for (int j = 0; j < 4; ++j) {
             if (pr[i] < 0 || pc[j] < 0 || (R == C && tm + i < tn + j)) continue;
             const int hi = max(pr[i], pc[j]), lo = min(pr[i], pc[j]);
-            double* t = a.Lpool + front_tile(p, hi / NB, lo / NB) * TILE_P;
+            double* t = Lpool + front_tile(p, hi / NB, lo / NB) * TILE_P;
             atomicAdd(t + (lo % NB) * LDT + hi % NB, acc[i][j]);
             if (hi / NB == lo / NB && hi != lo) atomicAdd(t + (hi % NB) * LDT + lo % NB, acc[i][j]);
         }
@@ -469,28 +481,32 @@ __global__ void __launch_bounds__(kTdThreads, 2) nd_factor_kernel(NdFactorArgs a
     __shared__ int s_bad;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int tm = (tid & 15) * 4, tn = (tid >> 4) * 4;
-    int* abort_flag = a.ready + a.n_tiles;
     if (tid == 0) mbar_init(&full, 1);
     fence_proxy_async();
     __syncthreads();
     uint32_t phase = 0;
 
-    for (int t = blockIdx.x; t < a.n_tasks; t += gridDim.x) {
-        const int4 tk = a.tasks[t];
+    for (int t = blockIdx.x; t < a.n_tasks * a.n_slots; t += gridDim.x) {
+        const int slot = t % a.n_slots;
+        const int4 tk = a.tasks[t / a.n_slots];
+        double* const Lpool = a.Lpool + slot * a.band_stride;
+        double* const linv = a.linv + slot * a.band_stride;
+        int* const ready = a.ready + 2 * slot * a.band_stride;
+        int* const abort_flag = ready + a.n_tiles;
         const FrontDesc f = a.fronts[tk.x];
         const int R = tk.y, C = tk.z;
         const bool diag = R == C;
-        double* my_tile = a.Lpool + front_tile(f, R, C) * TILE_P;
+        double* my_tile = Lpool + front_tile(f, R, C) * TILE_P;
         const int nJ = min(C, f.nsT);
 
         auto issue = [&](int J) {                    // thread 0: wait for the operand tiles, then fetch them by TMA
             const long long tR = front_tile(f, R, J), tC = front_tile(f, C, J);
-            wait_flag(a.ready + tR, 1, abort_flag);
-            if (!diag) wait_flag(a.ready + tC, 1, abort_flag);
+            wait_flag(ready + tR, 1, abort_flag);
+            if (!diag) wait_flag(ready + tC, 1, abort_flag);
             fence_proxy_async();
             mbar_expect_tx(&full, diag ? TILE_P_BYTES : 2 * TILE_P_BYTES);
-            tma_load_ptile(pA, a.Lpool + tR * TILE_P, &full);
-            if (!diag) tma_load_ptile(pB, a.Lpool + tC * TILE_P, &full);
+            tma_load_ptile(pA, Lpool + tR * TILE_P, &full);
+            if (!diag) tma_load_ptile(pB, Lpool + tC * TILE_P, &full);
         };
         if (tid == 0 && nJ > 0) issue(0);
         double acc[4][4];
@@ -516,7 +532,7 @@ __global__ void __launch_bounds__(kTdThreads, 2) nd_factor_kernel(NdFactorArgs a
 
         if (C >= f.nsT) {
             // ---- trailing tile: this front's update matrix, added straight into the parent's front --------------------------
-            if (f.parent >= 0) scatter_to_parent(acc, a, f, R, C, tm, tn);
+            if (f.parent >= 0) scatter_to_parent(acc, a, Lpool, f, R, C, tm, tn);
             else regs_to_tile_ld<LDT>(acc, my_tile, tm, tn);     // root: entry (rhs, rhs) = -||y||^2
         } else if (diag) {
             // ---- diagonal tile: Cholesky + inverse in registers ---------------------------------------------------------------
@@ -535,21 +551,21 @@ __global__ void __launch_bounds__(kTdThreads, 2) nd_factor_kernel(NdFactorArgs a
                 for (int j = 0; j < 4; ++j) {
                     if (tm + i < tn + j) { acc[i][j] = 0.0; V[i][j] = 0.0; }
                 }
-            regs_to_tile_ld<LDT>(V, a.linv + (long long)(f.linv_base + C) * TILE_P, tm, tn);
+            regs_to_tile_ld<LDT>(V, linv + (long long)(f.linv_base + C) * TILE_P, tm, tn);
             regs_to_tile_ld<LDT>(acc, my_tile, tm, tn);
             __threadfence();
             __syncthreads();
             if (tid == 0) {
-                st_release(a.ready + front_tile(f, C, C), 1);
-                if (first_bad >= 0) atomicMin(a.ready + a.n_tiles + 1, a.idx[f.idx_off + C * NB + first_bad] + 1);
+                st_release(ready + front_tile(f, C, C), 1);
+                if (first_bad >= 0) atomicMin(ready + a.n_tiles + 1, a.idx[f.idx_off + C * NB + first_bad] + 1);
             }
         } else {
             // ---- sub-diagonal tile: L(R,C) = A L(C,C)^-T -------------------------------------------------------------------------
             if (tid == 0) {
-                wait_flag(a.ready + front_tile(f, C, C), 1, abort_flag);
+                wait_flag(ready + front_tile(f, C, C), 1, abort_flag);
                 fence_proxy_async();
                 mbar_expect_tx(&full, TILE_P_BYTES);
-                tma_load_ptile(pB, a.linv + (long long)(f.linv_base + C) * TILE_P, &full);
+                tma_load_ptile(pB, linv + (long long)(f.linv_base + C) * TILE_P, &full);
             }
             regs_to_tile_ld<LDT>(acc, pA, tm, tn);   // A(m, k) at [k*LDT + m]
             __syncthreads();
@@ -569,7 +585,7 @@ __global__ void __launch_bounds__(kTdThreads, 2) nd_factor_kernel(NdFactorArgs a
             regs_to_tile_ld<LDT>(L, my_tile, tm, tn);
             __threadfence();
             __syncthreads();
-            if (tid == 0) st_release(a.ready + front_tile(f, R, C), 1);
+            if (tid == 0) st_release(ready + front_tile(f, R, C), 1);
         }
         __syncthreads();
     }
@@ -577,12 +593,18 @@ __global__ void __launch_bounds__(kTdThreads, 2) nd_factor_kernel(NdFactorArgs a
 
 // log|P| = 2 sum log L_jj (deterministic: fixed slices, tree reductions, the last block to finish adds the slices in order),
 // ||y_d||^2 = -(root update entry (rhs_d, rhs_d)), info, and tau.  scal_out[0] = log|P|, scal_out[q_slot + d] = ||y_d||^2,
-// scal_out[info_slot] = info.
+// scal_out[info_slot] = info.  Slot blockIdx.y of a batch: its band buffer at blockIdx.y band_stride doubles (Lpool, ready and
+// scal_keep move with it), its scalars at scal_out + blockIdx.y scal_stride.
 __global__ void __launch_bounds__(256) nd_scalars_kernel(const long long* __restrict__ doff, int M, const double* __restrict__ Lpool,
                                                          const long long* __restrict__ quad_off, int R, int q_slot, int info_slot,
                                                          int* __restrict__ ready, long long n_tiles,
-                                                         double* __restrict__ scal_out, double* __restrict__ scal_keep) {
+                                                         double* __restrict__ scal_out, double* __restrict__ scal_keep,
+                                                         long long band_stride, int scal_stride) {
     __shared__ double s[256];
+    Lpool += blockIdx.y * band_stride;
+    ready += 2 * blockIdx.y * band_stride;
+    scal_keep += blockIdx.y * band_stride;
+    scal_out += blockIdx.y * scal_stride;
     __shared__ bool last;
     double acc = 0.0;
     for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < M; j += gridDim.x * blockDim.x) acc += log(__ldcg(Lpool + doff[j]));
@@ -622,11 +644,14 @@ __global__ void __launch_bounds__(256) nd_scalars_kernel(const long long* __rest
 // ---------------------------------------------------------------------------------------------------------------------
 // Pre-pass over every tile (R, C), C < nsT, of every front, fully parallel: off-diagonal tiles become Y^T
 // (Y = L(R,C) L(C,C)^-1, stored transposed so that it is a plain operand later), diagonal tiles seed
-// Sigma(C,C) = L(C,C)^-T L(C,C)^-1.
+// Sigma(C,C) = L(C,C)^-T L(C,C)^-1.  Slot blockIdx.y of a batch: Lpool, linv + blockIdx.y band_stride, sig_lower + blockIdx.y sig_stride.
 __global__ void __launch_bounds__(kTdThreads) nd_ypass_kernel(const FrontDesc* __restrict__ fronts, const int4* __restrict__ tasks,
                                                               int n_tasks, double* __restrict__ Lpool, const double* __restrict__ linv,
-                                                              double* __restrict__ sig_lower) {
+                                                              double* __restrict__ sig_lower, long long band_stride, long long sig_stride) {
     extern __shared__ __align__(16) unsigned char yp_smem[];
+    Lpool += blockIdx.y * band_stride;
+    linv += blockIdx.y * band_stride;
+    sig_lower += blockIdx.y * sig_stride;
     double* pL = reinterpret_cast<double*>(yp_smem);         // L tile as the A operand: L[m][k] at [k*LDT + m]
     double* pI = pL + TILE_P;                                // Linv transposed: Linv[k][n] at [k*LDT + n]
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -662,9 +687,13 @@ struct NdGatherArgs {
     double *sig_lower, *sig_upper;
     const double* scal_keep;        // [1] = tau
     int n_rhs;
+    long long band_stride, sig_stride;      // slot blockIdx.y: scal_keep + y band_stride, sig_* + y sig_stride
 };
 __global__ void __launch_bounds__(256) nd_gather_kernel(NdGatherArgs a) {
     __shared__ double s_t[NB][NB + 1];
+    a.sig_lower += blockIdx.y * a.sig_stride;
+    a.sig_upper += blockIdx.y * a.sig_stride;
+    a.scal_keep += blockIdx.y * a.band_stride;
     for (int t = blockIdx.x; t < a.n_tasks; t += gridDim.x) {
         const int4 tk = a.tasks[t];
         const FrontDesc f = a.fronts[tk.x];
@@ -707,6 +736,8 @@ struct NdSelArgs {
     int* sready;            // [n_tiles] tile flags, [n_cnt] per-block-column counters, abort
     long long n_tiles;
     int n_cnt;
+    int n_slots;            // tasks dealt task-major over the slots, as in nd_factor_kernel
+    long long band_stride, sig_stride, work_stride;     // doubles between the slots' buffers
 };
 
 // A diagonal Sigma tile is symmetric only up to rounding (a sum of REDs of termwise unsymmetric products): the operand handed
@@ -724,6 +755,9 @@ __device__ __forceinline__ void symmetrise_ptile(double* __restrict__ s, int tid
     for (int j = 0; j < 16; ++j) s[c * LDT + ((c + g * 16 + j) & (NB - 1))] = v[j];
 }
 
+// kBatched = false is the single-setting kernel (one slot; the kernel sits at its 128-register cap, and the slot arithmetic of
+// the batched instance would make it spill).
+template <bool kBatched>
 __global__ void __launch_bounds__(kTdThreads, 2) nd_selinv_kernel(NdSelArgs a) {
     extern __shared__ __align__(128) unsigned char td_smem[];
     double* const pA = reinterpret_cast<double*>(td_smem);
@@ -731,15 +765,20 @@ __global__ void __launch_bounds__(kTdThreads, 2) nd_selinv_kernel(NdSelArgs a) {
     __shared__ __align__(8) uint64_t full;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int tm = (tid & 15) * 4, tn = (tid >> 4) * 4;
-    int* cnt = a.sready + a.n_tiles;
-    int* abort_flag = cnt + a.n_cnt;
     if (tid == 0) mbar_init(&full, 1);
     fence_proxy_async();
     __syncthreads();
     uint32_t phase = 0;
 
-    for (int t = blockIdx.x; t < a.n_tasks; t += gridDim.x) {
-        const int4 tk = a.tasks[t];
+    for (int t = blockIdx.x; t < a.n_tasks * (kBatched ? a.n_slots : 1); t += gridDim.x) {
+        const int slot = kBatched ? t % a.n_slots : 0;
+        const int4 tk = a.tasks[kBatched ? t / a.n_slots : t];
+        const double* const Lpool = a.Lpool + slot * a.band_stride;
+        double* const sig_lower = a.sig_lower + slot * a.sig_stride;
+        double* const sig_upper = a.sig_upper + slot * a.sig_stride;
+        int* const sready = a.sready + 2 * slot * a.work_stride;
+        int* const cnt = sready + a.n_tiles;
+        int* const abort_flag = cnt + a.n_cnt;
         const FrontDesc f = a.fronts[tk.x];
         const int R = tk.y, C = tk.z;                // R > C, C < nsT
         const int Kmax = f.nT - 1, nK = Kmax - C;
@@ -748,18 +787,18 @@ __global__ void __launch_bounds__(kTdThreads, 2) nd_selinv_kernel(NdSelArgs a) {
             const int* flag = nullptr;
             int want = 1;
             if (K == R) {
-                src = a.sig_lower + front_tile(f, R, R) * TILE_P;
+                src = sig_lower + front_tile(f, R, R) * TILE_P;
                 if (R < f.nsT) { flag = cnt + f.cnt_base + R; want = f.nT - 1 - R; }      // all shares in
             } else if (K < R) {
-                src = a.sig_lower + front_tile(f, R, K) * TILE_P;
-                if (K < f.nsT) flag = a.sready + front_tile(f, R, K);
+                src = sig_lower + front_tile(f, R, K) * TILE_P;
+                if (K < f.nsT) flag = sready + front_tile(f, R, K);
             } else {
-                src = a.sig_upper + front_tile(f, K, R) * TILE_P;
-                if (R < f.nsT) flag = a.sready + front_tile(f, K, R);
+                src = sig_upper + front_tile(f, K, R) * TILE_P;
+                if (R < f.nsT) flag = sready + front_tile(f, K, R);
             }
             // the Y^T operand is there since the pre-pass: it is requested before the wait, only Sigma(R,K) after it
             mbar_expect_tx(&full, 2 * TILE_P_BYTES);
-            tma_load_ptile(pB, a.Lpool + front_tile(f, K, C) * TILE_P, &full);
+            tma_load_ptile(pB, Lpool + front_tile(f, K, C) * TILE_P, &full);
             if (flag != nullptr) wait_flag(flag, want, abort_flag);
             fence_proxy_async();
             tma_load_ptile(pA, src, &full);
@@ -779,17 +818,17 @@ __global__ void __launch_bounds__(kTdThreads, 2) nd_selinv_kernel(NdSelArgs a) {
                 } else {
                     // after the last product: fetch this tile's own Y^T for the diagonal contribution below
                     mbar_expect_tx(&full, TILE_P_BYTES);
-                    tma_load_ptile(pB, a.Lpool + front_tile(f, R, C) * TILE_P, &full);
+                    tma_load_ptile(pB, Lpool + front_tile(f, R, C) * TILE_P, &full);
                 }
             }
         }
         frags_subtract(acc, cf, pA, warp, lane, tm, tn);                // acc = -sum_K Sigma(R,K) Y(K,C)
         const long long me = front_tile(f, R, C);
-        regs_to_tile_ld<LDT>(acc, a.sig_lower + me * TILE_P, tm, tn);
+        regs_to_tile_ld<LDT>(acc, sig_lower + me * TILE_P, tm, tn);
         regs_to_tile_t_ld<LDT>(acc, pA, tm, tn);         // T[m][a] at [m*LDT + a]  ==  A'(a, k=m) at [k*LDT + a]
         __syncthreads();
         {
-            double* up = a.sig_upper + me * TILE_P;
+            double* up = sig_upper + me * TILE_P;
 #pragma unroll
             for (int idx = tid; idx < TILE / 2; idx += kTdThreads) {
                 const int c = idx >> 5, r = (idx & 31) * 2;
@@ -798,14 +837,14 @@ __global__ void __launch_bounds__(kTdThreads, 2) nd_selinv_kernel(NdSelArgs a) {
         }
         __threadfence();
         __syncthreads();
-        if (tid == 0) st_release(a.sready + me, 1);
+        if (tid == 0) st_release(sready + me, 1);
         mbar_wait(&full, phase);
         phase ^= 1u;
         {
             // D[a][b] = sum_m T[m][a] Y[m][b]: this tile's share of Sigma(C,C), added as REDs
             double D[8][2] = {};
             dmma_tile(D, pA, pB, warp, lane);
-            double* Sd = a.sig_lower + front_tile(f, C, C) * TILE_P;
+            double* Sd = sig_lower + front_tile(f, C, C) * TILE_P;
             const int row = warp * 8 + (lane >> 2), col = (lane & 3) * 2;
 #pragma unroll
             for (int cb = 0; cb < 8; ++cb) {
@@ -820,9 +859,15 @@ __global__ void __launch_bounds__(kTdThreads, 2) nd_selinv_kernel(NdSelArgs a) {
 }
 
 // x[d M + j] = x_d,j = -Sigma'(rhs_d, j) / tau  (t < R M)
+// Slot blockIdx.y of a batch: sig_lower + y sig_stride, scal_keep + y band_stride, abort_flag + 2 y work_stride, x + y RM.
 __global__ void __launch_bounds__(256) nd_x_kernel(const long long* __restrict__ xoff, int RM, const double* __restrict__ sig_lower,
                                                    const double* __restrict__ scal_keep, const int* __restrict__ abort_flag,
-                                                   double* __restrict__ x) {
+                                                   double* __restrict__ x, long long band_stride, long long sig_stride,
+                                                   long long work_stride) {
+    sig_lower += blockIdx.y * sig_stride;
+    scal_keep += blockIdx.y * band_stride;
+    abort_flag += 2 * blockIdx.y * work_stride;
+    x += (long long)blockIdx.y * RM;
     const double inv_tau = -1.0 / scal_keep[1];
     const bool aborted = *abort_flag != 0;
     for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < RM; j += gridDim.x * blockDim.x)
@@ -837,13 +882,19 @@ __device__ __forceinline__ double nd_rank_correction(const double* __restrict__ 
     return c;
 }
 
-// stencil entries of P^-1 = Sigma' - tau sum_d x_d x_d^T
+// stencil entries of P^-1 = Sigma' - tau sum_d x_d x_d^T.  Slot blockIdx.y of a batch: as nd_x_kernel, out + y total.
 __global__ void __launch_bounds__(256) nd_stencil_kernel(const long long* __restrict__ sigoff, int m1, int m2, int K, int R,
                                                          const double* __restrict__ sig_lower, const double* __restrict__ x,
                                                          const double* __restrict__ scal_keep, const int* __restrict__ abort_flag,
-                                                         double* __restrict__ out) {
+                                                         double* __restrict__ out, long long band_stride, long long sig_stride,
+                                                         long long work_stride) {
     const int NS = 2 * K + 1, n_e = (K + 1) * NS;
     const long long M = (long long)m1 * m2, total = M * n_e;
+    sig_lower += blockIdx.y * sig_stride;
+    scal_keep += blockIdx.y * band_stride;
+    abort_flag += 2 * blockIdx.y * work_stride;
+    x += blockIdx.y * M * R;
+    out += blockIdx.y * total;
     const double tau = scal_keep[1];
     const bool aborted = *abort_flag != 0;
     for (long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x; t < total; t += (long long)gridDim.x * blockDim.x) {
@@ -981,54 +1032,77 @@ static int64_t nd_plan_info(int m1, int m2, int order, int n_rhs, double* out, i
 
 
 // ---- shared bodies of the Kronecker and the dense entry points -----------------------------------------------------------------
+// A batch of B settings on one plan: slot s owns band + s band, sig_band + s sig, work + s work (strides in doubles, 0 for the
+// single calls), its scalars at scal + s scal_stride and its x at x_out + s n_rhs M.
+struct NdBatch {
+    int B = 1;
+    long long band = 0, sig = 0, work = 0;
+    int scal = 0;
+};
+// CTAs per slot of the fully parallel kernels: the single call's `cap`, shared out over the slots
+static int nd_grid_x(long long n, int cap, int B) { return (int)std::max<long long>(1, std::min<long long>(n, (cap + B - 1) / B)); }
+
 // multi = false: scal = { log|P|, Q, info } (single-rhs layout); true: scal = { log|P|, info, Q_1 ... Q_R }
-static int nd_factor_run(const NdPlan& P, NdAssembleArgs aa, double* band, double* scal, bool multi, cudaStream_t st) {
+static int nd_factor_run(const NdPlan& P, NdAssembleArgs aa, double* band, double* scal, bool multi, cudaStream_t st,
+                         const NdBatch& nb = NdBatch()) {
     const NdLayout lay = nd_layout(P);
     int* flags = reinterpret_cast<int*>(band + lay.flags);
-    ASVGP_CUDA_OK(cudaMemsetAsync(flags, 0, (size_t)lay.n_flag_ints * sizeof(int), st));
-    ASVGP_CUDA_OK(cudaMemsetAsync(flags + P.n_tiles + 1, 0x7f, sizeof(int), st));                       // first bad pivot = "none"
+    for (int s = 0; s < nb.B; ++s) {
+        int* f = flags + 2 * s * nb.band;
+        ASVGP_CUDA_OK(cudaMemsetAsync(f, 0, (size_t)lay.n_flag_ints * sizeof(int), st));
+        ASVGP_CUDA_OK(cudaMemsetAsync(f + P.n_tiles + 1, 0x7f, sizeof(int), st));                       // first bad pivot = "none"
+    }
     const int n_all = (int)P.all_tasks.size();
     aa.fronts = P.d_fronts; aa.tasks = P.d_all_tasks; aa.n_tasks = n_all; aa.idx = P.d_idx; aa.M = P.M; aa.Lpool = band;
-    nd_assemble_kernel<<<std::min(n_all, 148 * 16), 256, 0, st>>>(aa); ASVGP_LAUNCHED();
+    aa.band_stride = nb.band;
+    nd_assemble_kernel<<<dim3(nd_grid_x(n_all, 148 * 16, nb.B), nb.B), 256, 0, st>>>(aa); ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     for (int lev = P.n_levels - 1; lev >= 0; --lev) {
         const int n_tasks = (int)P.factor_tasks[lev].size();
-        NdFactorArgs fa{P.d_fronts, P.d_factor_tasks[lev], n_tasks, P.d_idx, P.d_pmap, band, band + lay.linv, flags, P.n_tiles};
-        if (int rc = nd_launch_persistent(nd_factor_kernel, &fa, n_tasks, st)) return rc;
+        NdFactorArgs fa{P.d_fronts, P.d_factor_tasks[lev], n_tasks, P.d_idx, P.d_pmap, band, band + lay.linv, flags, P.n_tiles,
+                        nb.B, nb.band};
+        if (int rc = nd_launch_persistent(nd_factor_kernel, &fa, n_tasks * nb.B, st)) return rc;
     }
-    nd_scalars_kernel<<<kNdScalarBlocks, 256, 0, st>>>(P.d_doff, P.M, band, P.d_quad_off, P.R, multi ? 2 : 1, multi ? 1 : 2, flags,
-                                                       P.n_tiles, scal, band + lay.scal); ASVGP_LAUNCHED();
+    nd_scalars_kernel<<<dim3(kNdScalarBlocks, nb.B), 256, 0, st>>>(P.d_doff, P.M, band, P.d_quad_off, P.R, multi ? 2 : 1, multi ? 1 : 2,
+                                                                   flags, P.n_tiles, scal, band + lay.scal, nb.band, nb.scal);
+    ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     return kOk;
 }
 
-// selected inverse of every front + x_d = P^-1 b_d; returns the abort flag's address for the extraction kernels
+// selected inverse of every front + x_d = P^-1 b_d; returns the abort flag's address (slot 0's) for the extraction kernels
 static int nd_selinv_run(const NdPlan& P, double* band, double* sig_band, double* x_out, double* work, cudaStream_t st,
-                         const int** abort_flag_out) {
+                         const int** abort_flag_out, const NdBatch& nb = NdBatch()) {
     const NdLayout lay = nd_layout(P);
     int* flags = reinterpret_cast<int*>(work);
-    ASVGP_CUDA_OK(cudaMemsetAsync(flags, 0, (size_t)lay.n_work_ints * sizeof(int), st));
+    for (int s = 0; s < nb.B; ++s)
+        ASVGP_CUDA_OK(cudaMemsetAsync(flags + 2 * s * nb.work, 0, (size_t)lay.n_work_ints * sizeof(int), st));
     double* sigL = sig_band;
     double* sigU = sig_band + lay.sig_upper;
     const size_t yp_smem = (size_t)(2 * TILE_P) * sizeof(double);
     ASVGP_CUDA_OK(cudaFuncSetAttribute(nd_ypass_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)yp_smem));
     const int n_yp = (int)P.ypass_tasks.size();
-    nd_ypass_kernel<<<std::min(n_yp, 148 * 3), kTdThreads, yp_smem, st>>>(P.d_fronts, P.d_ypass_tasks, n_yp, band, band + lay.linv, sigL);
+    nd_ypass_kernel<<<dim3(nd_grid_x(n_yp, 148 * 3, nb.B), nb.B), kTdThreads, yp_smem, st>>>(P.d_fronts, P.d_ypass_tasks, n_yp, band,
+                                                                                          band + lay.linv, sigL, nb.band, nb.sig);
     ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     for (int lev = 0; lev < P.n_levels; ++lev) {
         const int n_g = (int)P.gather_tasks[lev].size();
-        NdGatherArgs ga{P.d_fronts, P.d_gather_tasks[lev], n_g, P.d_pmap, sigL, sigU, band + lay.scal, P.R};
-        nd_gather_kernel<<<std::min(n_g, 148 * 8), 256, 0, st>>>(ga); ASVGP_LAUNCHED();
+        NdGatherArgs ga{P.d_fronts, P.d_gather_tasks[lev], n_g, P.d_pmap, sigL, sigU, band + lay.scal, P.R, nb.band, nb.sig};
+        nd_gather_kernel<<<dim3(nd_grid_x(n_g, 148 * 8, nb.B), nb.B), 256, 0, st>>>(ga); ASVGP_LAUNCHED();
         ASVGP_CUDA_OK(cudaGetLastError());
         const int n_s = (int)P.selinv_tasks[lev].size();
         if (n_s == 0) continue;
-        NdSelArgs sa{P.d_fronts, P.d_selinv_tasks[lev], n_s, band, sigL, sigU, flags, P.n_tiles, P.n_cnt};
-        if (int rc = nd_launch_persistent(nd_selinv_kernel, &sa, n_s, st)) return rc;
+        NdSelArgs sa{P.d_fronts, P.d_selinv_tasks[lev], n_s, band, sigL, sigU, flags, P.n_tiles, P.n_cnt, nb.B, nb.band, nb.sig, nb.work};
+        const int rc = nb.B > 1 ? nd_launch_persistent(nd_selinv_kernel<true>, &sa, n_s * nb.B, st)
+                                : nd_launch_persistent(nd_selinv_kernel<false>, &sa, n_s, st);
+        if (rc) return rc;
     }
     const int* abort_flag = flags + P.n_tiles + P.n_cnt;
     const int RM = P.M * P.R;
-    nd_x_kernel<<<(RM + 255) / 256, 256, 0, st>>>(P.d_xoff, RM, sigL, band + lay.scal, abort_flag, x_out); ASVGP_LAUNCHED();
+    nd_x_kernel<<<dim3((RM + 255) / 256, nb.B), 256, 0, st>>>(P.d_xoff, RM, sigL, band + lay.scal, abort_flag, x_out, nb.band, nb.sig,
+                                                              nb.work);
+    ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     *abort_flag_out = abort_flag;
     return kOk;
@@ -1039,7 +1113,7 @@ static int nd_kron_factor(const double* K1, const double* K2, const double* Gs, 
     const NdPlan* Pp = nullptr;
     if (int rc = nd_plan_device(m1, m2, order, n_rhs, &Pp)) return rc;
     NdAssembleArgs aa{};
-    aa.K1 = K1; aa.K2 = K2; aa.Gs = Gs; aa.b = rhs_io; aa.sigma2 = sigma2; aa.m1 = m1; aa.m2 = m2; aa.K = order; aa.dense = nullptr;
+    aa.K1 = K1; aa.K2 = K2; aa.Gs = Gs; aa.b = rhs_io; aa.sigma2[0] = sigma2; aa.m1 = m1; aa.m2 = m2; aa.K = order; aa.dense = nullptr;
     return nd_factor_run(*Pp, aa, band, scal, multi, static_cast<cudaStream_t>(stream));
 }
 
@@ -1055,7 +1129,7 @@ static int nd_kron_selinv(double* band, int m1, int m2, int order, int n_rhs, do
     const int64_t total = (int64_t)P.M * (order + 1) * (2 * order + 1);
     nd_stencil_kernel<<<(int)std::min<int64_t>((total + 255) / 256, 148 * 16), 256, 0, st>>>(P.d_sigoff, m1, m2, order, P.R, sig_band,
                                                                                           x_io, band + lay.scal, abort_flag,
-                                                                                          sigma_stencil);
+                                                                                          sigma_stencil, 0, 0, 0);
     ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     return kOk;
@@ -1095,6 +1169,88 @@ extern "C" int asvgp_kron_selinv_multi(double* band, int m1, int m2, int order, 
     return nd_kron_selinv(band, m1, m2, order, n_rhs, sig_band, x_io, sigma_stencil, work, stream);
 }
 
+// ---- B hyper-parameter settings through one plan ----------------------------------------------------------------------------------
+// Every slot runs the kernels of the single-setting calls on its own buffers; the persistent launches deal the tasks of all
+// slots task-major.  Slot strides are rounded to 32 doubles so that every slot's tiles keep the 256-byte alignment of the bulk
+// copies.
+static long long nd_slot_doubles(long long n) { return (n + 31) & ~31LL; }
+
+static NdBatch nd_batch(const NdPlan& P, int B) {
+    const NdLayout L = nd_layout(P);
+    NdBatch nb;
+    nb.B = B; nb.band = nd_slot_doubles(L.band_total); nb.sig = nd_slot_doubles(L.sig_total); nb.work = nd_slot_doubles(L.work_total);
+    nb.scal = 2 + P.R;
+    return nb;
+}
+
+#define ND_CHECK_BATCH(name) ASVGP_REQUIRE(B >= 1 && B <= ASVGP_MAX_BATCH, name ": B=%d not in 1..%d", B, ASVGP_MAX_BATCH)
+
+extern "C" int asvgp_kron_doubles_batched(int m1, int m2, int order, int n_rhs, int B, int64_t* h_sizes) {
+    ND_CHECK_ARGS("kron_doubles_batched");
+    ND_CHECK_RHS("kron_doubles_batched");
+    ND_CHECK_BATCH("kron_doubles_batched");
+    ASVGP_REQUIRE(h_sizes != nullptr, "kron_doubles_batched: h_sizes is NULL");
+    const NdPlan& P = *nd_plan_host(m1, m2, order, n_rhs);
+    const NdBatch nb = nd_batch(P, B);
+    h_sizes[0] = B * nb.band; h_sizes[1] = B * nb.sig; h_sizes[2] = B * nb.work;
+    h_sizes[3] = (int64_t)B * n_rhs * P.M;
+    h_sizes[4] = (int64_t)B * nb.scal;
+    h_sizes[5] = (int64_t)B * (order + 1) * (2 * order + 1) * P.M;
+    return kOk;
+}
+
+extern "C" int asvgp_kron_factor_batched(const double* K1, const double* K2, const double* Gs, const double* b, int m1, int m2,
+                                         int order, int n_rhs, int B, const double* h_sigma2, double* band, int64_t band_doubles,
+                                         double* scal, void* stream) {
+    ND_CHECK_ARGS("kron_factor_batched");
+    ND_CHECK_RHS("kron_factor_batched");
+    ND_CHECK_BATCH("kron_factor_batched");
+    ASVGP_REQUIRE(h_sigma2 != nullptr, "kron_factor_batched: h_sigma2 is NULL");
+    ASVGP_REQUIRE(K1 != nullptr && K2 != nullptr && Gs != nullptr && b != nullptr && band != nullptr && scal != nullptr,
+                  "kron_factor_batched: NULL buffer");
+    for (int s = 0; s < B; ++s)
+        ASVGP_REQUIRE(h_sigma2[s] > 0.0, "kron_factor_batched: slot %d: sigma2=%g must be positive", s, h_sigma2[s]);
+    const NdBatch need = nd_batch(*nd_plan_host(m1, m2, order, n_rhs), B);
+    ASVGP_REQUIRE(band_doubles >= B * need.band, "kron_factor_batched: band holds %lld doubles, %lld needed", (long long)band_doubles,
+                  (long long)(B * need.band));
+    const NdPlan* Pp = nullptr;
+    if (int rc = nd_plan_device(m1, m2, order, n_rhs, &Pp)) return rc;
+    NdAssembleArgs aa{};
+    aa.K1 = K1; aa.K2 = K2; aa.Gs = Gs; aa.b = b; aa.m1 = m1; aa.m2 = m2; aa.K = order; aa.dense = nullptr;
+    aa.k1_stride = (long long)(order + 1) * m1; aa.k2_stride = (long long)(order + 1) * m2;
+    for (int s = 0; s < B; ++s) aa.sigma2[s] = h_sigma2[s];
+    return nd_factor_run(*Pp, aa, band, scal, true, static_cast<cudaStream_t>(stream), need);
+}
+
+extern "C" int asvgp_kron_selinv_batched(double* band, int m1, int m2, int order, int n_rhs, int B, int64_t band_doubles,
+                                         double* sig_band, int64_t sig_doubles, double* work, int64_t work_doubles, double* x_out,
+                                         double* sigma_stencil, void* stream) {
+    ND_CHECK_ARGS("kron_selinv_batched");
+    ND_CHECK_RHS("kron_selinv_batched");
+    ND_CHECK_BATCH("kron_selinv_batched");
+    ASVGP_REQUIRE(band != nullptr && sig_band != nullptr && work != nullptr && x_out != nullptr && sigma_stencil != nullptr,
+                  "kron_selinv_batched: NULL buffer");
+    const NdBatch nb = nd_batch(*nd_plan_host(m1, m2, order, n_rhs), B);
+    ASVGP_REQUIRE(band_doubles >= B * nb.band && sig_doubles >= B * nb.sig && work_doubles >= B * nb.work,
+                  "kron_selinv_batched: buffers of %lld / %lld / %lld doubles, %lld / %lld / %lld needed", (long long)band_doubles,
+                  (long long)sig_doubles, (long long)work_doubles, (long long)(B * nb.band), (long long)(B * nb.sig),
+                  (long long)(B * nb.work));
+    const NdPlan* Pp = nullptr;
+    if (int rc = nd_plan_device(m1, m2, order, n_rhs, &Pp)) return rc;
+    const NdPlan& P = *Pp;
+    const NdLayout lay = nd_layout(P);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int* abort_flag = nullptr;
+    if (int rc = nd_selinv_run(P, band, sig_band, x_out, work, st, &abort_flag, nb)) return rc;
+    const int64_t total = (int64_t)P.M * (order + 1) * (2 * order + 1);
+    nd_stencil_kernel<<<dim3(nd_grid_x((total + 255) / 256, 148 * 16, B), B), 256, 0, st>>>(P.d_sigoff, m1, m2, order, P.R, sig_band, x_out,
+                                                                                         band + lay.scal, abort_flag, sigma_stencil,
+                                                                                         nb.band, nb.sig, nb.work);
+    ASVGP_LAUNCHED();
+    ASVGP_CUDA_OK(cudaGetLastError());
+    return kOk;
+}
+
 // ---- dense symmetric positive definite matrices on the same kernels (one front) -----------------------------------------------------
 // What GPR_additive needs (reference gpr.py:192-195, 221-231: tf.linalg.cholesky / triangular_solve of a DENSE (sum m_d)^2
 // matrix): log|A|, b^T A^-1 b, A^-1 b and A^-1, from the tile-DAG factorisation and the blocked Takahashi recursion above.
@@ -1124,7 +1280,7 @@ static int nd_dense_factor(const double* A, int n, int n_rhs, const double* rhs,
     const NdPlan* Pp = nullptr;
     if (int rc = nd_plan_device(n, 1, -1, n_rhs, &Pp)) return rc;
     NdAssembleArgs aa{};
-    aa.b = rhs; aa.sigma2 = 1.0; aa.m1 = n; aa.m2 = 1; aa.K = 0; aa.dense = A;
+    aa.b = rhs; aa.sigma2[0] = 1.0; aa.m1 = n; aa.m2 = 1; aa.K = 0; aa.dense = A;
     return nd_factor_run(*Pp, aa, band, scal, multi, static_cast<cudaStream_t>(stream));
 }
 

@@ -569,10 +569,14 @@ __global__ void __launch_bounds__(256) td_extract_stencil_kernel(TileGeom g, con
 //   out[4 + o] = x^T Op x
 // plus the Kronecker trace terms  out[8..10] = sum G[(i),(j)] T1[i1,j1] T2[i2,j2] for (T1,T2) in
 //   (S1,S2), (dS1,S2), (S1,dS2)   (reference gpr.py:307 trace(cholesky_solve(L_Kuu, KufKfu)) and its derivatives).
+// A batch (asvgp_kron_terms_batched): blockIdx.y = b D + d for slot b and output column d; slot b reads SigP + b sig_stride, the
+// per-dimension bands + b k1_stride / k2_stride, x + (b D + d) M, and writes out + (b D + d) 11.  Gs is shared.
 struct StencilTerms {
     const double *SigP, *Gs, *x;
     const double *K1, *dK1, *K2, *dK2;        // lower bands (K+1) x m
     const double *S1, *dS1, *S2, *dS2;        // lower bands of K1^-1, d(K1^-1), K2^-1, d(K2^-1)
+    long long sig_stride, k1_stride, k2_stride;
+    int n_cols;
 };
 
 __device__ __forceinline__ double band_sym(const double* B, int m, int i, int j) {
@@ -584,6 +588,14 @@ __global__ void __launch_bounds__(256) td_terms_kernel(int m1, int m2, int K, St
     const int NS = 2 * K + 1, n_e = (K + 1) * NS;
     const int64_t M = (int64_t)m1 * m2;
     const int64_t total = M * n_e;
+    {
+        const int b = blockIdx.y / a.n_cols;
+        a.SigP += b * a.sig_stride;
+        a.x += blockIdx.y * M;
+        a.K1 += b * a.k1_stride; a.dK1 += b * a.k1_stride; a.S1 += b * a.k1_stride; a.dS1 += b * a.k1_stride;
+        a.K2 += b * a.k2_stride; a.dK2 += b * a.k2_stride; a.S2 += b * a.k2_stride; a.dS2 += b * a.k2_stride;
+        out += blockIdx.y * 11;
+    }
     double acc[11];
 #pragma unroll
     for (int i = 0; i < 11; ++i) acc[i] = 0.0;
@@ -722,9 +734,30 @@ extern "C" int asvgp_kron_terms(const double* SigP, const double* Gs, const doub
     ASVGP_REQUIRE(m1 > 0 && m2 > 0 && order >= 1 && order <= kMaxOrder, "kron_terms: m=%d,%d order=%d", m1, m2, order);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     ASVGP_CUDA_OK(cudaMemsetAsync(out, 0, 11 * sizeof(double), st));
-    StencilTerms a{SigP, Gs, x, K1, dK1, K2, dK2, S1, dS1, S2, dS2};
+    StencilTerms a{SigP, Gs, x, K1, dK1, K2, dK2, S1, dS1, S2, dS2, 0, 0, 0, 1};
     const int64_t total = (int64_t)m1 * m2 * (order + 1) * (2 * order + 1);
     td_terms_kernel<<<(int)std::min<int64_t>((total + 255) / 256, 148 * 4), 256, 0, st>>>(m1, m2, order, a, out); ASVGP_LAUNCHED();
+    ASVGP_CUDA_OK(cudaGetLastError());
+    return kOk;
+}
+
+// B settings x D output columns in one launch: SigP[B][(order+1)(2 order+1)][M], x[B][D][M], per-dimension bands [B][order+1][m_i],
+// Gs shared; out[B][D][11] (device, zeroed here), entry (b, d) as asvgp_kron_terms on slot b's operands and column d.
+extern "C" int asvgp_kron_terms_batched(const double* SigP, const double* Gs, const double* x, const double* K1,
+                                        const double* dK1, const double* K2, const double* dK2, const double* S1,
+                                        const double* dS1, const double* S2, const double* dS2, int m1, int m2, int order,
+                                        int B, int D, double* out, void* stream) {
+    ASVGP_REQUIRE(m1 > 0 && m2 > 0 && order >= 1 && order <= kMaxOrder, "kron_terms_batched: m=%d,%d order=%d", m1, m2, order);
+    ASVGP_REQUIRE(B >= 1 && B <= ASVGP_MAX_BATCH, "kron_terms_batched: B=%d not in 1..%d", B, ASVGP_MAX_BATCH);
+    ASVGP_REQUIRE(D >= 1 && D <= ASVGP_MAX_RHS, "kron_terms_batched: D=%d not in 1..%d", D, ASVGP_MAX_RHS);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    ASVGP_CUDA_OK(cudaMemsetAsync(out, 0, (size_t)B * D * 11 * sizeof(double), st));
+    const int n_e = (order + 1) * (2 * order + 1);
+    StencilTerms a{SigP, Gs, x, K1, dK1, K2, dK2, S1, dS1, S2, dS2, (long long)n_e * m1 * m2, (long long)(order + 1) * m1,
+                   (long long)(order + 1) * m2, D};
+    const int64_t total = (int64_t)m1 * m2 * n_e;
+    const int per = (int)std::max<int64_t>(1, std::min<int64_t>((total + 255) / 256, (148 * 4 + B * D - 1) / (B * D)));
+    td_terms_kernel<<<dim3(per, B * D), 256, 0, st>>>(m1, m2, order, a, out); ASVGP_LAUNCHED();
     ASVGP_CUDA_OK(cudaGetLastError());
     return kOk;
 }

@@ -708,6 +708,83 @@ class GPR_kron(_PerDimension):
         """Variational bound on the log marginal likelihood (reference gpr.py:282-308)."""
         return np.float64(self._evaluate(False)[0])
 
+    def training_loss_and_gradients_batch(self, U, max_slots=None):
+        """training_loss_and_gradients at B settings at once, without changing the model's parameters.
+
+        U[B, len(trainable_variables)]: unconstrained values in the order of `trainable_variables` (1 <= B <= 64; 3 columns when
+        one kernel object serves both dimensions).  Returns (loss[B], grad[B, len(trainable_variables)], info[B]); row b equals
+        training_loss_and_gradients() with the parameters set to U[b] up to the summation order of the factorisation's fp64
+        REDs.  info is the first non-zero of the pivots of P and of the two per-dimension factors; such a setting gets loss =
+        +inf and NaN gradients (nothing is raised).  All settings share the accumulator: each group of settings is one
+        factorisation of P per setting through one plan (asvgp_kron_factor_batched and friends), and its results come back in
+        one device-to-host copy.  Groups hold at most `max_slots` settings (default: as many as fit in the free device
+        memory; a slot takes ~1.1 GB at 200 x 200, order 3); the results do not depend on the grouping."""
+        params = self.trainable_variables
+        U = np.asarray(U, dtype=np.float64)
+        if U.ndim != 2 or U.shape[1] != len(params):
+            raise ValueError("U must be [B, %d] (unconstrained values of trainable_variables), got shape %s"
+                             % (len(params), U.shape))
+        if not 1 <= U.shape[0] <= _lib.MAX_BATCH:
+            raise ValueError("U has %d rows; a batch holds 1..%d settings" % (U.shape[0], _lib.MAX_BATCH))
+        if not np.isfinite(U).all():
+            raise ValueError("U must be finite")
+        if (getattr(self, "_method", None) or ops.KRON_METHOD) != "nd":
+            raise NotImplementedError("batched evaluation runs the nested-dissection factorisation (method='nd')")
+        vals = _values_at(params, U)
+        # columns of vals holding (v1, l1, v2, l2, sigma2); one shared kernel object maps both dimensions to the same columns
+        roles = [self.kernels[0].variance, self.kernels[0].lengthscales, self.kernels[1].variance, self.kernels[1].lengthscales,
+                 self.likelihood.variance]
+        col = [next(j for j, p in enumerate(params) if p is r) for r in roles]
+        m1, m2, D = self.bases[0].m, self.bases[1].m, self.n_outputs
+        slot_bytes = ops.kron_batch_slot_bytes(m1, m2, self.order, D)
+        groups = ops.kron_batch_groups(len(U), slot_bytes, ops.kron_batch_free_bytes(m1, m2, self.order, D), max_slots)
+        bounds = []
+        for first, n in groups:
+            bounds += self._evaluate_batch(vals[first:first + n], col, params)
+        return _losses(bounds, params, U)
+
+    def _evaluate_batch(self, vals, col, params):
+        """(elbo, grad[len(params)], info) of each row of vals (constrained values of params) through one batch of slots."""
+        B = len(vals)
+        v1, l1, v2, l2, s2 = (vals[:, c] for c in col)
+        m1, m2, D = self.bases[0].m, self.bases[1].m, self.n_outputs
+        Ks, dKs = [], []
+        for feat, kern, ell, var in zip(self.inducing_features, self.kernels, (l1, l2), (v1, v2)):
+            K, dK = feat.make_Kuu_device_batched(kern, ell, var, want_grad=True)
+            Ks.append(K); dKs.append(dK)
+        Ss, dSs, scals, join = ops.band_inverses_beside(Ks, dKs, self.bases)
+        ws = ops.kron_batch_workspace(m1, m2, self.order, D, B)
+        ops.kron_factor_batched(Ks[0], Ks[1], self._acc, self.bases, s2, ws, b=self._rhs())
+        SigP, x = ops.kron_selinv_batched(self.bases, ws, B)
+        join()
+        ops.kron_terms_batched(SigP, self._acc, x, Ks[0], dKs[0], Ks[1], dKs[1], Ss[0], dSs[0], Ss[1], dSs[1], self.bases,
+                               ws.terms[:B])
+        yy_rest = [] if self._extra is None else [self._extra[:, -2]]          # sum(y_d^2) of columns 2 ... D
+        packed = torch.cat([scals[0].view(-1), scals[1].view(-1), ws.scal[:B].reshape(-1), ws.terms[:B].reshape(-1), self._scal]
+                           + yy_rest).cpu().numpy()                             # one D2H read
+        p = 0
+        sc1 = packed[p: p + 4 * B].reshape(B, 4); p += 4 * B
+        sc2 = packed[p: p + 4 * B].reshape(B, 4); p += 4 * B
+        scal = packed[p: p + (2 + D) * B].reshape(B, 2 + D); p += (2 + D) * B        # {log|P|, info, Q_1 ... Q_D} per slot
+        Ts = packed[p: p + 11 * D * B].reshape(B, D, 11); p += 11 * D * B
+        N = packed[p + 1]
+        yys = [packed[p], *packed[p + 2:]]
+        roles = [self.kernels[0].variance, self.kernels[0].lengthscales, self.kernels[1].variance, self.kernels[1].lengthscales,
+                 self.likelihood.variance]
+        out = []
+        for b in range(B):
+            infos = [scal[b, 1], sc1[b, 2], sc2[b, 2]]
+            if any(i != 0 for i in infos):
+                out.append((np.nan, np.full(len(params), np.nan), next(i for i in infos if i != 0)))
+                continue
+            v = [v1[b], v2[b]]
+            cols = [_kron_column_bound(N, s2[b], v, m1, m2, sc1[b], sc2[b], scal[b, 0], scal[b, 2 + d], yys[d], Ts[b, d], True)
+                    for d in range(D)]
+            elbo, g, info = _combine_columns([c[0] for c in cols], infos, lambda: _kron_shared(N, s2[b], v, Ts[b, 0]))
+            gd = _grad_dict(zip(roles, g))
+            out.append((elbo, np.array([gd[id(p)] for p in params]), info))
+        return out
+
     # -- prediction ----------------------------------------------------------------------------------------------
     def posterior_weights(self):
         """(alpha, SigP stencil, S1, S2) on the device: alpha = P^-1 Kuf_y / sigma2 ([D, M] for D > 1 output columns),

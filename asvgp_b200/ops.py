@@ -770,17 +770,43 @@ def band_inverse_1d(A, dA, basis, chunks=0, slot=0):
     return sig, dsig, scal
 
 
+def band_inverse_1d_batched(A, dA, basis, chunks=0, slot=0):
+    """band_inverse_1d for B matrices of one basis, A / dA [B, k+1, m], in one launch: (sig, dsig [B, k+1, m], scal [B, 4]);
+    slot b equals band_inverse_1d(A[b], dA[b]) bit for bit."""
+    k, m = basis.order, basis.m
+    B = A.shape[0]
+    if A.dim() != 3 or tuple(A.shape[1:]) != (k + 1, m) or tuple(dA.shape) != tuple(A.shape) or not 1 <= B <= _lib.MAX_BATCH:
+        raise ValueError("band_inverse_1d_batched: A and dA must be [B, %d, %d] with 1 <= B <= %d, got %s / %s"
+                         % (k + 1, m, _lib.MAX_BATCH, tuple(A.shape), tuple(dA.shape)))
+    dev = device()
+    key = (dev, m, k, chunks, "band_inverse_batched", slot)
+    ws = _WORKSPACES.get(key)
+    nbytes = _lib.load().asvgp_workspace_bytes_band_inverse_1d_batched(m, k, int(chunks), B)
+    if nbytes < 0:
+        raise _lib.AsvgpNativeError("asvgp_workspace_bytes_band_inverse_1d_batched rejected m=%d order=%d B=%d" % (m, k, B))
+    if ws is None or ws.numel() < nbytes:          # one scratch per (basis shape, stream slot), grown to the largest B asked for
+        ws = _WORKSPACES[key] = torch.empty(nbytes, dtype=torch.uint8, device=dev)
+    sig = torch.empty((B, k + 1, m), dtype=F64, device=A.device)
+    dsig = torch.empty_like(sig)
+    scal = torch.empty((B, 4), dtype=F64, device=A.device)
+    _lib.call("asvgp_band_inverse_1d_batched", _p(A), _p(dA), m, k, int(chunks), B, _p(sig), _p(dsig), _p(scal), _p(ws),
+              ws.numel(), _stream())
+    return sig, dsig, scal
+
+
 def band_inverses_beside(Ks, dKs, bases):
     """band_inverse_1d of every per-dimension factor (Ks[i], dKs[i]) on a side stream of its own, ordered after the current
     stream's work so far.  These short chains (~0.1 ms each) then overlap what the caller launches next on the current stream,
-    e.g. the factorisation of P.  Returns (Ss, dSs, scals, join): call join() before the current stream reads any of them."""
+    e.g. the factorisation of P.  Returns (Ss, dSs, scals, join): call join() before the current stream reads any of them.
+    Batched factors [B, k+1, m] go through band_inverse_1d_batched, one launch per dimension."""
     main = torch.cuda.current_stream()
     side = side_streams(len(bases))
     Ss, dSs, scals = [], [], []
     for i, (stream, basis) in enumerate(zip(side, bases)):
         stream.wait_stream(main)
+        inverse = band_inverse_1d_batched if Ks[i].dim() == 3 else band_inverse_1d
         with torch.cuda.stream(stream):
-            S, dS, sc = band_inverse_1d(Ks[i], dKs[i], basis, slot=1 + i)
+            S, dS, sc = inverse(Ks[i], dKs[i], basis, slot=1 + i)
         for t in (S, dS, sc):
             t.record_stream(main)
         Ss.append(S); dSs.append(dS); scals.append(sc)
@@ -941,6 +967,109 @@ def kron_terms(SigP, acc, x, K1, dK1, K2, dK2, S1, dS1, S2, dS2, bases, out):
     Gs, _, _ = split_accum_2d(acc, bases)
     _lib.call("asvgp_kron_terms", _p(SigP), _p(Gs), _p(x), _p(K1), _p(dK1), _p(K2), _p(dK2), _p(S1), _p(dS1), _p(S2),
               _p(dS2), m1, m2, k, _p(out), _stream())
+    return out
+
+
+# ---- B hyper-parameter settings of the Kronecker factorisation through one plan ------------------------------------------------
+class KronBatchWorkspace:
+    """Device buffers of `slots` settings of the nested-dissection factorisation (asvgp_kron_*_batched) for one plan (m1, m2,
+    order, n_rhs): the opaque band / sig / work pools, and per slot scal [2 + n_rhs] (the _multi layout, also for n_rhs = 1),
+    x [n_rhs, M], the stencil of P^-1 and the contractions [n_rhs, 11].  A batch of B <= slots uses the first B slots."""
+
+    def __init__(self, m1, m2, order, n_rhs, slots):
+        self.m1, self.m2, self.order, self.n_rhs, self.slots = m1, m2, order, _check_n_rhs(n_rhs), int(slots)
+        self.M = m1 * m2
+        sizes = kron_batch_doubles(m1, m2, order, n_rhs, slots)
+        dev = device()
+        self.band = torch.empty(sizes[0], dtype=F64, device=dev)
+        self.sig_band = torch.empty(sizes[1], dtype=F64, device=dev)
+        self.work = torch.empty(sizes[2], dtype=F64, device=dev)
+        self.x = torch.empty((slots, n_rhs, self.M), dtype=F64, device=dev)
+        self.scal = torch.empty((slots, 2 + n_rhs), dtype=F64, device=dev)
+        self.sigma_stencil = torch.empty((slots, stencil_rows(order), self.M), dtype=F64, device=dev)
+        self.terms = torch.empty((slots, n_rhs, 11), dtype=F64, device=dev)
+
+    def nbytes(self):
+        return 8 * sum(t.numel() for t in (self.band, self.sig_band, self.work, self.x, self.scal, self.sigma_stencil, self.terms))
+
+
+def kron_batch_doubles(m1, m2, order, n_rhs, B):
+    """Doubles of the six buffers of B slots (asvgp_kron_doubles_batched): band, sig, work, x, scal, sigma_stencil."""
+    sizes = (ctypes.c_int64 * 6)()
+    _lib.call("asvgp_kron_doubles_batched", m1, m2, order, int(n_rhs), int(B), ctypes.cast(sizes, ctypes.c_void_p))
+    return [int(v) for v in sizes]
+
+
+def kron_batch_slot_bytes(m1, m2, order, n_rhs):
+    """Device bytes one slot of a KronBatchWorkspace takes (the contractions included)."""
+    return 8 * (sum(kron_batch_doubles(m1, m2, order, n_rhs, 1)) + 11 * int(n_rhs))
+
+
+def kron_batch_groups(B, slot_bytes, free_bytes, max_slots=None, headroom=0.8):
+    """How a batch of B settings is run: [(first slot, count)], groups of at most max_slots in order.  max_slots=None takes as
+    many slots as `headroom` of free_bytes holds (at least one, at most B); the results do not depend on the grouping."""
+    if max_slots is None:
+        max_slots = int(headroom * free_bytes // slot_bytes)
+    max_slots = max(1, min(int(max_slots), int(B), _lib.MAX_BATCH))
+    return [(s, min(max_slots, B - s)) for s in range(0, B, max_slots)]
+
+
+_KRON_BATCH_WS = {}
+
+
+def kron_batch_workspace(m1, m2, order, n_rhs, slots):
+    """The cached KronBatchWorkspace of this plan on the current device with at least `slots` slots.  One workspace is kept
+    per (device, m1, m2, order, n_rhs): a request for more slots replaces it (at 200 x 200, order 3 a slot is ~1.1 GB)."""
+    key = (device(), m1, m2, order, int(n_rhs))
+    ws = _KRON_BATCH_WS.get(key)
+    if ws is None or ws.slots < slots:
+        _KRON_BATCH_WS.pop(key, None)
+        del ws
+        _KRON_BATCH_WS[key] = ws = KronBatchWorkspace(m1, m2, order, n_rhs, slots)
+    return ws
+
+
+def kron_batch_free_bytes(m1, m2, order, n_rhs):
+    """Free device memory plus what the cached batch workspace of this plan holds (it is replaced, not added to)."""
+    free, _ = torch.cuda.mem_get_info(device())
+    ws = _KRON_BATCH_WS.get((device(), m1, m2, order, int(n_rhs)))
+    return free + (ws.nbytes() if ws is not None else 0)
+
+
+def kron_factor_batched(K1, K2, acc, bases, sigma2s, ws, b=None):
+    """Factorisations of P_s = K1[s] (x) K2[s] + G / sigma2s[s] for the B = len(sigma2s) settings (K1 [B, k+1, m1], K2 [B, k+1,
+    m2], sigma2s on the host) in the first B slots of ws; b: the shared right-hand sides [n_rhs, M] (default: the projection in
+    acc), read and not overwritten.  Scalars land in ws.scal[:B] ({log|P|, info, Q_1 ... Q_n_rhs} per slot)."""
+    k, m1, m2 = _check_bases_2d(bases)
+    Gs, b_acc, _ = split_accum_2d(acc, bases)
+    b = b_acc if b is None else b
+    sigma2s = np.ascontiguousarray(sigma2s, dtype=np.float64).reshape(-1)
+    B = sigma2s.size
+    if not 1 <= B <= ws.slots or tuple(K1.shape) != (B, k + 1, m1) or tuple(K2.shape) != (B, k + 1, m2):
+        raise ValueError("kron_factor_batched: %d settings for %d slots, K1 %s, K2 %s" % (B, ws.slots, tuple(K1.shape), tuple(K2.shape)))
+    if b.numel() != ws.n_rhs * ws.M or not b.is_contiguous():
+        raise ValueError("b must be contiguous and hold n_rhs = %d columns of %d entries" % (ws.n_rhs, ws.M))
+    _lib.call("asvgp_kron_factor_batched", _p(K1), _p(K2), _p(Gs), _p(b), m1, m2, k, ws.n_rhs, B,
+              ctypes.c_void_p(sigma2s.ctypes.data), _p(ws.band), ws.band.numel(), _p(ws.scal), _stream())
+    return ws
+
+
+def kron_selinv_batched(bases, ws, B):
+    """Selected inverses of the first B slots' factors: (stencils of P_s^-1 [B, rows, M], x_s = P_s^-1 b [B, n_rhs, M])."""
+    k, m1, m2 = _check_bases_2d(bases)
+    _lib.call("asvgp_kron_selinv_batched", _p(ws.band), m1, m2, k, ws.n_rhs, int(B), ws.band.numel(), _p(ws.sig_band),
+              ws.sig_band.numel(), _p(ws.work), ws.work.numel(), _p(ws.x), _p(ws.sigma_stencil), _stream())
+    return ws.sigma_stencil[:B], ws.x[:B]
+
+
+def kron_terms_batched(SigP, acc, x, K1, dK1, K2, dK2, S1, dS1, S2, dS2, bases, out):
+    """asvgp_kron_terms for B slots and D columns in one launch: SigP [B, rows, M], x [B, D, M], the per-dimension bands [B, k+1,
+    m_i]; out [B, D, 11]."""
+    k, m1, m2 = _check_bases_2d(bases)
+    Gs, _, _ = split_accum_2d(acc, bases)
+    B, D = x.shape[0], x.shape[1]
+    _lib.call("asvgp_kron_terms_batched", _p(SigP), _p(Gs), _p(x), _p(K1), _p(dK1), _p(K2), _p(dK2), _p(S1), _p(dS1), _p(S2),
+              _p(dS2), m1, m2, k, B, D, _p(out), _stream())
     return out
 
 

@@ -332,6 +332,44 @@ ASVGP_API int asvgp_kron_factor_multi(const double* K1, const double* K2, const 
 ASVGP_API int asvgp_kron_selinv_multi(double* band, int m1, int m2, int order, int n_rhs, double* sig_band, double* x_io,
                                       double* sigma_stencil, double* work, void* stream);
 
+/* ---- B hyper-parameter settings through one plan (batched evaluation of the bound) -----------------------------------------------
+ * B settings (K1_b, K2_b, sigma2_b) of P_b = K1_b (x) K2_b + G / sigma2_b on one grid, one order and one set of n_rhs right-hand
+ * sides.  G and b are shared; every slot b owns its own slice of the buffers (tiles, flags, abort word, scalars, x).  The kernels
+ * are those of the single calls with a slot index; the persistent launches deal the tasks of all slots task-major, so the
+ * chain-bound top levels of different slots overlap.  Slot b equals asvgp_kron_factor_multi / asvgp_kron_selinv_multi on its own
+ * operands up to the order of the fp64 REDs of the extend-add (the single calls are not bitwise reproducible either).
+ *   asvgp_kron_doubles_batched: h_sizes[6] (HOST) = { band, sig, work, x, scal, sigma_stencil } doubles for B slots, each B
+ *     times a per-slot size (per-slot buffers are rounded up to 32 doubles).
+ *   asvgp_kron_factor_batched: K1 [B][order+1][m1], K2 [B][order+1][m2] (lower bands), Gs shared, b [n_rhs][M] shared and
+ *     read only; h_sigma2 is a HOST array [B].  scal[B][2 + n_rhs] in the layout of asvgp_kron_factor_multi; a non-positive
+ *     pivot or an internal time-out in slot b is reported in slot b's info alone.
+ *   asvgp_kron_selinv_batched: from the factors (consumed): x_out[B][n_rhs][M] = P_b^-1 b_d and sigma_stencil[B][(order+1)
+ *     (2 order+1)][M]; a slot that timed out gets NaN outputs, the others are unaffected.
+ * B outside 1..ASVGP_MAX_BATCH, n_rhs outside 1..ASVGP_MAX_RHS, a non-positive or NaN sigma2_b, NULL arrays and buffers
+ * shorter than the query's sizes are rejected before any CUDA call (asvgp_last_error says which).  No host synchronisation.
+ *
+ * asvgp_band_inverse_1d_batched: asvgp_band_inverse_1d for B matrices of one size, A / dA [B][order+1][M] ->
+ *   sig_val / sig_tan [B][order+1][M], scal[B][4]; slot b equals asvgp_band_inverse_1d on (A_b, dA_b) bit for bit.  The
+ *   workspace needs asvgp_workspace_bytes_band_inverse_1d_batched(M, order, chunks, B) bytes (-1 for arguments out of range).
+ * asvgp_kron_terms_batched: asvgp_kron_terms for B slots and D output columns in one launch: SigP[B][(order+1)(2 order+1)][M],
+ *   x[B][D][M], K1, dK1, S1, dS1 [B][order+1][m1], K2, dK2, S2, dS2 [B][order+1][m2], Gs shared; out[B][D][11] (device, zeroed
+ *   here) holds the 11 slots of asvgp_kron_terms for slot b and column d.  D lies in 1..ASVGP_MAX_RHS. */
+ASVGP_API int asvgp_kron_doubles_batched(int m1, int m2, int order, int n_rhs, int B, int64_t* h_sizes);
+ASVGP_API int asvgp_kron_factor_batched(const double* K1, const double* K2, const double* Gs, const double* b, int m1, int m2,
+                                        int order, int n_rhs, int B, const double* h_sigma2, double* band, int64_t band_doubles,
+                                        double* scal, void* stream);
+ASVGP_API int asvgp_kron_selinv_batched(double* band, int m1, int m2, int order, int n_rhs, int B, int64_t band_doubles,
+                                        double* sig_band, int64_t sig_doubles, double* work, int64_t work_doubles, double* x_out,
+                                        double* sigma_stencil, void* stream);
+ASVGP_API int64_t asvgp_workspace_bytes_band_inverse_1d_batched(int M, int order, int chunks, int B);
+ASVGP_API int asvgp_band_inverse_1d_batched(const double* A, const double* dA, int M, int order, int chunks, int B,
+                                            double* sig_val, double* sig_tan, double* scal, void* work, int64_t work_bytes,
+                                            void* stream);
+ASVGP_API int asvgp_kron_terms_batched(const double* SigP, const double* Gs, const double* x, const double* K1,
+                                       const double* dK1, const double* K2, const double* dK2, const double* S1,
+                                       const double* dS1, const double* S2, const double* dS2, int m1, int m2, int order,
+                                       int B, int D, double* out, void* stream);
+
 /* asvgp_kronband_*: the same two operations on the scalar band of P in the natural order (bandwidth order*(m2+1), gpr.py:262)
  * as one tile DAG over the band (csrc/tiledag_2d.cu) — a single chain over all m1 m2 columns, 10x slower at 200 x 200; kept
  * as an independent second implementation (the tests compare the two).  Same arguments, except that rhs_io has
